@@ -20,6 +20,10 @@ The JSON line:
                launches / their CUDA-event time, against MEASURED_PEAKS.json (sustained figure: the kernel is
                timed inside a long step)
   cpu_baseline oracle port of the reference arithmetic on the host cores, bounded sample (rank 0, N=1 only)
+
+--dump-outputs DIR writes what the last timed step of the round trip returned (rank 0's shard) as float32 .npy files:
+DIR/decoded.npy [16, 2, 442368] and DIR/latent.npy [16, 64, 216], 57.5 MB together.  Weights, audio and sampler noise
+come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -238,6 +242,14 @@ def gpu_eager_baseline(dev, steps=3):
     return out
 
 
+def dump_outputs(out_dir, tensors):
+    """name -> tensor, written as out_dir/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def workload_config(n_gpus):
     return {"workload": "BASELINE configs[1]: SAO-shape sigmaVAE encode -> sample('fix') -> decode round trip, "
                         f"{BATCH_PER_GPU} clips x 10.03 s per GPU, bf16 tensor-core mode, fp32 I/O",
@@ -282,8 +294,12 @@ def run_cuda(args):
         _ms, z = ae.encode_and_sample(x)
         return ae.decode(z), z
 
+    last = {}                            # outputs of the latest step, kept only for --dump-outputs
+
     def step_resident():
-        y, _ = roundtrip(x_dev)
+        y, z = roundtrip(x_dev)
+        if args.dump_outputs:
+            last["decoded"], last["latent"] = y, z
         return y
 
     # end-to-end leg: the public host-buffer pipeline (kalle_audio_b200.HostPipeline) -- every step copies its input
@@ -448,6 +464,9 @@ def run_cuda(args):
             except Exception as exc:                       # never lose the main line to an extra leg
                 extra[name] = {"error": f"{type(exc).__name__}: {exc}"}
             torch.cuda.empty_cache()
+    if args.dump_outputs and rank == 0:  # after every timed leg: no file I/O between them
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     if rank == 0:
         line.update(extra)
         print(json.dumps(line), flush=True)
@@ -991,7 +1010,14 @@ def main():
     ap.add_argument("--main-only", action="store_true",
                     help="only the configs[1] line (skip the extra keys: configs[2] strong scaling, configs[3] streaming, "
                          "configs[4] training step, torch-eager GPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the decoded waveform and the sampled latent of the last timed "
+                         "round-trip step as DIR/decoded.npy and DIR/latent.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "cuda" or args.workload != "roundtrip"):
+        ap.error("--dump-outputs applies to the CUDA round trip (--impl cuda --workload roundtrip)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "train":
