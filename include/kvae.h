@@ -271,6 +271,32 @@ int kvae_mrstft_loss(const void* input, const void* target, int B, int C, long l
  * `downsample.lowpass.filter` buffers (device fp32). */
 int kvae_aa_act_fwd(const void* x, void* y, const float* alpha, const float* beta, int logscale, const float* filt_up,
                     const float* filt_down, int B, int C, long long T, int dtype, void* stream);
+/* Window form of kvae_aa_act_fwd for the streaming decoder (BigVGANStreamingDecoder; every Activation1d of flows.py:266,
+   312, 443).  x holds the absolute rows [x0, x0 + nx) of each of the B*C rows at pitch ldx; outputs t in [o0, o1) are
+   written to y + row * ldy + (t - o0).  Replicate padding happens only at absolute row 0 and, when t_end >= 0, at the
+   stream end t_end; t_end < 0 = the stream continues.  Rows [max(0, o0 - 5), min(o1 + 5, t_end)) must lie in the
+   window.  Per-sample arithmetic is the whole-row kernel's: kvae_aa_act_fwd is the case x0 = o0 = 0, o1 = t_end = T.
+   Replicate padding at the start only ever touches rows < 0, and outputs o >= 5 read no such row: a window whose
+   outputs all lie at o0 >= 5 may therefore be addressed from any origin that keeps o0 >= 5 (the streaming decoder
+   passes window-relative rows, x0 = 0, o0 = 5, so that its captured launches repeat from push to push). */
+int kvae_aa_act_win_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy, long long o0,
+                        long long o1, long long t_end, const float* alpha, const float* beta, int logscale,
+                        const float* filt_up, const float* filt_down, int B, int C, int dtype, void* stream);
+/* Window form of the conv layers of BigVGANFlowVAE for the streaming decoder (Conv1d / ConvTranspose1d, flows.py:336-391,
+   566-620).  kvae_conv1d_pack packs a folded fp32 weight ([Cout, Cin, K], transposed: [Cin, Cout, K]) once, for engine
+   0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split, into kvae_conv1d_packed_bytes.  kvae_conv1d_win_fwd
+   runs the conv (padding `padding`) of the T-row window x ([B, Cin] rows at pitch ldx) with those weights and writes only
+   its output rows [o0, o1) to y ([B, Cout] rows at pitch ldy, row o0 first); tcgen05 engines need o0 and o1 to be
+   multiples of the stride of a transposed conv and kvae_conv1d_win_scratch_bytes of scratch.  Per output row the
+   arithmetic is that of kvae_conv1d_fwd / kvae_conv1d_tc_fwd. */
+size_t kvae_conv1d_packed_bytes(int Cin, int Cout, int K, int engine);
+int kvae_conv1d_pack(const float* w, int transposed, int Cin, int Cout, int K, int engine, void* packed,
+                     size_t packed_bytes, void* stream);
+size_t kvae_conv1d_win_scratch_bytes(int B, int Cin, long long T, int engine);
+int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, const void* packed, const float* bias,
+                        int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation,
+                        int padding, long long o0, long long o1, int dtype, int engine, void* scratch,
+                        size_t scratch_bytes, void* stream);
 /* op 0: nn.LeakyReLU(param) (flows.py:181-217), op 1: tanh (:527) */
 int kvae_unary_fwd(const void* x, void* y, size_t n, int op, float param, int dtype, void* stream);
 /* out = alpha*a + beta*b: the residual adds of the AMP blocks (:283) and their average (:519-520) */

@@ -22,6 +22,7 @@ from .hostio import HostPipeline
 from .glue import LatentGlue
 from .dataset import LatentExtractor
 from .bigvgan import BigVGANFlowVAE
+from .bigvgan_stream import BigVGANStreamingDecoder, bigvgan_stream_geometry
 from .losses import MultiResolutionSTFTLoss, SumAndDifferenceSTFTLoss, aw_fir_taps
 from .discriminators import OobleckDiscriminator, get_hinge_losses
 from .utils import load_ckpt_state_dict, prepare_audio, remove_weight_norm_from_model, to_pcm16
@@ -37,4 +38,5 @@ __all__ = [
     "get_activation", "load_ckpt_state_dict", "prepare_audio", "remove_weight_norm_from_model", "sample",
     "snake_beta", "vae_sample", "to_pcm16", "AutoencoderTrainer", "FlatAdamW", "GradSync", "flatten_parameters",
     "gaussian_nll", "vae_sample_with_grad", "StreamingDecoder", "decoder_context_frames", "HostPipeline", "LatentGlue", "LatentExtractor", "BigVGANFlowVAE",
+    "BigVGANStreamingDecoder", "bigvgan_stream_geometry",
 ]

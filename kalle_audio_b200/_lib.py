@@ -80,6 +80,17 @@ SIGNATURES = {
     "kvae_plan_fused_pcm_supported": (C.c_int, [C.c_void_p]),
     "kvae_aa_act_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                   C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_aa_act_win_fwd": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_longlong,
+                                      C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int,
+                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "kvae_conv1d_packed_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "kvae_conv1d_pack": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
+                                   C.c_void_p]),
+    "kvae_conv1d_win_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong, C.c_int]),
+    "kvae_conv1d_win_fwd": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p,
+                                      C.c_int, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int,
+                                      C.c_int, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
+                                      C.c_void_p]),
     "kvae_unary_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_int, C.c_void_p]),
     "kvae_axpby": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_int, C.c_void_p]),
     "kvae_gauss_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

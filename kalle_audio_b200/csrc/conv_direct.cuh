@@ -36,6 +36,8 @@ struct DirectParams {
   const float* snake_a;
   const float* snake_inv_b;
   int tanh_out;
+  int q_base;                     // window form: first output row index q computed (blocks start there)
+  int t_lo;                       // window form: outputs t < t_lo are not stored; out_raw holds t - t_lo
 };
 
 constexpr int kDirectKC = 16;
@@ -54,7 +56,7 @@ conv_direct_kernel(const __grid_constant__ DirectParams p) {
   const int tx = tid % (BN / TN);
   const int ty = tid / (BN / TN);
   const int phi = blockIdx.x % p.P_out;
-  const int q0 = (blockIdx.x / p.P_out) * BT;
+  const int q0 = (blockIdx.x / p.P_out) * BT + p.q_base;
   const int n0 = blockIdx.y * BN;
   const int b = blockIdx.z;
   const int t_lo = p.tap_begin[phi], t_hi = p.tap_begin[phi + 1];
@@ -116,7 +118,7 @@ conv_direct_kernel(const __grid_constant__ DirectParams p) {
     const int q = q0 + ty * TM + i;
     if (q >= p.Tq_out) continue;
     const long long t_out = static_cast<long long>(q) * p.P_out + phi;
-    if (t_out >= T_out) continue;
+    if (t_out >= T_out || t_out < p.t_lo) continue;
     const size_t cl_row = (static_cast<size_t>(b) * T_out + t_out) * p.Cout;
 #pragma unroll
     for (int j = 0; j < TN; ++j) {
@@ -129,7 +131,7 @@ conv_direct_kernel(const __grid_constant__ DirectParams p) {
                             : __bfloat162float(static_cast<const __nv_bfloat16*>(p.residual)[cl_row + co]);
       if (p.tanh_out) v = tanhf(v);
       if (p.out_raw) {
-        const long long off = b * p.o_sB + t_out * p.o_sT + co * p.o_sC;
+        const long long off = b * p.o_sB + (t_out - p.t_lo) * p.o_sT + co * p.o_sC;
         if (p.out_raw_f32) static_cast<float*>(p.out_raw)[off] = v;
         else static_cast<__nv_bfloat16*>(p.out_raw)[off] = __float2bfloat16(v);
       }

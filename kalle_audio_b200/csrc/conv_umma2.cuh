@@ -53,6 +53,7 @@ struct ConvParams2 {
                            //    (fp32 in registers and TMEM); 0: fp32.  Inference plans use fp16: it halves the
                            //    stream traffic of the HBM-bound 128-channel stages for +4e-5 of the 1e-3 budget
   void* out_cf;            // raw_mode 2: [B, Cout, T_out]
+  long long cf_ld;         // raw_mode 2: elements between channel rows of out_cf (0: T_out)
   int out_cf_f32;
   int act_mode;            // 0 none, 1 bf16 channels-last via TMA (tmO)
   int one_producer;        // 1: activation and weight slabs requested by one thread in one FIFO (A/B switch)
@@ -819,7 +820,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             for (int j = 0; j < 32; ++j) {
               const int q = r0 + j;
               if (q < p.Tq_out) {
-                const size_t o = (static_cast<size_t>(b) * p.Cout + c) * T_out + static_cast<size_t>(q) * p.P_out + phi;
+                const size_t o = (static_cast<size_t>(b) * p.Cout + c) * (p.cf_ld ? p.cf_ld : T_out) + static_cast<size_t>(q) * p.P_out + phi;
                 if (p.out_cf_f32) static_cast<float*>(p.out_cf)[o] = v[j];
                 else static_cast<__nv_bfloat16*>(p.out_cf)[o] = __float2bfloat16(v[j]);
                 fused_sigma_sample(p, b, c, static_cast<size_t>(q) * p.P_out + phi, T_out, v[j]);
@@ -898,15 +899,16 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           const int q = r0 + lane;
           if (q < p.Tq_out) {
             const size_t t_out = static_cast<size_t>(q) * p.P_out + phi;
-            const size_t o0 = (static_cast<size_t>(b) * p.Cout + cbase) * T_out + t_out;
+            const size_t ld = p.cf_ld ? static_cast<size_t>(p.cf_ld) : static_cast<size_t>(T_out);
+            const size_t o0 = (static_cast<size_t>(b) * p.Cout + cbase) * ld + t_out;
             if (p.out_cf_f32) {
               float* op = static_cast<float*>(p.out_cf) + o0;
 #pragma unroll
-              for (int j = 0; j < 32; ++j) op[static_cast<size_t>(j) * T_out] = v[j];
+              for (int j = 0; j < 32; ++j) op[static_cast<size_t>(j) * ld] = v[j];
             } else {
               __nv_bfloat16* op = static_cast<__nv_bfloat16*>(p.out_cf) + o0;
 #pragma unroll
-              for (int j = 0; j < 32; ++j) op[static_cast<size_t>(j) * T_out] = __float2bfloat16(v[j]);
+              for (int j = 0; j < 32; ++j) op[static_cast<size_t>(j) * ld] = __float2bfloat16(v[j]);
             }
             if (p.samp_noise) {
 #pragma unroll

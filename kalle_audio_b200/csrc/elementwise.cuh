@@ -56,14 +56,15 @@ __global__ void snake_params_kernel(const float* alpha, const float* beta, int l
 // split = 1: y is [B, T, 2C] with the bf16 (hi | lo) halves of the fp32 value (fp32-mode tensor-core operand)
 // y_pitch (0 = T): rows between clips in y (the streaming decoder writes into a window buffer)
 __global__ void cf_to_cl_bf16_kernel(const void* x, int f32, __nv_bfloat16* y, int C, int T, int split,
-                                     long long y_pitch = 0) {
+                                     long long y_pitch = 0, long long x_pitch = 0) {
   const long long YP = y_pitch ? y_pitch : T;
+  const long long XP = x_pitch ? x_pitch : T;          // elements between channel rows of x
   __shared__ float tile[32][33];
   const int b = blockIdx.z;
   const int t0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += 8) {
     const int c = c0 + i, t = t0 + threadIdx.x;
-    tile[i][threadIdx.x] = (c < C && t < T) ? ld_elem(x, (static_cast<size_t>(b) * C + c) * T + t, f32) : 0.f;
+    tile[i][threadIdx.x] = (c < C && t < T) ? ld_elem(x, (static_cast<size_t>(b) * C + c) * XP + t, f32) : 0.f;
   }
   __syncthreads();
   for (int i = threadIdx.y; i < 32; i += 8) {

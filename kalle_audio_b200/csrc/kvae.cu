@@ -2000,6 +2000,134 @@ int kvae_conv1d_tc_fwd(const void* x, void* y, const float* w, const float* bias
   return 0;
 }
 
+// Window form of the layer-level conv for the streaming BigVGAN decoder: weights packed once (kvae_conv1d_pack), input
+// and output pitched, and only the output rows [o0, o1) of the conv of the T-row window computed.  Engines: 0 = CUDA
+// cores fp32 (conv_direct_kernel), 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split -- the arithmetic of kvae_conv1d_fwd /
+// kvae_conv1d_tc_fwd per output row.
+namespace {
+size_t win_pack_main_bytes(int Cin, int Cout, int K, int engine) {
+  const size_t n = static_cast<size_t>(Cin) * Cout * K;
+  return engine == 0 ? align_up(n * 4, 1024) : align_up(n * 2 * (engine == 2 ? 2 : 1), 1024);
+}
+}  // namespace
+
+size_t kvae_conv1d_packed_bytes(int Cin, int Cout, int K, int engine) {
+  if (engine < 0 || engine > 2) return 0;
+  const size_t n = static_cast<size_t>(Cin) * Cout * K;
+  return win_pack_main_bytes(Cin, Cout, K, engine) + (engine == 2 ? align_up(n * 4, 1024) : 0);
+}
+
+int kvae_conv1d_pack(const float* w, int transposed, int Cin, int Cout, int K, int engine, void* packed,
+                     size_t packed_bytes, void* stream) {
+  if (!w || !packed) return fail("null argument");
+  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
+  if (Cin <= 0 || Cout <= 0 || K <= 0) return fail("empty weight");
+  if (packed_bytes < kvae_conv1d_packed_bytes(Cin, Cout, K, engine)) return fail("packed buffer too small");
+  DeviceGuard guard(device_of(w));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t n = static_cast<size_t>(Cin) * Cout * K;
+  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 4096));
+  uint8_t* base = static_cast<uint8_t*>(packed);
+  if (engine == 0) {
+    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, reinterpret_cast<float*>(base));
+  } else if (engine == 1) {
+    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, reinterpret_cast<__nv_bfloat16*>(base), nullptr);
+  } else {
+    float* w_direct = reinterpret_cast<float*>(base + win_pack_main_bytes(Cin, Cout, K, 2));
+    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, w_direct);
+    KV_CUDA(cudaGetLastError());
+    split_pack_kernel<<<blocks, 256, 0, st>>>(w_direct, K, Cin, Cout, reinterpret_cast<__nv_bfloat16*>(base));
+    ++g_launches;
+  }
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+size_t kvae_conv1d_win_scratch_bytes(int B, int Cin, long long T, int engine) {
+  if (engine == 0) return 0;
+  return align_up(static_cast<size_t>(B) * T * Cin * 2 * (engine == 2 ? 2 : 1), 1024);
+}
+
+int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, const void* packed, const float* bias,
+                        int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation,
+                        int padding, long long o0, long long o1, int dtype, int engine, void* scratch,
+                        size_t scratch_bytes, void* stream) {
+  if (!x || !y || !packed) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
+  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
+  if (!transposed && stride != 1) return fail("window form: stride-1 or transposed convs");
+  if (ldx < T) return fail("ldx < T");
+  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
+  const long long T_nat = g.out_len(static_cast<int>(T));
+  if (o0 < 0 || o1 <= o0 || o1 > T_nat) return fail("output rows must satisfy 0 <= o0 < o1 <= the conv's output length");
+  if (ldy < o1 - o0) return fail("ldy < o1 - o0");
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int P_out = transposed ? stride : 1;
+  if (engine == 0) {
+    TapPlan tp;
+    std::string err;
+    if (!build_taps(g, false, tp, err)) return fail(err);
+    DirectParams d;
+    std::memset(&d, 0, sizeof(d));
+    d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
+    d.Tq_out = static_cast<int>((o1 + tp.P_out - 1) / tp.P_out); d.T_out = static_cast<int>(o1);
+    d.q_base = static_cast<int>(o0 / tp.P_out); d.t_lo = static_cast<int>(o0);
+    d.T_in = static_cast<int>(T); d.Cin = Cin; d.Cout = Cout; d.span = tp.span;
+    for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
+    for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+    d.x = x; d.x_f32 = (dtype == KVAE_F32);
+    d.x_sB = static_cast<long long>(Cin) * ldx; d.x_sT = 1; d.x_sC = ldx;
+    d.w = static_cast<const float*>(packed); d.bias = bias;
+    d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
+    d.o_sB = static_cast<long long>(Cout) * ldy; d.o_sT = 1; d.o_sC = ldy;
+    const int cfg = direct_cfg_for(Cout);
+    int BT, BN;
+    direct_tile(cfg, BT, BN);
+    dim3 grid(ceil_div(d.Tq_out - d.q_base, BT) * tp.P_out, ceil_div(Cout, BN), B);
+    const size_t smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
+    KV_CUDA(launch_direct(d, grid, cfg, smem, st));
+    ++g_launches;
+    return 0;
+  }
+  if (!kvae_conv1d_tc_supported(Cin, Cout, K, stride, dilation, transposed))
+    return fail("kvae_conv1d_win_fwd: the tcgen05 engine needs channel counts that are multiples of 64");
+  if (o0 % P_out || o1 % P_out) return fail("tcgen05 engine: o0 and o1 must be multiples of the stride (transposed)");
+  if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, Cin, T, engine) || !scratch) return fail("scratch too small");
+  const int split = engine == 2 ? 2 : 1;
+  __nv_bfloat16* xcl = static_cast<__nv_bfloat16*>(scratch);
+  {
+    dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(Cin, 32), B), block(32, 8);
+    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, Cin, static_cast<int>(T), split == 2 ? 1 : 0,
+                                                 0, ldx);
+    KV_CUDA(cudaGetLastError());
+  }
+  ConvEpilogue ep;
+  ep.bias = bias;
+  ep.out_raw = y;
+  ep.out_raw_cf = 1;
+  ep.out_raw_f32 = (dtype == KVAE_F32);
+  if (split == 2) { ep.split3 = 1; ep.precise = 1; }
+  ConvTuning2 tune;
+  ConvLaunch2 L;
+  std::string err;
+  StreamGeom sg;                 // rows q of the window's output from o0 / P_out on: taps shifted by that many rows
+  sg.in_rows = static_cast<int>(T);
+  sg.out_q = static_cast<int>((o1 - o0) / P_out);
+  sg.row_bias = static_cast<int>(o0 / P_out);
+  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(T), static_cast<const __nv_bfloat16*>(packed), ep, tune, L, err, &sg))
+    return fail(err);
+  L.p.cf_ld = ldy;
+  KV_CUDA(launch_conv_umma2(L, st));
+  g_launches += 2;
+  return 0;
+}
+
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)
 namespace {
 int mrstft_signals(int B, int C, int sum_diff) { return sum_diff ? 2 * B : B * C; }
@@ -2411,15 +2539,26 @@ int kvae_sigma_sample(const void* mean, const void* noise, void* out, size_t n, 
 // ------------------------------------------------------------------ BigVGANFlowVAE leaf kernels (bigvgan.cuh)
 int kvae_aa_act_fwd(const void* x, void* y, const float* alpha, const float* beta, int logscale, const float* filt_up,
                     const float* filt_down, int B, int C, long long T, int dtype, void* stream) {
+  return kvae_aa_act_win_fwd(x, T, 0, T, y, T, 0, T, T, alpha, beta, logscale, filt_up, filt_down, B, C, dtype, stream);
+}
+
+int kvae_aa_act_win_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy, long long o0,
+                        long long o1, long long t_end, const float* alpha, const float* beta, int logscale,
+                        const float* filt_up, const float* filt_down, int B, int C, int dtype, void* stream) {
   if (!x || !y || !alpha || !filt_up || !filt_down) return fail("null argument");
   if (!check_dtype(dtype)) return fail("bad dtype");
-  if (B <= 0 || C <= 0 || T <= 0) return 0;
+  if (B <= 0 || C <= 0 || o1 <= o0) return 0;
   if (static_cast<long long>(B) * C > 65535) return fail("B*C too large");
+  const long long te = t_end < 0 ? kAaNoEnd : t_end;
+  if (x0 < 0 || nx <= 0 || o0 < 0 || o1 > te || ldx < nx || ldy < o1 - o0)
+    return fail("aa_act window: need 0 <= x0, 0 <= o0 < o1 <= t_end, nx <= ldx, o1 - o0 <= ldy");
+  if (std::max(0ll, o0 - kAaHalo) < x0 || std::min(o1 + kAaHalo, te) > x0 + nx)
+    return fail("aa_act window: the input rows [o0 - 5, o1 + 5) (clipped to the stream) must be inside [x0, x0 + nx)");
   DeviceGuard guard(device_of(x));
   if (!guard.ok) return fail("cannot select the tensor's device");
-  dim3 grid(static_cast<unsigned>((T + kAaTile - 1) / kAaTile), B * C);
-  aa_act_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, y, alpha, beta, logscale, filt_up, filt_down, C, T,
-                                                                     dtype == KVAE_F32);
+  dim3 grid(static_cast<unsigned>((o1 - o0 + kAaTile - 1) / kAaTile), B * C);
+  aa_act_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, ldx, x0, nx, y, ldy, o0, o1, te, alpha, beta,
+                                                                     logscale, filt_up, filt_down, C, dtype == KVAE_F32);
   KV_CUDA(cudaGetLastError());
   ++g_launches;
   return 0;
