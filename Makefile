@@ -19,17 +19,11 @@ build/tma_copy_probe: tools/tma_copy_probe.cu $(CSRC)/ptx.cuh
 	@mkdir -p build
 	$(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo -o $@ $< -lcuda
 
-# A/B build used by tools/run_ab_*.sh (KVAE_LIB=build/libkvae_nu.so): plain threadIdx.x >> 5 warp index, i.e. TMA
-# operands in vector registers (the state before ptx::warp_idx)
-build/libkvae_nu.so: $(CSRC)/kvae.cu $(HDRS)
-	@mkdir -p build
-	$(NVCC) $(NVFLAGS) -DKVAE_UNIFORM_WARP=0 -shared -o $@ $<
-
 oracle:
 	$(MAKE) -C oracle
 
 clean:
-	rm -f $(LIB) build/umma_probe build/tma_copy_probe build/libkvae_nu.so
+	rm -f $(LIB) build/umma_probe build/tma_copy_probe
 	$(MAKE) -C oracle clean
 
 .PHONY: all clean oracle

@@ -11,7 +11,7 @@
 #include <cuda_bf16.h>
 #include <cstdint>
 
-#include "conv_umma.cuh"  // Tap, kMaxTaps, kMaxPhases, snake_beta
+#include "conv_common.cuh"  // Tap, kMaxTaps, kMaxPhases, snake_beta
 
 namespace kvae {
 

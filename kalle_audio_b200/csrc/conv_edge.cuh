@@ -14,7 +14,7 @@
 #include <cuda_fp16.h>
 #include <cstdint>
 
-#include "conv_umma.cuh"    // snake_beta
+#include "conv_common.cuh"  // snake_beta
 #include "elementwise.cuh"  // ld_elem / st_elem
 #include "ptx.cuh"
 

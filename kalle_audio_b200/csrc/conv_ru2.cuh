@@ -1,21 +1,77 @@
-// conv_ru2: the fused ResidualUnit of conv_ru.cuh (reference autoencoders.py:39-62) with the tensor pipe kept busy
-// across tiles.  conv_ru_kernel runs GEMM1 -> EPI1 -> GEMM2 of a tile as a serial chain on one accumulator; the
-// ablation in profiles/r01_ru_ablation.txt shows that chain alone (no HBM traffic at all) costs 0.35 of the 0.47 ms
-// per launch, against 0.19 ms of tensor work.  Here:
+// conv_ru2: one-kernel ResidualUnit for 128-channel stages (reference autoencoders.py:39-62):
+//     x' = x + conv_k1( SnakeBeta2( conv_k7_dil_d( SnakeBeta1(x) ) ) )
+// The producer of x already wrote a = SnakeBeta1(x) (bf16 operand) and x (the fp16 residual stream); this kernel never
+// materialises the intermediate h = SnakeBeta2(conv_k7(a)) in HBM.  Per output row it moves 256 B (a) + 256 B (x) in and
+// 256 B (x') + 256 B (a' = next layer's operand) out = 1024 B instead of the 1536 B of the two-kernel form, which also
+// writes and reads h -- these stages are HBM-bound, so that is the speed-up.
+//
+// Orientation (see conv_umma2.cuh "swap"): out-channels on the MMA M side (TMEM lanes), 256 time rows on N.
+//   GEMM1  D1[co, t]  = sum_{tap,ci} W7[tap][co, ci] * a[t + shift(tap), ci]      (14 x 4 MMAs of 128x256x16)
+//   EPI1   h[t, c]    = bf16( SnakeBeta2( D1[c, t] + bias7[c] ) )  -> shared memory, K-major, 128-row halves
+//   GEMM2  D2[co2, t] = sum_c W1[co2, c] * h[t, c]                                 (2 halves x 2 x 4 MMAs of 128x128x16)
+//   EPI2   x'[t, c]   = D2[c, t] + bias1[c] + x[t, c]  -> fp16 stream (TMA store); a' = bf16(SnakeBeta_next(x')) (TMA store)
+// Warp roles (640 threads): 0 weight TMA producer, 1 UMMA issuer, 2 TMEM allocator, 3 activation-slab TMA producer, 4-19
+// epilogue.  All 16 epilogue warps (4 per TMEM lane quadrant) do BOTH epilogues, one after the other: their EPI1 share of
+// a tile, then their EPI2 share (4 of the 16 16-row items); with separate EPI1 / EPI2 warp groups the EPI1 warps idled
+// 70 % of the time waiting for GEMM1 (profiles/r01_conv_ru_unified_epilogue_B16.ncu-rep).  Every warp prefetches its
+// next skip-connection block by TMA and stores in place.
+//
+// The tensor pipe is kept busy across tiles.  Run as a serial GEMM1 -> EPI1 -> GEMM2 chain on one accumulator (the
+// first two generations of this kernel), the chain alone (no HBM traffic at all) cost 0.35 of the 0.47 ms per launch,
+// against 0.19 ms of tensor work (profiles/r01_ru_ablation.txt).  Here:
 //   * TMEM holds TWO 256-column accumulators; tile i uses buffer i & 1.  GEMM2 of a half writes D2 IN PLACE over the
 //     128 columns of D1 that EPI1 has just consumed, so two tiles are in flight in 512 columns.
 //   * The single MMA thread issues GEMM1 of tile i+1 slab by slab and slots the two GEMM2 halves of tile i in at
-//     fixed slab positions (k0, k1): the k=1 conv of tile i executes in the middle of the k=7 conv of tile i+1, the
-//     pipe never drains while the epilogue warps turn D1 into h, and EPI2 of tile i runs under the rest of GEMM1.
+//     fixed slab positions (kRuK0, kRuK1): the k=1 conv of tile i executes in the middle of the k=7 conv of tile i+1,
+//     the pipe never drains while the epilogue warps turn D1 into h, and EPI2 of tile i runs under the rest of GEMM1.
 //   * The weight ring is strictly FIFO in that issue order: W7 slabs of tile i+1 with the two W1 chunks of tile i
 //     inserted (twice, once per half) at the same positions.
-//   * Epilogue warps use the fragment mapping of conv_ru_kernel<1> (tcgen05.ld.16x256b, ldmatrix/stmatrix.trans,
-//     packed fp32 pairs).
-// Same RuParams / tensor maps / shared-memory layout as conv_ru_kernel; results are bit-identical to it.
+//   * Epilogue warps use the mma-style fragment mapping (tcgen05.ld.16x256b, ldmatrix/stmatrix.trans, packed fp32
+//     pairs).
+// Shared memory (227 KB): activation slab ring 2 x <=40 KB, weight ring of 16 KB stages (W7 taps, then the two W1
+// chunks of the tile), h half 32 KB, epilogue staging 16 x 3 KB.
 #pragma once
-#include "conv_ru.cuh"
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+#include <cstdint>
+
+#include "conv_umma2.cuh"
 
 namespace kvae {
+
+struct RuParams {
+  int B, T;                 // rows per clip (stride-1 conv: T_in == T_out)
+  int RB, nbox;             // activation slab = nbox TMA boxes of RB rows (256 + 6*dilation rows)
+  int SA, SB;
+  int q_tiles, total_tiles; // 256-row tiles
+  uint32_t tap_shift16[7];  // (tap*dilation*128 B) >> 4
+  int slab_row0;            // slab start row relative to the tile's first row (= -3*dilation)
+  const float* bias7;       // [128]
+  const float* s2_a;        // SnakeBeta between the two convs
+  const float* s2_inv_b;
+  const float* bias1;       // [128]
+  int raw_out;              // 1: fp16 stream out via tmR
+  int act_out;              // 1: bf16 operand out via tmO
+  const float* sn_a;        // SnakeBeta folded into the operand output (nullptr: plain cast)
+  const float* sn_inv_b;
+  int act_f16;              // the operand output is fp16 instead of bf16 (the unit in front of the decoder tail,
+                            // whose GEMM is kind::f16 -- conv_edge.cuh, WaveOutTcParams::preact)
+};
+
+constexpr int kRuC = 128;
+constexpr int kRuHBytes = 2 * 128 * 128;   // h half: 2 K-chunks x [128 rows x 128 B]
+constexpr int kRuActBlk = 16 * 64;         // 16 rows x 32 bf16 / fp16, SWIZZLE_64B
+constexpr int kRuThreads = 640;
+constexpr int kRuEpiWarps = 16;
+// GEMM2 half 0 / half 1 of tile i are issued before slab kRuK0 / kRuK1 of tile i+1's GEMM1 (14 slabs: 2 chunks x 7 taps)
+constexpr int kRuK0 = 3, kRuK1 = 6;
+
+// per epilogue warp: 2 fp16 stream blocks (skip in / stream out, in place) + 1 bf16 operand block
+__host__ __device__ inline int ru_stage_bytes_per_warp(int act_out) { return 2 * kRuActBlk + (act_out ? kRuActBlk : 0); }
+__host__ __device__ inline size_t ru_smem_bytes(const RuParams& p) {
+  return 1024 + 1024 + static_cast<size_t>(p.SA) * p.nbox * p.RB * 128 + static_cast<size_t>(p.SB) * kRuC * 128 +
+         kRuHBytes + kRuEpiWarps * ru_stage_bytes_per_warp(p.act_out);
+}
 
 __global__ void __launch_bounds__(kRuThreads, 1)
 conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW7,
@@ -74,7 +130,7 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   ptx::tc_fence_after();
   ptx::pdl_wait();
   const uint32_t tmem_base = *tmem_slot;
-  const int k0 = p.k0, k1 = p.k1;       // GEMM2 half 0 / half 1 of tile i are issued before slab k0 / k1 of tile i+1
+  constexpr int k0 = kRuK0, k1 = kRuK1;
 
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer: ring entries in MMA issue order
@@ -84,12 +140,8 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       auto load_w = [&](const CUtensorMap* tm, int c0, int c2) {
         ptx::mbar_wait(&b_empty[bs], bph ^ 1u);
         if (ptx::elect_one()) {
-          if (p.dbg & 32) {                                // ablation: no weight loads
-            ptx::mbar_arrive(&b_full[bs]);
-          } else {
-            ptx::mbar_expect_tx(&b_full[bs], b_bytes);
-            ptx::tma_load_3d(b_ring + static_cast<size_t>(bs) * b_bytes, tm, &b_full[bs], c0, 0, c2);
-          }
+          ptx::mbar_expect_tx(&b_full[bs], b_bytes);
+          ptx::tma_load_3d(b_ring + static_cast<size_t>(bs) * b_bytes, tm, &b_full[bs], c0, 0, c2);
         }
         __syncwarp();
         if (++bs == p.SB) { bs = 0; bph ^= 1u; }
@@ -117,34 +169,13 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
         const int b = tile / p.q_tiles;
         const int q0 = (tile % p.q_tiles) * 256;
-        if (p.pf && ptx::elect_one()) {
-          // HBM -> L2 one tile period ahead: the rows of this CTA's next tile are contiguous in both tensors
-          const int t2 = tile + gridDim.x;
-          if (t2 < p.total_tiles) {
-            const int b2 = t2 / p.q_tiles, q2 = (t2 % p.q_tiles) * 256;
-            if (p.pf & 1) {
-              const int lo = max(0, q2 + p.slab_row0), hi = min(p.T, q2 + 256 - p.slab_row0);
-              ptx::bulk_prefetch_l2(static_cast<const uint8_t*>(p.a_ptr) + (static_cast<size_t>(b2) * p.T + lo) * 256,
-                                    static_cast<uint32_t>(hi - lo) * 256u);
-            }
-            if (p.pf & 2) {
-              const int hi = min(p.T, q2 + 256);
-              ptx::bulk_prefetch_l2(static_cast<const uint8_t*>(p.x_ptr) + (static_cast<size_t>(b2) * p.T + q2) * 256,
-                                    static_cast<uint32_t>(hi - q2) * 256u);
-            }
-          }
-        }
         for (int ch = 0; ch < 2; ++ch) {
           ptx::mbar_wait(&a_empty[as], aph ^ 1u);
           if (ptx::elect_one()) {
-            if (p.dbg & 64) {                            // ablation: no activation loads
-              ptx::mbar_arrive(&a_full[as]);
-            } else {
-              ptx::mbar_expect_tx(&a_full[as], a_bytes);
-              for (int bx = 0; bx < p.nbox; ++bx)
-                ptx::tma_load_4d(a_ring + static_cast<size_t>(as) * a_bytes + bx * p.RB * 128, &tmA, &a_full[as], ch * 64, 0,
-                                 q0 + p.slab_row0 + bx * p.RB, b);
-            }
+            ptx::mbar_expect_tx(&a_full[as], a_bytes);
+            for (int bx = 0; bx < p.nbox; ++bx)
+              ptx::tma_load_4d(a_ring + static_cast<size_t>(as) * a_bytes + bx * p.RB * 128, &tmA, &a_full[as], ch * 64, 0,
+                               q0 + p.slab_row0 + bx * p.RB, b);
           }
           __syncwarp();
           if (++as == p.SA) { as = 0; aph ^= 1u; }
@@ -223,12 +254,10 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             const int cbs = bs;
             if (++bs == p.SB) { bs = 0; bph ^= 1u; }
             if (ptx::elect_one()) {
-              if (!(p.dbg & 16) || t == 0) {
-                ptx::umma_f16(dnext, desc_hi | bl, desc_hi | al, idesc1, s ? 1u : 0u);
-                ptx::umma_f16(dnext, desc_hi | (bl + 2), desc_hi | (al + 2), idesc1, 1u);
-                ptx::umma_f16(dnext, desc_hi | (bl + 4), desc_hi | (al + 4), idesc1, 1u);
-                ptx::umma_f16(dnext, desc_hi | (bl + 6), desc_hi | (al + 6), idesc1, 1u);
-              }
+              ptx::umma_f16(dnext, desc_hi | bl, desc_hi | al, idesc1, s ? 1u : 0u);
+              ptx::umma_f16(dnext, desc_hi | (bl + 2), desc_hi | (al + 2), idesc1, 1u);
+              ptx::umma_f16(dnext, desc_hi | (bl + 4), desc_hi | (al + 4), idesc1, 1u);
+              ptx::umma_f16(dnext, desc_hi | (bl + 6), desc_hi | (al + 6), idesc1, 1u);
               ptx::umma_commit(&b_empty[cbs]);
               if (s == 6 || s == 13) ptx::umma_commit(&a_empty[cur_a]);
               if (s == 13) ptx::umma_commit(&d1_full[(i + 1) & 1]);
@@ -240,7 +269,7 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       }
     }
   } else if (warp >= 4) {
-    // ------------------------------------------------------------ epilogue warps (fragment mapping, see conv_ru_kernel<1>)
+    // ------------------------------------------------------------ epilogue warps (fragment mapping)
     const int e = warp - 4;                            // 0..15
     const int quad = warp & 3;                         // TMEM lane quadrant = channels quad*32 .. +31
     const int sub = e >> 2;                            // 0..3
@@ -263,13 +292,12 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     const uint32_t ablk_lane = ring_lane + 2 * kRuActBlk;
     uint8_t* ablk = ring + 2 * kRuActBlk;
     uint64_t* my_res_full = res_full + e * 2;
-    const bool use_skip = !(p.dbg & 1);
     const bool has_snake = p.sn_a != nullptr;
     auto issue_skip = [&](int tb, int tq0, int item, int slot) {   // lane 0 only; (tb, tq0) = clip, first row of the tile
       ptx::mbar_expect_tx(&my_res_full[slot], kRuActBlk);
       ptx::tma_load_4d(ring + slot * kRuActBlk, &tmX, &my_res_full[slot], cbase, 0, tq0 + item * 16, tb);
     };
-    if (use_skip && static_cast<int>(blockIdx.x) < p.total_tiles && ptx::elect_one())
+    if (static_cast<int>(blockIdx.x) < p.total_tiles && ptx::elect_one())
       issue_skip(blockIdx.x / p.q_tiles, (blockIdx.x % p.q_tiles) * 256, sub, 0);
     int slot = 0;
     uint32_t he_ph = 0, d2f_ph = 0, res_ph = 0;
@@ -292,13 +320,10 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         for (int half = 0; half < 2; ++half) {
           uint32_t r[32], pk[16];
           __syncwarp();
-          if (!(p.dbg & 128)) {
-            ptx::tmem_ld_16x256b_x8(d1_lane + boff + half * 128, r);
-            ptx::tmem_ld_wait();
-          }
+          ptx::tmem_ld_16x256b_x8(d1_lane + boff + half * 128, r);
+          ptx::tmem_ld_wait();
 #pragma unroll
           for (int q = 0; q < 16; ++q) {                 // q = 2n + hi: column group n, channel c1 + 8 hi
-            if (p.dbg & 128) { pk[q] = 0u; continue; }     // ablation: epilogue warps run the barrier protocol only
             const uint64_t v = ptx::f2_add(ptx::f2_pack_u(r[2 * q], r[2 * q + 1]), kb[q & 1]);
             float t0, t1, y0, y1;
             ptx::f2_unpack(ptx::f2_mul(v, ka[q & 1]), t0, t1);
@@ -311,7 +336,7 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           he_ph ^= 1u;
 #pragma unroll
           for (int m = 0; m < 4; ++m)
-            if (!(p.dbg & 128)) ptx::stmatrix_x4_trans(h_lane + m * 2048, pk[4 * m], pk[4 * m + 1], pk[4 * m + 2], pk[4 * m + 3]);
+            ptx::stmatrix_x4_trans(h_lane + m * 2048, pk[4 * m], pk[4 * m + 1], pk[4 * m + 2], pk[4 * m + 3]);
           ptx::fence_proxy_async();
           ptx::tc_fence_before();                        // this half of D1 has been read: GEMM2 may overwrite it
           __syncwarp();
@@ -340,16 +365,8 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           // every store issued so far has read its shared-memory source: the other stream slot and the operand
           // block are free again; fetch the NEXT item's skip block into the other slot
           ptx::bulk_wait_read<0>();
-          if (use_skip) {
-            if (item + 4 < 16) issue_skip(b, q0, item + 4, slot ^ 1);
-            else if (ntile < p.total_tiles) issue_skip(nb, nq0, sub, slot ^ 1);
-          }
-        }
-        if (p.dbg & 128) {
-          if (use_skip) ptx::mbar_wait_parked(&my_res_full[slot], (res_ph >> slot) & 1u);
-          res_ph ^= (1u << slot);
-          slot ^= 1;
-          continue;
+          if (item + 4 < 16) issue_skip(b, q0, item + 4, slot ^ 1);
+          else if (ntile < p.total_tiles) issue_skip(nb, nq0, sub, slot ^ 1);
         }
         uint32_t r[16], sk[8];
         __syncwarp();
@@ -357,14 +374,9 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         ptx::tmem_ld_16x256b_x2(t2, r);
         ptx::tmem_ld_16x256b_x2(t2 + (16u << 16), r + 8);
         const uint32_t rb = ring_lane + slot * kRuActBlk;
-        if (use_skip) {
-          ptx::mbar_wait_parked(&my_res_full[slot], (res_ph >> slot) & 1u);
-          ptx::ldmatrix_x4_trans(rb, sk[0], sk[1], sk[2], sk[3]);
-          ptx::ldmatrix_x4_trans(rb ^ 32u, sk[4], sk[5], sk[6], sk[7]);
-        } else {
-#pragma unroll
-          for (int q = 0; q < 8; ++q) sk[q] = 0u;
-        }
+        ptx::mbar_wait_parked(&my_res_full[slot], (res_ph >> slot) & 1u);
+        ptx::ldmatrix_x4_trans(rb, sk[0], sk[1], sk[2], sk[3]);
+        ptx::ldmatrix_x4_trans(rb ^ 32u, sk[4], sk[5], sk[6], sk[7]);
         res_ph ^= (1u << slot);
         ptx::tmem_ld_wait();
         uint64_t v[8];                                     // q = 4 L + 2 n + hi
@@ -413,8 +425,8 @@ conv_ru2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         __syncwarp();
         if (ptx::elect_one()) {
           uint8_t* const rblk = ring + slot * kRuActBlk;
-          if (p.raw_out && !(p.dbg & 2)) ptx::tma_store_4d(&tmR, rblk, cbase, 0, r0, b);
-          if (p.act_out && !(p.dbg & 2)) ptx::tma_store_4d(&tmO, ablk, cbase, 0, r0, b);
+          if (p.raw_out) ptx::tma_store_4d(&tmR, rblk, cbase, 0, r0, b);
+          if (p.act_out) ptx::tma_store_4d(&tmO, ablk, cbase, 0, r0, b);
           ptx::bulk_commit();
         }
         slot ^= 1;

@@ -1,6 +1,12 @@
 // conv_umma2: persistent, double-buffered version of the tcgen05 implicit-GEMM convolution.
 //
-// Same GEMM view and tap decomposition as conv_umma.cuh (see there).  What changes is the schedule:
+// Implicit-GEMM 1-D convolution on the sm_100a tensor cores (tcgen05.mma, TMEM accumulators, TMA-fed operands).  One
+// kernel serves the three weight-normalised convolution shapes of the Oobleck stack (reference:
+// stable_audio_tools/models/autoencoders.py:39-114): Conv1d stride 1 dilation d, Conv1d stride s kernel 2s, and
+// ConvTranspose1d stride s (polyphase).  Activations are channels-last [B, T, C] bf16, so a tap shift is a whole
+// 128-byte-row offset of a K-major operand tile; weights are pre-packed [tap][Cout][Cin] bf16.  GEMM view per tile:
+// D[M, N] += A[time rows, 64 ch] * W[out-channels, 64 ch]^T summed over (64-channel chunk) x (tap); taps that read the
+// same input phase share one staged A slab (conv_common.cuh, Tap).  The schedule:
 //   * one CTA per SM loops over output tiles (static round-robin), so operand loads of tile i+1 are
 //     in flight while tile i is still being multiplied / written out;
 //   * the accumulator lives in TMEM twice (2 x MT*NT columns) when that fits in 512 columns: the UMMA
@@ -24,7 +30,7 @@
 #include <cuda_fp16.h>
 #include <cstdint>
 
-#include "conv_umma.cuh"
+#include "conv_common.cuh"
 #include "ptx.cuh"
 
 namespace kvae {
@@ -56,12 +62,9 @@ struct ConvParams2 {
   long long cf_ld;         // raw_mode 2: elements between channel rows of out_cf (0: T_out)
   int out_cf_f32;
   int act_mode;            // 0 none, 1 bf16 channels-last via TMA (tmO)
-  int one_producer;        // 1: activation and weight slabs requested by one thread in one FIFO (A/B switch)
-  int park;                // waits that use the barrier unit's suspend hint instead of a spin loop (KVAE_PARK): bit 0 epilogue
-                           // warps (t_full, skip blocks), bit 1 TMA producers (a_empty, b_empty), bit 2 the MMA thread's t_empty
   int fast;                // 1: conv_umma2_kernel<1> -- 16 epilogue warps on 16-row x 32-channel items (forward, swap orientation,
-                           //    2-byte stream / operand blocks only; see the kFast branch of the kernel)
-  int no_frag;             // 1: scalar swap epilogue even where the fragment-mapped one applies (A/B switch, KVAE_FRAG_EPI=0)
+                           //    2-byte stream / operand blocks only; see the kFast branch of the kernel);
+                           // 2: conv_umma2_kernel<2> -- the same epilogue with the fused SnakeBeta backward (bwd below)
   int split3;              // fp32-mode arithmetic on the tensor cores: both operands are stored as bf16 (hi | lo)
                            // halves -- activations [.., 2*Cin], weights [tap][Cout][2*Cin] -- and every K chunk is
                            // multiplied three times: hi*hi + lo*hi + hi*lo (the lo*lo term is below fp32 rounding).
@@ -75,7 +78,7 @@ struct ConvParams2 {
   // mean half of the latents, twj-style chunk(2, dim=1)): for channels c < samp_D,
   //   samp_out[b, c, t] = mean + samp_std * samp_noise[b, c, t], two separately rounded operations on the value AS STORED
   // (rounded to the output dtype first), i.e. bit-identical to torch on the stored latents.  Same dtype as out_cf.
-  // Training backward, data-gradient launches (fragment-mapped swap epilogue only): the SnakeBeta derivative and the
+  // Training backward, data-gradient launches (conv_umma2_kernel<2> only): the SnakeBeta derivative and the
   // skip-connection add of the layer BEFORE this conv are applied to the accumulator in the epilogue,
   //   G = dA * (1 + a * inv_b * sin(2 a x)) + skip        (dA = this conv's output, x = that layer's saved fp16 stream)
   // G leaves as bf16 through the operand path (act_mode 1), and the per-channel sums d alpha, d beta and the bias
@@ -121,9 +124,8 @@ __host__ __device__ inline int conv_umma2_raw_slots(int raw_mode, bool residual)
 }
 __host__ __device__ inline int conv_umma2_stage_bytes_per_warp(int raw_mode, int act_mode, bool residual, int raw_f16,
                                                                int act_split = 0, int bwd = 0, int fast = 0) {
-  if (fast && bwd) return 2 * (2 * kFastBlk) + 2 * kFastBlk;    // two slots of [x block | skip block], two bf16 output blocks
+  if (bwd) return 2 * (2 * kFastBlk) + 2 * kFastBlk;            // <2>: two slots of [x block | skip block], two bf16 output blocks
   if (fast) return conv_umma2_raw_slots(raw_mode, residual) * kFastBlk + (act_mode == 1 ? 2 * kFastBlk : 0);
-  if (bwd) return 2 * (2 * kActBlkBytes) + 2 * kActBlkBytes;      // two slots of [x block | skip block], two bf16 output blocks
   return conv_umma2_raw_slots(raw_mode, residual) * conv_umma2_raw_blk(raw_f16) +
          (act_mode == 1 ? 2 * kActBlkBytes * (act_split ? 2 : 1) : 0);
 }
@@ -201,16 +203,14 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   // Two TMA producer threads.  In ONE FIFO with the weight slabs an activation slab was requested only SB weight
   // stages (about a microsecond) before its first MMA -- less than an HBM round trip -- although its ring stage had
   // been free for much longer; on its own thread a slab is requested the moment its stage is released.
-  // KVAE_SPLIT_PRODUCER=0 (ConvParams2::one_producer) restores the single FIFO for A/B measurements.
   if (warp == 0 || warp == 3) {
     // (warp-uniform loops, one elected lane issues -- see the UMMA issuer below)
     {
-      const bool do_a = p.one_producer ? warp == 0 : warp == 3;
+      const bool do_a = warp == 3;
       const bool do_w = warp == 0;
       const int SA = p.SA, SB = p.SB, nbox = p.nbox, RB = p.RB;
       int as = 0, bs = 0;
       uint32_t aph = 0, bph = 0;
-      if (do_a || do_w)
       for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
         int b, q0, phi, n0;
         decode(tile, b, q0, phi, n0);
@@ -227,7 +227,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           for (int t = t_lo; t < t_hi; ++t) {
             const uint32_t tl = p.tap_ld[t];
             if (do_a && (p.tap_mma[t] & 0x10000u)) {
-              if (p.park & 2) ptx::mbar_wait_parked(&a_empty[as], aph ^ 1u); else ptx::mbar_wait(&a_empty[as], aph ^ 1u);
+              ptx::mbar_wait(&a_empty[as], aph ^ 1u);
               if (ptx::elect_one()) {
                 ptx::mbar_expect_tx(&a_full[as], a_bytes);
                 const int row = q0 + (static_cast<int32_t>(tl) >> 16);
@@ -239,7 +239,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
               if (++as == SA) { as = 0; aph ^= 1u; }
             }
             if (do_w) {
-              if (p.park & 2) ptx::mbar_wait_parked(&b_empty[bs], bph ^ 1u); else ptx::mbar_wait(&b_empty[bs], bph ^ 1u);
+              ptx::mbar_wait(&b_empty[bs], bph ^ 1u);
               if (ptx::elect_one()) {
                 ptx::mbar_expect_tx(&b_full[bs], b_bytes);
                 ptx::tma_load_3d(b_ring + static_cast<size_t>(bs) * b_bytes, &tmW, &b_full[bs], w_col, n0,
@@ -277,7 +277,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
         const int phi = (tile / p.n_tiles) % p.P_out;
         const int t_lo = p.tap_begin[phi], t_hi = p.tap_begin[phi + 1];
-        if (p.park & 4) ptx::mbar_wait_parked(&t_empty[acc], accph ^ 1u); else ptx::mbar_wait(&t_empty[acc], accph ^ 1u);   // epilogue has drained this accumulator buffer
+        ptx::mbar_wait(&t_empty[acc], accph ^ 1u);   // epilogue has drained this accumulator buffer
         ptx::tc_fence_after();
         const uint32_t d0 = tmem_base + acc * acc_cols;
         const uint32_t d1 = d0 + NT16;
@@ -551,20 +551,19 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     const int g = e >> 2;              // item parity handled by this warp
     const int quad = warp & 3;         // TMEM lane quadrant = rows quad*32 .. +31 of a 128-row sub-tile
     const int T_out = p.Tq_out * p.P_out;
-    const bool has_res = p.residual != nullptr || p.bwd;
-    const int R = p.bwd ? 2 : conv_umma2_raw_slots(p.raw_mode, has_res);
-    const int rawblk = p.bwd ? 2 * kActBlkBytes : conv_umma2_raw_blk(p.raw_f16);
-    const uint32_t res_tx = p.bwd ? (p.bwd_skip ? 2 * kActBlkBytes : kActBlkBytes) : rawblk;   // bytes one item's loads deliver
-    uint8_t* raw_ring = stage_base + e * conv_umma2_stage_bytes_per_warp(p.raw_mode, p.act_mode, has_res, p.raw_f16, p.act_split, p.bwd);
+    const bool has_res = p.residual != nullptr;
+    const int R = conv_umma2_raw_slots(p.raw_mode, has_res);
+    const int rawblk = conv_umma2_raw_blk(p.raw_f16);
+    uint8_t* raw_ring = stage_base + e * conv_umma2_stage_bytes_per_warp(p.raw_mode, p.act_mode, has_res, p.raw_f16, p.act_split);
     uint8_t* act_ring = raw_ring + R * rawblk;
     uint64_t* my_res_full = res_full + e * 3;
     // An item is one 32-row x 32-channel output block.  swap = 0: TMEM lane = time row, so a thread owns one
     // row x 32 channels (vector shared-memory accesses).  swap = 1: TMEM lane = channel, so a thread owns one
     // channel x 32 rows (scalar accesses into the same swizzled blocks; per-channel constants live in registers).
     const int ipt = p.swap ? 4 * p.MT : p.MT * (p.NT >> 5);
-    // fragment-mapped fast path of the swap orientation (inference plans in bf16 mode: fp16 stream, bf16 operand)
-    const bool frag = p.swap && !p.act_split && !p.precise && p.raw_mode != 2 &&
-                      (p.bwd || (!p.no_frag && (p.raw_f16 || (p.raw_mode == 0 && !has_res))));
+    // fragment-mapped path of the swap orientation for 2-byte stream / operand blocks: the launches that <1> takes
+    // unless KVAE_FAST_EPI=0 sends them here
+    const bool frag = p.swap && !p.act_split && !p.precise && p.raw_mode != 2 && (p.raw_f16 || (p.raw_mode == 0 && !has_res));
     // ldmatrix / stmatrix: this lane addresses row (lane & 7) of matrix (lane >> 3) inside a 16-row half of a
     // [32 rows x 64 B] SWIZZLE_64B block (lane half 1: address ^ 32, rows 16..31: + 1024)
     const int frag_row = ((lane >> 4) << 3) + (lane & 7);
@@ -586,12 +585,9 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     if (has_res && lane == 0 && static_cast<int>(blockIdx.x) < p.total_tiles && g < ipt) {
       int cb, ph, r0, bb;
       coords(blockIdx.x, g, cb, ph, r0, bb);
-      ptx::mbar_expect_tx(&my_res_full[0], res_tx);
+      ptx::mbar_expect_tx(&my_res_full[0], rawblk);
       ptx::tma_load_4d(raw_ring, &tmX, &my_res_full[0], cb, ph, r0, bb);
-      if (p.bwd_skip) ptx::tma_load_4d(raw_ring + kActBlkBytes, &tmR, &my_res_full[0], cb, ph, r0, bb);
     }
-    float bw_a[4] = {0.f, 0.f, 0.f, 0.f}, bw_ib[4] = {0.f, 0.f, 0.f, 0.f};          // bwd mode: this thread's 4 channels
-    float acc_da[4] = {0.f, 0.f, 0.f, 0.f}, acc_db[4] = {0.f, 0.f, 0.f, 0.f}, acc_bias[4] = {0.f, 0.f, 0.f, 0.f};
     for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
       int b, q0, phi, n0;
       decode(tile, b, q0, phi, n0);
@@ -610,21 +606,13 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           }
         }
       }
-      if (p.bwd) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int c = n0 + quad * 32 + (i >> 1) * 16 + (i & 1) * 8 + (lane >> 2);
-          bw_a[i] = __ldg(p.bwd_a + c);
-          bw_ib[i] = __ldg(p.bwd_inv_b + c);
-        }
-      }
       float bias_s = 0.f, sa_s = 1.f, sib_s = 0.f;
       if (p.swap && !frag) {
         const int c = n0 + quad * 32 + lane;
         if (p.bias) bias_s = __ldg(p.bias + c);
         if (p.snake_a) { sa_s = __ldg(p.snake_a + c); sib_s = __ldg(p.snake_inv_b + c); }
       }
-      if (p.park & 1) ptx::mbar_wait_parked(&t_full[acc], accph); else ptx::mbar_wait(&t_full[acc], accph);
+      ptx::mbar_wait(&t_full[acc], accph);
       ptx::tc_fence_after();
       const uint32_t acc_tmem = tmem_base + acc * acc_cols + (static_cast<uint32_t>(quad * 32) << 16);
       for (int item = g; item < ipt; item += 2) {
@@ -650,12 +638,11 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
               int cb, ph, rr, bb;
               coords(nt, ni, cb, ph, rr, bb);
               const int sn = (jr + 1) % R;
-              ptx::mbar_expect_tx(&my_res_full[sn], res_tx);
+              ptx::mbar_expect_tx(&my_res_full[sn], rawblk);
               ptx::tma_load_4d(raw_ring + sn * rawblk, &tmX, &my_res_full[sn], cb, ph, rr, bb);
-              if (p.bwd_skip) ptx::tma_load_4d(raw_ring + sn * rawblk + kActBlkBytes, &tmR, &my_res_full[sn], cb, ph, rr, bb);
             }
           }
-          if (p.park & 1) ptx::mbar_wait_parked(&my_res_full[jr], (res_ph >> jr) & 1u); else ptx::mbar_wait(&my_res_full[jr], (res_ph >> jr) & 1u);
+          ptx::mbar_wait(&my_res_full[jr], (res_ph >> jr) & 1u);
           res_ph ^= (1u << jr);
         }
         uint8_t* const rblk = raw_ring + jr * rawblk;
@@ -672,57 +659,6 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           ptx::tmem_ld_16x256b_x4(acc_tmem + tcol + (16u << 16), r + 16);
           uint32_t sk[16];                                   // sk[8 L + 4 m + j]: rows 16 m + 8 (j >> 1) .., channel group 2 L + (j & 1)
           const uint32_t rb = ptx::smem_u32(rblk) + frag_lane;
-          if (p.bwd) {
-            // ---- fused SnakeBeta backward (see ConvParams2::bwd): x block at rb, skip-gradient block behind it
-            uint32_t gs[16];
-#pragma unroll
-            for (int L = 0; L < 2; ++L)
-#pragma unroll
-              for (int m = 0; m < 2; ++m) {
-                ptx::ldmatrix_x4_trans((rb + m * 1024) ^ (L * 32u), sk[8 * L + 4 * m], sk[8 * L + 4 * m + 1],
-                                       sk[8 * L + 4 * m + 2], sk[8 * L + 4 * m + 3]);
-                if (p.bwd_skip)
-                  ptx::ldmatrix_x4_trans((rb + kActBlkBytes + m * 1024) ^ (L * 32u), gs[8 * L + 4 * m], gs[8 * L + 4 * m + 1],
-                                         gs[8 * L + 4 * m + 2], gs[8 * L + 4 * m + 3]);
-              }
-            ptx::tmem_ld_wait();
-            uint32_t w[16];
-#pragma unroll
-            for (int q = 0; q < 16; ++q) {
-              const int L = q >> 3, ci = 2 * L + (q & 1);
-              const int ri = 16 * L + 4 * (2 * ((q >> 2) & 1) + ((q >> 1) & 1)) + 2 * (q & 1);
-              const float2 xf = __half22float2(*reinterpret_cast<const __half2*>(&sk[q]));
-              float d0 = __uint_as_float(r[ri]), d1 = __uint_as_float(r[ri + 1]);
-              // rows past the end of the clip hold whatever the taps that still reach valid input produced: the TMA store
-              // clips them, the column sums must not see them
-              const int trow = r0 + 8 * (2 * ((q >> 2) & 1) + ((q >> 1) & 1)) + 2 * (lane & 3);
-              if (trow >= p.Tq_out) d0 = 0.f;
-              if (trow + 1 >= p.Tq_out) d1 = 0.f;
-              const float t0 = bw_a[ci] * xf.x, t1 = bw_a[ci] * xf.y;
-              const float sn0 = __sinf(t0), cs0 = __cosf(t0), sn1 = __sinf(t1), cs1 = __cosf(t1);
-              const float s20 = 2.f * sn0 * cs0, s21 = 2.f * sn1 * cs1;
-              acc_da[ci] = fmaf(d0 * xf.x, s20, fmaf(d1 * xf.y, s21, acc_da[ci]));
-              acc_db[ci] = fmaf(d0, sn0 * sn0, fmaf(d1, sn1 * sn1, acc_db[ci]));
-              const float k = bw_ib[ci] * bw_a[ci];
-              d0 *= fmaf(k, s20, 1.f);
-              d1 *= fmaf(k, s21, 1.f);
-              if (p.bwd_skip) {
-                const float2 gf = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&gs[q]));
-                d0 += gf.x;
-                d1 += gf.y;
-              }
-              acc_bias[ci] += d0 + d1;
-              const __nv_bfloat162 h2 = __floats2bfloat162_rn(d0, d1);
-              w[q] = *reinterpret_cast<const uint32_t*>(&h2);
-            }
-            const uint32_t ab = ptx::smem_u32(ablk) + frag_lane;
-#pragma unroll
-            for (int L = 0; L < 2; ++L)
-#pragma unroll
-              for (int m = 0; m < 2; ++m)
-                ptx::stmatrix_x4_trans((ab + m * 1024) ^ (L * 32u), w[8 * L + 4 * m], w[8 * L + 4 * m + 1],
-                                       w[8 * L + 4 * m + 2], w[8 * L + 4 * m + 3]);
-          } else {
           if (has_res) {
 #pragma unroll
             for (int L = 0; L < 2; ++L)
@@ -783,7 +719,6 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                 ptx::stmatrix_x4_trans((ab + m * 1024) ^ (L * 32u), w[8 * L + 4 * m], w[8 * L + 4 * m + 1],
                                        w[8 * L + 4 * m + 2], w[8 * L + 4 * m + 3]);
           }
-          }   // !bwd
         } else {
         uint32_t r[32];
         __syncwarp();
@@ -988,26 +923,6 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           }
           if (R > 0) jr = (jr + 1 == R) ? 0 : jr + 1;
           ja ^= 1;
-        }
-      }
-      if (p.bwd) {
-        // per-channel sums of this tile: the four lanes that share a channel (lane & 3 = time columns) combine, then
-        // one atomic per channel, warp and tile
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          float va = acc_da[i], vb = acc_db[i], vc = acc_bias[i];
-          va += __shfl_xor_sync(0xffffffffu, va, 1); va += __shfl_xor_sync(0xffffffffu, va, 2);
-          vb += __shfl_xor_sync(0xffffffffu, vb, 1); vb += __shfl_xor_sync(0xffffffffu, vb, 2);
-          vc += __shfl_xor_sync(0xffffffffu, vc, 1); vc += __shfl_xor_sync(0xffffffffu, vc, 2);
-          if ((lane & 3) == 0) {
-            const int c = n0 + quad * 32 + (i >> 1) * 16 + (i & 1) * 8 + (lane >> 2);
-            const float ib = bw_ib[i], a = bw_a[i];
-            const float eb = 1.f / ib - 1e-9f;                      // exp(beta)
-            atomicAdd(p.d_alpha + c, va * ib * (p.bwd_logscale ? a : 1.f));
-            atomicAdd(p.d_beta + c, -vb * ib * ib * (p.bwd_logscale ? eb : 1.f));
-            if (p.d_bias) atomicAdd(p.d_bias + c, vc);
-          }
-          acc_da[i] = 0.f; acc_db[i] = 0.f; acc_bias[i] = 0.f;
         }
       }
       // accumulator buffer fully read: hand it back to the UMMA issuer

@@ -13,9 +13,8 @@
 #include <string>
 #include <vector>
 
-#include "conv_umma.cuh"
+#include "conv_common.cuh"
 #include "conv_umma2.cuh"
-#include "conv_ru.cuh"
 #include "conv_ru2.cuh"
 #include "wgrad_umma.cuh"
 
@@ -61,8 +60,7 @@ struct TapPlan {
   std::vector<Tap> taps;
 };
 
-// per_tap_slab = true stages one A slab per tap (no row-shifted descriptors); used by the probe.
-inline bool build_taps(const ConvGeom& g, bool per_tap_slab, TapPlan& tp, std::string& err) {
+inline bool build_taps(const ConvGeom& g, TapPlan& tp, std::string& err) {
   tp = TapPlan();
   struct Raw { int a_phase, delta, w; };
   std::vector<std::vector<Raw>> by_out_phase;
@@ -103,22 +101,15 @@ inline bool build_taps(const ConvGeom& g, bool per_tap_slab, TapPlan& tp, std::s
         dmax = std::max(dmax, v[j].delta);
         ++j;
       }
-      if (!per_tap_slab) tp.span = std::max(tp.span, dmax - dmin);
+      tp.span = std::max(tp.span, dmax - dmin);
       for (size_t t = i; t < j; ++t) {
         Tap tap;
         tap.a_phase = static_cast<int16_t>(v[t].a_phase);
         tap.w_slab = static_cast<int16_t>(v[t].w);
-        if (per_tap_slab) {
-          tap.a_row = static_cast<int16_t>(v[t].delta);
-          tap.shift = 0;
-          tap.first = 1;
-          tap.last = 1;
-        } else {
-          tap.a_row = static_cast<int16_t>(dmin);
-          tap.shift = static_cast<int16_t>(v[t].delta - dmin);
-          tap.first = (t == i) ? 1 : 0;
-          tap.last = (t + 1 == j) ? 1 : 0;
-        }
+        tap.a_row = static_cast<int16_t>(dmin);
+        tap.shift = static_cast<int16_t>(v[t].delta - dmin);
+        tap.first = (t == i) ? 1 : 0;
+        tap.last = (t + 1 == j) ? 1 : 0;
         tp.taps.push_back(tap);
       }
       i = j;
@@ -217,8 +208,8 @@ struct ConvEpilogue {
   __nv_bfloat16* out_act = nullptr;
   const float* snake_a = nullptr;
   const float* snake_inv_b = nullptr;
-  int stream_f16 = 0;     // persistent kernel only: residual and channels-last out_raw are fp16 instead of fp32
-  // fp32-mode arithmetic on the tensor cores (persistent kernel only, see ConvParams2::split3)
+  int stream_f16 = 0;     // residual and channels-last out_raw are fp16 instead of fp32
+  // fp32-mode arithmetic on the tensor cores (see ConvParams2::split3)
   int split3 = 0;         // x is [B, T, 2*Cin] (hi | lo), wpacked is [K][Cout][2*Cin]
   int act_split = 0;      // out_act is [B, T, 2*Cout] (hi | lo)
   int precise = 0;        // sinf instead of MUFU sin in the fused SnakeBeta
@@ -230,13 +221,6 @@ struct ConvEpilogue {
   int bwd_logscale = 1;
 };
 
-struct ConvTuning {
-  int MT = 0;             // 0 = auto
-  int NT = 0;             // 0 = auto
-  int desc_mode = 0;
-  bool per_tap_slab = false;
-};
-
 inline bool umma_supported(const ConvGeom& g) {
   return g.Cin % 64 == 0 && g.Cout % 64 == 0 && g.Cout >= 64;
 }
@@ -245,72 +229,6 @@ inline int pick_nt(int Cout) {
   if (Cout % 256 == 0) return 256;
   if (Cout % 128 == 0) return 128;
   return 64;
-}
-
-// A prepared launch: everything that depends on (layer, B, T, pointers) but not on the data.
-struct ConvLaunch {
-  CUtensorMap tmA, tmW;
-  ConvParams p;
-  dim3 grid;
-  size_t smem = 0;
-  int T_out = 0;
-};
-
-inline bool prepare_conv_umma(const ConvGeom& g, const __nv_bfloat16* x, int B, int T_in,
-                              const __nv_bfloat16* wpacked, const ConvEpilogue& ep,
-                              const ConvTuning& tune, ConvLaunch& L, std::string& err) {
-  if (!umma_supported(g)) { err = "channel counts not multiples of 64"; return false; }
-  TapPlan tp;
-  if (!build_taps(g, tune.per_tap_slab, tp, err)) return false;
-  const int T_out = g.out_len(T_in);
-  if (T_out <= 0 || T_out % tp.P_out) { err = "bad output length"; return false; }
-  ConvParams& p = L.p;
-  std::memset(&p, 0, sizeof(p));
-  p.B = B;
-  p.P_out = tp.P_out;
-  p.Tq_out = T_out / tp.P_out;
-  p.Cout = g.Cout;
-  p.n_chunks = g.Cin / 64;
-  p.NT = tune.NT ? tune.NT : pick_nt(g.Cout);
-  if (g.Cout % p.NT || p.NT % 16 || p.NT > 256) { err = "bad NT"; return false; }
-  int MT = tune.MT ? tune.MT : (p.Tq_out > 128 ? 2 : 1);
-  if (MT * p.NT > 512) MT = 1;
-  p.MT = MT;
-  const int rows = 128 * MT + tp.span;
-  p.nbox = (rows + 255) / 256;
-  p.RB = (((rows + p.nbox - 1) / p.nbox) + 7) & ~7;
-  if (p.RB > 256) { err = "slab box too tall"; return false; }
-  p.desc_mode = tune.desc_mode;
-  int cols = 32;
-  while (cols < MT * p.NT) cols <<= 1;
-  p.tmem_cols = cols;
-  for (int i = 0; i <= kMaxPhases; ++i) p.tap_begin[i] = tp.tap_begin[i];
-  for (size_t i = 0; i < tp.taps.size(); ++i) p.taps[i] = tp.taps[i];
-  // ring depths from the 227 KB budget
-  const size_t budget = 227 * 1024 - 2048;
-  const size_t a_bytes = static_cast<size_t>(p.nbox) * p.RB * 128, b_bytes = static_cast<size_t>(p.NT) * 128;
-  p.SA = 2;
-  if (2 * a_bytes + 2 * b_bytes > budget) p.SA = 1;
-  if (p.SA * a_bytes + 2 * b_bytes > budget) { err = "tile does not fit shared memory"; return false; }
-  p.SB = static_cast<int>(std::min<size_t>(8, (budget - p.SA * a_bytes) / b_bytes));
-  // spend what is left on a deeper A ring (strided convs stage `stride` slabs per chunk)
-  while (p.SA < 4 && (p.SA + 1) * a_bytes + p.SB * b_bytes <= budget) ++p.SA;
-  p.bias = ep.bias;
-  p.residual = ep.residual;
-  p.residual_f32 = ep.residual_f32;
-  p.out_raw = ep.out_raw;
-  p.out_raw_f32 = ep.out_raw_f32;
-  p.out_raw_cf = ep.out_raw_cf;
-  p.out_act = ep.out_act;
-  p.snake_a = ep.snake_a;
-  p.snake_inv_b = ep.snake_inv_b;
-  if (!make_act_tmap(&L.tmA, x, B, T_in, g.Cin, tp.P_in, p.RB, err)) return false;
-  if (!make_w_tmap(&L.tmW, wpacked, g.K, g.Cout, g.Cin, p.NT, err)) return false;
-  const int q_tiles = (p.Tq_out + 128 * MT - 1) / (128 * MT);
-  L.grid = dim3(q_tiles * tp.P_out, g.Cout / p.NT, B);
-  L.smem = conv_umma_smem_bytes(p);
-  L.T_out = T_out;
-  return true;
 }
 
 // ------------------------------------------------------------------ persistent kernel (conv_umma2.cuh)
@@ -357,7 +275,7 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
   if (ep.residual && !ep.residual_f32 && !ep.stream_f16) { err = "residual must be fp32 (or the fp16 stream)"; return false; }
   if (ep.out_raw && !ep.out_raw_cf && !ep.out_raw_f32 && !ep.stream_f16) { err = "channels-last raw output must be fp32 (or the fp16 stream)"; return false; }
   TapPlan tp;
-  if (!build_taps(g, false, tp, err)) return false;
+  if (!build_taps(g, tp, err)) return false;
   if (sg) {
     if (tp.P_in != 1) { err = "streaming form needs a stride-1 or transposed conv"; return false; }
     T_in = sg->in_rows;
@@ -376,9 +294,6 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
   p.act_mode = ep.out_act ? 1 : 0;
   p.raw_f16 = ep.stream_f16 ? 1 : 0;
   p.split3 = ep.split3 ? 1 : 0;
-  if (const char* e = getenv("KVAE_SPLIT_PRODUCER")) p.one_producer = atoi(e) ? 0 : 1;
-  if (const char* e = getenv("KVAE_FRAG_EPI")) p.no_frag = atoi(e) ? 0 : 1;
-  if (const char* e = getenv("KVAE_PARK")) p.park = atoi(e);
   p.act_split = (ep.act_split && ep.out_act) ? 1 : 0;
   p.precise = ep.precise ? 1 : 0;
   p.Cin = g.Cin;
@@ -394,9 +309,10 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
     p.bwd_a = ep.bwd_a;
     p.bwd_inv_b = ep.bwd_inv_b;
   }
-  // (the 8-warp and 16-warp epilogues stage the same number of bytes per CTA: 16-row instead of 32-row blocks)
-  const size_t stage = 8 * static_cast<size_t>(conv_umma2_stage_bytes_per_warp(p.raw_mode, p.act_mode, ep.residual != nullptr,
-                                                                                p.raw_f16, p.act_split, p.bwd));
+  // (the 8-warp and 16-warp epilogues stage the same number of bytes per CTA: 16-row instead of 32-row blocks; the fused
+  // SnakeBeta backward only runs on the 16-warp one)
+  const size_t stage = (p.bwd ? 16 : 8) * static_cast<size_t>(conv_umma2_stage_bytes_per_warp(p.raw_mode, p.act_mode, ep.residual != nullptr,
+                                                                                               p.raw_f16, p.act_split, p.bwd));
   const size_t budget = 227 * 1024 - 2048 - stage;
   // candidate tilings, best first: double-buffered accumulators when they fit the 512 TMEM columns
   struct Cand { int MT, NT, acc; };
@@ -414,15 +330,12 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
     const bool starved = big_tiles * 10 < static_cast<long long>(sm_count()) * 6;
     if (starved && g.Cout % 128 == 0) cands.push_back({1, 128, 2});
     // Cout >= 512: 128-channel swap tiles (N = 256 time rows) with double-buffered accumulators, like the narrower
-    // layers.  256 x 256 tiles (KVAE_WIDE_TILES=2, the first choice until the end of round 1) fill all 512 TMEM columns
+    // layers.  256 x 256 tiles (the first choice until the end of round 1) fill all 512 TMEM columns
     // with ONE accumulator set, so their epilogue cannot overlap the next tile's MMAs: 63 % tensor-pipe activity at
     // C = 512 (profiles/r01_ncu_summary.txt); the swap tiles read the activation slab twice as often from L2 but
     // measured k7 C=512 0.295 -> 0.254 ms, k1 C=512 0.164 -> 0.121 ms, ConvTranspose 1024->512 0.249 -> 0.197 ms at
-    // B = 8 (profiles/r01_tile_shapes_B8.log).  KVAE_WIDE_TILES=1: 128 x 256 time-on-M tiles, double-buffered.
-    static const int wide = [] { const char* e = getenv("KVAE_WIDE_TILES"); return e ? atoi(e) : 0; }();
-    if (wide == 0 && g.Cout % 128 == 0) cands.push_back({mt, 128, 2});
-    if (wide == 1 && g.Cout % 256 == 0 && g.Cout >= 512) cands.push_back({1, 256, 2});
-    if (g.Cout % 256 == 0 && g.Cout >= 512) cands.push_back({mt, 256, mt * 256 * 2 <= 512 ? 2 : 1});
+    // B = 8 (profiles/r01_tile_shapes_B8.log).  (A 256-wide candidate after the 128-wide one could never be taken: it
+    // needs more shared memory for the same slab.)
     if (g.Cout % 128 == 0) cands.push_back({mt, 128, 2});
     if (g.Cout % 128 == 0) cands.push_back({1, 128, 2});
     cands.push_back({mt, 64, 2});
@@ -452,30 +365,21 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
       int n_slabs = 0;
       for (int t = tp.tap_begin[0]; t < tp.tap_begin[1]; ++t) n_slabs += tp.taps[t].first ? 1 : 0;
       const int n_taps = tp.tap_begin[1] - tp.tap_begin[0];
-      static const bool deep_a = [] { const char* e = getenv("KVAE_DEEP_A"); return !(e && e[0] == '0'); }();
-      if (deep_a && p.SA < 3 && n_taps <= 2 * std::max(1, n_slabs) && 3 * a_bytes + 2 * b_bytes <= budget) {
+      if (p.SA < 3 && n_taps <= 2 * std::max(1, n_slabs) && 3 * a_bytes + 2 * b_bytes <= budget) {
         p.SA = 3;
         p.SB = static_cast<int>(std::min<size_t>(8, (budget - 3 * a_bytes) / b_bytes));
       }
     }
-    if (const char* e = getenv("KVAE_SA")) {   // tuning experiments: deeper / shallower activation ring
-      const int sa = std::max(1, std::min(8, atoi(e)));
-      if (sa * a_bytes + 2 * b_bytes <= budget) {
-        p.SA = sa;
-        p.SB = static_cast<int>(std::min<size_t>(8, (budget - sa * a_bytes) / b_bytes));
-      }
-    }
-    if (const char* e = getenv("KVAE_SB")) p.SB = std::max(2, std::min(p.SB, atoi(e)));
     ok = true;
     break;
   }
   if (!ok) { err = "no tiling fits shared memory"; return false; }
   // conv_umma2_kernel<1>: forward launches in the swap orientation whose stream / operand blocks are 2-byte
+  // (KVAE_FAST_EPI=0 sends them to the generic epilogue of <0>); <2>: every fused SnakeBeta backward
   static const bool fast_on = [] { const char* e = getenv("KVAE_FAST_EPI"); return !(e && e[0] == '0'); }();
-  p.fast = (fast_on && p.swap && !p.bwd && !p.act_split && !p.precise && !p.no_frag && p.raw_mode != 2 &&
+  p.fast = (fast_on && p.swap && !p.bwd && !p.act_split && !p.precise && p.raw_mode != 2 &&
             (p.raw_f16 || (p.raw_mode == 0 && !ep.residual))) ? 1 : 0;
-  static const bool fast_bwd_on = [] { const char* e = getenv("KVAE_FAST_BWD"); return !(e && e[0] == '0'); }();
-  if (fast_on && fast_bwd_on && p.bwd && p.swap) p.fast = 2;
+  if (p.bwd) p.fast = 2;
   const int box_rows = p.fast ? 16 : 32;
   int cols = 32;
   while (cols < p.acc_stages * p.MT * p.NT) cols <<= 1;
@@ -521,11 +425,6 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
 }
 
 // Launch with programmatic stream serialization (ptx.cuh, pdl_*): the kernel may begin while its predecessor drains.
-// KVAE_PDL=0 restores plain stream-ordered launches (A/B measurements).
-inline bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("KVAE_PDL"); return !(e && e[0] == '0'); }();
-  return on;
-}
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -537,7 +436,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -559,13 +458,12 @@ inline cudaError_t launch_conv_umma2(const ConvLaunch2& L, cudaStream_t stream) 
   return launch_pdl(conv_umma2_kernel<0>, dim3(L.grid), dim3(384), L.smem, stream, L.tmA, L.tmW, L.tmR, L.tmO, L.tmX, L.p);
 }
 
-// ------------------------------------------------------------------ fused ResidualUnit (conv_ru.cuh)
+// ------------------------------------------------------------------ fused ResidualUnit (conv_ru2.cuh)
 struct RuLaunch {
   CUtensorMap tmA, tmW7, tmW1, tmR, tmO, tmX;
   RuParams p;
   int grid = 0;
   size_t smem = 0;
-  int epi = 2;   // kernel: 2 = conv_ru2_kernel, 0 / 1 = conv_ru_kernel<0 / 1> (KVAE_RU_EPI, read when the launch is prepared)
 };
 
 struct RuArgs {
@@ -608,35 +506,16 @@ inline bool prepare_conv_ru(const RuArgs& a, int B, int T, int dilation, RuLaunc
   p.act_out = a.out_act ? 1 : 0;
   const size_t a_bytes = static_cast<size_t>(p.nbox) * p.RB * 128, b_bytes = kRuC * 128;
   if (!a.stream_f16) { err = "fused RU: needs the fp16 residual stream"; return false; }
-  p.raw_f16 = 1;
   const int sdt = 2;
   const size_t budget = 227 * 1024 - 2048 - kRuHBytes - kRuEpiWarps * static_cast<size_t>(ru_stage_bytes_per_warp(p.act_out));
   p.SA = 2;
   if (2 * a_bytes + 3 * b_bytes > budget) { err = "fused RU does not fit shared memory"; return false; }
   p.SB = static_cast<int>(std::min<size_t>(8, (budget - 2 * a_bytes) / b_bytes));
-  if (const char* e = getenv("KVAE_RU_DBG")) p.dbg = atoi(e);
-  if (const char* e = getenv("KVAE_RU_SB")) {   // ring-depth experiments
-    const size_t cap = (227 * 1024 - 2048 - kRuHBytes - 2 * a_bytes - ((p.dbg & 131) == 131 ? 0 : kRuEpiWarps * static_cast<size_t>(ru_stage_bytes_per_warp(p.act_out)))) / b_bytes;
-    p.SB = static_cast<int>(std::max<size_t>(2, std::min<size_t>({static_cast<size_t>(atoi(e)), cap, static_cast<size_t>(16)})));
-  }
   p.q_tiles = (T + 255) / 256;
   p.total_tiles = p.q_tiles * B;
   p.bias7 = a.bias7; p.s2_a = a.s2_a; p.s2_inv_b = a.s2_inv_b; p.bias1 = a.bias1;
   p.sn_a = a.sn_a; p.sn_inv_b = a.sn_inv_b;
-  if (const char* e = getenv("KVAE_RU_DBG")) p.dbg = atoi(e);
-  // KVAE_RU_EPI (A/B measurements, parity test): 0 = first-generation kernel, 1 = fragment-mapped epilogue on the
-  // serial GEMM1 -> EPI1 -> GEMM2 chain, 2 (default) = conv_ru2_kernel
-  L.epi = 2;
-  if (const char* e = getenv("KVAE_RU_EPI")) L.epi = atoi(e);
   p.act_f16 = a.act_f16;
-  if (p.act_f16 && L.epi != 2) { err = "fused RU: the fp16 operand output needs conv_ru2_kernel"; return false; }
-  p.a_ptr = a.a; p.x_ptr = a.x;
-  p.pf = 0;
-  if (const char* e = getenv("KVAE_RU_PF")) p.pf = atoi(e);
-  p.k0 = 3; p.k1 = 6;
-  if (const char* e = getenv("KVAE_RU_K0")) p.k0 = atoi(e);
-  if (const char* e = getenv("KVAE_RU_K1")) p.k1 = atoi(e);
-  if (p.k0 < 0 || p.k1 <= p.k0 || p.k1 > 13) { err = "fused RU: need 0 <= k0 < k1 <= 13"; return false; }
   if (!make_act_tmap(&L.tmA, a.a, B, sg ? sg->in_rows : T, kRuC, 1, p.RB, err, sg ? sg->in_pitch : 0)) return false;
   if (!make_w_tmap(&L.tmW7, a.w7, 7, kRuC, kRuC, kRuC, err)) return false;
   if (!make_w_tmap(&L.tmW1, a.w1, 1, kRuC, kRuC, kRuC, err)) return false;
@@ -651,25 +530,14 @@ inline bool prepare_conv_ru(const RuArgs& a, int B, int T, int dilation, RuLaunc
 
 inline cudaError_t launch_conv_ru(const RuLaunch& L, cudaStream_t stream) {
   static bool attr_set[64] = {false};
-  const int epi = L.epi;
   int dev = 0;
   cudaGetDevice(&dev);
   if (!attr_set[dev & 63]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_ru_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(conv_ru_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(conv_ru2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(conv_ru2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return e;
     attr_set[dev & 63] = true;
   }
-  if (epi == 2)
-    return launch_pdl(conv_ru2_kernel, dim3(L.grid), dim3(kRuThreads), L.smem, stream, L.tmA, L.tmW7, L.tmW1, L.tmR, L.tmO, L.tmX, L.p);
-  else if (epi == 0)
-    conv_ru_kernel<0><<<L.grid, kRuThreads, L.smem, stream>>>(L.tmA, L.tmW7, L.tmW1, L.tmR, L.tmO, L.tmX, L.p);
-  else
-    conv_ru_kernel<1><<<L.grid, kRuThreads, L.smem, stream>>>(L.tmA, L.tmW7, L.tmW1, L.tmR, L.tmO, L.tmX, L.p);
-  return cudaGetLastError();
+  return launch_pdl(conv_ru2_kernel, dim3(L.grid), dim3(kRuThreads), L.smem, stream, L.tmA, L.tmW7, L.tmW1, L.tmR, L.tmO, L.tmX, L.p);
 }
 
 // ------------------------------------------------------------------ tensor-core weight gradient (wgrad_umma.cuh)
@@ -777,20 +645,6 @@ inline cudaError_t launch_wgrad_umma(const WgradLaunch& L, cudaStream_t stream) 
     attr_set[dev & 63] = true;
   }
   wgrad_umma_kernel<<<L.grid, 256, L.smem, stream>>>(L.tmD, L.tmS, L.p);
-  return cudaGetLastError();
-}
-
-inline cudaError_t launch_conv_umma(const ConvLaunch& L, cudaStream_t stream) {
-  static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr_set[dev & 63]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         227 * 1024);
-    if (e != cudaSuccess) return e;
-    attr_set[dev & 63] = true;
-  }
-  conv_umma_kernel<<<L.grid, 256, L.smem, stream>>>(L.tmA, L.tmW, L.p);
   return cudaGetLastError();
 }
 

@@ -4,7 +4,7 @@
 #include <cuda_bf16.h>
 #include <cstdint>
 
-#include "conv_umma.cuh"  // snake_beta
+#include "conv_common.cuh"  // snake_beta
 
 namespace kvae {
 

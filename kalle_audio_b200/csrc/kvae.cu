@@ -134,9 +134,7 @@ struct Layout {
 };
 
 struct PreparedRun {
-  std::vector<ConvLaunch> umma;     // per step (valid when that step is tensor-core, KVAE_CONV_V1=1)
-  std::vector<ConvLaunch2> umma2;   // per step (valid when that step is tensor-core; persistent kernel)
-  bool use_v1 = false;
+  std::vector<ConvLaunch2> umma2;   // per step (valid when that step is tensor-core)
   std::vector<DirectParams> direct; // per step (valid otherwise)
   std::vector<dim3> direct_grid;
   std::vector<int> direct_cfg;      // 0: 32x64 tile, 1: 128x4 tile
@@ -240,7 +238,7 @@ void add_conv(kvae_plan* p, int kind, int Cin, int Cout, int K, int stride, int 
   c.g = ConvGeom{kind, Cin, Cout, K, stride, dil, pad};
   c.has_bias = bias;
   c.umma = (p->precision == KVAE_PREC_BF16) && umma_supported(c.g);
-  c.umma32 = (p->precision == KVAE_PREC_F32) && umma_supported(c.g) && !env_flag("KVAE_F32_CUDA_CORES");
+  c.umma32 = (p->precision == KVAE_PREC_F32) && umma_supported(c.g);
   p->convs.push_back(c);
 }
 int add_snake(kvae_plan* p, int C) {
@@ -372,16 +370,15 @@ void finalize_steps(kvae_plan* p) {
   const int n = static_cast<int>(p->steps.size());
   // fp16 residual stream: only when every step runs on a kernel that knows about it (tensor-core convs and the
   // two waveform-edge kernels), i.e. the graded architectures in bf16 mode; anything else keeps fp32
-  p->stream_f16 = p->precision == KVAE_PREC_BF16 && !env_flag("KVAE_STREAM_F32") && !env_flag("KVAE_WAVE_OUT_CC") &&
-                  !env_flag("KVAE_CONV_V1");
+  p->stream_f16 = p->precision == KVAE_PREC_BF16;
   for (int k = 0; k < n && p->stream_f16; ++k)
     if (!p->convs[p->steps[k].conv].umma && !is_wave_in_step(p, p->steps, k) && !is_wave_out_step(p, p->steps, k))
       p->stream_f16 = false;
   // Training plans: the saved pre-activation stream is fp16 too when every step is a tensor-core conv or one of the
   // two waveform-edge convs (the graded architectures): the forward k=1 convs then move 1024 instead of 1536 bytes per
   // row and use the fragment-mapped epilogue, the SnakeBeta backward reads 2 instead of 4 bytes per element.  The
-  // 11 significant bits of fp16 are what the inference path already carries.  KVAE_TRAIN_STREAM_F32=1 keeps fp32.
-  p->train_stream_f16 = p->stream_f16 && !env_flag("KVAE_TRAIN_STREAM_F32") && n >= 3;
+  // 11 significant bits of fp16 are what the inference path already carries.
+  p->train_stream_f16 = p->stream_f16 && n >= 3;
   // a conv is a tensor-core step in bf16 mode (always) or in fp32 mode for inference (bf16x3 split); fp32-mode
   // training stays on the CUDA cores, so the two step lists can differ in who needs which tensor
   auto set_flags = [&](std::vector<Step>& steps, bool train) {
@@ -415,10 +412,9 @@ void finalize_steps(kvae_plan* p) {
     c.off_v = off; off += static_cast<long long>(c.numel()); p->param_sizes.push_back(static_cast<long long>(c.numel()));
   }
   p->n_params = off;
-  // ResidualUnits of 128-channel stages run as ONE kernel (conv_ru.cuh): k7 -> SnakeBeta -> k1 -> + skip
-  const char* nf = getenv("KVAE_NO_RU_FUSION");
-  const char* v1 = getenv("KVAE_CONV_V1");
-  if ((nf && nf[0] == '1') || (v1 && v1[0] == '1') || !p->stream_f16) return;   // the fused kernel reads / writes the fp16 stream
+  // ResidualUnits of 128-channel stages run as ONE kernel (conv_ru2.cuh): k7 -> SnakeBeta -> k1 -> + skip.
+  // KVAE_NO_RU_FUSION=1 keeps the two-kernel form (the reference of the fused kernel's tests).
+  if (env_flag("KVAE_NO_RU_FUSION") || !p->stream_f16) return;   // the fused kernel reads / writes the fp16 stream
   for (int k = 1; k + 1 < n; ++k) {
     Step& a = p->steps[k];
     Step& b = p->steps[k + 1];
@@ -440,7 +436,7 @@ void finalize_steps(kvae_plan* p) {
   // Decoder tail (conv_edge.cuh): when the unit in front of it is a fused ResidualUnit, that unit applies the tail's
   // SnakeBeta in its epilogue and writes the result in fp16; the tail's 16 transform warps (0.33 of its 0.49 ms at
   // 16 x 442 368 rows) have nothing left to do.  One rounding fewer than snake(fp16(x)).  KVAE_TAIL_RAW=1: old flow.
-  if (n >= 3 && !env_flag("KVAE_TAIL_RAW") && !env_flag("KVAE_WAVE_OUT_CC") && is_wave_out_step(p, p->steps, n - 1) &&
+  if (n >= 3 && !env_flag("KVAE_TAIL_RAW") && is_wave_out_step(p, p->steps, n - 1) &&
       p->steps[n - 2].fuse == 2 && p->steps[n - 1].pre_snake >= 0) {
     Step& b = p->steps[n - 2];
     b.needs_act = true;
@@ -537,13 +533,8 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
                  PreparedRun& R, std::string& err) {
   const int n = static_cast<int>(steps.size());
   if (!make_layout(p, steps, train, B, T, R.layout, err)) return false;
-  R.umma.resize(n);
   R.umma2.resize(n);
   R.ru.resize(n);
-  {
-    const char* e = getenv("KVAE_CONV_V1");   // development switch: the non-persistent first-generation kernel
-    R.use_v1 = e && e[0] == '1';
-  }
   R.direct.resize(n);
   R.direct_grid.resize(n);
   R.direct_cfg.assign(n, 0);
@@ -570,8 +561,8 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
     void* act = s.needs_act ? tptr(2 + 2 * k) : nullptr;
     const void* res = (s.residual_from >= 0) ? tptr(1 + 2 * s.residual_from) : nullptr;
     if (s.residual_from >= 0 && !res) { err = "internal: residual tensor missing"; return false; }
-    if (s.fuse == 2 && !R.use_v1) { R.kind[k] = 5; continue; }
-    if (s.fuse == 1 && !R.use_v1) {
+    if (s.fuse == 2) { R.kind[k] = 5; continue; }
+    if (s.fuse == 1) {
       const Step& s1 = steps[k + 1];
       const ConvLayer& c1 = p->convs[s1.conv];
       RuArgs ra;
@@ -611,8 +602,7 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
       w.tanh_out = (p->direction == KVAE_DECODER && p->arch.final_tanh) ? 1 : 0;
       w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
       R.kind[k] = 3;
-      const char* cc = getenv("KVAE_WAVE_OUT_CC");     // development switch: the CUDA-core tail
-      if (!(cc && cc[0] == '1') && p->precision == KVAE_PREC_BF16) {   // fp32 mode keeps the exact fp32 FMAs
+      if (p->precision == KVAE_PREC_BF16) {   // fp32 mode keeps the exact fp32 FMAs
         PreparedRun::WaveOutTc& t = R.wave_out_tc[k];
         std::memset(&t.p, 0, sizeof(t.p));
         t.p.pro_a = w.pro_a; t.p.pro_inv_b = w.pro_inv_b; t.p.w = w.w;
@@ -623,9 +613,6 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
         if (sf16) { if (!make_act_tmap(&t.tmX, w.x, B, w.T, 128, 1, kWoTcRows, err)) return false; }
         else if (!make_out_tmap(&t.tmX, w.x, B, w.T, 128, 1, 1, err, kWoTcRows)) return false;
         R.kind[k] = 6;
-      } else if (sf16) {
-        err = "internal: fp16 stream needs the tensor-core tail";
-        return false;
       }
       continue;
     }
@@ -693,27 +680,19 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
         ep.snake_inv_b = p->snakes[s.epi_snake].inv_b;
       }
       if (!c.umma) {               // fp32 mode on the tensor cores: bf16x3 split operands, sinf in the epilogue
-        if (R.use_v1) { err = "KVAE_CONV_V1 has no fp32-mode tensor-core path"; return false; }
         ep.split3 = 1;
         ep.act_split = 1;
         ep.precise = 1;
       }
-      if (R.use_v1) {
-        ConvTuning tune;
-        if (!prepare_conv_umma(c.g, static_cast<const __nv_bfloat16*>(in), B, static_cast<int>(T_in), c.w_umma, ep,
-                               tune, R.umma[k], err))
-          return false;
-      } else {
-        ConvTuning2 tune;
-        if (!prepare_conv_umma2(c.g, static_cast<const __nv_bfloat16*>(in), B, static_cast<int>(T_in), c.w_umma, ep,
-                                tune, R.umma2[k], err))
-          return false;
-      }
+      ConvTuning2 tune;
+      if (!prepare_conv_umma2(c.g, static_cast<const __nv_bfloat16*>(in), B, static_cast<int>(T_in), c.w_umma, ep,
+                              tune, R.umma2[k], err))
+        return false;
     } else {
       DirectParams& d = R.direct[k];
       std::memset(&d, 0, sizeof(d));
       TapPlan tp;
-      if (!build_taps(c.g, false, tp, err)) return false;
+      if (!build_taps(c.g, tp, err)) return false;
       d.B = B;
       d.P_out = tp.P_out;
       d.P_in = tp.P_in;
@@ -975,7 +954,7 @@ int run_plan(kvae_plan* p, bool train, const void* in, int in_dtype, void* out, 
       w.x = in;
       w.x_f32 = (in_dtype == KVAE_F32);
       KV_CUDA(launch_wave_in(w, c.g.Cin, B, st));
-    } else if (R.kind[k] == 0 && !R.use_v1) {
+    } else if (R.kind[k] == 0) {
       ConvLaunch2& L = R.umma2[k];
       if (k == n - 1) {
         L.p.out_cf = out;
@@ -986,14 +965,6 @@ int run_plan(kvae_plan* p, bool train, const void* in, int in_dtype, void* out, 
         L.p.samp_std = fs ? fs->std : 0.f;
       }
       KV_CUDA(launch_conv_umma2(L, st));
-    } else if (R.kind[k] == 0) {
-      ConvLaunch& L = R.umma[k];
-      if (k == n - 1) {
-        L.p.out_raw = out;
-        L.p.out_raw_f32 = (out_dtype == KVAE_F32);
-        L.p.out_raw_cf = 1;
-      }
-      KV_CUDA(launch_conv_umma(L, st));
     } else {
       DirectParams& d = R.direct[k];
       if (k == 0) { d.x = in; d.x_f32 = (in_dtype == KVAE_F32); }
@@ -1033,8 +1004,7 @@ void set_sb_grid(SnakeBwdParams& sb, dim3& grid) {
 
 cudaError_t launch_snake_bwd(const SnakeBwdParams& sb, dim3 grid, cudaStream_t st) {
   SnakeBwdStreamGeom gm;
-  static const bool no_stream = env_flag("KVAE_SNAKE_BWD_PLAIN");     // A/B switch: the latency-bound predecessor
-  if (!no_stream && snake_bwd_stream_geom(sb, gm)) {
+  if (snake_bwd_stream_geom(sb, gm)) {
     static bool attr_set[64] = {false};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1200,8 +1170,8 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
     const ConvGeom gd = dgrad_geom(c.g, static_cast<int>(T_in));
     if (gd.out_len(static_cast<int>(T_out)) != T_in) { err = "internal: dgrad length bookkeeping"; return false; }
     // bf16 mode: dA crosses HBM as bf16 (written by the data-gradient conv's fragment-mapped epilogue, read by the
-    // vectorised SnakeBeta backward); KVAE_BWD_DA_F32=1 keeps the fp32 hand-over (A/B, debugging)
-    const bool da_bf16 = c.umma && k >= 1 && p->precision == KVAE_PREC_BF16 && c.g.Cin % 4 == 0 && !env_flag("KVAE_BWD_DA_F32");
+    // vectorised SnakeBeta backward)
+    const bool da_bf16 = c.umma && k >= 1 && p->precision == KVAE_PREC_BF16 && c.g.Cin % 4 == 0;
     if (c.umma) {
       bw.dgrad_kind = 1;
       ConvEpilogue ep;
@@ -1230,7 +1200,7 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
       DirectParams& d = bw.dg_direct;
       std::memset(&d, 0, sizeof(d));
       TapPlan tp;
-      if (!build_taps(gd, false, tp, err)) return false;
+      if (!build_taps(gd, tp, err)) return false;
       d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
       d.Tq_out = static_cast<int>((T_in + tp.P_out - 1) / tp.P_out);
       d.T_out = static_cast<int>(T_in); d.T_in = static_cast<int>(T_out);
@@ -1275,7 +1245,7 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
           if (j != k + 1) { err = "internal: skip connection spans more than one ResidualUnit"; return false; }
           sb.skip = Gf(j);
           // bf16 mode: read the bf16 copy of that gradient (it exists whenever step j runs on the tensor cores)
-          if (p->convs[steps[j].conv].umma && p->precision == KVAE_PREC_BF16 && c.g.Cin % 4 == 0 && !env_flag("KVAE_BWD_DA_F32")) {
+          if (p->convs[steps[j].conv].umma && p->precision == KVAE_PREC_BF16 && c.g.Cin % 4 == 0) {
             sb.skip = reinterpret_cast<const float*>(Gb(j));
             sb.skip_bf16 = 1;
           }
@@ -1284,7 +1254,7 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
       // k1 conv of a ResidualUnit), the CUDA-core kernels, or the input-gradient of step 0
       // (the skip-connection reader takes the bf16 copy in bf16 mode, see above)
       bool skip_reader_bf16 = false;
-      if (steps[k - 1].residual_from >= 0 && p->precision == KVAE_PREC_BF16 && !env_flag("KVAE_BWD_DA_F32")) {
+      if (steps[k - 1].residual_from >= 0 && p->precision == KVAE_PREC_BF16) {
         const int rf = steps[k - 1].residual_from;          // G_{k-1} is added into G_{rf} by the pass at step rf + 1
         skip_reader_bf16 = cp.umma && rf + 1 < n && p->convs[steps[rf + 1].conv].g.Cin % 4 == 0;
       }
@@ -1297,9 +1267,7 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
       set_sb_grid(sb, bw.sb_grid);
       // Fuse this pass into the data-gradient conv's epilogue when its only product is the bf16 gradient: tensor-core
       // dgrad with 128-channel tiles, fp16 saved stream, bf16 skip gradient (or none), no fp32 copy of G wanted.
-      // KVAE_BWD_FUSE_SNAKE=0: separate pass (A/B).
-      static const bool no_fuse = [] { const char* e = getenv("KVAE_BWD_FUSE_SNAKE"); return e && e[0] == '0'; }();
-      if (!no_fuse && bw.dgrad_kind == 1 && da_bf16 && sb.a && sb.x_f16 && !sb.G && sb.Gb && (!sb.skip || sb.skip_bf16) &&
+      if (bw.dgrad_kind == 1 && da_bf16 && sb.a && sb.x_f16 && !sb.G && sb.Gb && (!sb.skip || sb.skip_bf16) &&
           gd.Cout % 128 == 0) {
         ConvEpilogue ep;
         ep.out_act = sb.Gb;
@@ -1367,7 +1335,7 @@ int run_backward(kvae_plan* p, const void* x, int x_dtype, const void* gy, int g
       if (bw.wg_edge_x_is_thin) { e.N = x; e.N_f32 = (x_dtype == KVAE_F32); }
       e.dW = grads + c.off_v;
       const int C4 = e.C / 4;
-      const bool vec = e.C % 4 == 0 && C4 >= 8 && C4 <= 256 && (C4 & (C4 - 1)) == 0 && (e.W_f16 || !env_flag("KVAE_WGRAD_EDGE_SCALAR"));
+      const bool vec = e.C % 4 == 0 && C4 >= 8 && C4 <= 256 && (C4 & (C4 - 1)) == 0;
       if (vec) {
         // + the lane-reduction scratch: 256 threads x NT x 4 floats behind the thin rows
         const size_t smem = bw.wg_edge_smem + 16 + 256 * 2 * 4 * sizeof(float);
@@ -1421,44 +1389,23 @@ int run_backward(kvae_plan* p, const void* x, int x_dtype, const void* gy, int g
   }
   // weight-norm backward: dW (folded-weight gradient; in place in the weight_v slot, or packed by the
   // tensor-core kernel) -> (dv, dg); without params the packed gradients are only re-ordered
-  bool batched = true;               // KVAE_LOAD_PARAMS_PER_LAYER=1: per-layer launches (A/B, debugging)
-  if (const char* e = getenv("KVAE_LOAD_PARAMS_PER_LAYER")) batched = !(e[0] == '1');
-  if (batched) {
-    if (!p->wn_desc) {
-      std::vector<WnBwdDesc> wd(p->convs.size());
-      int rows = 0;
-      for (size_t i = 0; i < p->convs.size(); ++i) {
-        const ConvLayer& c = p->convs[i];
-        const int R = c.dim0();
-        wd[i].off_v = c.off_v; wd[i].off_g = c.off_g; wd[i].off_dwp = c.off_dwp;
-        wd[i].R = R; wd[i].Cc = static_cast<int>(c.numel() / c.g.K / R); wd[i].K = c.g.K; wd[i].row0 = rows;
-        rows += R;
-      }
-      KV_CUDA(cudaMalloc(&p->wn_desc, wd.size() * sizeof(WnBwdDesc)));
-      KV_CUDA(cudaMemcpy(p->wn_desc, wd.data(), wd.size() * sizeof(WnBwdDesc), cudaMemcpyHostToDevice));
-      p->wn_rows = rows;
+  if (!p->wn_desc) {
+    std::vector<WnBwdDesc> wd(p->convs.size());
+    int rows = 0;
+    for (size_t i = 0; i < p->convs.size(); ++i) {
+      const ConvLayer& c = p->convs[i];
+      const int R = c.dim0();
+      wd[i].off_v = c.off_v; wd[i].off_g = c.off_g; wd[i].off_dwp = c.off_dwp;
+      wd[i].R = R; wd[i].Cc = static_cast<int>(c.numel() / c.g.K / R); wd[i].K = c.g.K; wd[i].row0 = rows;
+      rows += R;
     }
-    weight_norm_bwd_all_kernel<<<p->wn_rows, 256, 0, st>>>(params, grads, p->dwp, p->wn_desc,
-                                                          static_cast<int>(p->convs.size()));
-    KV_CUDA(cudaGetLastError());
-    ++g_launches;
-    return 0;
+    KV_CUDA(cudaMalloc(&p->wn_desc, wd.size() * sizeof(WnBwdDesc)));
+    KV_CUDA(cudaMemcpy(p->wn_desc, wd.data(), wd.size() * sizeof(WnBwdDesc), cudaMemcpyHostToDevice));
+    p->wn_rows = rows;
   }
-  for (const ConvLayer& c : p->convs) {
-    const int R = c.dim0(), inner = static_cast<int>(c.numel() / R);
-    if (c.off_dwp >= 0) {
-      weight_norm_bwd_packed_kernel<<<R, 256, 0, st>>>(params ? params + c.off_v : nullptr,
-                                                       params ? params + c.off_g : nullptr, p->dwp + c.off_dwp,
-                                                       grads + c.off_v, grads + c.off_g, R, inner / c.g.K, c.g.K);
-    } else if (params) {
-      weight_norm_bwd_kernel<<<R, 256, 0, st>>>(params + c.off_v, params + c.off_g, grads + c.off_v, grads + c.off_v,
-                                                grads + c.off_g, inner);
-    } else {
-      continue;
-    }
-    KV_CUDA(cudaGetLastError());
-    ++g_launches;
-  }
+  weight_norm_bwd_all_kernel<<<p->wn_rows, 256, 0, st>>>(params, grads, p->dwp, p->wn_desc, static_cast<int>(p->convs.size()));
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
   return 0;
 }
 
@@ -1704,7 +1651,7 @@ int kvae_encode_sample(kvae_plan* p, const void* wav, int wav_dtype, void* lat, 
   if (!check_dtype(wav_dtype) || !check_dtype(lat_dtype)) return fail("bad dtype");
   if (D <= 0 || D > p->arch.latent_dim) return fail("D must be in 1 .. latent_dim");
   const ConvLayer& cl = p->convs[p->steps.back().conv];
-  if (!conv_tc(cl, false) || env_flag("KVAE_CONV_V1"))
+  if (!conv_tc(cl, false))
     return fail("fused sampling needs a tensor-core output conv (use kvae_encode + kvae_sigma_sample)");
   FusedSample fs;
   fs.noise = noise; fs.out = z; fs.D = D; fs.std = std;
@@ -1713,7 +1660,7 @@ int kvae_encode_sample(kvae_plan* p, const void* wav, int wav_dtype, void* lat, 
 
 int kvae_plan_fused_sample_supported(const kvae_plan* p) {
   if (!p) return 0;
-  return p->direction == KVAE_ENCODER && conv_tc(p->convs[p->steps.back().conv], false) && !env_flag("KVAE_CONV_V1") ? 1 : 0;
+  return p->direction == KVAE_ENCODER && conv_tc(p->convs[p->steps.back().conv], false) ? 1 : 0;
 }
 
 double kvae_plan_flops(const kvae_plan* p, int B, long long T) {
@@ -1808,7 +1755,7 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
   if (!guard.ok) return fail("cannot select the tensor's device");
   TapPlan tp;
   std::string err;
-  if (!build_taps(g, false, tp, err)) return fail(err);
+  if (!build_taps(g, tp, err)) return fail(err);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* wd = static_cast<float*>(scratch);
   const size_t n = static_cast<size_t>(Cin) * Cout * K;
@@ -1893,7 +1840,7 @@ int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, flo
   const ConvGeom gd = dgrad_geom(g, static_cast<int>(T));
   TapPlan tp;
   std::string err;
-  if (!build_taps(gd, false, tp, err)) return fail(err);
+  if (!build_taps(gd, tp, err)) return fail(err);
   float* wd = static_cast<float*>(scratch);
   pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
       w, gd.kind == kConvT, gd.Cout, gd.Cin, K, nullptr, wd);
@@ -2072,7 +2019,7 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
   if (engine == 0) {
     TapPlan tp;
     std::string err;
-    if (!build_taps(g, false, tp, err)) return fail(err);
+    if (!build_taps(g, tp, err)) return fail(err);
     DirectParams d;
     std::memset(&d, 0, sizeof(d));
     d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
@@ -2234,8 +2181,7 @@ int kvae_plan_load_params(kvae_plan* p, const float* params, int logscale, int t
     for (const ConvLayer& c : p->convs) m = std::max(m, c.dim0());
     KV_CUDA(cudaMalloc(&p->scale_scratch, static_cast<size_t>(m) * 4));
   }
-  bool batched = true;               // KVAE_LOAD_PARAMS_PER_LAYER=1: the per-layer launches below (A/B, debugging)
-  if (const char* e = getenv("KVAE_LOAD_PARAMS_PER_LAYER")) batched = !(e[0] == '1');
+  bool batched = true;               // one scale + one pack + one SnakeBeta-constant launch for the whole plan
   for (const ConvLayer& c : p->convs) {
     if (c.g.K > kPackMaxK) return fail("kernel size > 16 unsupported by kvae_plan_load_params");
     if (c.umma32) batched = false;   // fp32-mode inference operands need the extra split pass per layer
@@ -2340,11 +2286,9 @@ int kvae_plan_load_params(kvae_plan* p, const float* params, int logscale, int t
   }
   }
   if (train && !p->dwp) {
-    const char* e = getenv("KVAE_WGRAD_DIRECT");     // development switch: CUDA-core weight gradients everywhere
-    const bool direct = e && e[0] == '1';
     size_t off = 0;
     for (ConvLayer& c : p->convs)
-      if (c.umma && !direct) { c.off_dwp = static_cast<long long>(off); off += c.numel(); }
+      if (c.umma) { c.off_dwp = static_cast<long long>(off); off += c.numel(); }
     p->dwp_floats = off;
     if (off) KV_CUDA(cudaMalloc(&p->dwp, off * 4));
   }
@@ -2498,8 +2442,7 @@ int kvae_decode_pcm16(kvae_plan* p, const void* z, int z_dtype, void* wav, int w
 
 int kvae_plan_fused_pcm_supported(const kvae_plan* p) {
   if (!p || p->direction != KVAE_DECODER) return 0;
-  return (p->precision == KVAE_PREC_BF16 && p->stream_f16 && !env_flag("KVAE_WAVE_OUT_CC") &&
-          is_wave_out_step(p, p->steps, static_cast<int>(p->steps.size()) - 1)) ? 1 : 0;
+  return (p->precision == KVAE_PREC_BF16 && p->stream_f16 && is_wave_out_step(p, p->steps, static_cast<int>(p->steps.size()) - 1)) ? 1 : 0;
 }
 
 int kvae_pcm16(const void* wav, int dtype, int16_t* out, size_t n, void* scratch, void* stream) {

@@ -16,15 +16,8 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 // Warp index broadcast from lane 0: ptxas then treats it (and everything derived from it -- staging addresses, TMA
 // coordinates, loop counters) as warp-uniform and keeps it in uniform registers.  With a plain threadIdx.x >> 5 every
 // TMA issue under `lane == 0` is wrapped in a per-operand R2UR waterfall loop (~25 instructions per issue).
-#ifndef KVAE_UNIFORM_WARP
-#define KVAE_UNIFORM_WARP 1
-#endif
 __device__ __forceinline__ int warp_idx() {
-#if KVAE_UNIFORM_WARP
   return __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
-#else
-  return static_cast<int>(threadIdx.x >> 5);
-#endif
 }
 
 __device__ __forceinline__ bool elect_one() {

@@ -107,7 +107,7 @@ void stream_reset(kvae_stream* s) {
 // per-step tap statistics of the decoder's convs (all stride-1 convs or transposed convs)
 bool stream_step_geometry(const ConvGeom& g, StreamStep& st, std::string& err) {
   TapPlan tp;
-  if (!build_taps(g, false, tp, err)) return false;
+  if (!build_taps(g, tp, err)) return false;
   if (tp.P_in != 1) { err = "streaming: strided convolutions (encoders) are not supported"; return false; }
   int dmin = 1 << 30, dmax = -(1 << 30);
   for (const Tap& t : tp.taps) {

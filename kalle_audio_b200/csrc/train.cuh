@@ -14,7 +14,7 @@
 #include <cuda_fp16.h>
 #include <cstdint>
 
-#include "conv_umma.cuh"    // snake_beta
+#include "conv_common.cuh"  // snake_beta
 #include "elementwise.cuh"  // ld_elem / st_elem
 
 namespace kvae {
@@ -866,11 +866,6 @@ __device__ __forceinline__ void weight_norm_bwd_packed_row(float (*red)[32], con
     if (k2 >= K) { k2 -= K; ++c2; }
   }
   if (g && threadIdx.x == 0) dg[i] = dot / n;
-}
-__global__ void weight_norm_bwd_packed_kernel(const float* v, const float* g, const float* dwp, float* dv, float* dg,
-                                              int R, int Cc, int K) {
-  __shared__ float red[2][32];
-  weight_norm_bwd_packed_row(red, v, g, dwp, dv, dg, R, Cc, K, blockIdx.x);
 }
 
 // All layers of a plan in ONE launch (72 launches of ~16 us each before): grid = sum of dim-0 rows, a block finds its

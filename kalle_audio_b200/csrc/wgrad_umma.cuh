@@ -17,7 +17,7 @@
 // split over gridDim.y CTAs per tile (split-K); CTAs of the same split run side by side (tile index is the
 // fast grid dimension), so the D / S rows they share come from L2.  Partial sums are added to a packed fp32
 // buffer [K][Cd][Cs] with vector reductions (red.global.add.v4.f32); the weight-norm backward reads that
-// layout directly (train.cuh::weight_norm_bwd_packed_kernel).
+// layout directly (train.cuh::weight_norm_bwd_packed_row).
 //
 // Warp roles (256 threads): warp 0 TMA producer, warp 1 UMMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue.
 #pragma once

@@ -414,16 +414,14 @@ def test_fused_residual_unit_matches_two_kernel_path(dev):
     assert float((y_fused - y_split).abs().max()) <= 2e-5 * float(ref.abs().max())
 
 
-def test_pipelined_residual_unit_bit_identical_to_serial_kernels(dev):
-    """conv_ru2_kernel (two TMEM accumulators, GEMM2 of tile i inside GEMM1 of tile i+1, fragment-mapped epilogues)
-    against its predecessors conv_ru_kernel<0> (one channel per thread, scalar fp32) and <1> on the same plan: the
-    packed fp32 pairs round like the scalar instructions and the MMA order per tile is unchanged, so the waveform
-    must be bit-identical.  KVAE_RU_GRID=5 forces ~20 tiles per CTA through the cross-tile pipeline."""
+def test_pipelined_residual_unit_bit_identical_across_grids(dev):
+    """conv_ru2_kernel (two TMEM accumulators, GEMM2 of tile i inside GEMM1 of tile i+1) carries state from tile to
+    tile of a CTA: the waveform must be bit-identical whatever the number of tiles per CTA.  KVAE_RU_GRID=5 and 7 force
+    ~20 and ~14 of the 99 tiles per CTA through the cross-tile pipeline."""
     import os
     z = torch.randn(3, 64, 211, generator=torch.Generator().manual_seed(4)).to(dev)
     outs = {}
-    for name, env in (("ru2", {}), ("ru2_few_ctas", {"KVAE_RU_GRID": "5"}), ("serial0", {"KVAE_RU_EPI": "0"}),
-                      ("serial1", {"KVAE_RU_EPI": "1", "KVAE_RU_GRID": "7"})):
+    for name, env in (("ru2", {}), ("ru2_grid5", {"KVAE_RU_GRID": "5"}), ("ru2_grid7", {"KVAE_RU_GRID": "7"})):
         os.environ.update(env)
         try:
             m = H.build("mid", 0, snake_seed=7).to(dev).set_precision("bf16")
@@ -433,7 +431,7 @@ def test_pipelined_residual_unit_bit_identical_to_serial_kernels(dev):
             for key in env:
                 del os.environ[key]
     assert bool(torch.isfinite(outs["ru2"]).all())
-    for name in ("ru2_few_ctas", "serial0", "serial1"):
+    for name in ("ru2_grid5", "ru2_grid7"):
         assert torch.equal(outs["ru2"], outs[name]), name
 
 

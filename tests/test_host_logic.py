@@ -191,3 +191,24 @@ def test_layer_model_flops_match_survey():
     for arch, want in (("sao", 1089.145), ("o12", 1255.219)):
         total = sum(lm.model(l)["gflop"] for l in lm.decoder_layers(lm.ARCH[arch], 1))
         assert abs(total - want) < 2e-3 * want, (arch, total)
+
+
+def test_library_environment_switches_are_the_kept_set():
+    """The native library reads exactly these environment switches: KVAE_NO_RU_FUSION (the two-kernel reference of
+    the fused ResidualUnit), KVAE_RU_GRID (many tiles per CTA) and KVAE_FAST_EPI / KVAE_WAVE_IN_CC / KVAE_TAIL_RAW (the
+    kernel variants test_gpu_variants.py compares).  A new switch has to be added here on purpose."""
+    import os
+    import re
+    csrc = os.path.join(os.path.dirname(k.__file__), "csrc")
+    names, other = set(), []
+    for fn in sorted(os.listdir(csrc)):
+        with open(os.path.join(csrc, fn)) as f:
+            src = f.read()
+        for arg in re.findall(r"\b(?:getenv|env_flag)\(([^)]*)\)", src):
+            lit = re.fullmatch(r'\s*"([^"]+)"\s*', arg)
+            if lit:
+                names.add(lit.group(1))
+            elif arg.strip() not in ("name", "const char* name"):   # env_flag's own definition
+                other.append((fn, arg))
+    assert not other, other
+    assert names == {"KVAE_NO_RU_FUSION", "KVAE_RU_GRID", "KVAE_FAST_EPI", "KVAE_WAVE_IN_CC", "KVAE_TAIL_RAW"}

@@ -1,5 +1,5 @@
-"""Development aid: SAO decode + encode at B=8 under the current environment (KVAE_LIB, KVAE_RU_EPI, ...): per-step
-CUDA-event profile summed by kernel class, plus the parity numbers against the golden anchor.  One line per run."""
+"""Development aid: SAO decode + encode at B=8 with the library KVAE_LIB names (and the kept switches of tools/README.md):
+per-step CUDA-event profile summed by kernel class, plus the parity numbers against the golden anchor.  One line per run."""
 import os
 import sys
 

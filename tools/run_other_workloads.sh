@@ -3,10 +3,9 @@ mkdir -p gpurun_out
 for w in stream o12_decode train; do
   python bench.py --workload $w --no-cpu-baseline --steps 20 > gpurun_out/bench_$w.json 2> gpurun_out/bench_$w.err; echo "$w exit $?"
 done
-KVAE_LIB=$PWD/build/libkvae_nu.so KVAE_RU_EPI=0 KVAE_SPLIT_PRODUCER=0 python bench.py --workload stream --no-cpu-baseline --steps 20 > gpurun_out/bench_stream_old.json 2>/dev/null
 python - <<'PY'
 import json
-for w in ['stream','stream_old','o12_decode','train']:
+for w in ['stream','o12_decode','train']:
     try:
         j=json.loads(open(f'gpurun_out/bench_{w}.json').read().strip().split('\n')[-1])
         keys=['value','ms_per_step','per_chunk_ms','first_chunk_wall_ms_incl_d2h','exact_context_stream','tflops','clocks']

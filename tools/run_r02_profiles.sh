@@ -16,7 +16,6 @@ ncu --set full --clock-control none --import-source on -k regex:conv_umma2_kerne
 PROF_STEPS=1 python tools/prof_sao_b16.py 16 > gpurun_out/r02_step_profile_sao_b16.txt 2>&1
 python tools/prof_o12_b1.py 128 1 > gpurun_out/r02_step_profile_o12_b1.txt 2>&1
 python tools/prof_o12_b1.py 96 1 >> gpurun_out/r02_step_profile_o12_b1.txt 2>&1
-bash tools/run_train_list2.sh > gpurun_out/r02_train_step_launches.txt 2>&1
 python bench.py --workload train --steps 10 --warmup 3 > gpurun_out/r02_bench_train_n1.json 2>/dev/null
 python bench.py --workload stream --steps 30 --warmup 5 > gpurun_out/r02_bench_stream.json 2>/dev/null
 python bench.py --workload bigvgan --steps 6 > gpurun_out/r02_bench_bigvgan.json 2>/dev/null

@@ -1,9 +1,12 @@
-// Stand-alone probe for the tcgen05 convolution kernel (kalle_audio_b200/csrc/conv_umma.cuh).
+// Stand-alone probe for the tcgen05 convolution kernels (kalle_audio_b200/csrc/conv_umma2.cuh, conv_ru2.cuh).
 // Each invocation runs ONE case so a trap in one case cannot poison the others:
-//   umma_probe <case> <variant>     variant 0: one A slab per tap (no shifted descriptors)
-//                                   variant 1: shared slab, descriptor base_offset = 0
-//                                   variant 2: shared slab, base_offset = (addr >> 7) & 7
-//   umma_probe perf <idx>           timing of full-size layers (no CPU check)
+//   umma_probe <case> <variant>     variant 3: automatic tiling
+//                                   variant 4: a grid of 3 CTAs, so every CTA loops over many tiles
+//                                   variant 5: 128-row tiles at most 128 channels wide
+//                                   variant 6: operand swap disabled (time rows on the M side)
+//   umma_probe perf <idx> <version> <epilogue>   timing of full-size layers (no CPU check); version 2: automatic
+//                                   tiling, 3: the table's MT / NT, 4: operand swap disabled
+//   umma_probe ru <dilation> <B> <T> [perf]       the fused ResidualUnit against the CPU loops (or timed)
 // The check is a double-precision channels-last convolution over the same bf16-rounded operands.
 #include <cmath>
 #include <cstdio>
@@ -141,41 +144,21 @@ static int run_case(int idx, int variant) {
     ep.snake_inv_b = dsib;
   }
   std::string err;
-  if (variant >= 3) {
-    // persistent double-buffered kernel; variant 4 forces a tiny grid so every CTA loops over many tiles
-    ConvTuning2 tune2;
-    if (variant == 4) tune2.max_ctas = 3;
-    if (variant == 5) { tune2.MT = 1; tune2.NT = c.NT > 128 ? 128 : c.NT; }
-    if (variant == 6) tune2.swap = 0;   // time rows on the M side even for 128-channel tiles
-    ConvLaunch2 L2;
-    if (!prepare_conv_umma2(g, dx, c.B, c.T, dw, ep, tune2, L2, err)) {
-      printf("CASE %d %s variant %d: prepare failed: %s\n", idx, c.name, variant, err.c_str());
-      return 3;
-    }
-    printf("CASE %d %s variant %d: grid %d smem %zu MT %d NT %d acc %d RB %d nbox %d SA %d SB %d tmem %d tiles %d\n",
-           idx, c.name, variant, L2.grid, L2.smem, L2.p.MT, L2.p.NT, L2.p.acc_stages, L2.p.RB, L2.p.nbox, L2.p.SA,
-           L2.p.SB, L2.p.tmem_cols, L2.p.total_tiles);
-    fflush(stdout);
-    CK(launch_conv_umma2(L2, 0));
-    CK(cudaDeviceSynchronize());
-  } else {
-  ConvTuning tune;
-  tune.MT = c.MT;
-  tune.NT = c.NT;
-  tune.per_tap_slab = (variant == 0);
-  tune.desc_mode = (variant == 2) ? 1 : 0;
-  ConvLaunch L;
-  if (!prepare_conv_umma(g, dx, c.B, c.T, dw, ep, tune, L, err)) {
+  ConvTuning2 tune2;
+  if (variant == 4) tune2.max_ctas = 3;
+  if (variant == 5) { tune2.MT = 1; tune2.NT = c.NT > 128 ? 128 : c.NT; }
+  if (variant == 6) tune2.swap = 0;   // time rows on the M side even for 128-channel tiles
+  ConvLaunch2 L2;
+  if (!prepare_conv_umma2(g, dx, c.B, c.T, dw, ep, tune2, L2, err)) {
     printf("CASE %d %s variant %d: prepare failed: %s\n", idx, c.name, variant, err.c_str());
     return 3;
   }
-  printf("CASE %d %s variant %d: grid (%d,%d,%d) smem %zu MT %d NT %d RB %d nbox %d SA %d SB %d tmem %d taps %d\n",
-         idx, c.name, variant, L.grid.x, L.grid.y, L.grid.z, L.smem, L.p.MT, L.p.NT, L.p.RB, L.p.nbox,
-         L.p.SA, L.p.SB, L.p.tmem_cols, L.p.tap_begin[L.p.P_out]);
+  printf("CASE %d %s variant %d: grid %d smem %zu MT %d NT %d acc %d RB %d nbox %d SA %d SB %d tmem %d tiles %d\n",
+         idx, c.name, variant, L2.grid, L2.smem, L2.p.MT, L2.p.NT, L2.p.acc_stages, L2.p.RB, L2.p.nbox, L2.p.SA,
+         L2.p.SB, L2.p.tmem_cols, L2.p.total_tiles);
   fflush(stdout);
-  CK(launch_conv_umma(L, 0));
+  CK(launch_conv_umma2(L2, 0));
   CK(cudaDeviceSynchronize());
-  }
   std::vector<float> raw(nout);
   std::vector<__nv_bfloat16> act(nout);
   CK(cudaMemcpy(raw.data(), draw, nout * 4, cudaMemcpyDeviceToHost));
@@ -277,26 +260,15 @@ static int run_perf(int idx, int ver, int epi) {
     ep.residual = dres; ep.residual_f32 = 1; ep.out_raw = draw; ep.out_raw_f32 = 1;
   }
   std::string err;
-  ConvLaunch L;
   ConvLaunch2 L2;
-  if (ver == 1) {
-    ConvTuning tune;
-    tune.MT = c.MT;
-    tune.NT = c.NT;
-    if (!prepare_conv_umma(g, dx, c.B, c.T, dw, ep, tune, L, err)) {
-      printf("PERF %s: prepare failed: %s\n", c.name, err.c_str());
-      return 3;
-    }
-  } else {
-    ConvTuning2 tune2;
-    if (ver == 3) { tune2.MT = c.MT; tune2.NT = c.NT; }
-    if (ver == 4) tune2.swap = 0;
-    if (!prepare_conv_umma2(g, dx, c.B, c.T, dw, ep, tune2, L2, err)) {
-      printf("PERF %s: prepare failed: %s\n", c.name, err.c_str());
-      return 3;
-    }
+  ConvTuning2 tune2;
+  if (ver == 3) { tune2.MT = c.MT; tune2.NT = c.NT; }
+  if (ver == 4) tune2.swap = 0;
+  if (!prepare_conv_umma2(g, dx, c.B, c.T, dw, ep, tune2, L2, err)) {
+    printf("PERF %s: prepare failed: %s\n", c.name, err.c_str());
+    return 3;
   }
-  auto launch = [&]() { return ver == 1 ? launch_conv_umma(L, 0) : launch_conv_umma2(L2, 0); };
+  auto launch = [&]() { return launch_conv_umma2(L2, 0); };
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0));
   CK(cudaEventCreate(&e1));
@@ -313,13 +285,9 @@ static int run_perf(int idx, int ver, int epi) {
   const double taps_eff = (g.kind == kConv) ? (double)g.K * T_out : (double)g.K * c.T;
   const double flops = 2.0 * c.B * taps_eff * g.Cin * g.Cout;
   const double bytes = (nin + nout) * 2.0 + (epi >= 2 ? nout * 8.0 : 0.0);
-  if (ver == 1)
-    printf("PERF v1 epi%d %s: %.3f ms  %.1f TFLOP/s  %.1f GB/s  MT %d NT %d smem %zu SA %d SB %d\n", epi, c.name, ms,
-           flops / ms * 1e-9, bytes / ms * 1e-6, L.p.MT, L.p.NT, L.smem, L.p.SA, L.p.SB);
-  else
-    printf("PERF v%d epi%d %s: %.3f ms  %.1f TFLOP/s  %.1f GB/s  MT %d NT %d swap %d acc %d grid %d smem %zu SA %d SB %d\n",
-           ver, epi, c.name, ms, flops / ms * 1e-9, bytes / ms * 1e-6, L2.p.MT, L2.p.NT, L2.p.swap, L2.p.acc_stages,
-           L2.grid, L2.smem, L2.p.SA, L2.p.SB);
+  printf("PERF v%d epi%d %s: %.3f ms  %.1f TFLOP/s  %.1f GB/s  MT %d NT %d swap %d acc %d grid %d smem %zu SA %d SB %d\n",
+         ver, epi, c.name, ms, flops / ms * 1e-9, bytes / ms * 1e-6, L2.p.MT, L2.p.NT, L2.p.swap, L2.p.acc_stages,
+         L2.grid, L2.smem, L2.p.SA, L2.p.SB);
   return 0;
 }
 
@@ -443,7 +411,8 @@ int main(int argc, char** argv) {
   if (argc >= 3 && std::string(argv[1]) == "perf") {
     int idx = atoi(argv[2]);
     if (idx < 0 || idx >= kNumPerf) return 4;
-    const int ver = argc >= 4 ? atoi(argv[3]) : 1, epi = argc >= 5 ? atoi(argv[4]) : 0;
+    const int ver = argc >= 4 ? atoi(argv[3]) : 2, epi = argc >= 5 ? atoi(argv[4]) : 0;
+    if (ver < 2 || ver > 4) return 4;
     return run_perf(idx, ver, epi);
   }
   if (argc >= 2 && std::string(argv[1]) == "count") {
@@ -451,11 +420,11 @@ int main(int argc, char** argv) {
     return 0;
   }
   if (argc < 3) {
-    printf("usage: umma_probe <case 0..%d> <variant 0..2> | perf <0..%d> | count\n", kNumCases - 1,
-           kNumPerf - 1);
+    printf("usage: umma_probe <case 0..%d> <variant 3..6> | perf <0..%d> [2..4] [0..2] | ru <dil> <B> <T> [1] | count\n",
+           kNumCases - 1, kNumPerf - 1);
     return 4;
   }
   int idx = atoi(argv[1]), variant = atoi(argv[2]);
-  if (idx < 0 || idx >= kNumCases) return 4;
+  if (idx < 0 || idx >= kNumCases || variant < 3 || variant > 6) return 4;
   return run_case(idx, variant);
 }
