@@ -147,6 +147,28 @@ int kvae_decode_stream_push(kvae_stream* s, const void* z, int z_dtype, int n_fr
 int kvae_decode_stream_end(kvae_stream* s, void* wav, int wav_dtype, long long wav_capacity, long long* n_samples,
                            void* stream);
 void kvae_decode_stream_destroy(kvae_stream* s);
+/* ---- stateful streaming encode: the same engine in the encoder's direction, for callers that receive audio
+ * incrementally (live input to a speech LM) or encode long recordings in bounded memory.  Every layer keeps the tail
+ * of its own input; the strided convs keep whole groups of `stride` rows, so the emitted latents equal kvae_encode of
+ * the whole clip bit for bit, and for a length L that is not a multiple of the ratio they are the
+ * kvae_plan_out_length(L) frames of the reference's floor arithmetic (kvae_encode_ragged).
+ *   begin      window buffers for pushes of up to max_samples samples; use_graphs as for the decoder stream
+ *   frames     how many latent frames the next push of n_samples (or, end != 0, the end call) will emit
+ *   lookahead  samples past a frame's last sample that must have arrived before the frame is emitted (the encoder's
+ *              right receptive field: 14 885 for the SAO strides, 9 925 for the 12.5 Hz strides)
+ *   push       wav [B, io_channels, n_samples] -> lat [B, latent_dim, *n_frames] (packed with that length)
+ *   end        emits the remaining frames (right edge zero-padded like the whole-clip encode) and resets the stream
+ *   destroy    frees the stream
+ * Encoder plans whose every step has a tensor-core kernel (channels / latent_dim multiples of 64, a 128-channel head),
+ * bf16 or fp32 mode; other architectures get an error from begin. */
+int kvae_encode_stream_begin(kvae_plan* plan, int B, long long max_samples, int use_graphs, kvae_stream** out);
+long long kvae_encode_stream_frames(kvae_stream* s, long long n_samples, int end);
+long long kvae_encode_stream_lookahead(const kvae_stream* s);
+int kvae_encode_stream_push(kvae_stream* s, const void* wav, int wav_dtype, long long n_samples, void* lat,
+                            int lat_dtype, long long lat_capacity, long long* n_frames, void* stream);
+int kvae_encode_stream_end(kvae_stream* s, void* lat, int lat_dtype, long long lat_capacity, long long* n_frames,
+                           void* stream);
+void kvae_encode_stream_destroy(kvae_stream* s);
 /* kvae_encode with the sigma-VAE sample fused into the last conv's epilogue: lat [B, latent_dim, T] as kvae_encode,
  * and z [B, D, T] = lat[:, :D] + std * noise (sample(mean, 'fix') of model_sigmaVAE.py:187-213 applied to the mean
  * half of the encoder output, D = latent_dim / 2 for the mean | scale layout of twj_dataset.py:251), evaluated on the

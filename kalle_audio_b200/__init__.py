@@ -17,7 +17,7 @@ from .factory import create_model_from_config, create_model_from_config_path, cr
 from .layers import SnakeBeta, WNConv1d, WNConvTranspose1d, snake_beta
 from .pretransforms import AutoencoderPretransform, Pretransform
 from .sampling import SigmaVAESampler, sample
-from .streaming import StreamingDecoder, decoder_context_frames
+from .streaming import StreamingDecoder, StreamingEncoder, decoder_context_frames, encoder_context_samples
 from .hostio import HostPipeline
 from .glue import LatentGlue
 from .dataset import LatentExtractor
@@ -38,5 +38,5 @@ __all__ = [
     "get_activation", "load_ckpt_state_dict", "prepare_audio", "remove_weight_norm_from_model", "sample",
     "snake_beta", "vae_sample", "to_pcm16", "AutoencoderTrainer", "FlatAdamW", "GradSync", "flatten_parameters",
     "gaussian_nll", "vae_sample_with_grad", "StreamingDecoder", "decoder_context_frames", "HostPipeline", "LatentGlue", "LatentExtractor", "BigVGANFlowVAE",
-    "BigVGANStreamingDecoder", "bigvgan_stream_geometry",
+    "BigVGANStreamingDecoder", "bigvgan_stream_geometry", "StreamingEncoder", "encoder_context_samples",
 ]

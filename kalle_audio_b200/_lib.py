@@ -72,6 +72,14 @@ SIGNATURES = {
     "kvae_decode_stream_end": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_longlong, C.POINTER(C.c_longlong),
                                          C.c_void_p]),
     "kvae_decode_stream_destroy": (None, [C.c_void_p]),
+    "kvae_encode_stream_begin": (C.c_int, [C.c_void_p, C.c_int, C.c_longlong, C.c_int, C.POINTER(C.c_void_p)]),
+    "kvae_encode_stream_frames": (C.c_longlong, [C.c_void_p, C.c_longlong, C.c_int]),
+    "kvae_encode_stream_lookahead": (C.c_longlong, [C.c_void_p]),
+    "kvae_encode_stream_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_longlong, C.c_void_p, C.c_int, C.c_longlong,
+                                          C.POINTER(C.c_longlong), C.c_void_p]),
+    "kvae_encode_stream_end": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_longlong, C.POINTER(C.c_longlong),
+                                         C.c_void_p]),
+    "kvae_encode_stream_destroy": (None, [C.c_void_p]),
     "kvae_encode_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                      C.c_float, C.c_int, C.c_longlong, C.c_void_p, C.c_size_t, C.c_void_p]),
     "kvae_plan_fused_sample_supported": (C.c_int, [C.c_void_p]),

@@ -443,7 +443,12 @@ struct WaveInParams {
   __nv_bfloat16* out_act; // [B, T, Cout] bf16 or nullptr
   const float* snake_a;   // epilogue SnakeBeta of the first ResidualUnit (or nullptr: plain cast)
   const float* snake_inv_b;
-  int T, Cout;
+  int T, Cout;            // T: output rows
+  // input geometry as in WaveOutParams (a whole clip: T_in = T, in_row0 = -3, x_pitch = T; the streaming encoder passes
+  // its sample window): output t reads samples t + in_row0 .. t + in_row0 + 6, those outside [0, T_in) are zero padding
+  int T_in, in_row0;
+  long long x_pitch;      // samples between channel rows of x
+  long long out_pitch;    // rows between clips in out_raw / out_act
 };
 
 constexpr int kWaveInTile = 64;
@@ -459,8 +464,8 @@ __global__ void __launch_bounds__(128) conv_wave_in_kernel(const WaveInParams p)
   const int co = blockIdx.y * 128 + lane * 4;
   for (int i = threadIdx.x; i < CIN * RS; i += 128) {
     const int c = i / RS, r = i % RS;
-    const int t = t0 - 3 + r;
-    xs[c][r] = (t >= 0 && t < p.T) ? ld_elem(p.x, (static_cast<size_t>(b) * CIN + c) * p.T + t, p.x_f32) : 0.f;
+    const int t = t0 + p.in_row0 + r;
+    xs[c][r] = (t >= 0 && t < p.T_in) ? ld_elem(p.x, (static_cast<size_t>(b) * CIN + c) * p.x_pitch + t, p.x_f32) : 0.f;
   }
   float w[7][CIN][4];
 #pragma unroll
@@ -489,7 +494,7 @@ __global__ void __launch_bounds__(128) conv_wave_in_kernel(const WaveInParams p)
         v0 = fmaf(xv, w[k][c][0], v0); v1 = fmaf(xv, w[k][c][1], v1);
         v2 = fmaf(xv, w[k][c][2], v2); v3 = fmaf(xv, w[k][c][3], v3);
       }
-    const size_t o = (static_cast<size_t>(b) * p.T + t) * p.Cout + co;
+    const size_t o = (static_cast<size_t>(b) * p.out_pitch + t) * p.Cout + co;
     if (p.out_raw) {
       if (p.raw_f16) {
         *reinterpret_cast<uint2*>(static_cast<__half*>(p.out_raw) + o) =
@@ -510,7 +515,7 @@ __global__ void __launch_bounds__(128) conv_wave_in_kernel(const WaveInParams p)
       }
       __nv_bfloat162 h0 = __floats2bfloat162_rn(v0, v1), h1 = __floats2bfloat162_rn(v2, v3);
       if (p.act_split) {
-        const size_t o2 = (static_cast<size_t>(b) * p.T + t) * 2 * p.Cout + co;
+        const size_t o2 = (static_cast<size_t>(b) * p.out_pitch + t) * 2 * p.Cout + co;
         const float2 f0 = __bfloat1622float2(h0), f1 = __bfloat1622float2(h1);
         __nv_bfloat162 l0 = __floats2bfloat162_rn(v0 - f0.x, v1 - f0.y), l1 = __floats2bfloat162_rn(v2 - f1.x, v3 - f1.y);
         *reinterpret_cast<uint2*>(p.out_act + o2) =
@@ -541,8 +546,10 @@ struct WaveInColParams {
   __nv_bfloat16* col;     // [B, T, 64]
   const float* w;         // [7][CIN][Cout] fp32 (folded weight-norm weights)
   __nv_bfloat16* wp;      // [Cout][64]
-  int T, B, Cout, CIN;
+  int T, B, Cout, CIN;    // T: output rows
   int row_blocks;         // blocks that write im2col rows (kColRows rows each); the rest pack weights
+  int T_in, in_row0;      // input geometry, as in WaveInParams
+  long long x_pitch;
 };
 
 constexpr int kColRows = 512;   // im2col rows per block
@@ -570,8 +577,8 @@ __global__ void __launch_bounds__(256) wave_in_im2col_kernel(const WaveInColPara
   const int b = blockIdx.x / tiles_per_clip, t0 = (blockIdx.x % tiles_per_clip) * kColRows;
   for (int i = threadIdx.x; i < (p.CIN + 1) * RS; i += 256) {
     const int c = i / RS, r = i - c * RS;
-    const int t = t0 - 3 + r;
-    xs[i] = (c < p.CIN && t >= 0 && t < p.T) ? ld_elem(p.x, (static_cast<size_t>(b) * p.CIN + c) * p.T + t, p.x_f32) : 0.f;
+    const int t = t0 + p.in_row0 + r;
+    xs[i] = (c < p.CIN && t >= 0 && t < p.T_in) ? ld_elem(p.x, (static_cast<size_t>(b) * p.CIN + c) * p.x_pitch + t, p.x_f32) : 0.f;
   }
   // two threads per row: thread h owns columns 8h .. 8h+7 of every block, i.e. 16 bytes of the hi block (written
   // twice), 16 bytes of the lo block and 16 bytes of zeros -- a lane pair writes 32 contiguous bytes per store

@@ -260,7 +260,9 @@ inline int sm_count() {
 // added to all of them), and exactly out_q output rows per phase are produced -- those whose receptive field lies
 // inside the window (or, at the end of the stream, beyond its last row, where TMA's out-of-bounds zero fill is the
 // conv's zero padding).  Output / skip pointers are passed already offset to their first row; *_pitch = rows between
-// clips in those buffers.
+// clips in those buffers.  A strided conv (the encoder's downsampling, input viewed as [T/s, s, C]) keeps its phase
+// assignment: window row 0 is an absolute input row = 0 (mod s), in_rows and in_pitch are multiples of s and row_bias
+// counts groups of s rows.
 struct StreamGeom {
   int in_rows = 0, out_q = 0, row_bias = 0;
   long long in_pitch = 0, raw_pitch = 0, act_pitch = 0, res_pitch = 0;
@@ -277,7 +279,7 @@ inline bool prepare_conv_umma2(const ConvGeom& g, const __nv_bfloat16* x, int B,
   TapPlan tp;
   if (!build_taps(g, tp, err)) return false;
   if (sg) {
-    if (tp.P_in != 1) { err = "streaming form needs a stride-1 or transposed conv"; return false; }
+    if (sg->in_rows % tp.P_in || sg->in_pitch % tp.P_in) { err = "streaming form of a strided conv needs whole phase groups"; return false; }
     T_in = sg->in_rows;
     for (Tap& t : tp.taps) t.a_row = static_cast<int16_t>(t.a_row + sg->row_bias);
   }

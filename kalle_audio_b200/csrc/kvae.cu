@@ -635,6 +635,7 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
         w.snake_inv_b = nullptr;
       }
       w.T = static_cast<int>(T_out);
+      w.T_in = w.T; w.in_row0 = -3; w.x_pitch = w.T; w.out_pitch = w.T;
       w.Cout = c.g.Cout;
       R.kind[k] = 2;
       if (head_on_tc(p, steps, train)) {
@@ -644,6 +645,7 @@ bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B
         h.w = c.w_direct;
         h.wp = c.w_head;
         h.T = static_cast<int>(T_out); h.B = B; h.Cout = c.g.Cout; h.CIN = c.g.Cin;
+        h.T_in = h.T; h.in_row0 = -3; h.x_pitch = h.T;
         h.row_blocks = B * static_cast<int>((T_out + kColRows - 1) / kColRows);
         if (!h.col || !h.wp) { err = "internal: head operand missing"; return false; }
         ConvGeom g1 = c.g;
@@ -2549,6 +2551,7 @@ int kvae_gauss_sample(const void* mean, const void* logs, const void* noise, voi
 
 // ------------------------------------------------------------------ stateful streaming decode
 int kvae_decode_stream_begin(kvae_plan* plan, int B, int max_frames, int use_graphs, kvae_stream** out) {
+  if (plan && plan->direction != KVAE_DECODER) return fail("streaming: plan is not a decoder");
   return stream_create(plan, B, max_frames, use_graphs, out);
 }
 
@@ -2568,8 +2571,8 @@ long long kvae_decode_stream_samples(kvae_stream* s, int n_frames, int end) {
   if (!s) return fail("null stream");
   if (n_frames < 0 || n_frames > s->max_frames) return fail("streaming: n_frames out of range (0 .. max_frames)");
   DeviceGuard guard(s->plan->device);
-  PreparedPush* P = stream_get(s, end ? 0 : n_frames, end != 0, KVAE_F32);
-  return P ? P->n_samples : -1;
+  PreparedPush* P = stream_get(s, end ? 0 : n_frames, end != 0, KVAE_F32, KVAE_F32);
+  return P ? P->n_out : -1;
 }
 
 long long kvae_decode_stream_lookahead(const kvae_stream* s) {
@@ -2597,6 +2600,52 @@ int kvae_decode_stream_end(kvae_stream* s, void* wav, int wav_dtype, long long w
   if (!s) return fail("null stream");
   if (!check_dtype(wav_dtype)) return fail("bad dtype");
   return stream_run(s, nullptr, KVAE_F32, 0, true, wav, wav_dtype, wav_capacity, n_samples, static_cast<cudaStream_t>(stream));
+}
+
+// ------------------------------------------------------------------ stateful streaming encode
+int kvae_encode_stream_begin(kvae_plan* plan, int B, long long max_samples, int use_graphs, kvae_stream** out) {
+  if (plan && plan->direction != KVAE_ENCODER) return fail("streaming: plan is not an encoder");
+  return stream_create(plan, B, max_samples, use_graphs, out);
+}
+
+void kvae_encode_stream_destroy(kvae_stream* s) { kvae_decode_stream_destroy(s); }
+
+long long kvae_encode_stream_frames(kvae_stream* s, long long n_samples, int end) {
+  if (!s || !s->enc) return fail("null or non-encoder stream");
+  if (n_samples < 0 || n_samples > s->max_in) return fail("streaming: n_samples out of range (0 .. max_samples)");
+  DeviceGuard guard(s->plan->device);
+  PreparedPush* P = stream_get(s, end ? 0 : static_cast<int>(n_samples), end != 0, KVAE_F32, KVAE_F32);
+  return P ? P->n_out : -1;
+}
+
+long long kvae_encode_stream_lookahead(const kvae_stream* s) {
+  if (!s || !s->enc) return fail("null or non-encoder stream");
+  // last sample frame t reads is t * ratio + reach, accumulated back to front; the lookahead is what lies beyond
+  // the frame's own last sample
+  long long reach = 0;
+  for (int k = static_cast<int>(s->ss.size()) - 1; k >= 0; --k) {
+    if (s->ss[k].kind == 5) continue;                    // the k = 1 half of a fused unit reads its own row
+    reach = reach * s->ss[k].P_in + s->ss[k].dmax;
+  }
+  return reach - (s->ratio - 1);
+}
+
+int kvae_encode_stream_push(kvae_stream* s, const void* wav, int wav_dtype, long long n_samples, void* lat, int lat_dtype,
+                            long long lat_capacity, long long* n_frames, void* stream) {
+  if (!s || !s->enc) return fail("null or non-encoder stream");
+  if (n_samples > 0 && !wav) return fail("null wav");
+  if (!check_dtype(wav_dtype) || !check_dtype(lat_dtype)) return fail("bad dtype");
+  if (!lat && lat_capacity > 0) return fail("null latents");
+  if (n_samples < 0 || n_samples > s->max_in) return fail("streaming: n_samples out of range (0 .. max_samples)");
+  return stream_run(s, wav, wav_dtype, static_cast<int>(n_samples), false, lat, lat_dtype, lat_capacity, n_frames,
+                    static_cast<cudaStream_t>(stream));
+}
+
+int kvae_encode_stream_end(kvae_stream* s, void* lat, int lat_dtype, long long lat_capacity, long long* n_frames,
+                           void* stream) {
+  if (!s || !s->enc) return fail("null or non-encoder stream");
+  if (!check_dtype(lat_dtype)) return fail("bad dtype");
+  return stream_run(s, nullptr, KVAE_F32, 0, true, lat, lat_dtype, lat_capacity, n_frames, static_cast<cudaStream_t>(stream));
 }
 
 int kvae_lm_glue_step(const void* hidden, int hidden_dtype, const float* w1, const float* b1, const float* w2,

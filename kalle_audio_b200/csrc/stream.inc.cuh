@@ -18,6 +18,15 @@
 //   * after a call the last `span` rows of every buffer move to its front (one batched copy kernel).
 // A call with the same buffer fill and frame count as an earlier one re-uses its prepared launches, and (optionally)
 // replays them as one CUDA graph: the steady state of a constant-hop stream is one graph launch per hop.
+//
+// The encoder (kvae_encode_stream_*) runs the same engine in the other direction: the input is a channels-first fp32
+// sample window [B, io, cap] (its carry: the head's 6-sample halo), the rates go down by each strided conv's stride s,
+// and the last conv writes channels-first latents into a staging buffer.  A strided conv keeps the phase assignment of
+// the batch path, which views its input as [T/s, s, C]: its window starts at an absolute row = 0 (mod s), its carry is
+// a whole number of s-row groups and its bias counts groups; it emits output q once every row q reads has arrived
+// (rows of a partly filled group feed only outputs that are not stored).  At the end of the stream the rows of the
+// last partial group past the true end are zeroed by a memset in the prepared launch list, so every layer's output
+// count follows the reference's floor arithmetic (ConvGeom::out_len).
 
 struct StreamOut {            // geometry shared by the raw (stream) and act (operand) tensors one step produces
   long long rows = 0;         // valid rows per clip currently in the buffers
@@ -27,13 +36,17 @@ struct StreamOut {            // geometry shared by the raw (stream) and act (op
   int init_rows = 0;          // zero rows at the start of a stream (the consumer's -dmin)
   size_t off_raw = 0, off_act = 0;
   int raw_row_bytes = 0, act_row_bytes = 0;   // 0: tensor not produced
+  int cf = 0;                 // > 0: channels-first fp32 [B, cf, cap] (the encoder's sample window; raw_row_bytes = 4)
 };
 
 struct StreamStep {
   int kind = -1;              // 0 tensor-core conv, 4 fused ResidualUnit (this step + next), 5 second half of a fused unit,
-                              // 6 tensor-core tail, 3 CUDA-core tail
-  int bias = 0, span = 0, dmax = 0;   // in input rows
-  int P_out = 1;
+                              // 6 tensor-core tail, 3 CUDA-core tail, 7 encoder head as im2col + k = 1 tensor-core conv,
+                              // 2 CUDA-core encoder head
+  int bias = 0;               // in input groups of P_in rows: added to every tap offset
+  int span = 0;               // last window row output 0 reads (input rows): the rows kept between calls
+  int dmax = 0;               // last input row output q reads, relative to row q * P_in
+  int P_in = 1, P_out = 1;
   int in_out = -1;            // index of the StreamOut this step reads (-1: the stream's input buffer, slot 0 of `outs`)
 };
 
@@ -49,6 +62,15 @@ __global__ void stream_carry_kernel(const StreamCarry* d, int n_desc) {
   (void)n_desc;
 }
 
+// one clip-strided 2D region: `height` rows of `width` bytes, `pitch` bytes apart
+struct StreamRegion { uint8_t* dst; const uint8_t* src; size_t width, pitch, height; };
+
+__global__ void stream_append_cf_kernel(const void* x, int x_f32, float* y, long long n, long long y_pitch) {
+  const size_t row = blockIdx.y;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n; i += static_cast<long long>(gridDim.x) * blockDim.x)
+    y[row * y_pitch + i] = ld_elem(x, row * n + i, x_f32);
+}
+
 struct PreparedPush {
   std::vector<int> launch;                 // per step: 1 = launch
   std::vector<ConvLaunch2> umma2;
@@ -56,10 +78,14 @@ struct PreparedPush {
   PreparedRun::WaveOutTc wo_tc;
   WaveOutParams wo_cc;
   int wo_cout = 0;
-  long long n_samples = 0;
-  int in_rows0 = 0;                        // row of the input buffer where the new frames go
+  WaveInColParams wi_col;                  // encoder head, kind 7 (its k = 1 conv is umma2[0])
+  WaveInParams wi_cc;                      // encoder head, kind 2
+  long long n_out = 0;                     // rows the call emits (samples / latent frames)
+  int in_rows0 = 0;                        // row of the input buffer where the new rows go
+  std::vector<StreamRegion> zero;          // end of stream: rows of a strided conv's last partial group past the end
   std::vector<StreamCarry> carry;          // non-overlapping moves (one kernel)
   std::vector<StreamCarry> carry_overlap;  // overlapping moves (through scratch)
+  std::vector<StreamRegion> carry_cf;      // the channels-first sample window (through scratch)
   StreamCarry* carry_dev = nullptr;
   std::vector<StreamOut> after;            // state after this call
   cudaGraphExec_t graph = nullptr;
@@ -74,17 +100,21 @@ struct PreparedPush {
 
 struct kvae_stream {
   kvae_plan* plan = nullptr;
+  bool enc = false;                 // encoder: samples in, latent frames out
   int B = 0, max_frames = 0;
   bool use_graphs = false;
   uint8_t* ws = nullptr;
   size_t ws_bytes = 0;
-  std::vector<StreamOut> outs;      // [0] = channels-last copy of the latent input, [1 + k] = outputs of step k
+  std::vector<StreamOut> outs;      // [0] = the input window (decoder: channels-last latents, encoder: channels-first
+                                    // samples), [1 + k] = outputs of step k
   std::vector<StreamStep> ss;
   uint8_t* z_stage = nullptr;       // [B, latent, max_frames] in the caller's dtype (4 bytes per element reserved)
-  float* wav_stage = nullptr;       // [B, io, max_samples]
+  float* wav_stage = nullptr;       // [B, io, max_samples] (the encoder's input: caller's dtype)
+  __nv_bfloat16* col = nullptr;     // encoder head on the tensor cores: im2col operand [B, rows, 64] (inside ws)
   uint8_t* scratch = nullptr;       // overlapping carry moves
   size_t scratch_bytes = 0;
   long long max_samples = 0;
+  long long max_in = 0;             // input rows one call takes (max_frames / max_samples)
   long long ratio = 1;
   bool stream_f16 = false;
   std::map<std::vector<long long>, std::unique_ptr<PreparedPush>> cache;
@@ -104,26 +134,27 @@ void stream_reset(kvae_stream* s) {
   s->samples_out = 0;
 }
 
-// per-step tap statistics of the decoder's convs (all stride-1 convs or transposed convs)
+// per-step tap statistics: input groups (of P_in rows; rows for stride-1 and transposed convs) and input rows read
 bool stream_step_geometry(const ConvGeom& g, StreamStep& st, std::string& err) {
   TapPlan tp;
   if (!build_taps(g, tp, err)) return false;
-  if (tp.P_in != 1) { err = "streaming: strided convolutions (encoders) are not supported"; return false; }
-  int dmin = 1 << 30, dmax = -(1 << 30);
+  int dmin = 1 << 30, dmax = -(1 << 30), rmax = -(1 << 30);
   for (const Tap& t : tp.taps) {
     dmin = std::min(dmin, t.a_row + t.shift);
     dmax = std::max(dmax, t.a_row + t.shift);
+    rmax = std::max(rmax, (t.a_row + t.shift) * tp.P_in + t.a_phase);
   }
   st.bias = -dmin;
-  st.dmax = dmax;
-  st.span = dmax - dmin;
+  st.dmax = rmax;
+  st.span = rmax + st.bias * tp.P_in;
+  st.P_in = tp.P_in;
   st.P_out = tp.P_out;
   if (dmin > 0 || dmax < 0) { err = "streaming: one-sided receptive field unsupported"; return false; }
   return true;
 }
 
 // Lays out one call: how many rows every step produces, the launches, the carry moves and the state afterwards.
-bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, PreparedPush& P, std::string& err) {
+bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, PreparedPush& P, std::string& err) {
   kvae_plan* p = s->plan;
   const std::vector<Step>& steps = p->steps;
   const int n = static_cast<int>(steps.size());
@@ -135,12 +166,13 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
   P.umma2.resize(n);
   P.ru.resize(n);
   P.in_rows0 = static_cast<int>(cur[0].rows);
-  cur[0].rows += n_frames;
+  cur[0].rows += n_in;
   if (cur[0].rows > cur[0].cap) { err = "streaming: input buffer overflow"; return false; }
   uint8_t* base = s->ws;
   auto raw_ptr = [&](const StreamOut& o, long long row) -> uint8_t* { return base + o.off_raw + static_cast<size_t>(row) * o.raw_row_bytes; };
   auto act_ptr = [&](const StreamOut& o, long long row) -> uint8_t* { return base + o.off_act + static_cast<size_t>(row) * o.act_row_bytes; };
-  P.n_samples = 0;
+  P.n_out = 0;
+  std::vector<long long> consumed(cur.size(), 0);   // rows of each buffer its consumer is done with after this call
   for (int k = 0; k < n; ++k) {
     const StreamStep& st = s->ss[k];
     if (st.kind == 5) continue;
@@ -150,16 +182,26 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
     const int ko = (st.kind == 4) ? k + 1 : k;              // the step whose tensors receive the result
     StreamOut& out = cur[ko + 1];
     const bool last = (ko == n - 1);
-    long long out_q = in.rows - st.span + (flush ? st.dmax : 0);
+    // every output whose input rows have all arrived; at the end of the stream, all the conv's output rows (its
+    // right zero padding lies past the window).  in.abs_base is a multiple of P_in.
+    const long long out_q = flush ? c.g.out_len(static_cast<int>(in.rows)) / st.P_out - st.bias
+                                  : (in.rows > st.span ? (in.rows - 1 - st.span) / st.P_in + 1 : 0);
     if (out_q <= 0) continue;
     const long long out_rows = out_q * st.P_out;
-    const long long out_abs = (in.abs_base + st.bias) * st.P_out;
+    const long long out_abs = (in.abs_base / st.P_in + st.bias) * st.P_out;
     if (!last) {
       if (out.abs_base + out.rows != out_abs) { err = "internal: streaming row bookkeeping at step " + std::to_string(k); return false; }
       if (out.rows + out_rows > out.cap) { err = "streaming: window buffer overflow at step " + std::to_string(k); return false; }
     }
     StreamGeom sg;
-    sg.in_rows = static_cast<int>(in.rows);
+    sg.in_rows = static_cast<int>((in.rows + st.P_in - 1) / st.P_in * st.P_in);   // whole phase groups
+    if (sg.in_rows > in.cap) { err = "internal: strided window exceeds its buffer"; return false; }
+    if (flush && sg.in_rows > in.rows) {
+      // rows of the last partial group past the end of the stream are the conv's zero padding
+      if (!in.act_row_bytes) { err = "internal: strided conv without operand tensor"; return false; }
+      P.zero.push_back({act_ptr(in, in.rows), nullptr, static_cast<size_t>(sg.in_rows - in.rows) * in.act_row_bytes,
+                        static_cast<size_t>(in.cap) * in.act_row_bytes, static_cast<size_t>(B)});
+    }
     sg.out_q = static_cast<int>(out_q);
     sg.row_bias = st.bias;
     sg.in_pitch = in.cap;
@@ -191,6 +233,47 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
       ra.act_f16 = s1.act_f16 ? 1 : 0;
       if (s1.epi_snake >= 0) { ra.sn_a = p->snakes[s1.epi_snake].a; ra.sn_inv_b = p->snakes[s1.epi_snake].inv_b; }
       if (!prepare_conv_ru(ra, B, 0, c.g.dilation, P.ru[k], err, &sg)) return false;
+    } else if (st.kind == 7 || st.kind == 2) {
+      // encoder head: reads the channels-first sample window, output q reads window samples q .. q + 6
+      const int io = c.g.Cin;
+      const float* snake_a = sp.epi_snake >= 0 ? p->snakes[sp.epi_snake].a : nullptr;
+      const float* snake_inv_b = sp.epi_snake >= 0 ? p->snakes[sp.epi_snake].inv_b : nullptr;
+      void* o_raw = out.raw_row_bytes ? raw_ptr(out, out.rows) : nullptr;
+      __nv_bfloat16* o_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
+      if (st.kind == 7) {
+        WaveInColParams& h = P.wi_col;
+        std::memset(&h, 0, sizeof(h));
+        h.x = raw_ptr(in, 0); h.x_f32 = 1;
+        h.col = s->col; h.w = c.w_direct; h.wp = c.w_head;
+        h.T = static_cast<int>(out_rows); h.B = B; h.Cout = c.g.Cout; h.CIN = io;
+        h.row_blocks = B * ((h.T + kColRows - 1) / kColRows);
+        h.T_in = static_cast<int>(in.rows); h.in_row0 = 0; h.x_pitch = in.cap;
+        if (out_rows > in.cap) { err = "internal: head operand overflow"; return false; }
+        ConvGeom g1 = c.g;
+        g1.Cin = 64; g1.K = 1; g1.pad = 0; g1.dilation = 1; g1.stride = 1;
+        ConvEpilogue ep;
+        ep.bias = c.bias;
+        ep.stream_f16 = 1;
+        ep.out_raw = o_raw;
+        ep.out_act = o_act;
+        ep.snake_a = snake_a; ep.snake_inv_b = snake_inv_b;
+        StreamGeom sg1;
+        sg1.in_rows = h.T; sg1.out_q = h.T; sg1.in_pitch = h.T; sg1.raw_pitch = out.cap; sg1.act_pitch = out.cap;
+        ConvTuning2 tune;
+        if (!prepare_conv_umma2(g1, s->col, B, 0, c.w_head, ep, tune, P.umma2[k], err, &sg1)) return false;
+      } else {
+        WaveInParams& w = P.wi_cc;
+        std::memset(&w, 0, sizeof(w));
+        w.x = raw_ptr(in, 0); w.x_f32 = 1;
+        w.w = c.w_direct; w.bias = c.bias;
+        w.out_raw = o_raw; w.raw_f16 = sf16;
+        w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
+        w.act_split = (o_act && p->precision == KVAE_PREC_F32) ? 1 : 0;
+        w.out_act = o_act;
+        w.snake_a = snake_a; w.snake_inv_b = snake_inv_b;
+        w.T = static_cast<int>(out_rows); w.Cout = c.g.Cout;
+        w.T_in = static_cast<int>(in.rows); w.in_row0 = 0; w.x_pitch = in.cap; w.out_pitch = out.cap;
+      }
     } else if (st.kind == 6 || st.kind == 3) {
       // decoder tail: reads the stream (raw) tensor of the previous step, writes the staging waveform [B, io, out_rows]
       const bool preact = p->tail_preact && st.kind == 6;    // the last unit wrote SnakeBeta(x) in fp16 (kvae.cu, finalize_steps)
@@ -220,7 +303,7 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
         w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
         w.T_in = static_cast<int>(in.rows); w.in_row0 = 0; w.x_pitch = in.cap;
       }
-      P.n_samples = out_rows;
+      P.n_out = out_rows;
     } else {
       ConvEpilogue ep;
       ep.bias = c.has_bias ? c.bias : nullptr;
@@ -232,12 +315,22 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
       ep.out_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
       if (sp.epi_snake >= 0) { ep.snake_a = p->snakes[sp.epi_snake].a; ep.snake_inv_b = p->snakes[sp.epi_snake].inv_b; }
       if (!c.umma) { ep.split3 = 1; ep.act_split = 1; ep.precise = 1; }
+      if (last) {
+        // encoder output conv: channels-first latents into the staging buffer, in the caller's dtype
+        if (out_rows > s->max_frames) { err = "streaming: latent staging overflow"; return false; }
+        ep.out_raw = s->z_stage;
+        ep.out_raw_cf = 1;
+        ep.out_raw_f32 = (out_dtype == KVAE_F32) ? 1 : 0;
+        P.n_out = out_rows;
+      }
       ConvTuning2 tune;
       if (!prepare_conv_umma2(c.g, reinterpret_cast<const __nv_bfloat16*>(act_ptr(in, 0)), B, 0, c.w_umma, ep, tune,
                               P.umma2[k], err, &sg))
         return false;
+      if (last) P.umma2[k].p.cf_ld = s->max_frames;
     }
     P.launch[k] = 1;
+    consumed[st.in_out + 1] = out_q * st.P_in;
     if (!last) out.rows += out_rows;
     (void)split;
   }
@@ -245,9 +338,13 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
   for (size_t j = 0; j < cur.size(); ++j) {
     StreamOut& o = cur[j];
     if (!o.cap) continue;
-    const long long keep = flush ? 0 : std::min<long long>(o.rows, o.keep);
+    const long long keep = flush ? 0 : o.rows - consumed[j];
     const long long drop = o.rows - keep;
-    if (drop > 0 && keep > 0) {
+    if (drop > 0 && keep > 0 && o.cf) {
+      uint8_t* b0 = base + o.off_raw;
+      P.carry_cf.push_back({b0, b0 + static_cast<size_t>(drop) * 4, static_cast<size_t>(keep) * 4, static_cast<size_t>(o.cap) * 4,
+                            static_cast<size_t>(B) * o.cf});
+    } else if (drop > 0 && keep > 0) {
       for (int which = 0; which < 2; ++which) {
         const int rb = which ? o.act_row_bytes : o.raw_row_bytes;
         if (!rb) continue;
@@ -263,6 +360,8 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
   }
   for (const StreamCarry& c : P.carry_overlap)
     if (c.bytes * static_cast<size_t>(B) > s->scratch_bytes) { err = "internal: carry scratch too small"; return false; }
+  for (const StreamRegion& c : P.carry_cf)
+    if (c.width * c.height > s->scratch_bytes) { err = "internal: carry scratch too small"; return false; }
   if (!P.carry.empty()) {
     if (cudaMalloc(&P.carry_dev, P.carry.size() * sizeof(StreamCarry)) != cudaSuccess) { err = "cudaMalloc(carry table) failed"; return false; }
     if (cudaMemcpy(P.carry_dev, P.carry.data(), P.carry.size() * sizeof(StreamCarry), cudaMemcpyHostToDevice) != cudaSuccess) {
@@ -271,7 +370,6 @@ bool stream_prepare(kvae_stream* s, int n_frames, bool flush, int z_dtype, Prepa
     }
   }
   P.after = cur;
-  (void)z_dtype;
   return true;
 }
 
@@ -279,7 +377,20 @@ cudaError_t stream_launch_all(kvae_stream* s, PreparedPush& P, int n_frames, int
   kvae_plan* p = s->plan;
   const int n = static_cast<int>(p->steps.size());
   const ConvLayer& c0 = p->convs[p->steps[0].conv];
-  if (n_frames > 0) {
+  for (const StreamRegion& z : P.zero) {
+    cudaError_t e = cudaMemset2DAsync(z.dst, z.pitch, 0, z.width, z.height, st);
+    if (e != cudaSuccess) return e;
+  }
+  if (n_frames > 0 && s->enc) {
+    // [B, io, n] staging (caller's dtype) -> fp32 rows appended to the sample window
+    const StreamOut& o = s->outs[0];
+    dim3 grid(std::min(ceil_div(n_frames, 256), 16), s->B * o.cf);
+    stream_append_cf_kernel<<<grid, 256, 0, st>>>(s->wav_stage, z_f32, reinterpret_cast<float*>(s->ws + o.off_raw) + P.in_rows0,
+                                                  n_frames, o.cap);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    ++g_launches;
+  } else if (n_frames > 0) {
     // [B, D, n_frames] (staging) -> channels-last rows appended to the input window
     const StreamOut& o = s->outs[0];
     dim3 grid(ceil_div(n_frames, 32), ceil_div(c0.g.Cin, 32), s->B), block(32, 8);
@@ -313,6 +424,15 @@ cudaError_t stream_launch_all(kvae_stream* s, PreparedPush& P, int n_frames, int
       else e = launch_pdl(conv_wave_out_tc_kernel<false>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<false>(), st, P.wo_tc.tmX, P.wo_tc.p);
     } else if (kind == 3) {
       e = launch_wave_out(P.wo_cc, P.wo_cout, s->B, st);
+    } else if (kind == 7) {
+      const WaveInColParams& h = P.wi_col;
+      wave_in_im2col_kernel<<<h.row_blocks + (h.Cout * 64 + 255) / 256, 256, 0, st>>>(h);
+      e = cudaGetLastError();
+      if (e != cudaSuccess) return e;
+      ++g_launches;
+      e = launch_conv_umma2(P.umma2[k], st);
+    } else if (kind == 2) {
+      e = launch_wave_in(P.wi_cc, p->convs[p->steps[k].conv].g.Cin, s->B, st);
     }
     if (e != cudaSuccess) return e;
     ++g_launches;
@@ -331,28 +451,36 @@ cudaError_t stream_launch_all(kvae_stream* s, PreparedPush& P, int n_frames, int
     if (e == cudaSuccess) e = cudaMemcpy2DAsync(c.dst, c.pitch, s->scratch, c.bytes, c.bytes, s->B, cudaMemcpyDeviceToDevice, st);
     if (e != cudaSuccess) return e;
   }
+  for (const StreamRegion& c : P.carry_cf) {               // a few samples per channel row: through scratch
+    cudaError_t e = cudaMemcpy2DAsync(s->scratch, c.width, c.src, c.pitch, c.width, c.height, cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpy2DAsync(c.dst, c.pitch, s->scratch, c.width, c.width, c.height, cudaMemcpyDeviceToDevice, st);
+    if (e != cudaSuccess) return e;
+  }
   return cudaSuccess;
 }
 
 void stream_zero_initial_rows(kvae_stream* s, cudaStream_t st);
 
-PreparedPush* stream_get(kvae_stream* s, int n_frames, bool flush, int z_dtype) {
+// out_dtype: the encoder's latent dtype (its output conv writes it); the decoder converts its fp32 staging instead
+PreparedPush* stream_get(kvae_stream* s, int n_frames, bool flush, int z_dtype, int out_dtype) {
   std::vector<long long> key;
   key.push_back(n_frames); key.push_back(flush ? 1 : 0); key.push_back(z_dtype);
+  if (s->enc) key.push_back(out_dtype);
   for (const StreamOut& o : s->outs) key.push_back(o.rows);
   auto it = s->cache.find(key);
   if (it == s->cache.end()) {
     auto P = std::make_unique<PreparedPush>();
     std::string err;
-    if (!stream_prepare(s, n_frames, flush, z_dtype, *P, err)) { fail(err); return nullptr; }
+    if (!stream_prepare(s, n_frames, flush, out_dtype, *P, err)) { fail(err); return nullptr; }
     if (s->cache.size() > 64) s->cache.clear();
     it = s->cache.emplace(key, std::move(P)).first;
   }
   return it->second.get();
 }
 
-int stream_run(kvae_stream* s, const void* z, int z_dtype, int n_frames, bool flush, void* wav, int wav_dtype,
-               long long wav_capacity, long long* n_samples, cudaStream_t st) {
+// in: [B, C_in, n_in] (decoder: latents, encoder: samples); out: [B, C_out, *n_out] (decoder: samples, encoder: frames)
+int stream_run(kvae_stream* s, const void* in, int in_dtype, int n_in, bool flush, void* out, int out_dtype,
+               long long out_capacity, long long* n_out, cudaStream_t st) {
   kvae_plan* p = s->plan;
   for (const ConvLayer& c : p->convs)
     if (!c.set) return fail("plan weights not set (kvae_plan_set_conv / kvae_plan_load_params)");
@@ -360,31 +488,37 @@ int stream_run(kvae_stream* s, const void* z, int z_dtype, int n_frames, bool fl
     if (!sn.set) return fail("plan SnakeBeta parameters not set");
   DeviceGuard guard(p->device);
   if (!guard.ok) return fail("cannot select device");
-  if (n_frames < 0 || n_frames > s->max_frames) return fail("streaming: n_frames out of range (0 .. max_frames)");
-  PreparedPush* Pp = stream_get(s, n_frames, flush, z_dtype);
+  if (n_in < 0 || n_in > s->max_in)
+    return fail(s->enc ? "streaming: n_samples out of range (0 .. max_samples)" : "streaming: n_frames out of range (0 .. max_frames)");
+  PreparedPush* Pp = stream_get(s, n_in, flush, in_dtype, out_dtype);
   if (!Pp) return -1;
   PreparedPush& P = *Pp;
   if (s->needs_zero) {
     stream_zero_initial_rows(s, st);
     s->needs_zero = false;
   }
-  if (P.n_samples > wav_capacity) return fail("wav buffer too small for this call (kvae_decode_stream_samples tells the size)");
+  if (P.n_out > out_capacity)
+    return fail(s->enc ? "latent buffer too small for this call (kvae_encode_stream_frames tells the size)"
+                       : "wav buffer too small for this call (kvae_decode_stream_samples tells the size)");
   const int io = p->arch.io_channels;
-  if (n_frames > 0) {
-    const size_t zb = static_cast<size_t>(s->B) * p->arch.latent_dim * n_frames * (z_dtype == KVAE_F32 ? 4 : 2);
-    KV_CUDA(cudaMemcpyAsync(s->z_stage, z, zb, cudaMemcpyDeviceToDevice, st));
-  }
+  const int D = p->arch.latent_dim;
+  const size_t ies = in_dtype == KVAE_F32 ? 4 : 2, oes = out_dtype == KVAE_F32 ? 4 : 2;
+  if (n_in > 0)
+    KV_CUDA(cudaMemcpyAsync(s->enc ? static_cast<void*>(s->wav_stage) : static_cast<void*>(s->z_stage), in,
+                            static_cast<size_t>(s->B) * (s->enc ? io : D) * n_in * ies, cudaMemcpyDeviceToDevice, st));
   if (s->use_graphs) {
     if (!P.graph) {
       // the first call with this geometry runs eagerly (sets kernel attributes, fills caches), the second is captured
       // (captured on a stream of our own: the caller's may be the legacy default stream, which cannot capture)
       cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
       if (st) KV_CUDA(cudaStreamIsCapturing(st, &cs));
-      if (cs == cudaStreamCaptureStatusNone && P.eager_done && P.carry_overlap.empty()) {
+      // (the encoder's short pushes move overlapping carries at every deep stage: 2D copies through scratch, which a
+      // graph captures like any other copy; the decoder stream runs such calls eagerly, as it always has)
+      if (cs == cudaStreamCaptureStatusNone && P.eager_done && (s->enc || P.carry_overlap.empty())) {
         if (!s->cap_stream) KV_CUDA(cudaStreamCreateWithFlags(&s->cap_stream, cudaStreamNonBlocking));
         cudaGraph_t g = nullptr;
         KV_CUDA(cudaStreamBeginCapture(s->cap_stream, cudaStreamCaptureModeThreadLocal));
-        cudaError_t e = stream_launch_all(s, P, n_frames, z_dtype == KVAE_F32, s->cap_stream);
+        cudaError_t e = stream_launch_all(s, P, n_in, in_dtype == KVAE_F32, s->cap_stream);
         cudaError_t e2 = cudaStreamEndCapture(s->cap_stream, &g);
         if (e != cudaSuccess) { if (g) cudaGraphDestroy(g); return cuda_fail(e, "stream capture"); }
         KV_CUDA(e2);
@@ -396,28 +530,32 @@ int stream_run(kvae_stream* s, const void* z, int z_dtype, int n_frames, bool fl
     if (P.graph) {
       KV_CUDA(cudaGraphLaunch(P.graph, st));
     } else {
-      KV_CUDA(stream_launch_all(s, P, n_frames, z_dtype == KVAE_F32, st));
+      KV_CUDA(stream_launch_all(s, P, n_in, in_dtype == KVAE_F32, st));
       P.eager_done = true;
     }
   } else {
-    KV_CUDA(stream_launch_all(s, P, n_frames, z_dtype == KVAE_F32, st));
+    KV_CUDA(stream_launch_all(s, P, n_in, in_dtype == KVAE_F32, st));
   }
-  if (P.n_samples > 0) {
+  if (P.n_out > 0 && s->enc) {
+    // staging [B, D, max_frames] (already in the caller's dtype) -> the caller's buffer [B, D, n]
+    KV_CUDA(cudaMemcpy2DAsync(out, P.n_out * oes, s->z_stage, static_cast<size_t>(s->max_frames) * oes, P.n_out * oes,
+                              static_cast<size_t>(s->B) * D, cudaMemcpyDeviceToDevice, st));
+  } else if (P.n_out > 0) {
     // staging [B, io, n] fp32 -> the caller's buffer [B, io, n] (dtype conversion included)
-    const size_t cnt = static_cast<size_t>(s->B) * io * P.n_samples;
-    if (wav_dtype == KVAE_F32) {
-      KV_CUDA(cudaMemcpyAsync(wav, s->wav_stage, cnt * 4, cudaMemcpyDeviceToDevice, st));
+    const size_t cnt = static_cast<size_t>(s->B) * io * P.n_out;
+    if (out_dtype == KVAE_F32) {
+      KV_CUDA(cudaMemcpyAsync(out, s->wav_stage, cnt * 4, cudaMemcpyDeviceToDevice, st));
     } else {
       const int blocks = static_cast<int>(std::min<size_t>((cnt + 255) / 256, 148 * 8));
-      f32_to_bf16_kernel<<<blocks, 256, 0, st>>>(s->wav_stage, static_cast<__nv_bfloat16*>(wav), cnt);
+      f32_to_bf16_kernel<<<blocks, 256, 0, st>>>(s->wav_stage, static_cast<__nv_bfloat16*>(out), cnt);
       KV_CUDA(cudaGetLastError());
       ++g_launches;
     }
   }
   s->outs = P.after;
-  s->frames_in += n_frames;
-  s->samples_out += P.n_samples;
-  if (n_samples) *n_samples = P.n_samples;
+  s->frames_in += n_in;
+  s->samples_out += P.n_out;
+  if (n_out) *n_out = P.n_out;
   if (flush) {
     stream_reset(s);
     s->needs_zero = true;
@@ -425,25 +563,35 @@ int stream_run(kvae_stream* s, const void* z, int z_dtype, int n_frames, bool fl
   return 0;
 }
 
-// decides which kernels serve the steps and sizes the persistent window buffers
-int stream_create(kvae_plan* p, int B, int max_frames, int use_graphs, kvae_stream** out) {
+// decides which kernels serve the steps and sizes the persistent window buffers; max_in: input rows one call takes
+// (decoder: latent frames, encoder: samples)
+int stream_create(kvae_plan* p, int B, long long max_in, int use_graphs, kvae_stream** out) {
   if (!p || !out) return fail("null argument");
-  if (p->direction != KVAE_DECODER) return fail("streaming: plan is not a decoder");
-  if (B <= 0 || max_frames <= 0) return fail("streaming: bad batch / max_frames");
+  const bool enc = p->direction == KVAE_ENCODER;
+  if (B <= 0 || max_in <= 0) return fail(enc ? "streaming: bad batch / max_samples" : "streaming: bad batch / max_frames");
+  if (max_in > (1 << 26)) return fail("streaming: too many input rows per call");
   DeviceGuard guard(p->device);
   if (!guard.ok) return fail("cannot select device");
   const std::vector<Step>& steps = p->steps;
   const int n = static_cast<int>(steps.size());
   auto s = std::make_unique<kvae_stream>();
-  s->plan = p; s->B = B; s->max_frames = max_frames; s->use_graphs = use_graphs != 0;
+  s->plan = p; s->enc = enc; s->B = B; s->max_in = max_in; s->use_graphs = use_graphs != 0;
   s->stream_f16 = p->stream_f16;
   s->ratio = p->ratio;
+  // output staging: decoder samples, encoder latent frames (the stream's lag is far below 24 frames)
+  if (enc) {
+    s->max_samples = max_in;
+    s->max_frames = static_cast<int>((max_in + 24 * p->ratio) / p->ratio + 1);
+  } else {
+    s->max_frames = static_cast<int>(max_in);
+    s->max_samples = static_cast<long long>(max_in + 24) * p->ratio;
+  }
   s->ss.resize(n);
   s->outs.assign(n + 1, StreamOut());
   std::string err;
   const int split = (p->precision == KVAE_PREC_F32) ? 2 : 1;
   const ConvLayer& c0 = p->convs[steps[0].conv];
-  if (!conv_tc(c0, false)) return fail("streaming: needs a tensor-core first layer (latent_dim and channels multiples of 64)");
+  if (!enc && !conv_tc(c0, false)) return fail("streaming: needs a tensor-core first layer (latent_dim and channels multiples of 64)");
   // step kinds and geometry
   for (int k = 0; k < n; ++k) {
     const Step& sp = steps[k];
@@ -453,16 +601,18 @@ int stream_create(kvae_plan* p, int B, int max_frames, int use_graphs, kvae_stre
     if (sp.fuse == 2) { st.kind = 5; continue; }
     if (!stream_step_geometry(c.g, st, err)) return fail(err);
     if (sp.fuse == 1) st.kind = 4;
-    else if (is_wave_out_step(p, steps, k)) st.kind = (p->precision == KVAE_PREC_BF16 && s->stream_f16) ? 6 : 3;
+    else if (!enc && is_wave_out_step(p, steps, k)) st.kind = (p->precision == KVAE_PREC_BF16 && s->stream_f16) ? 6 : 3;
+    else if (enc && k == 0 && is_wave_in_step(p, steps, k)) st.kind = head_on_tc(p, steps, false) ? 7 : 2;
     else if (conv_tc(c, false)) st.kind = 0;
     else return fail("streaming: step " + std::to_string(k) + " has no tensor-core kernel (channels must be multiples of 64; "
                      "the 128-channel tail is required)");
     if (st.kind == 3 && (c.g.Cin != 128)) return fail("streaming: CUDA-core tail needs 128 input channels");
-    if (k == n - 1 && st.kind == 0) return fail("streaming: tensor-core output conv unsupported");
+    if (!enc && k == n - 1 && st.kind == 0) return fail("streaming: tensor-core output conv unsupported");
   }
-  // rate of every tensor relative to the latent frame rate, keep / init rows from the consumer
+  // rate of every tensor relative to the input rate, keep / init rows from the consumer
   std::vector<double> rates(n + 1, 1.0);
-  for (int k = 0; k < n; ++k) rates[k + 1] = static_cast<double>(step_len(steps[k], 1000)) / 1000.0;
+  for (int k = 0; k < n; ++k) rates[k + 1] = static_cast<double>(steps[k].len_num) / steps[k].len_den;
+  const long long in_slack = enc ? 24 * p->ratio : 24;
   size_t off = 0;
   auto consumer_of = [&](int j) -> int {   // first step that reads StreamOut j (j = -1: the input)
     for (int k = j + 1; k < n; ++k)
@@ -477,11 +627,20 @@ int stream_create(kvae_plan* p, int B, int max_frames, int use_graphs, kvae_stre
     if (j >= 0 && s->ss[j].kind == 4) continue;          // the k7 half of a fused unit produces no tensor
     const int cons = consumer_of(j);
     if (cons < 0) return fail("internal: streaming tensor without consumer");
-    o.keep = s->ss[cons].span;
-    o.init_rows = s->ss[cons].bias;
+    const StreamStep& cs = s->ss[cons];
+    o.keep = cs.span;
+    o.init_rows = cs.bias * cs.P_in;
     const double r = rates[j + 1];
-    o.cap = static_cast<long long>(std::ceil(r * (max_frames + 24))) + o.keep + 64;
-    o.cap = (o.cap + 7) / 8 * 8;
+    o.cap = static_cast<long long>(std::ceil(r * (max_in + in_slack))) + o.keep + 64;
+    o.cap = (o.cap + 8 * cs.P_in - 1) / (8 * cs.P_in) * (8 * cs.P_in);   // whole phase groups of a strided consumer
+    if (enc && j < 0) {
+      // channels-first fp32 sample window [B, io, cap]
+      o.cf = c0.g.Cin;
+      o.raw_row_bytes = 4;
+      o.off_raw = off;
+      off += align_up(static_cast<size_t>(B) * o.cf * o.cap * 4, 1024);
+      continue;
+    }
     const int C = (j < 0) ? c0.g.Cin : p->convs[steps[j].conv].g.Cout;
     const bool needs_raw = j >= 0 && steps[j].needs_raw;
     const bool needs_act = j < 0 || steps[j].needs_act;
@@ -496,15 +655,20 @@ int stream_create(kvae_plan* p, int B, int max_frames, int use_graphs, kvae_stre
       off += align_up(static_cast<size_t>(B) * o.cap * o.act_row_bytes, 1024);
     }
   }
+  size_t off_col = 0;
+  if (enc && s->ss[0].kind == 7) {                       // im2col operand of the head: at most a window of rows
+    off_col = off;
+    off += align_up(static_cast<size_t>(B) * s->outs[0].cap * 64 * 2, 1024);
+  }
   s->ws_bytes = std::max<size_t>(off, 1024);
-  s->max_samples = static_cast<long long>(max_frames + 24) * p->ratio;
   size_t max_carry = 1024;
   for (const StreamOut& o : s->outs)
-    max_carry = std::max<size_t>(max_carry, static_cast<size_t>(o.keep) * std::max(o.raw_row_bytes, o.act_row_bytes));
+    max_carry = std::max<size_t>(max_carry, static_cast<size_t>(o.keep) * std::max(o.raw_row_bytes, o.act_row_bytes) * std::max(o.cf, 1));
   s->scratch_bytes = max_carry * B;
   KV_CUDA(cudaMalloc(&s->ws, s->ws_bytes));
   KV_CUDA(cudaMemset(s->ws, 0, s->ws_bytes));            // the initial carry rows are zeros (conv left padding)
-  KV_CUDA(cudaMalloc(&s->z_stage, static_cast<size_t>(B) * p->arch.latent_dim * max_frames * 4));
+  if (off_col) s->col = reinterpret_cast<__nv_bfloat16*>(s->ws + off_col);
+  KV_CUDA(cudaMalloc(&s->z_stage, static_cast<size_t>(B) * p->arch.latent_dim * s->max_frames * 4));
   KV_CUDA(cudaMalloc(&s->wav_stage, static_cast<size_t>(B) * p->arch.io_channels * s->max_samples * 4));
   KV_CUDA(cudaMalloc(&s->scratch, s->scratch_bytes));
   stream_reset(s.get());
@@ -517,7 +681,8 @@ void stream_zero_initial_rows(kvae_stream* s, cudaStream_t st) {
   for (const StreamOut& o : s->outs) {
     if (!o.cap || !o.init_rows) continue;
     if (o.raw_row_bytes)
-      cudaMemset2DAsync(s->ws + o.off_raw, static_cast<size_t>(o.cap) * o.raw_row_bytes, 0, static_cast<size_t>(o.init_rows) * o.raw_row_bytes, s->B, st);
+      cudaMemset2DAsync(s->ws + o.off_raw, static_cast<size_t>(o.cap) * o.raw_row_bytes, 0, static_cast<size_t>(o.init_rows) * o.raw_row_bytes,
+                        static_cast<size_t>(s->B) * std::max(o.cf, 1), st);
     if (o.act_row_bytes)
       cudaMemset2DAsync(s->ws + o.off_act, static_cast<size_t>(o.cap) * o.act_row_bytes, 0, static_cast<size_t>(o.init_rows) * o.act_row_bytes, s->B, st);
   }

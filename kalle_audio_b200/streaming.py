@@ -1,4 +1,4 @@
-"""Incremental latent -> waveform decoding.
+"""Incremental latent -> waveform decoding, and incremental waveform -> latent encoding (``StreamingEncoder``).
 
 Two engines behind one class:
 
@@ -49,6 +49,123 @@ def decoder_context_frames(strides: Sequence[int]) -> Tuple[int, int]:
         hi = (hi + p) // s
     lo, hi = lo - 3, hi + 3                  # first conv
     return f0 - lo, hi - (f1 - 1)
+
+
+def encoder_context_samples(strides: Sequence[int]) -> Tuple[int, int]:
+    """(left, right) input samples an OobleckEncoder latent frame depends on beyond its own ``ratio`` samples.
+
+    Walks the stack backwards with interval arithmetic (autoencoders.py:64-81, 130-141): final conv k3 pad 1; per
+    EncoderBlock, in reverse, the strided Conv1d(k = 2s, stride s, pad ceil(s / 2)) and three ResidualUnits (k7,
+    dilation 9 / 3 / 1: 39 rows each way at that block's rate); head conv k7 pad 3.  ``strides`` in constructor order."""
+    ratio = int(math.prod(strides))
+    f0 = 1000                                # one frame far from the edges
+    lo, hi = f0 - 1, f0 + 1                  # final conv
+    for s in reversed(strides):
+        p = math.ceil(s / 2)
+        lo, hi = lo * s - p, hi * s + 2 * s - 1 - p   # output t reads rows t*s - p .. t*s + 2s - 1 - p
+        lo, hi = lo - 39, hi + 39            # ResidualUnits: 3 * (1 + 3 + 9)
+    lo, hi = lo - 3, hi + 3                  # head conv
+    return f0 * ratio - lo, hi - ((f0 + 1) * ratio - 1)
+
+
+class StreamingEncoder:
+    """Feed audio as it arrives; get latent frames back as soon as they are final.
+
+        se = StreamingEncoder(autoencoder.encoder)
+        for x in audio_chunks:               # x: [B, io_channels, n], any n >= 0
+            z = se.push(x)                   # [B, latent_dim, m], m = frames that became final (possibly 0)
+        tail = se.flush()                    # the last frames (right edge zero-padded like the whole-clip encode)
+
+    ``torch.cat`` of everything returned equals ``encoder(torch.cat(audio_chunks, -1))`` bit for bit when the total
+    length is a multiple of ``ratio``; otherwise it is the ``kvae_plan_out_length(L)`` frames the reference's floor
+    arithmetic gives (``encoder(x, valid_len=...)``).  Every layer keeps the tail of its own input inside libkvae
+    (``kvae_encode_stream_*``), so no sample is encoded twice; a frame comes out once ``lookahead`` samples past its
+    last sample have arrived.  Needs an encoder whose every layer has a tensor-core kernel (channels and latent_dim
+    multiples of 64, a 128-channel head): other architectures raise ``KvaeError`` on the first push."""
+
+    def __init__(self, encoder, max_samples: Optional[int] = None, use_cuda_graphs: bool = True):
+        """``max_samples``: the longest push the stream takes in one library call (longer pushes are split)."""
+        if not hasattr(encoder, "_arch") or encoder._direction != _lib.KVAE_ENCODER:
+            raise TypeError("StreamingEncoder wraps a kalle_audio_b200.OobleckEncoder")
+        self.encoder = encoder
+        strides = [encoder._arch.strides[i] for i in range(encoder._arch.n_stages)]
+        self.ratio = int(math.prod(strides))
+        self.max_samples = int(max_samples or max(65536, 4 * self.ratio))
+        if self.max_samples < 1:
+            raise ValueError("max_samples must be >= 1")
+        self._use_graphs = bool(use_cuda_graphs)
+        self._native = None            # (handle, finalizer, runner, batch) once the first push fixes device and batch
+        self._last_dtype = None
+        self.lookahead: Optional[int] = None   # samples; set by the library when the first push starts the stream
+
+    def reset(self) -> None:
+        """Drops the stream and its state; the next push starts a new one."""
+        if self._native is not None:
+            self._native[1]()
+            self._native = None
+
+    def _stream(self, audio: torch.Tensor):
+        import ctypes as C
+        import weakref
+        if self._native is not None:
+            if self._native[3] != audio.shape[0]:
+                raise ValueError("batch size changed inside a stream")
+            return self._native
+        L = _lib.lib()
+        r = self.encoder.runner(audio.device)
+        r.sync_weights()
+        h = C.c_void_p()
+        _lib.check(L.kvae_encode_stream_begin(r.handle, audio.shape[0], self.max_samples, int(self._use_graphs),
+                                              C.byref(h)))
+        fin = weakref.finalize(self, L.kvae_encode_stream_destroy, h)
+        self._native = (h, fin, r, audio.shape[0])
+        self.lookahead = int(L.kvae_encode_stream_lookahead(h))
+        return self._native
+
+    def _call(self, x: Optional[torch.Tensor], end: bool) -> torch.Tensor:
+        import ctypes as C
+        L = _lib.lib()
+        h, _, r, B = self._native
+        r.sync_weights()
+        dev = r.device
+        out_dt = self.encoder._out_dtype(x) if x is not None else self._last_dtype
+        self._last_dtype = out_dt
+        kdt = out_dt if out_dt in (torch.float32, torch.bfloat16) else torch.float32
+        n = 0 if x is None else x.shape[2]
+        nf = int(L.kvae_encode_stream_frames(h, n, int(end)))
+        if nf < 0:
+            raise _lib.KvaeError(L.kvae_last_error().decode())
+        lat = torch.empty((B, self.encoder._out_channels_for_plan, nf), dtype=kdt, device=dev)
+        got = C.c_longlong(0)
+        if end:
+            _lib.check(L.kvae_encode_stream_end(h, lat.data_ptr(), _lib.dtype_code(kdt), nf, C.byref(got),
+                                                _lib.stream_ptr(dev)))
+        else:
+            xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
+            xin = xin.contiguous()
+            _lib.check(L.kvae_encode_stream_push(h, xin.data_ptr(), _lib.dtype_code(xin.dtype), n, lat.data_ptr(),
+                                                 _lib.dtype_code(kdt), nf, C.byref(got), _lib.stream_ptr(dev)))
+        assert got.value == nf
+        return lat if lat.dtype == out_dt else lat.to(out_dt)
+
+    def push(self, audio: torch.Tensor) -> torch.Tensor:
+        """audio [B, io_channels, n] -> the latent frames [B, latent_dim, m] that became final."""
+        _lib.require_cuda(audio, "StreamingEncoder.push")
+        if audio.dim() != 3:
+            raise ValueError("expected [B, C, n]")
+        self._stream(audio)
+        pieces = [self._call(audio[:, :, i:i + self.max_samples], False)
+                  for i in range(0, audio.shape[2], self.max_samples)]
+        if not pieces:
+            return audio.new_zeros((audio.shape[0], self.encoder._out_channels_for_plan, 0),
+                                   dtype=self.encoder._out_dtype(audio))
+        return pieces[0] if len(pieces) == 1 else torch.cat(pieces, dim=2)
+
+    def flush(self) -> torch.Tensor:
+        """Everything not yet emitted (end of stream).  The stream starts over with the next push."""
+        if self._native is None:
+            raise ValueError("nothing was pushed")
+        return self._call(None, True)
 
 
 class StreamingDecoder:
