@@ -133,31 +133,48 @@ struct Layout {
   size_t total = 0;
 };
 
+// The kernel that serves one step of a plan (step_kind); the whole-clip run and the stream both launch these.
+enum StepKind {
+  kTcConv,      // tensor-core conv (conv_umma2.cuh)
+  kDirect,      // CUDA-core conv (conv_direct.cuh)
+  kWaveIn,      // encoder head on the CUDA cores (conv_edge.cuh)
+  kWaveOut,     // decoder tail on the CUDA cores
+  kRuFused,     // fused ResidualUnit (conv_ru2.cuh): this step and the next
+  kRuSecond,    // the k = 1 half of a fused unit: computed by the previous step's launch
+  kWaveOutTc,   // decoder tail on the tensor cores (TF32, or fp16 with the fp16 stream)
+  kWaveInTc,    // encoder head as im2col + a k = 1 tensor-core conv
+};
+
+struct DirectLaunch {             // conv_direct_kernel: parameters, tile configuration (direct_cfg_for), grid, smem
+  DirectParams d;
+  dim3 grid;
+  int cfg = 0;
+  size_t smem = 0;
+};
+
+// what one step needs at launch time; only the members of its kind are filled
+struct StepLaunch {
+  StepKind kind = kTcConv;
+  int k = 0;                      // index of the step
+  ConvLaunch2 umma2;              // kTcConv, and the k = 1 conv of kWaveInTc
+  RuLaunch ru;                    // kRuFused
+  WaveInParams wave_in;           // kWaveIn
+  WaveInColParams head_col;       // kWaveInTc: im2col + weight pack in front of the k = 1 conv
+  WaveOutParams wave_out;         // kWaveOut
+  CUtensorMap wo_tmX;             // kWaveOutTc
+  WaveOutTcParams wave_out_tc;
+  DirectLaunch direct;            // kDirect
+};
+
 struct PreparedRun {
-  std::vector<ConvLaunch2> umma2;   // per step (valid when that step is tensor-core)
-  std::vector<DirectParams> direct; // per step (valid otherwise)
-  std::vector<dim3> direct_grid;
-  std::vector<int> direct_cfg;      // 0: 32x64 tile, 1: 128x4 tile
-  std::vector<size_t> direct_smem;
-  std::vector<int> kind;            // per step: 0 tensor-core, 1 generic, 2 waveform-in, 3 waveform-out,
-                                    //           4 fused ResidualUnit (this step + the next), 5 done by the previous step, 6 tensor-core tail,
-                                    //           7 encoder head as im2col + k = 1 tensor-core conv
-  std::vector<RuLaunch> ru;
-  std::vector<WaveInParams> wave_in;
-  WaveInColParams head_col;         // kind 7: im2col + weight pack in front of the head conv on the tensor cores
-  std::vector<WaveOutParams> wave_out;
-  struct WaveOutTc { CUtensorMap tmX; WaveOutTcParams p; };
-  std::vector<WaveOutTc> wave_out_tc;   // kind 6: decoder tail on the tensor cores (TF32, or fp16 with the fp16 stream)
+  std::vector<StepLaunch> steps;    // one per step of the plan
   bool stream_f16 = false;
   Layout layout;
   // ---- training runs only: the backward pass over the saved activations
   struct Bwd {
     int dgrad_kind = 0;             // 0 none, 1 tensor-core (conv_umma2 under the dgrad geometry), 2 CUDA-core
     ConvLaunch2 dg_umma;
-    DirectParams dg_direct;
-    dim3 dg_grid;
-    int dg_cfg = 0;
-    size_t dg_smem = 0;
+    DirectLaunch dg_direct;
     int wg_kind = 0;                // 0 CUDA-core (torch-layout atomics), 1 tensor-core (packed accumulator),
                                     // 2 waveform-edge streaming kernel
     EdgeWgradParams wg_edge;
@@ -226,8 +243,6 @@ namespace {
 
 int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
-int direct_cfg_for(int Cout);
-void direct_tile(int cfg, int& BT, int& BN);
 bool env_flag(const char* name) {
   const char* e = getenv(name);
   return e && e[0] == '1';
@@ -365,6 +380,15 @@ bool is_wave_in_step(const kvae_plan* p, const std::vector<Step>& steps, int k) 
 bool head_on_tc(const kvae_plan* p, const std::vector<Step>& steps, bool train) {
   return !train && p->precision == KVAE_PREC_BF16 && p->stream_f16 && is_wave_in_step(p, steps, 0) &&
          p->convs[steps[0].conv].g.Cin <= 2 && !env_flag("KVAE_WAVE_IN_CC");
+}
+StepKind step_kind(const kvae_plan* p, const std::vector<Step>& steps, int k, bool train) {
+  const Step& s = steps[k];
+  if (s.fuse == 2) return kRuSecond;
+  if (s.fuse == 1) return kRuFused;
+  // fp32 mode keeps the tail's exact fp32 FMAs
+  if (is_wave_out_step(p, steps, k)) return p->precision == KVAE_PREC_BF16 ? kWaveOutTc : kWaveOut;
+  if (is_wave_in_step(p, steps, k)) return head_on_tc(p, steps, train) ? kWaveInTc : kWaveIn;
+  return conv_tc(p->convs[s.conv], train) ? kTcConv : kDirect;
 }
 void finalize_steps(kvae_plan* p) {
   const int n = static_cast<int>(p->steps.size());
@@ -529,233 +553,41 @@ bool make_layout(const kvae_plan* p, const std::vector<Step>& steps, bool train,
   return true;
 }
 
-bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B, long long T, void* ws,
-                 PreparedRun& R, std::string& err) {
-  const int n = static_cast<int>(steps.size());
-  if (!make_layout(p, steps, train, B, T, R.layout, err)) return false;
-  R.umma2.resize(n);
-  R.ru.resize(n);
-  R.direct.resize(n);
-  R.direct_grid.resize(n);
-  R.direct_cfg.assign(n, 0);
-  R.direct_smem.assign(n, 0);
-  R.kind.assign(n, 1);
-  R.stream_f16 = train ? p->train_stream_f16 : p->stream_f16;
-  const int sf16 = R.stream_f16 ? 1 : 0;
-  R.wave_in.resize(n);
-  R.wave_out.resize(n);
-  R.wave_out_tc.resize(n);
-  uint8_t* base = static_cast<uint8_t*>(ws);
-  auto tptr = [&](int id) -> void* { return R.layout.t[id].bytes ? base + R.layout.t[id].offset : nullptr; };
-  for (int k = 0; k < n; ++k) {
-    const Step& s = steps[k];
-    const ConvLayer& c = p->convs[s.conv];
-    const long long T_in = (k == 0) ? T : step_len(steps[k - 1], T);
-    const long long T_out = step_len(s, T);
-    if (c.g.out_len(static_cast<int>(T_in)) != T_out) {
-      err = "length bookkeeping mismatch at step " + std::to_string(k) + " (input length must be a multiple of the stride product)";
-      return false;
-    }
-    const bool last = (k == n - 1);
-    void* raw = (s.needs_raw && !last) ? tptr(1 + 2 * k) : nullptr;
-    void* act = s.needs_act ? tptr(2 + 2 * k) : nullptr;
-    const void* res = (s.residual_from >= 0) ? tptr(1 + 2 * s.residual_from) : nullptr;
-    if (s.residual_from >= 0 && !res) { err = "internal: residual tensor missing"; return false; }
-    if (s.fuse == 2) { R.kind[k] = 5; continue; }
-    if (s.fuse == 1) {
-      const Step& s1 = steps[k + 1];
-      const ConvLayer& c1 = p->convs[s1.conv];
-      RuArgs ra;
-      ra.a = static_cast<const __nv_bfloat16*>(tptr(2 + 2 * (k - 1)));
-      ra.x = tptr(1 + 2 * (k - 1));
-      ra.stream_f16 = sf16;
-      ra.w7 = c.w_umma;
-      ra.w1 = c1.w_umma;
-      ra.bias7 = c.bias;
-      ra.s2_a = p->snakes[s.epi_snake].a;
-      ra.s2_inv_b = p->snakes[s.epi_snake].inv_b;
-      ra.bias1 = c1.bias;
-      ra.out_raw = s1.needs_raw ? tptr(1 + 2 * (k + 1)) : nullptr;
-      ra.out_act = s1.needs_act ? static_cast<__nv_bfloat16*>(tptr(2 + 2 * (k + 1))) : nullptr;
-      ra.act_f16 = s1.act_f16 ? 1 : 0;
-      if (s1.epi_snake >= 0) {
-        ra.sn_a = p->snakes[s1.epi_snake].a;
-        ra.sn_inv_b = p->snakes[s1.epi_snake].inv_b;
-      }
-      if (!prepare_conv_ru(ra, B, static_cast<int>(T_out), c.g.dilation, R.ru[k], err)) return false;
-      R.kind[k] = 4;
-      continue;
-    }
-    if (is_wave_out_step(p, steps, k)) {
-      // decoder tail (conv_edge.cuh)
-      WaveOutParams& w = R.wave_out[k];
-      const bool preact = p->tail_preact && !train;
-      w.x = static_cast<const float*>(preact ? tptr(2 + 2 * (k - 1)) : tptr(1 + 2 * (k - 1)));
-      if (!w.x) { err = "internal: raw input missing"; return false; }
-      w.pro_a = p->snakes[s.pre_snake].a;
-      w.pro_inv_b = p->snakes[s.pre_snake].inv_b;
-      w.w = c.w_direct;
-      w.y = nullptr;  // patched per call
-      w.T = static_cast<int>(T_out);
-      w.T_in = w.T; w.in_row0 = -3; w.x_pitch = w.T;
-      w.Cin = c.g.Cin;
-      w.tanh_out = (p->direction == KVAE_DECODER && p->arch.final_tanh) ? 1 : 0;
-      w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
-      R.kind[k] = 3;
-      if (p->precision == KVAE_PREC_BF16) {   // fp32 mode keeps the exact fp32 FMAs
-        PreparedRun::WaveOutTc& t = R.wave_out_tc[k];
-        std::memset(&t.p, 0, sizeof(t.p));
-        t.p.pro_a = w.pro_a; t.p.pro_inv_b = w.pro_inv_b; t.p.w = w.w;
-        t.p.T = w.T; t.p.B = B; t.p.COUT = c.g.Cout; t.p.tanh_out = w.tanh_out; t.p.in_row0 = -3;
-        t.p.preact = preact ? 1 : 0;
-        t.p.tiles_per_clip = (w.T + kWoTcTile - 1) / kWoTcTile;
-        t.p.total_tiles = t.p.tiles_per_clip * B;
-        if (sf16) { if (!make_act_tmap(&t.tmX, w.x, B, w.T, 128, 1, kWoTcRows, err)) return false; }
-        else if (!make_out_tmap(&t.tmX, w.x, B, w.T, 128, 1, 1, err, kWoTcRows)) return false;
-        R.kind[k] = 6;
-      }
-      continue;
-    }
-    if (is_wave_in_step(p, steps, k)) {
-      // encoder head (conv_edge.cuh)
-      WaveInParams& w = R.wave_in[k];
-      w.x = nullptr;  // patched per call
-      w.w = c.w_direct;
-      w.bias = c.bias;
-      w.out_raw = raw;
-      w.raw_f16 = sf16;
-      w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
-      w.act_split = (act && p->precision == KVAE_PREC_F32 && !train) ? 1 : 0;
-      w.out_act = static_cast<__nv_bfloat16*>(act);
-      if (s.epi_snake >= 0) {
-        w.snake_a = p->snakes[s.epi_snake].a;
-        w.snake_inv_b = p->snakes[s.epi_snake].inv_b;
-      } else {
-        w.snake_a = nullptr;
-        w.snake_inv_b = nullptr;
-      }
-      w.T = static_cast<int>(T_out);
-      w.T_in = w.T; w.in_row0 = -3; w.x_pitch = w.T; w.out_pitch = w.T;
-      w.Cout = c.g.Cout;
-      R.kind[k] = 2;
-      if (head_on_tc(p, steps, train)) {
-        WaveInColParams& h = R.head_col;
-        h.x = nullptr;  // patched per call
-        h.col = static_cast<__nv_bfloat16*>(tptr(0));
-        h.w = c.w_direct;
-        h.wp = c.w_head;
-        h.T = static_cast<int>(T_out); h.B = B; h.Cout = c.g.Cout; h.CIN = c.g.Cin;
-        h.T_in = h.T; h.in_row0 = -3; h.x_pitch = h.T;
-        h.row_blocks = B * static_cast<int>((T_out + kColRows - 1) / kColRows);
-        if (!h.col || !h.wp) { err = "internal: head operand missing"; return false; }
-        ConvGeom g1 = c.g;
-        g1.Cin = 64; g1.K = 1; g1.pad = 0; g1.dilation = 1; g1.stride = 1;
-        ConvEpilogue ep;
-        ep.bias = c.bias;
-        ep.stream_f16 = 1;
-        ep.out_raw = raw;
-        ep.out_act = static_cast<__nv_bfloat16*>(act);
-        ep.snake_a = w.snake_a;
-        ep.snake_inv_b = w.snake_inv_b;
-        ConvTuning2 tune;
-        if (!prepare_conv_umma2(g1, h.col, B, static_cast<int>(T_out), c.w_head, ep, tune, R.umma2[k], err)) return false;
-        R.kind[k] = 7;
-      }
-      continue;
-    }
-    if (conv_tc(c, train)) {
-      R.kind[k] = 0;
-      const void* in = (k == 0) ? tptr(0) : tptr(2 + 2 * (k - 1));
-      if (!in) { err = "internal: tensor-core operand missing"; return false; }
-      ConvEpilogue ep;
-      ep.bias = c.has_bias ? c.bias : nullptr;
-      ep.residual = res;
-      ep.residual_f32 = sf16 ? 0 : 1;
-      ep.stream_f16 = sf16;
-      ep.out_raw = raw;            // external output patched at call time when last
-      ep.out_raw_f32 = (sf16 && !last) ? 0 : 1;
-      ep.out_raw_cf = last ? 1 : 0;
-      if (last) ep.out_raw = reinterpret_cast<void*>(0x1);  // placeholder, patched per call
-      ep.out_act = static_cast<__nv_bfloat16*>(act);
-      if (s.epi_snake >= 0) {
-        ep.snake_a = p->snakes[s.epi_snake].a;
-        ep.snake_inv_b = p->snakes[s.epi_snake].inv_b;
-      }
-      if (!c.umma) {               // fp32 mode on the tensor cores: bf16x3 split operands, sinf in the epilogue
-        ep.split3 = 1;
-        ep.act_split = 1;
-        ep.precise = 1;
-      }
-      ConvTuning2 tune;
-      if (!prepare_conv_umma2(c.g, static_cast<const __nv_bfloat16*>(in), B, static_cast<int>(T_in), c.w_umma, ep,
-                              tune, R.umma2[k], err))
-        return false;
-    } else {
-      DirectParams& d = R.direct[k];
-      std::memset(&d, 0, sizeof(d));
-      TapPlan tp;
-      if (!build_taps(c.g, tp, err)) return false;
-      d.B = B;
-      d.P_out = tp.P_out;
-      d.P_in = tp.P_in;
-      d.Tq_out = static_cast<int>((T_out + tp.P_out - 1) / tp.P_out);
-      d.T_out = static_cast<int>(T_out);
-      d.T_in = static_cast<int>(T_in);
-      d.Cin = c.g.Cin;
-      d.Cout = c.g.Cout;
-      d.span = tp.span;
-      for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
-      for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
-      if (k == 0) {  // external input, API layout [B, C, T]; pointer / dtype patched per call
-        d.x = nullptr;
-        d.x_sB = static_cast<long long>(c.g.Cin) * T_in;
-        d.x_sT = 1;
-        d.x_sC = T_in;
-      } else {
-        const Step& prev = steps[k - 1];
-        d.x = tptr(1 + 2 * (k - 1));
-        if (!prev.needs_raw || !d.x) { err = "internal: raw input missing"; return false; }
-        d.x_f32 = 1;
-        d.x_sB = T_in * c.g.Cin;
-        d.x_sT = c.g.Cin;
-        d.x_sC = 1;
-      }
-      if (s.pre_snake >= 0) {
-        d.pro_a = p->snakes[s.pre_snake].a;
-        d.pro_inv_b = p->snakes[s.pre_snake].inv_b;
-      }
-      d.w = c.w_direct;
-      d.bias = c.has_bias ? c.bias : nullptr;
-      d.residual = res;
-      d.residual_f32 = 1;
-      if (last) {  // external output, API layout; pointer / dtype patched per call
-        d.out_raw = nullptr;
-        d.o_sB = static_cast<long long>(c.g.Cout) * T_out;
-        d.o_sT = 1;
-        d.o_sC = T_out;
-        d.tanh_out = (p->direction == KVAE_DECODER && p->arch.final_tanh) ? 1 : 0;
-      } else {
-        d.out_raw = raw;
-        d.out_raw_f32 = 1;
-        d.o_sB = T_out * c.g.Cout;
-        d.o_sT = c.g.Cout;
-        d.o_sC = 1;
-      }
-      d.out_act = static_cast<__nv_bfloat16*>(act);
-      d.act_split = (act && p->precision == KVAE_PREC_F32 && !train) ? 1 : 0;
-      if (s.epi_snake >= 0) {
-        d.snake_a = p->snakes[s.epi_snake].a;
-        d.snake_inv_b = p->snakes[s.epi_snake].inv_b;
-      }
-      const int cfg = direct_cfg_for(c.g.Cout);
-      int BT, BN;
-      direct_tile(cfg, BT, BN);
-      R.direct_cfg[k] = cfg;
-      R.direct_grid[k] = dim3(ceil_div(d.Tq_out, BT) * tp.P_out, ceil_div(c.g.Cout, BN), B);
-      R.direct_smem[k] = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
-    }
-  }
+// CUDA-core conv tile (time rows x out-channels per 128-thread block) by output width: the 64-wide tile left 50-75 % of
+// the threads without a channel on the 32- and 16-channel stages of BigVGANFlowVAE.  The per-output summation order does
+// not depend on the tile, so every configuration gives the same bits.
+int direct_cfg_for(int Cout) { return Cout <= 4 ? 1 : Cout <= 16 ? 2 : Cout <= 32 ? 3 : 0; }
+void direct_tile(int cfg, int& BT, int& BN) {
+  BT = cfg == 1 ? 128 : cfg == 2 ? 128 : cfg == 3 ? 64 : 32;
+  BN = cfg == 1 ? 4 : cfg == 2 ? 16 : cfg == 3 ? 32 : 64;
+}
+// conv_direct_kernel for output rows [t_lo, T_out) of the conv of a T_in-row input: taps, geometry, tile, grid and
+// shared memory.  Operands, strides and epilogue are zero; the caller fills them.
+bool prepare_direct(const ConvGeom& g, int B, long long T_in, long long T_out, long long t_lo, DirectLaunch& L,
+                    std::string& err) {
+  TapPlan tp;
+  if (!build_taps(g, tp, err)) return false;
+  DirectParams& d = L.d;
+  std::memset(&d, 0, sizeof(d));
+  d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
+  d.Tq_out = static_cast<int>((T_out + tp.P_out - 1) / tp.P_out); d.T_out = static_cast<int>(T_out);
+  d.q_base = static_cast<int>(t_lo / tp.P_out); d.t_lo = static_cast<int>(t_lo);
+  d.T_in = static_cast<int>(T_in); d.Cin = g.Cin; d.Cout = g.Cout; d.span = tp.span;
+  for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
+  for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+  L.cfg = direct_cfg_for(g.Cout);
+  int BT, BN;
+  direct_tile(L.cfg, BT, BN);
+  L.grid = dim3(ceil_div(d.Tq_out - d.q_base, BT) * tp.P_out, ceil_div(g.Cout, BN), B);
+  L.smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
   return true;
+}
+cudaError_t launch_direct(const DirectLaunch& L, cudaStream_t st) {
+  if (L.cfg == 1) conv_direct_kernel<128, 4, 1, 4><<<L.grid, 128, L.smem, st>>>(L.d);
+  else if (L.cfg == 2) conv_direct_kernel<128, 16, 4, 4><<<L.grid, 128, L.smem, st>>>(L.d);
+  else if (L.cfg == 3) conv_direct_kernel<64, 32, 4, 4><<<L.grid, 128, L.smem, st>>>(L.d);
+  else conv_direct_kernel<32, 64, 4, 4><<<L.grid, 128, L.smem, st>>>(L.d);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_wave_out(WaveOutParams& w, int Cout, int B, cudaStream_t st) {
@@ -779,6 +611,21 @@ cudaError_t launch_wave_out(WaveOutParams& w, int Cout, int B, cudaStream_t st) 
   return cudaGetLastError();
 }
 
+cudaError_t launch_wave_out_tc(const CUtensorMap& tmX, const WaveOutTcParams& t, bool stream_f16, cudaStream_t st) {
+  static bool attr_set[64] = {false};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (!attr_set[dev & 63]) {
+    cudaError_t e = cudaFuncSetAttribute(conv_wave_out_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_wave_out_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e != cudaSuccess) return e;
+    attr_set[dev & 63] = true;
+  }
+  const int grid = std::min(t.total_tiles, sm_count());
+  if (stream_f16) return launch_pdl(conv_wave_out_tc_kernel<true>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<true>(), st, tmX, t);
+  return launch_pdl(conv_wave_out_tc_kernel<false>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<false>(), st, tmX, t);
+}
+
 cudaError_t launch_wave_in(const WaveInParams& w, int Cin, int B, cudaStream_t st) {
   dim3 grid((w.T + kWaveInTile - 1) / kWaveInTile, w.Cout / 128, B);
   if (Cin == 1) conv_wave_in_kernel<1><<<grid, 128, 0, st>>>(w);
@@ -786,20 +633,242 @@ cudaError_t launch_wave_in(const WaveInParams& w, int Cin, int B, cudaStream_t s
   return cudaGetLastError();
 }
 
-// CUDA-core conv tile (time rows x out-channels per 128-thread block) by output width: the 64-wide tile left 50-75 % of
-// the threads without a channel on the 32- and 16-channel stages of BigVGANFlowVAE.  The per-output summation order does
-// not depend on the tile, so every configuration gives the same bits.
-int direct_cfg_for(int Cout) { return Cout <= 4 ? 1 : Cout <= 16 ? 2 : Cout <= 32 ? 3 : 0; }
-void direct_tile(int cfg, int& BT, int& BN) {
-  BT = cfg == 1 ? 128 : cfg == 2 ? 128 : cfg == 3 ? 64 : 32;
-  BN = cfg == 1 ? 4 : cfg == 2 ? 16 : cfg == 3 ? 32 : 64;
+// Where one step reads and writes.  The whole-clip run points into its workspace (a padded clip: in_row0 = -3, the
+// caller's input and output are patched in per call); the stream points into its window buffers (in_row0 = 0, and a
+// StreamGeom for the tensor-core kernels, which also carries the output and skip pitches).
+struct StepIO {
+  const void* in_act = nullptr;       // bf16 operand of the input
+  const void* in_raw = nullptr;       // stream tensor of the input (the head: the channels-first samples)
+  long long in_rows = 0, in_pitch = 0;
+  int in_row0 = 0;                    // edge kernels: input row of output 0's first tap
+  long long out_rows = 0, out_pitch = 0;
+  void* out_raw = nullptr;            // stream tensor of the output
+  __nv_bfloat16* out_act = nullptr;   // operand tensor of the output
+  const void* res = nullptr;          // skip connection, row-aligned with the output
+  void* ext = nullptr;                // last step: the caller's (or the staging) output, channels-first
+  int ext_f32 = 1;
+  long long cf_ld = 0;                // its rows per channel (0: out_rows)
+  __nv_bfloat16* col = nullptr;       // im2col operand of the head on the tensor cores
+  const StreamGeom* sg = nullptr;
+};
+
+// Prepares the launch of step k (kRuFused: k and k + 1, whose tensors io describes) for the whole-clip run and the
+// stream alike.
+bool prepare_step(const kvae_plan* p, const std::vector<Step>& steps, int k, bool train, int B, const StepIO& io,
+                  StepLaunch& L, std::string& err) {
+  const Step& s = steps[k];
+  const ConvLayer& c = p->convs[s.conv];
+  const bool last = k == static_cast<int>(steps.size()) - 1;
+  const int sf16 = (train ? p->train_stream_f16 : p->stream_f16) ? 1 : 0;
+  const int precise = p->precision == KVAE_PREC_F32 ? 1 : 0;
+  const int T_in = static_cast<int>(io.in_rows), T_out = static_cast<int>(io.out_rows);
+  const float* snake_a = s.epi_snake >= 0 ? p->snakes[s.epi_snake].a : nullptr;
+  const float* snake_inv_b = s.epi_snake >= 0 ? p->snakes[s.epi_snake].inv_b : nullptr;
+  L.kind = step_kind(p, steps, k, train);
+  L.k = k;
+  switch (L.kind) {
+    case kRuSecond:
+      return true;
+    case kRuFused: {
+      const Step& s1 = steps[k + 1];
+      const ConvLayer& c1 = p->convs[s1.conv];
+      RuArgs ra;
+      ra.a = static_cast<const __nv_bfloat16*>(io.in_act);
+      ra.x = io.res;
+      ra.stream_f16 = sf16;
+      ra.w7 = c.w_umma; ra.w1 = c1.w_umma;
+      ra.bias7 = c.bias; ra.bias1 = c1.bias;
+      ra.s2_a = snake_a; ra.s2_inv_b = snake_inv_b;
+      ra.out_raw = io.out_raw;
+      ra.out_act = io.out_act;
+      ra.act_f16 = s1.act_f16 ? 1 : 0;
+      if (s1.epi_snake >= 0) { ra.sn_a = p->snakes[s1.epi_snake].a; ra.sn_inv_b = p->snakes[s1.epi_snake].inv_b; }
+      return prepare_conv_ru(ra, B, T_out, c.g.dilation, L.ru, err, io.sg);
+    }
+    case kWaveOut:
+    case kWaveOutTc: {
+      // decoder tail (conv_edge.cuh): reads the stream tensor of the previous step, or its operand tensor when the
+      // last unit wrote SnakeBeta(x) in fp16 (finalize_steps, tail_preact)
+      const bool preact = p->tail_preact && !train;
+      const void* x = preact ? io.in_act : io.in_raw;
+      if (!x) { err = "internal: raw input missing"; return false; }
+      const int tanh_out = (p->direction == KVAE_DECODER && p->arch.final_tanh) ? 1 : 0;
+      const SnakeLayer& sn = p->snakes[s.pre_snake];
+      if (L.kind == kWaveOut) {
+        WaveOutParams& w = L.wave_out;
+        std::memset(&w, 0, sizeof(w));
+        w.x = static_cast<const float*>(x);
+        w.pro_a = sn.a; w.pro_inv_b = sn.inv_b; w.w = c.w_direct;
+        w.y = io.ext; w.y_f32 = io.ext_f32;
+        w.T = T_out; w.Cin = c.g.Cin; w.tanh_out = tanh_out; w.precise = precise;
+        w.T_in = T_in; w.in_row0 = io.in_row0; w.x_pitch = io.in_pitch;
+        return true;
+      }
+      WaveOutTcParams& t = L.wave_out_tc;
+      std::memset(&t, 0, sizeof(t));
+      t.pro_a = sn.a; t.pro_inv_b = sn.inv_b; t.w = c.w_direct;
+      t.y = io.ext; t.y_f32 = io.ext_f32;
+      t.T = T_out; t.B = B; t.COUT = c.g.Cout; t.tanh_out = tanh_out; t.in_row0 = io.in_row0;
+      t.preact = preact ? 1 : 0;
+      t.tiles_per_clip = (t.T + kWoTcTile - 1) / kWoTcTile;
+      t.total_tiles = t.tiles_per_clip * B;
+      if (sf16) return make_act_tmap(&L.wo_tmX, x, B, T_in, 128, 1, kWoTcRows, err, io.in_pitch);
+      return make_out_tmap(&L.wo_tmX, x, B, T_in, 128, 1, 1, err, kWoTcRows, io.in_pitch);
+    }
+    case kWaveIn: {
+      // encoder head (conv_edge.cuh): reads the channels-first samples
+      WaveInParams& w = L.wave_in;
+      std::memset(&w, 0, sizeof(w));
+      w.x = io.in_raw; w.x_f32 = 1;
+      w.w = c.w_direct; w.bias = c.bias;
+      w.out_raw = io.out_raw; w.raw_f16 = sf16;
+      w.precise = precise;
+      w.act_split = (io.out_act && precise && !train) ? 1 : 0;
+      w.out_act = io.out_act;
+      w.snake_a = snake_a; w.snake_inv_b = snake_inv_b;
+      w.T = T_out; w.Cout = c.g.Cout;
+      w.T_in = T_in; w.in_row0 = io.in_row0; w.x_pitch = io.in_pitch; w.out_pitch = io.out_pitch;
+      return true;
+    }
+    case kWaveInTc: {
+      WaveInColParams& h = L.head_col;
+      std::memset(&h, 0, sizeof(h));
+      h.x = io.in_raw; h.x_f32 = 1;
+      h.col = io.col; h.w = c.w_direct; h.wp = c.w_head;
+      h.T = T_out; h.B = B; h.Cout = c.g.Cout; h.CIN = c.g.Cin;
+      h.T_in = T_in; h.in_row0 = io.in_row0; h.x_pitch = io.in_pitch;
+      h.row_blocks = B * ((T_out + kColRows - 1) / kColRows);
+      if (!h.col || !h.wp) { err = "internal: head operand missing"; return false; }
+      ConvGeom g1 = c.g;
+      g1.Cin = 64; g1.K = 1; g1.pad = 0; g1.dilation = 1; g1.stride = 1;
+      ConvEpilogue ep;
+      ep.bias = c.bias;
+      ep.stream_f16 = 1;
+      ep.out_raw = io.out_raw;
+      ep.out_act = io.out_act;
+      ep.snake_a = snake_a; ep.snake_inv_b = snake_inv_b;
+      StreamGeom sg1;   // window form: the k = 1 conv reads all T_out rows of the im2col operand
+      if (io.sg) { sg1.in_rows = sg1.out_q = T_out; sg1.in_pitch = T_out; sg1.raw_pitch = io.sg->raw_pitch; sg1.act_pitch = io.sg->act_pitch; }
+      return prepare_conv_umma2(g1, h.col, B, T_out, c.w_head, ep, ConvTuning2(), L.umma2, err, io.sg ? &sg1 : nullptr);
+    }
+    case kTcConv: {
+      if (!io.in_act) { err = "internal: tensor-core operand missing"; return false; }
+      ConvEpilogue ep;
+      ep.bias = c.has_bias ? c.bias : nullptr;
+      ep.residual = io.res;
+      ep.residual_f32 = sf16 ? 0 : 1;
+      ep.stream_f16 = sf16;
+      ep.out_raw = last ? io.ext : io.out_raw;
+      ep.out_raw_f32 = last ? io.ext_f32 : (sf16 ? 0 : 1);
+      ep.out_raw_cf = last ? 1 : 0;
+      ep.out_act = io.out_act;
+      ep.snake_a = snake_a; ep.snake_inv_b = snake_inv_b;
+      if (!c.umma) {               // fp32 mode on the tensor cores: bf16x3 split operands, sinf in the epilogue
+        ep.split3 = 1;
+        ep.act_split = 1;
+        ep.precise = 1;
+      }
+      if (!prepare_conv_umma2(c.g, static_cast<const __nv_bfloat16*>(io.in_act), B, T_in, c.w_umma, ep, ConvTuning2(),
+                              L.umma2, err, io.sg))
+        return false;
+      if (last) L.umma2.p.cf_ld = io.cf_ld;
+      return true;
+    }
+    case kDirect: {
+      // the first step reads the caller's input [B, C, T], the last writes the caller's output; the rest of the chain
+      // is channels-last fp32
+      if (!prepare_direct(c.g, B, T_in, T_out, 0, L.direct, err)) return false;
+      DirectParams& d = L.direct.d;
+      d.x = io.in_raw; d.x_f32 = 1;
+      if (k == 0) {
+        d.x_sB = static_cast<long long>(c.g.Cin) * io.in_pitch; d.x_sT = 1; d.x_sC = io.in_pitch;
+      } else {
+        if (!d.x) { err = "internal: raw input missing"; return false; }
+        d.x_sB = io.in_pitch * c.g.Cin; d.x_sT = c.g.Cin; d.x_sC = 1;
+      }
+      if (s.pre_snake >= 0) { d.pro_a = p->snakes[s.pre_snake].a; d.pro_inv_b = p->snakes[s.pre_snake].inv_b; }
+      d.w = c.w_direct;
+      d.bias = c.has_bias ? c.bias : nullptr;
+      d.residual = io.res;
+      d.residual_f32 = 1;
+      if (last) {
+        d.out_raw = io.ext; d.out_raw_f32 = io.ext_f32;
+        d.o_sB = static_cast<long long>(c.g.Cout) * io.out_pitch; d.o_sT = 1; d.o_sC = io.out_pitch;
+        d.tanh_out = (p->direction == KVAE_DECODER && p->arch.final_tanh) ? 1 : 0;
+      } else {
+        d.out_raw = io.out_raw; d.out_raw_f32 = 1;
+        d.o_sB = io.out_pitch * c.g.Cout; d.o_sT = c.g.Cout; d.o_sC = 1;
+      }
+      d.out_act = io.out_act;
+      d.act_split = (io.out_act && precise && !train) ? 1 : 0;
+      d.snake_a = snake_a; d.snake_inv_b = snake_inv_b;
+      return true;
+    }
+  }
+  err = "internal: unknown step kind";
+  return false;
 }
-cudaError_t launch_direct(const DirectParams& d, dim3 grid, int cfg, size_t smem, cudaStream_t st) {
-  if (cfg == 1) conv_direct_kernel<128, 4, 1, 4><<<grid, 128, smem, st>>>(d);
-  else if (cfg == 2) conv_direct_kernel<128, 16, 4, 4><<<grid, 128, smem, st>>>(d);
-  else if (cfg == 3) conv_direct_kernel<64, 32, 4, 4><<<grid, 128, smem, st>>>(d);
-  else conv_direct_kernel<32, 64, 4, 4><<<grid, 128, smem, st>>>(d);
-  return cudaGetLastError();
+
+// One step's kernels on stream st; g is the step's conv.  Counts every launch in g_launches.
+cudaError_t launch_step(StepLaunch& L, const ConvGeom& g, int B, bool stream_f16, cudaStream_t st) {
+  cudaError_t e = cudaSuccess;
+  switch (L.kind) {
+    case kRuSecond: return cudaSuccess;
+    case kRuFused: e = launch_conv_ru(L.ru, st); break;
+    case kTcConv: e = launch_conv_umma2(L.umma2, st); break;
+    case kWaveOutTc: e = launch_wave_out_tc(L.wo_tmX, L.wave_out_tc, stream_f16, st); break;
+    case kWaveOut: e = launch_wave_out(L.wave_out, g.Cout, B, st); break;
+    case kWaveIn: e = launch_wave_in(L.wave_in, g.Cin, B, st); break;
+    case kDirect: e = launch_direct(L.direct, st); break;
+    case kWaveInTc: {
+      const WaveInColParams& h = L.head_col;
+      wave_in_im2col_kernel<<<h.row_blocks + (h.Cout * 64 + 255) / 256, 256, 0, st>>>(h);
+      e = cudaGetLastError();
+      if (e != cudaSuccess) return e;
+      ++g_launches;
+      e = launch_conv_umma2(L.umma2, st);
+      break;
+    }
+  }
+  if (e == cudaSuccess) ++g_launches;
+  return e;
+}
+
+bool prepare_run(kvae_plan* p, const std::vector<Step>& steps, bool train, int B, long long T, void* ws,
+                 PreparedRun& R, std::string& err) {
+  const int n = static_cast<int>(steps.size());
+  if (!make_layout(p, steps, train, B, T, R.layout, err)) return false;
+  R.steps.assign(n, StepLaunch());
+  R.stream_f16 = train ? p->train_stream_f16 : p->stream_f16;
+  uint8_t* base = static_cast<uint8_t*>(ws);
+  auto tptr = [&](int id) -> void* { return R.layout.t[id].bytes ? base + R.layout.t[id].offset : nullptr; };
+  for (int k = 0; k < n; ++k) {
+    const Step& s = steps[k];
+    const ConvLayer& c = p->convs[s.conv];
+    const long long T_in = (k == 0) ? T : step_len(steps[k - 1], T);
+    const long long T_out = step_len(s, T);
+    if (c.g.out_len(static_cast<int>(T_in)) != T_out) {
+      err = "length bookkeeping mismatch at step " + std::to_string(k) + " (input length must be a multiple of the stride product)";
+      return false;
+    }
+    const int ko = (s.fuse == 1) ? k + 1 : k;    // the step whose tensors receive the result
+    const Step& so = steps[ko];
+    // tensor 0: the channels-last copy of the input for a tensor-core first layer, or the head's im2col operand
+    StepIO io;
+    io.in_act = tptr(k == 0 ? 0 : 2 + 2 * (k - 1));
+    io.in_raw = (k == 0) ? nullptr : tptr(1 + 2 * (k - 1));   // k == 0: the caller's input, patched per call
+    io.in_rows = io.in_pitch = T_in;
+    io.in_row0 = -3;
+    io.out_rows = io.out_pitch = T_out;
+    io.out_raw = (so.needs_raw && ko != n - 1) ? tptr(1 + 2 * ko) : nullptr;
+    io.out_act = so.needs_act ? static_cast<__nv_bfloat16*>(tptr(2 + 2 * ko)) : nullptr;
+    io.res = (so.residual_from >= 0) ? tptr(1 + 2 * so.residual_from) : nullptr;
+    if (so.residual_from >= 0 && !io.res) { err = "internal: residual tensor missing"; return false; }
+    io.ext = reinterpret_cast<void*>(0x1);      // placeholder: the caller's output, patched per call
+    io.col = static_cast<__nv_bfloat16*>(tptr(0));
+    if (!prepare_step(p, steps, k, train, B, io, R.steps[k], err)) return false;
+  }
+  return true;
 }
 
 bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R, std::string& err);
@@ -917,63 +986,35 @@ int run_plan(kvae_plan* p, bool train, const void* in, int in_dtype, void* out, 
     p->prof_valid = true;
   }
   for (int k = 0; k < n; ++k) {
-    const ConvLayer& c = p->convs[steps[k].conv];
-    if (R.kind[k] == 5) {
-      // computed by the fused ResidualUnit launch of the previous step
-    } else if (R.kind[k] == 4) {
-      KV_CUDA(launch_conv_ru(R.ru[k], st));
-    } else if (R.kind[k] == 6) {
-      PreparedRun::WaveOutTc& t = R.wave_out_tc[k];
-      t.p.y = out;
-      t.p.y_f32 = (out_dtype == KVAE_F32);
-      t.p.peak_bits = fs ? fs->peak : nullptr;
-      static bool attr_set[64] = {false};
-      int dev = 0;
-      cudaGetDevice(&dev);
-      if (!attr_set[dev & 63]) {
-        KV_CUDA(cudaFuncSetAttribute(conv_wave_out_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KV_CUDA(cudaFuncSetAttribute(conv_wave_out_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        attr_set[dev & 63] = true;
-      }
-      const int grid = std::min(t.p.total_tiles, sm_count());
-      if (R.stream_f16) KV_CUDA(launch_pdl(conv_wave_out_tc_kernel<true>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<true>(), st, t.tmX, t.p));
-      else KV_CUDA(launch_pdl(conv_wave_out_tc_kernel<false>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<false>(), st, t.tmX, t.p));
-    } else if (R.kind[k] == 3) {
-      WaveOutParams& w = R.wave_out[k];
-      w.y = out;
-      w.y_f32 = (out_dtype == KVAE_F32);
-      KV_CUDA(launch_wave_out(w, c.g.Cout, B, st));
-    } else if (R.kind[k] == 7) {
-      WaveInColParams& h = R.head_col;
-      h.x = in;
-      h.x_f32 = (in_dtype == KVAE_F32);
-      wave_in_im2col_kernel<<<h.row_blocks + (h.Cout * 64 + 255) / 256, 256, 0, st>>>(h);
-      KV_CUDA(cudaGetLastError());
-      ++g_launches;
-      KV_CUDA(launch_conv_umma2(R.umma2[k], st));
-    } else if (R.kind[k] == 2) {
-      WaveInParams& w = R.wave_in[k];
-      w.x = in;
-      w.x_f32 = (in_dtype == KVAE_F32);
-      KV_CUDA(launch_wave_in(w, c.g.Cin, B, st));
-    } else if (R.kind[k] == 0) {
-      ConvLaunch2& L = R.umma2[k];
-      if (k == n - 1) {
-        L.p.out_cf = out;
-        L.p.out_cf_f32 = (out_dtype == KVAE_F32);
-        L.p.samp_noise = (fs && fs->out) ? fs->noise : nullptr;
-        L.p.samp_out = fs ? fs->out : nullptr;
-        L.p.samp_D = fs ? fs->D : 0;
-        L.p.samp_std = fs ? fs->std : 0.f;
-      }
-      KV_CUDA(launch_conv_umma2(L, st));
-    } else {
-      DirectParams& d = R.direct[k];
-      if (k == 0) { d.x = in; d.x_f32 = (in_dtype == KVAE_F32); }
-      if (k == n - 1) { d.out_raw = out; d.out_raw_f32 = (out_dtype == KVAE_F32); }
-      KV_CUDA(launch_direct(d, R.direct_grid[k], R.direct_cfg[k], R.direct_smem[k], st));
+    StepLaunch& S = R.steps[k];
+    const bool f32_in = in_dtype == KVAE_F32, f32_out = out_dtype == KVAE_F32;
+    switch (S.kind) {   // the caller's tensors
+      case kWaveOutTc:
+        S.wave_out_tc.y = out;
+        S.wave_out_tc.y_f32 = f32_out;
+        S.wave_out_tc.peak_bits = fs ? fs->peak : nullptr;
+        break;
+      case kWaveOut: S.wave_out.y = out; S.wave_out.y_f32 = f32_out; break;
+      case kWaveInTc: S.head_col.x = in; S.head_col.x_f32 = f32_in; break;
+      case kWaveIn: S.wave_in.x = in; S.wave_in.x_f32 = f32_in; break;
+      case kTcConv:
+        if (k == n - 1) {
+          ConvParams2& cp = S.umma2.p;
+          cp.out_cf = out;
+          cp.out_cf_f32 = f32_out;
+          cp.samp_noise = (fs && fs->out) ? fs->noise : nullptr;
+          cp.samp_out = fs ? fs->out : nullptr;
+          cp.samp_D = fs ? fs->D : 0;
+          cp.samp_std = fs ? fs->std : 0.f;
+        }
+        break;
+      case kDirect:
+        if (k == 0) { S.direct.d.x = in; S.direct.d.x_f32 = f32_in; }
+        if (k == n - 1) { S.direct.d.out_raw = out; S.direct.d.out_raw_f32 = f32_out; }
+        break;
+      default: break;
     }
-    if (R.kind[k] != 5) ++g_launches;
+    KV_CUDA(launch_step(S, p->convs[steps[k].conv].g, B, R.stream_f16, st));
     if (valid && k != n - 1) KV_CUDA(zero_step_tails(p, steps, R, k, B, T, ws, valid_rows[k], train, st));
     if (prof) KV_CUDA(cudaEventRecord(p->events[k + 1], st));
   }
@@ -1199,16 +1240,8 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
       e.rows_per_block = tmp.rows_per_block; e.blocks_per_clip = tmp.blocks_per_clip;
     } else {
       bw.dgrad_kind = 2;
-      DirectParams& d = bw.dg_direct;
-      std::memset(&d, 0, sizeof(d));
-      TapPlan tp;
-      if (!build_taps(gd, tp, err)) return false;
-      d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
-      d.Tq_out = static_cast<int>((T_in + tp.P_out - 1) / tp.P_out);
-      d.T_out = static_cast<int>(T_in); d.T_in = static_cast<int>(T_out);
-      d.Cin = gd.Cin; d.Cout = gd.Cout; d.span = tp.span;
-      for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
-      for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+      if (!prepare_direct(gd, B, T_out, T_in, 0, bw.dg_direct, err)) return false;
+      DirectParams& d = bw.dg_direct.d;
       d.x = Gf(k); d.x_f32 = 1;
       d.x_sB = T_out * gd.Cin; d.x_sT = gd.Cin; d.x_sC = 1;
       d.w = c.w_direct_d;
@@ -1219,12 +1252,6 @@ bool prepare_backward(kvae_plan* p, int B, long long T, void* ws, PreparedRun& R
         d.out_raw = dA; d.out_raw_f32 = 1;
         d.o_sB = T_in * gd.Cout; d.o_sT = gd.Cout; d.o_sC = 1;
       }
-      const int cfg = direct_cfg_for(gd.Cout);
-      int BT, BN;
-      direct_tile(cfg, BT, BN);
-      bw.dg_cfg = cfg;
-      bw.dg_grid = dim3(ceil_div(d.Tq_out, BT) * tp.P_out, ceil_div(gd.Cout, BN), B);
-      bw.dg_smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
     }
     // ---- SnakeBeta backward producing G_{k-1}
     if (k >= 1) {
@@ -1372,9 +1399,9 @@ int run_backward(kvae_plan* p, const void* x, int x_dtype, const void* gy, int g
       }
       KV_CUDA(launch_conv_umma2(L, st));
     } else {
-      DirectParams& d = bw.dg_direct;
+      DirectParams& d = bw.dg_direct.d;
       if (k == 0) { d.out_raw = gx; d.out_raw_f32 = (gx_dtype == KVAE_F32); }
-      KV_CUDA(launch_direct(d, bw.dg_grid, bw.dg_cfg, bw.dg_smem, st));
+      KV_CUDA(launch_direct(bw.dg_direct, st));
     }
     ++g_launches;
     if (bw.has_sb && !bw.sb_fused) {
@@ -1755,33 +1782,22 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
   if (T_out <= 0) return fail("input shorter than the kernel");
   DeviceGuard guard(device_of(x));
   if (!guard.ok) return fail("cannot select the tensor's device");
-  TapPlan tp;
+  DirectLaunch L;
   std::string err;
-  if (!build_taps(g, tp, err)) return fail(err);
+  if (!prepare_direct(g, B, T, T_out, 0, L, err)) return fail(err);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* wd = static_cast<float*>(scratch);
   const size_t n = static_cast<size_t>(Cin) * Cout * K;
   pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
       w, transposed, Cout, Cin, K, nullptr, wd);
   KV_CUDA(cudaGetLastError());
-  DirectParams d;
-  std::memset(&d, 0, sizeof(d));
-  d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
-  d.Tq_out = static_cast<int>((T_out + tp.P_out - 1) / tp.P_out); d.T_out = static_cast<int>(T_out);
-  d.T_in = static_cast<int>(T); d.Cin = Cin; d.Cout = Cout; d.span = tp.span;
-  for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
-  for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+  DirectParams& d = L.d;
   d.x = x; d.x_f32 = (dtype == KVAE_F32);
   d.x_sB = static_cast<long long>(Cin) * T; d.x_sT = 1; d.x_sC = T;
   d.w = wd; d.bias = bias;
   d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
   d.o_sB = static_cast<long long>(Cout) * T_out; d.o_sT = 1; d.o_sC = T_out;
-  const int cfg = direct_cfg_for(Cout);
-  int BT, BN;
-  direct_tile(cfg, BT, BN);
-  dim3 grid(ceil_div(d.Tq_out, BT) * tp.P_out, ceil_div(Cout, BN), B);
-  const size_t smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
-  KV_CUDA(launch_direct(d, grid, cfg, smem, st));
+  KV_CUDA(launch_direct(L, st));
   g_launches += 2;
   return 0;
 }
@@ -1840,31 +1856,20 @@ int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, flo
   if (!gx) return 0;
   // ---- data gradient: the forward kernel under the opposite kind, same weight tensor
   const ConvGeom gd = dgrad_geom(g, static_cast<int>(T));
-  TapPlan tp;
+  DirectLaunch L;
   std::string err;
-  if (!build_taps(gd, tp, err)) return fail(err);
+  if (!prepare_direct(gd, B, T_out, T, 0, L, err)) return fail(err);
   float* wd = static_cast<float*>(scratch);
   pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
       w, gd.kind == kConvT, gd.Cout, gd.Cin, K, nullptr, wd);
   KV_CUDA(cudaGetLastError());
-  DirectParams d;
-  std::memset(&d, 0, sizeof(d));
-  d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
-  d.Tq_out = static_cast<int>((T + tp.P_out - 1) / tp.P_out); d.T_out = static_cast<int>(T);
-  d.T_in = static_cast<int>(T_out); d.Cin = gd.Cin; d.Cout = gd.Cout; d.span = tp.span;
-  for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
-  for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+  DirectParams& d = L.d;
   d.x = gy; d.x_f32 = f32;
   d.x_sB = gsB; d.x_sT = 1; d.x_sC = T_out;
   d.w = wd;
   d.out_raw = gx; d.out_raw_f32 = f32;
   d.o_sB = xsB; d.o_sT = 1; d.o_sC = T;
-  const int cfg = direct_cfg_for(gd.Cout);
-  int BT, BN;
-  direct_tile(cfg, BT, BN);
-  dim3 grid(ceil_div(d.Tq_out, BT) * tp.P_out, ceil_div(gd.Cout, BN), B);
-  const size_t smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
-  KV_CUDA(launch_direct(d, grid, cfg, smem, st));
+  KV_CUDA(launch_direct(L, st));
   g_launches += 2;
   return 0;
 }
@@ -2019,28 +2024,16 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int P_out = transposed ? stride : 1;
   if (engine == 0) {
-    TapPlan tp;
+    DirectLaunch L;
     std::string err;
-    if (!build_taps(g, tp, err)) return fail(err);
-    DirectParams d;
-    std::memset(&d, 0, sizeof(d));
-    d.B = B; d.P_out = tp.P_out; d.P_in = tp.P_in;
-    d.Tq_out = static_cast<int>((o1 + tp.P_out - 1) / tp.P_out); d.T_out = static_cast<int>(o1);
-    d.q_base = static_cast<int>(o0 / tp.P_out); d.t_lo = static_cast<int>(o0);
-    d.T_in = static_cast<int>(T); d.Cin = Cin; d.Cout = Cout; d.span = tp.span;
-    for (int i = 0; i <= kMaxPhases; ++i) d.tap_begin[i] = tp.tap_begin[i];
-    for (size_t i = 0; i < tp.taps.size(); ++i) d.taps[i] = tp.taps[i];
+    if (!prepare_direct(g, B, T, o1, o0, L, err)) return fail(err);
+    DirectParams& d = L.d;
     d.x = x; d.x_f32 = (dtype == KVAE_F32);
     d.x_sB = static_cast<long long>(Cin) * ldx; d.x_sT = 1; d.x_sC = ldx;
     d.w = static_cast<const float*>(packed); d.bias = bias;
     d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
     d.o_sB = static_cast<long long>(Cout) * ldy; d.o_sT = 1; d.o_sC = ldy;
-    const int cfg = direct_cfg_for(Cout);
-    int BT, BN;
-    direct_tile(cfg, BT, BN);
-    dim3 grid(ceil_div(d.Tq_out - d.q_base, BT) * tp.P_out, ceil_div(Cout, BN), B);
-    const size_t smem = (static_cast<size_t>(BT + tp.span) * (kDirectKC + 1) + kDirectKC * BN) * sizeof(float);
-    KV_CUDA(launch_direct(d, grid, cfg, smem, st));
+    KV_CUDA(launch_direct(L, st));
     ++g_launches;
     return 0;
   }
@@ -2580,7 +2573,7 @@ long long kvae_decode_stream_lookahead(const kvae_stream* s) {
   // samples by which the emitted waveform trails the pushed latents in steady state
   long long lag = 0;                       // in rows of the current rate, accumulated front to back
   for (size_t k = 0; k < s->ss.size(); ++k) {
-    if (s->ss[k].kind == 5) continue;
+    if (s->ss[k].kind == kRuSecond) continue;
     lag = (lag + s->ss[k].dmax) * s->ss[k].P_out;
   }
   return lag;
@@ -2624,7 +2617,7 @@ long long kvae_encode_stream_lookahead(const kvae_stream* s) {
   // the frame's own last sample
   long long reach = 0;
   for (int k = static_cast<int>(s->ss.size()) - 1; k >= 0; --k) {
-    if (s->ss[k].kind == 5) continue;                    // the k = 1 half of a fused unit reads its own row
+    if (s->ss[k].kind == kRuSecond) continue;            // the k = 1 half of a fused unit reads its own row
     reach = reach * s->ss[k].P_in + s->ss[k].dmax;
   }
   return reach - (s->ratio - 1);

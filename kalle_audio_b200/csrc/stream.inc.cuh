@@ -40,9 +40,7 @@ struct StreamOut {            // geometry shared by the raw (stream) and act (op
 };
 
 struct StreamStep {
-  int kind = -1;              // 0 tensor-core conv, 4 fused ResidualUnit (this step + next), 5 second half of a fused unit,
-                              // 6 tensor-core tail, 3 CUDA-core tail, 7 encoder head as im2col + k = 1 tensor-core conv,
-                              // 2 CUDA-core encoder head
+  StepKind kind = kTcConv;
   int bias = 0;               // in input groups of P_in rows: added to every tap offset
   int span = 0;               // last window row output 0 reads (input rows): the rows kept between calls
   int dmax = 0;               // last input row output q reads, relative to row q * P_in
@@ -72,14 +70,7 @@ __global__ void stream_append_cf_kernel(const void* x, int x_f32, float* y, long
 }
 
 struct PreparedPush {
-  std::vector<int> launch;                 // per step: 1 = launch
-  std::vector<ConvLaunch2> umma2;
-  std::vector<RuLaunch> ru;
-  PreparedRun::WaveOutTc wo_tc;
-  WaveOutParams wo_cc;
-  int wo_cout = 0;
-  WaveInColParams wi_col;                  // encoder head, kind 7 (its k = 1 conv is umma2[0])
-  WaveInParams wi_cc;                      // encoder head, kind 2
+  std::vector<StepLaunch> steps;           // the steps that run in this call, in order
   long long n_out = 0;                     // rows the call emits (samples / latent frames)
   int in_rows0 = 0;                        // row of the input buffer where the new rows go
   std::vector<StreamRegion> zero;          // end of stream: rows of a strided conv's last partial group past the end
@@ -159,12 +150,7 @@ bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, Prepare
   const std::vector<Step>& steps = p->steps;
   const int n = static_cast<int>(steps.size());
   const int B = s->B;
-  const int sf16 = s->stream_f16 ? 1 : 0;
-  const int split = (p->precision == KVAE_PREC_F32) ? 2 : 1;
   std::vector<StreamOut> cur = s->outs;
-  P.launch.assign(n, 0);
-  P.umma2.resize(n);
-  P.ru.resize(n);
   P.in_rows0 = static_cast<int>(cur[0].rows);
   cur[0].rows += n_in;
   if (cur[0].rows > cur[0].cap) { err = "streaming: input buffer overflow"; return false; }
@@ -175,11 +161,10 @@ bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, Prepare
   std::vector<long long> consumed(cur.size(), 0);   // rows of each buffer its consumer is done with after this call
   for (int k = 0; k < n; ++k) {
     const StreamStep& st = s->ss[k];
-    if (st.kind == 5) continue;
-    const Step& sp = steps[k];
-    const ConvLayer& c = p->convs[sp.conv];
+    if (st.kind == kRuSecond) continue;
+    const ConvLayer& c = p->convs[steps[k].conv];
     StreamOut& in = cur[st.in_out + 1];
-    const int ko = (st.kind == 4) ? k + 1 : k;              // the step whose tensors receive the result
+    const int ko = (st.kind == kRuFused) ? k + 1 : k;       // the step whose tensors receive the result
     StreamOut& out = cur[ko + 1];
     const bool last = (ko == n - 1);
     // every output whose input rows have all arrived; at the end of the stream, all the conv's output rows (its
@@ -192,6 +177,14 @@ bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, Prepare
     if (!last) {
       if (out.abs_base + out.rows != out_abs) { err = "internal: streaming row bookkeeping at step " + std::to_string(k); return false; }
       if (out.rows + out_rows > out.cap) { err = "streaming: window buffer overflow at step " + std::to_string(k); return false; }
+    } else {
+      // decoder: the tail writes the waveform staging [B, io, max_samples] (fp32); encoder: the output conv writes
+      // channels-first latents [B, latent, max_frames] in the caller's dtype
+      if (out_rows > (s->enc ? s->max_frames : s->max_samples)) {
+        err = s->enc ? "streaming: latent staging overflow" : "streaming: waveform staging overflow";
+        return false;
+      }
+      P.n_out = out_rows;
     }
     StreamGeom sg;
     sg.in_rows = static_cast<int>((in.rows + st.P_in - 1) / st.P_in * st.P_in);   // whole phase groups
@@ -207,132 +200,35 @@ bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, Prepare
     sg.in_pitch = in.cap;
     sg.raw_pitch = out.cap;
     sg.act_pitch = out.cap;
-    const Step& so = steps[ko];
+    StepIO io;
     // skip connection: rows of the residual-source stream aligned with this step's output rows
-    const uint8_t* res = nullptr;
+    const Step& so = steps[ko];
     if (so.residual_from >= 0) {
       const StreamOut& r = cur[so.residual_from + 1];
       const long long rel = out_abs - r.abs_base;
       if (!r.raw_row_bytes || rel < 0 || rel + out_rows > r.rows) { err = "internal: streaming skip rows unavailable at step " + std::to_string(k); return false; }
-      res = raw_ptr(r, rel);
+      io.res = raw_ptr(r, rel);
       sg.res_pitch = r.cap;
     }
-    if (st.kind == 4) {
-      const Step& s1 = steps[k + 1];
-      const ConvLayer& c1 = p->convs[s1.conv];
-      RuArgs ra;
-      ra.a = reinterpret_cast<const __nv_bfloat16*>(act_ptr(in, 0));
-      ra.x = res;
-      ra.stream_f16 = sf16;
-      ra.w7 = c.w_umma; ra.w1 = c1.w_umma;
-      ra.bias7 = c.bias;
-      ra.s2_a = p->snakes[sp.epi_snake].a; ra.s2_inv_b = p->snakes[sp.epi_snake].inv_b;
-      ra.bias1 = c1.bias;
-      ra.out_raw = out.raw_row_bytes ? raw_ptr(out, out.rows) : nullptr;
-      ra.out_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
-      ra.act_f16 = s1.act_f16 ? 1 : 0;
-      if (s1.epi_snake >= 0) { ra.sn_a = p->snakes[s1.epi_snake].a; ra.sn_inv_b = p->snakes[s1.epi_snake].inv_b; }
-      if (!prepare_conv_ru(ra, B, 0, c.g.dilation, P.ru[k], err, &sg)) return false;
-    } else if (st.kind == 7 || st.kind == 2) {
-      // encoder head: reads the channels-first sample window, output q reads window samples q .. q + 6
-      const int io = c.g.Cin;
-      const float* snake_a = sp.epi_snake >= 0 ? p->snakes[sp.epi_snake].a : nullptr;
-      const float* snake_inv_b = sp.epi_snake >= 0 ? p->snakes[sp.epi_snake].inv_b : nullptr;
-      void* o_raw = out.raw_row_bytes ? raw_ptr(out, out.rows) : nullptr;
-      __nv_bfloat16* o_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
-      if (st.kind == 7) {
-        WaveInColParams& h = P.wi_col;
-        std::memset(&h, 0, sizeof(h));
-        h.x = raw_ptr(in, 0); h.x_f32 = 1;
-        h.col = s->col; h.w = c.w_direct; h.wp = c.w_head;
-        h.T = static_cast<int>(out_rows); h.B = B; h.Cout = c.g.Cout; h.CIN = io;
-        h.row_blocks = B * ((h.T + kColRows - 1) / kColRows);
-        h.T_in = static_cast<int>(in.rows); h.in_row0 = 0; h.x_pitch = in.cap;
-        if (out_rows > in.cap) { err = "internal: head operand overflow"; return false; }
-        ConvGeom g1 = c.g;
-        g1.Cin = 64; g1.K = 1; g1.pad = 0; g1.dilation = 1; g1.stride = 1;
-        ConvEpilogue ep;
-        ep.bias = c.bias;
-        ep.stream_f16 = 1;
-        ep.out_raw = o_raw;
-        ep.out_act = o_act;
-        ep.snake_a = snake_a; ep.snake_inv_b = snake_inv_b;
-        StreamGeom sg1;
-        sg1.in_rows = h.T; sg1.out_q = h.T; sg1.in_pitch = h.T; sg1.raw_pitch = out.cap; sg1.act_pitch = out.cap;
-        ConvTuning2 tune;
-        if (!prepare_conv_umma2(g1, s->col, B, 0, c.w_head, ep, tune, P.umma2[k], err, &sg1)) return false;
-      } else {
-        WaveInParams& w = P.wi_cc;
-        std::memset(&w, 0, sizeof(w));
-        w.x = raw_ptr(in, 0); w.x_f32 = 1;
-        w.w = c.w_direct; w.bias = c.bias;
-        w.out_raw = o_raw; w.raw_f16 = sf16;
-        w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
-        w.act_split = (o_act && p->precision == KVAE_PREC_F32) ? 1 : 0;
-        w.out_act = o_act;
-        w.snake_a = snake_a; w.snake_inv_b = snake_inv_b;
-        w.T = static_cast<int>(out_rows); w.Cout = c.g.Cout;
-        w.T_in = static_cast<int>(in.rows); w.in_row0 = 0; w.x_pitch = in.cap; w.out_pitch = out.cap;
-      }
-    } else if (st.kind == 6 || st.kind == 3) {
-      // decoder tail: reads the stream (raw) tensor of the previous step, writes the staging waveform [B, io, out_rows]
-      const bool preact = p->tail_preact && st.kind == 6;    // the last unit wrote SnakeBeta(x) in fp16 (kvae.cu, finalize_steps)
-      if (preact ? !in.act_row_bytes : !in.raw_row_bytes) { err = "internal: streaming tail needs the stream tensor"; return false; }
-      if (out_rows > s->max_samples) { err = "streaming: waveform staging overflow"; return false; }
-      const int tanh_out = (p->arch.final_tanh) ? 1 : 0;
-      P.wo_cout = c.g.Cout;
-      if (st.kind == 6) {
-        PreparedRun::WaveOutTc& t = P.wo_tc;
-        std::memset(&t.p, 0, sizeof(t.p));
-        t.p.pro_a = p->snakes[sp.pre_snake].a; t.p.pro_inv_b = p->snakes[sp.pre_snake].inv_b; t.p.w = c.w_direct;
-        t.p.T = static_cast<int>(out_rows); t.p.B = B; t.p.COUT = c.g.Cout; t.p.tanh_out = tanh_out;
-        t.p.tiles_per_clip = (t.p.T + kWoTcTile - 1) / kWoTcTile;
-        t.p.total_tiles = t.p.tiles_per_clip * B;
-        t.p.in_row0 = 0;                                   // -3 + bias 3
-        t.p.y = s->wav_stage; t.p.y_f32 = 1;
-        t.p.preact = preact ? 1 : 0;
-        if (sf16) { if (!make_act_tmap(&t.tmX, preact ? act_ptr(in, 0) : raw_ptr(in, 0), B, static_cast<int>(in.rows), 128, 1, kWoTcRows, err, in.cap)) return false; }
-        else if (!make_out_tmap(&t.tmX, raw_ptr(in, 0), B, static_cast<int>(in.rows), 128, 1, 1, err, kWoTcRows, in.cap)) return false;
-      } else {
-        WaveOutParams& w = P.wo_cc;
-        std::memset(&w, 0, sizeof(w));
-        w.x = reinterpret_cast<const float*>(raw_ptr(in, 0));
-        w.pro_a = p->snakes[sp.pre_snake].a; w.pro_inv_b = p->snakes[sp.pre_snake].inv_b; w.w = c.w_direct;
-        w.y = s->wav_stage; w.y_f32 = 1;
-        w.T = static_cast<int>(out_rows); w.Cin = c.g.Cin; w.tanh_out = tanh_out;
-        w.precise = (p->precision == KVAE_PREC_F32) ? 1 : 0;
-        w.T_in = static_cast<int>(in.rows); w.in_row0 = 0; w.x_pitch = in.cap;
-      }
-      P.n_out = out_rows;
-    } else {
-      ConvEpilogue ep;
-      ep.bias = c.has_bias ? c.bias : nullptr;
-      ep.residual = res;
-      ep.residual_f32 = sf16 ? 0 : 1;
-      ep.stream_f16 = sf16;
-      ep.out_raw = out.raw_row_bytes ? raw_ptr(out, out.rows) : nullptr;
-      ep.out_raw_f32 = sf16 ? 0 : 1;
-      ep.out_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
-      if (sp.epi_snake >= 0) { ep.snake_a = p->snakes[sp.epi_snake].a; ep.snake_inv_b = p->snakes[sp.epi_snake].inv_b; }
-      if (!c.umma) { ep.split3 = 1; ep.act_split = 1; ep.precise = 1; }
-      if (last) {
-        // encoder output conv: channels-first latents into the staging buffer, in the caller's dtype
-        if (out_rows > s->max_frames) { err = "streaming: latent staging overflow"; return false; }
-        ep.out_raw = s->z_stage;
-        ep.out_raw_cf = 1;
-        ep.out_raw_f32 = (out_dtype == KVAE_F32) ? 1 : 0;
-        P.n_out = out_rows;
-      }
-      ConvTuning2 tune;
-      if (!prepare_conv_umma2(c.g, reinterpret_cast<const __nv_bfloat16*>(act_ptr(in, 0)), B, 0, c.w_umma, ep, tune,
-                              P.umma2[k], err, &sg))
-        return false;
-      if (last) P.umma2[k].p.cf_ld = s->max_frames;
-    }
-    P.launch[k] = 1;
+    if (st.kind == kWaveInTc && out_rows > in.cap) { err = "internal: head operand overflow"; return false; }
+    io.in_act = in.act_row_bytes ? act_ptr(in, 0) : nullptr;
+    io.in_raw = in.raw_row_bytes ? raw_ptr(in, 0) : nullptr;
+    io.in_rows = in.rows;
+    io.in_pitch = in.cap;
+    io.in_row0 = 0;                                          // edge kernels: the clip's -3 plus the window's bias of 3
+    io.out_rows = out_rows;
+    io.out_pitch = out.cap;
+    io.out_raw = out.raw_row_bytes ? raw_ptr(out, out.rows) : nullptr;
+    io.out_act = out.act_row_bytes ? reinterpret_cast<__nv_bfloat16*>(act_ptr(out, out.rows)) : nullptr;
+    io.ext = s->enc ? static_cast<void*>(s->z_stage) : static_cast<void*>(s->wav_stage);
+    io.ext_f32 = s->enc ? (out_dtype == KVAE_F32) : 1;
+    io.cf_ld = s->max_frames;
+    io.col = s->col;
+    io.sg = &sg;
+    P.steps.emplace_back();
+    if (!prepare_step(p, steps, k, false, B, io, P.steps.back(), err)) return false;
     consumed[st.in_out + 1] = out_q * st.P_in;
     if (!last) out.rows += out_rows;
-    (void)split;
   }
   // carry: keep the last `keep` rows of every buffer (all of them while a layer is still starved)
   for (size_t j = 0; j < cur.size(); ++j) {
@@ -375,7 +271,6 @@ bool stream_prepare(kvae_stream* s, int n_in, bool flush, int out_dtype, Prepare
 
 cudaError_t stream_launch_all(kvae_stream* s, PreparedPush& P, int n_frames, int z_f32, cudaStream_t st) {
   kvae_plan* p = s->plan;
-  const int n = static_cast<int>(p->steps.size());
   const ConvLayer& c0 = p->convs[p->steps[0].conv];
   for (const StreamRegion& z : P.zero) {
     cudaError_t e = cudaMemset2DAsync(z.dst, z.pitch, 0, z.width, z.height, st);
@@ -401,41 +296,9 @@ cudaError_t stream_launch_all(kvae_stream* s, PreparedPush& P, int n_frames, int
     if (e != cudaSuccess) return e;
     ++g_launches;
   }
-  for (int k = 0; k < n; ++k) {
-    if (!P.launch[k]) continue;
-    const int kind = s->ss[k].kind;
-    cudaError_t e = cudaSuccess;
-    if (kind == 4) {
-      e = launch_conv_ru(P.ru[k], st);
-    } else if (kind == 0) {
-      e = launch_conv_umma2(P.umma2[k], st);
-    } else if (kind == 6) {
-      static bool attr_set[64] = {false};
-      int dev = 0;
-      cudaGetDevice(&dev);
-      if (!attr_set[dev & 63]) {
-        e = cudaFuncSetAttribute(conv_wave_out_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_wave_out_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev & 63] = true;
-      }
-      const int grid = std::min(P.wo_tc.p.total_tiles, sm_count());
-      if (s->stream_f16) e = launch_pdl(conv_wave_out_tc_kernel<true>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<true>(), st, P.wo_tc.tmX, P.wo_tc.p);
-      else e = launch_pdl(conv_wave_out_tc_kernel<false>, dim3(grid), dim3(kWoTcThreads), wave_out_tc_smem<false>(), st, P.wo_tc.tmX, P.wo_tc.p);
-    } else if (kind == 3) {
-      e = launch_wave_out(P.wo_cc, P.wo_cout, s->B, st);
-    } else if (kind == 7) {
-      const WaveInColParams& h = P.wi_col;
-      wave_in_im2col_kernel<<<h.row_blocks + (h.Cout * 64 + 255) / 256, 256, 0, st>>>(h);
-      e = cudaGetLastError();
-      if (e != cudaSuccess) return e;
-      ++g_launches;
-      e = launch_conv_umma2(P.umma2[k], st);
-    } else if (kind == 2) {
-      e = launch_wave_in(P.wi_cc, p->convs[p->steps[k].conv].g.Cin, s->B, st);
-    }
+  for (StepLaunch& S : P.steps) {
+    cudaError_t e = launch_step(S, p->convs[p->steps[S.k].conv].g, s->B, s->stream_f16, st);
     if (e != cudaSuccess) return e;
-    ++g_launches;
   }
   if (!P.carry.empty()) {
     size_t maxb = 0;
@@ -594,20 +457,17 @@ int stream_create(kvae_plan* p, int B, long long max_in, int use_graphs, kvae_st
   if (!enc && !conv_tc(c0, false)) return fail("streaming: needs a tensor-core first layer (latent_dim and channels multiples of 64)");
   // step kinds and geometry
   for (int k = 0; k < n; ++k) {
-    const Step& sp = steps[k];
-    const ConvLayer& c = p->convs[sp.conv];
+    const ConvLayer& c = p->convs[steps[k].conv];
     StreamStep& st = s->ss[k];
     st.in_out = k - 1;
-    if (sp.fuse == 2) { st.kind = 5; continue; }
+    st.kind = step_kind(p, steps, k, false);
+    if (st.kind == kRuSecond) continue;
     if (!stream_step_geometry(c.g, st, err)) return fail(err);
-    if (sp.fuse == 1) st.kind = 4;
-    else if (!enc && is_wave_out_step(p, steps, k)) st.kind = (p->precision == KVAE_PREC_BF16 && s->stream_f16) ? 6 : 3;
-    else if (enc && k == 0 && is_wave_in_step(p, steps, k)) st.kind = head_on_tc(p, steps, false) ? 7 : 2;
-    else if (conv_tc(c, false)) st.kind = 0;
-    else return fail("streaming: step " + std::to_string(k) + " has no tensor-core kernel (channels must be multiples of 64; "
-                     "the 128-channel tail is required)");
-    if (st.kind == 3 && (c.g.Cin != 128)) return fail("streaming: CUDA-core tail needs 128 input channels");
-    if (!enc && k == n - 1 && st.kind == 0) return fail("streaming: tensor-core output conv unsupported");
+    if (st.kind == kDirect)
+      return fail("streaming: step " + std::to_string(k) + " has no tensor-core kernel (channels must be multiples of 64; "
+                  "the 128-channel tail is required)");
+    if (st.kind == kWaveOut && (c.g.Cin != 128)) return fail("streaming: CUDA-core tail needs 128 input channels");
+    if (!enc && k == n - 1 && st.kind == kTcConv) return fail("streaming: tensor-core output conv unsupported");
   }
   // rate of every tensor relative to the input rate, keep / init rows from the consumer
   std::vector<double> rates(n + 1, 1.0);
@@ -616,15 +476,15 @@ int stream_create(kvae_plan* p, int B, long long max_in, int use_graphs, kvae_st
   size_t off = 0;
   auto consumer_of = [&](int j) -> int {   // first step that reads StreamOut j (j = -1: the input)
     for (int k = j + 1; k < n; ++k)
-      if (s->ss[k].kind != 5 && s->ss[k].in_out == j) return k;
+      if (s->ss[k].kind != kRuSecond && s->ss[k].in_out == j) return k;
     return -1;
   };
   // a fused unit at step k writes the tensors of step k+1; its consumer is step k+2 reading StreamOut k+1
   for (int k = 0; k < n; ++k)
-    if (s->ss[k].kind != 5 && k > 0 && s->ss[k - 1].kind == 5) s->ss[k].in_out = k - 1;
+    if (s->ss[k].kind != kRuSecond && k > 0 && s->ss[k - 1].kind == kRuSecond) s->ss[k].in_out = k - 1;
   for (int j = -1; j < n - 1; ++j) {
     StreamOut& o = s->outs[j + 1];
-    if (j >= 0 && s->ss[j].kind == 4) continue;          // the k7 half of a fused unit produces no tensor
+    if (j >= 0 && s->ss[j].kind == kRuFused) continue;         // the k7 half of a fused unit produces no tensor
     const int cons = consumer_of(j);
     if (cons < 0) return fail("internal: streaming tensor without consumer");
     const StreamStep& cs = s->ss[cons];
@@ -656,7 +516,7 @@ int stream_create(kvae_plan* p, int B, long long max_in, int use_graphs, kvae_st
     }
   }
   size_t off_col = 0;
-  if (enc && s->ss[0].kind == 7) {                       // im2col operand of the head: at most a window of rows
+  if (enc && s->ss[0].kind == kWaveInTc) {                      // im2col operand of the head: at most a window of rows
     off_col = off;
     off += align_up(static_cast<size_t>(B) * s->outs[0].cap * 64 * 2, 1024);
   }
