@@ -304,6 +304,20 @@ int kvae_aa_act_fwd(const void* x, void* y, const float* alpha, const float* bet
 int kvae_aa_act_win_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy, long long o0,
                         long long o1, long long t_end, const float* alpha, const float* beta, int logscale,
                         const float* filt_up, const float* filt_down, int B, int C, int dtype, void* stream);
+/* Ragged form of kvae_aa_act_fwd for BigVGANFlowVAE batches of clips with different lengths (every Activation1d of
+   flows.py:266, 312, 443 under extract_latents / inference_from_latents(valid_len=...)).  valid_len: HOST array of
+   B <= 64 ints in [1, T].  Each (b, c) row is its own signal ending at valid_len[b]: replicate padding happens at that
+   end, so outputs t < valid_len[b] equal kvae_aa_act_fwd on the row's first valid_len[b] samples bit for bit, and
+   outputs t >= valid_len[b] are stored as 0 (a following conv reads them as its zero padding).  Rows of x past a
+   clip's end are never read. */
+int kvae_aa_act_ragged_fwd(const void* x, void* y, const float* alpha, const float* beta, int logscale,
+                           const float* filt_up, const float* filt_down, int B, int C, long long T,
+                           const int* valid_len, int dtype, void* stream);
+/* y[b, c, t] = 0 for t in [valid_len[b], T): channels-first [B, C] rows of T samples at pitch ldy >= T, valid_len a
+   HOST array of B <= 64 ints in [0, T].  Re-creates a clip's end-of-signal zero padding inside a padded BigVGANFlowVAE
+   batch where the next op reads past the clip's end (the input, the input of a non-causal ConvTranspose1d
+   (flows.py:336-391), the inputs of the encoder's convs (:139-189), the final output). */
+int kvae_zero_tail_cf(void* y, int B, int C, long long T, long long ldy, const int* valid_len, int dtype, void* stream);
 /* Window form of the conv layers of BigVGANFlowVAE for the streaming decoder (Conv1d / ConvTranspose1d, flows.py:336-391,
    566-620).  kvae_conv1d_pack packs a folded fp32 weight ([Cout, Cin, K], transposed: [Cin, Cout, K]) once, for engine
    0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split, into kvae_conv1d_packed_bytes.  kvae_conv1d_win_fwd

@@ -91,6 +91,10 @@ SIGNATURES = {
     "kvae_aa_act_win_fwd": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_longlong,
                                       C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int,
                                       C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "kvae_aa_act_ragged_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                         C.c_int, C.c_int, C.c_longlong, C.POINTER(C.c_int), C.c_int, C.c_void_p]),
+    "kvae_zero_tail_cf": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_longlong, C.POINTER(C.c_int),
+                                    C.c_int, C.c_void_p]),
     "kvae_conv1d_packed_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "kvae_conv1d_pack": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
                                    C.c_void_p]),

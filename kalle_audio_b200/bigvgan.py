@@ -8,6 +8,9 @@ only; kept as a parameter container so checkpoints load), ``conv_pre``, ``ups``,
     extract_latents(x)                      :494-496   waveform [B, 1, L] -> [B, 2 D, L / prod(downsample_rates)]
     inference_from_latents(x, do_sample)    :498-529   latents -> waveform [B, 1, T * prod(upsample_rates)]
 
+Both take ``valid_len`` for a batch of clips of different lengths, each clip bit-identical to its own call (the
+ragged path below ``_run_ragged``; ``latent_length`` / ``wav_length`` give the per-clip output lengths).
+
 Every step runs through libkvae: convolutions and transposed convolutions (causal or not) through the generic conv
 kernels (``kvae_conv1d_fwd``; weight norm folded on the device), the anti-aliased Snake / SnakeBeta activation as ONE
 fused kernel (``kvae_aa_act_fwd``: x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager
@@ -17,14 +20,17 @@ This is the parity-first form of SURVEY section 8(f) item 2: CUDA end to end, no
 """
 from __future__ import annotations
 
+import ctypes
 import math
-from typing import List, Optional
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 from torch import nn
 
 from . import _lib
-from .layers import WNConv1d, WNConvTranspose1d
+from .layers import TC_MIN_ROWS, WNConv1d, WNConvTranspose1d
+
+_RAGGED_MAX_CLIPS = 64       # kRaggedMaxClips (elementwise.cuh): lengths travel by value into the kernels
 
 
 def _kaiser_sinc_filter1d(cutoff: float, half_width: float, kernel_size: int) -> torch.Tensor:
@@ -133,6 +139,22 @@ class Activation1d(nn.Module):
                                               _lib.dtype_code(xin.dtype), _lib.stream_ptr(x.device)))
         return y if y.dtype == x.dtype else y.to(x.dtype)
 
+    def ragged(self, x, valid_len):
+        """forward on a batch whose row b ends at valid_len[b] (kvae_aa_act_ragged_fwd): rows t < valid_len[b] equal
+        forward(x[b:b+1, :, :valid_len[b]]), rows past it are 0.  x: contiguous fp32 / bf16 [B, C, T]."""
+        B, C, T = x.shape
+        y = torch.empty_like(x)
+        beta = getattr(self.act, "beta", None)
+        fu = self.upsample.filter.detach().float().reshape(-1).contiguous()
+        fd = self.downsample.lowpass.filter.detach().float().reshape(-1).contiguous()
+        _lib.check(_lib.lib().kvae_aa_act_ragged_fwd(x.data_ptr(), y.data_ptr(),
+                                                     self.act.alpha.detach().float().contiguous().data_ptr(),
+                                                     None if beta is None else beta.detach().float().contiguous().data_ptr(),
+                                                     int(self.act.alpha_logscale), fu.data_ptr(), fd.data_ptr(), B, C, T,
+                                                     (ctypes.c_int * B)(*valid_len), _lib.dtype_code(x.dtype),
+                                                     _lib.stream_ptr(x.device)))
+        return y
+
 
 class Conv1d(WNConv1d):
     """flows.py:566-620: weight-normed Conv1d, 'same' padding or causal (left padding d (K - 1), :607-608).  A causal conv
@@ -143,13 +165,13 @@ class Conv1d(WNConv1d):
         pad = dilation * (kernel_size - 1) if causal else int((kernel_size * dilation - dilation) / 2)
         super().__init__(in_channels, out_channels, kernel_size, stride=stride, padding=pad, dilation=dilation, bias=bias)
 
-    def forward(self, x):
+    def forward(self, x, tc=True):
         if self.causal and self.kernel_size[0] > 1:
-            y = self._forward_tc(x, keep=x.shape[2])         # tensor-core layers truncate inside the kernel
+            y = self._forward_tc(x, keep=x.shape[2]) if tc else None   # tensor-core layers truncate inside the kernel
             if y is not None:
                 return y
-            return super().forward(x)[:, :, :x.shape[2]].contiguous()
-        return super().forward(x)
+            return super().forward(x, tc=False)[:, :, :x.shape[2]].contiguous()
+        return super().forward(x, tc)
 
 
 class ConvTranspose1d(WNConvTranspose1d):
@@ -163,13 +185,13 @@ class ConvTranspose1d(WNConvTranspose1d):
                          padding=0 if causal else (kernel_size - stride) // 2)
         self._drop = stride if causal else 0
 
-    def forward(self, x):
+    def forward(self, x, tc=True):
         if self._drop:
-            y = self._forward_tc(x, keep=x.shape[2] * self.stride[0])
+            y = self._forward_tc(x, keep=x.shape[2] * self.stride[0]) if tc else None
             if y is not None:
                 return y
-            return super().forward(x)[:, :, :-self._drop].contiguous()
-        return super().forward(x)
+            return super().forward(x, tc=False)[:, :, :-self._drop].contiguous()
+        return super().forward(x, tc)
 
 
 class Conv1d_S(nn.Module):
@@ -287,6 +309,275 @@ class _FlowParams(nn.Module):
             self.flows.append(nn.Module())      # Flip: no parameters
 
 
+# ------------------------------------------------------------------------------------------------- layer descriptions
+_AA_HALO = 5            # Activation1d: y[t] reads x[t - 5 .. t + 5] (12-tap x2 filters, bigvgan.cuh)
+
+
+def _program(h) -> Tuple[List[tuple], str]:
+    """The inference path as a list of ops over named streams (flows.py:506-527 in execution order).
+
+    ("conv", module, src, dst)  ("convT", module, src, dst)  ("act", module, src, dst)
+    ("axpby", a, b, dst, alpha, beta)  ("tanh", src, dst).  Module paths are ``BigVGANFlowVAE`` attribute paths."""
+    ops: List[tuple] = [("conv", "conv_pre", "z", "x0")]
+    nk = len(h["resblock_kernel_sizes"])
+    x = "x0"
+    for i in range(len(h["upsample_rates"])):
+        up = f"u{i}"
+        ops.append(("convT", f"ups.{i}.0", x, up))
+        xs = None
+        for j, dil in enumerate(h["resblock_dilation_sizes"]):
+            rb, cur = f"resblocks.{i * nk + j}", up
+            if h["resblock"] == "1":
+                for q in range(len(dil)):
+                    t = f"{rb}.{q}"
+                    ops += [("act", f"{rb}.activations.{2 * q}", cur, t + "a1"),
+                            ("conv", f"{rb}.convs1.{q}", t + "a1", t + "c1"),
+                            ("act", f"{rb}.activations.{2 * q + 1}", t + "c1", t + "a2"),
+                            ("conv", f"{rb}.convs2.{q}", t + "a2", t + "c2"),
+                            ("axpby", t + "c2", cur, t + "r", 1.0, 1.0)]
+                    cur = t + "r"
+            else:
+                for q in range(len(dil)):
+                    t = f"{rb}.{q}"
+                    ops += [("act", f"{rb}.activations.{q}", cur, t + "a"),
+                            ("conv", f"{rb}.convs.{q}", t + "a", t + "c"),
+                            ("axpby", t + "c", cur, t + "r", 1.0, 1.0)]
+                    cur = t + "r"
+            if xs is None:
+                xs = cur
+            else:
+                ops.append(("axpby", xs, cur, f"s{i}.{j}", 1.0, 1.0))
+                xs = f"s{i}.{j}"
+        x = f"x{i + 1}"
+        ops.append(("axpby", xs, xs, x, 1.0 / nk, 0.0))
+    ops += [("act", "activation_post", x, "ap"), ("conv", "conv_post", "ap", "cp"), ("tanh", "cp", "wav")]
+    return ops, "wav"
+
+
+def _conv_shape(h, path: str) -> Tuple[int, int, int, bool]:
+    """(kernel, dilation, stride, causal) of a conv / transposed conv of the program, from ``h`` alone."""
+    causal = bool(h["causal"])
+    if path == "conv_pre":
+        return 7, 1, 1, False
+    if path == "conv_post":
+        return 7, 1, 1, causal
+    parts = path.split(".")
+    if parts[0] == "ups":
+        i = int(parts[1])
+        return int(h["upsample_kernel_sizes"][i]), 1, int(h["upsample_rates"][i]), causal
+    nk = len(h["resblock_kernel_sizes"])
+    j = int(parts[1]) % nk
+    k = int(h["resblock_kernel_sizes"][j])
+    d = int(h["resblock_dilation_sizes"][j][int(parts[3])]) if parts[2] in ("convs1", "convs") else 1
+    return k, d, 1, causal
+
+
+class _Geom:
+    """Integer form of one op: how many output rows are final once ``R`` input rows have arrived."""
+
+    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False):
+        self.kind, self.K, self.d, self.s, self.causal = kind, K, d, s, causal
+        if kind == "conv":
+            self.span = d * (K - 1)
+            self.pl = self.span if causal else d * (K - 1) // 2        # left zero rows (flows.py:607-608)
+            self.pr = 0 if causal else self.pl                           # right zero rows at the stream end
+        elif kind == "convT":
+            self.span = K - 1
+            self.p = 0 if causal else (K - s) // 2                       # flows.py:336-391
+        elif kind == "act":
+            self.span = 2 * _AA_HALO
+
+    def total(self, R: int) -> int:
+        """Output rows of the whole-utterance op on R input rows."""
+        if self.kind == "conv":
+            return R + self.pl + self.pr - self.span
+        if self.kind == "convT":
+            return R * self.s if self.causal else (R - 1) * self.s - 2 * self.p + self.K
+        return R
+
+    def avail(self, R: int, end: bool) -> int:
+        if end:
+            return max(0, self.total(R)) if R > 0 else 0
+        if self.kind == "conv":
+            return max(0, R + self.pl - self.span)
+        if self.kind == "convT":
+            return max(0, R * self.s - self.p)
+        if self.kind == "act":
+            return max(0, R - _AA_HALO)
+        return R
+
+    def lookahead(self) -> int:
+        """Rows after an output's own position that it reads (in output rows)."""
+        if self.kind == "conv":
+            return self.span - self.pl
+        if self.kind == "convT":
+            return self.p
+        return _AA_HALO if self.kind == "act" else 0
+
+
+def _geom_of(h, op) -> _Geom:
+    if op[0] in ("conv", "convT"):
+        K, d, s, causal = _conv_shape(h, op[1])
+        return _Geom(op[0], K, d, s, causal)
+    return _Geom(op[0])
+
+
+def _encoder_program(h) -> Tuple[List[tuple], str]:
+    """Encoder.generator (flows.py:191-241) as a list of ops over named streams, in execution order:
+
+    ("conv", module, src, dst, (K, stride, dilation, padding))  ("lrelu", module, src, dst)  ("add", a, b, dst).
+    Conv1d_S pads d (K - 1) // 2, so the strided conv (K = 2 f, stride f) maps L rows to (L - 2) // f + 1; the ResStack
+    has 6 layers at dilations 1 .. 32 (``Encoder``'s stacks / stack_dilation_base)."""
+    p = "audio_encoder.generator"
+    ops: List[tuple] = [("conv", f"{p}.0.layer", "x", "h", (3, 1, 1, 1)), ("lrelu", f"{p}.1", "h", "a0")]
+    x, idx = "a0", 2
+    for i, f in enumerate(h["downsample_rates"]):
+        f = int(f)
+        ops.append(("conv", f"{p}.{idx}.layer", x, f"s{i}", (2 * f, f, 1, f - 1)))
+        x = f"s{i}"
+        for j in range(6):
+            rs, t = f"{p}.{idx + 1}.layers.{j}", f"s{i}.{j}"
+            ops += [("lrelu", f"{rs}.0", x, t + "a"), ("conv", f"{rs}.1", t + "a", t + "c", (3, 1, 2 ** j, 2 ** j)),
+                    ("lrelu", f"{rs}.2", t + "c", t + "b"), ("conv", f"{rs}.3", t + "b", t + "d", (3, 1, 1, 1)),
+                    ("add", x, t + "d", t + "r")]
+            x = t + "r"
+        ops.append(("lrelu", f"{p}.{idx + 2}", x, f"a{i + 1}"))
+        x, idx = f"a{i + 1}", idx + 3
+    ops.append(("conv", f"{p}.{idx}.layer", x, "lat", (3, 1, 1, 1)))
+    return ops, "lat"
+
+
+def _lengths(h, encoder: bool, n: int) -> Dict[str, int]:
+    """Rows of every stream of the encoder's (``encoder``) or the decoder's op list for one clip of ``n`` input rows;
+    0 from the first op on that would get no rows (the clip's own call raises there)."""
+    ops, _ = _encoder_program(h) if encoder else _program(h)
+    R = {"x" if encoder else "z": int(n)}
+    for op in ops:
+        kind = op[0]
+        if kind == "add":
+            R[op[3]] = R[op[1]]
+        elif kind == "axpby":
+            R[op[3]] = min(R[op[1]], R[op[2]])
+        elif kind == "tanh":
+            R[op[2]] = R[op[1]]
+        elif kind == "lrelu":
+            R[op[3]] = R[op[2]]
+        elif kind == "conv" and encoder:
+            K, s, d, p = op[4]
+            R[op[3]] = max(0, (R[op[2]] + 2 * p - d * (K - 1) - 1) // s + 1) if R[op[2]] > 0 else 0
+        else:
+            R[op[3]] = max(0, _geom_of(h, op).total(R[op[2]])) if R[op[2]] > 0 else 0
+    return R
+
+
+def latent_length(h, n_samples: int) -> int:
+    """Latent frames ``extract_latents`` returns for ``n_samples`` samples: the chained floors of the encoder's convs."""
+    return _lengths(h, True, n_samples)["lat"]
+
+
+def wav_length(h, n_frames: int) -> int:
+    """Samples ``inference_from_latents`` returns for ``n_frames`` latent frames, from the decoder's layer arithmetic."""
+    return _lengths(h, False, n_frames)[_program(h)[1]]
+
+
+# ------------------------------------------------------------------------------------------------- ragged batches
+def ragged_order(valid_len: Sequence[int]) -> Tuple[List[int], List[int]]:
+    """(order, inverse): ``order`` lists the clips longest first (ties keep their index order), ``inverse[b]`` is clip
+    b's position in it, so ``sorted_batch[inverse]`` restores the caller's order."""
+    order = sorted(range(len(valid_len)), key=lambda b: -int(valid_len[b]))
+    inverse = [0] * len(order)
+    for i, b in enumerate(order):
+        inverse[b] = i
+    return order, inverse
+
+
+def tc_split(rows: Sequence[int]) -> int:
+    """Clips of a longest-first batch whose own call runs a tensor-core layer on the tensor cores: those with at least
+    ``TC_MIN_ROWS`` input rows there, a prefix of the batch."""
+    n = sum(1 for r in rows if r >= TC_MIN_ROWS)
+    if any(r < TC_MIN_ROWS for r in rows[:n]):
+        raise ValueError("tc_split: rows must be sorted longest first")
+    return n
+
+
+def _check_valid_len(valid_len, B: int, T: int, out_len, what: str) -> List[int]:
+    if isinstance(valid_len, torch.Tensor):
+        valid_len = valid_len.tolist()
+    lens = [int(v) for v in valid_len]
+    if len(lens) != B:
+        raise ValueError(f"{what}: valid_len has {len(lens)} entries for a batch of {B}")
+    if B > _RAGGED_MAX_CLIPS:
+        raise ValueError(f"{what}: at most {_RAGGED_MAX_CLIPS} clips per ragged call, got {B}")
+    for b, v in enumerate(lens):
+        if not 1 <= v <= T:
+            raise ValueError(f"{what}: valid_len[{b}] = {v} is outside 1 .. {T} (the padded length)")
+        if out_len(v) < 1:
+            raise ValueError(f"{what}: clip {b} ({v} rows) is too short to give any output row")
+    return lens
+
+
+def _zero_tail(x: torch.Tensor, rows: Sequence[int]) -> None:
+    """x[b, :, rows[b]:] = 0 in place (x: a contiguous [B, C, T] tensor of fp32 or bf16)."""
+    B, C, T = x.shape
+    _lib.check(_lib.lib().kvae_zero_tail_cf(x.data_ptr(), B, C, T, T, (ctypes.c_int * B)(*rows),
+                                            _lib.dtype_code(x.dtype), _lib.stream_ptr(x.device)))
+
+
+def _conv_ragged(m, x: torch.Tensor, rows: Sequence[int]) -> torch.Tensor:
+    """m(x) on a longest-first batch, each clip on the engine its own call picks: at most two launches."""
+    n = tc_split(rows) if m.tc_layer() else 0
+    if n in (0, x.shape[0]):
+        return m(x, tc=n > 0)
+    return torch.cat([m(x[:n], tc=True), m(x[n:], tc=False)], dim=0)
+
+
+def _run_ragged(model, encoder: bool, x: torch.Tensor, lens: List[int]) -> torch.Tensor:
+    """The encoder's or decoder's op list on the longest-first batch ``x`` (rows past each clip's end: anything), clip b
+    holding lens[b] input rows.  Rows past a clip's end are zeroed where the next op reads them as padding: the input
+    of every non-causal conv (the decoder's activations already store zeros there) and of a non-causal transposed
+    conv, and the output."""
+    h = model.h
+    ops, out = _encoder_program(h) if encoder else _program(h)
+    R = [_lengths(h, encoder, n) for n in lens]
+    src = "x" if encoder else "z"
+    last = {}                                     # stream -> index of the op that reads it last
+    for i, op in enumerate(ops):
+        for name in {"add": op[1:3], "axpby": op[1:3], "tanh": op[1:2]}.get(op[0], op[2:3]):
+            last[name] = i
+    vals = {src: x}
+    _zero_tail(x, [r[src] for r in R])
+    for i, op in enumerate(ops):
+        kind = op[0]
+        if kind in ("conv", "convT"):
+            m, xin = _module(model, op[1]), vals[op[2]]
+            rows = [r[op[2]] for r in R]
+            if encoder and op[2] != src or kind == "convT" and not m.causal:
+                _zero_tail(xin, rows)
+            vals[op[3]] = _conv_ragged(m, xin, rows)
+        elif kind == "act":
+            vals[op[3]] = _module(model, op[1]).ragged(vals[op[2]], [r[op[2]] for r in R])
+        elif kind == "lrelu":
+            vals[op[3]] = _module(model, op[1])(vals[op[2]])
+        elif kind == "add":
+            vals[op[3]] = _axpby(vals[op[1]], vals[op[2]], 1.0, 1.0)
+        elif kind == "axpby":
+            vals[op[3]] = _axpby(vals[op[1]], vals[op[2]], op[4], op[5])
+        else:
+            vals[op[2]] = _unary(vals[op[1]], 1)
+        for name in [k for k, j in last.items() if j == i]:
+            vals.pop(name, None)
+    y = vals[out]
+    _zero_tail(y, [r[out] for r in R])
+    return y
+
+
+def _module(model, path: str):
+    m = model
+    for p in path.split("."):
+        m = m[int(p)] if p.isdigit() else getattr(m, p)
+    return m
+
+
 class BigVGANFlowVAE(nn.Module):
     def __init__(self, h):
         super().__init__()
@@ -331,12 +622,41 @@ class BigVGANFlowVAE(nn.Module):
         raise NotImplementedError("BigVGANFlowVAE.forward (the training pass through the flow, flows.py:454-492) is "
                                   "outside the hot path; use extract_latents / inference_from_latents")
 
+    def latent_length(self, n_samples: int) -> int:
+        """Latent frames ``extract_latents`` returns for a clip of ``n_samples`` samples (0: too short for any)."""
+        return latent_length(self.h, n_samples)
+
+    def wav_length(self, n_frames: int) -> int:
+        """Samples ``inference_from_latents`` returns for ``n_frames`` latent frames."""
+        return wav_length(self.h, n_frames)
+
+    def _ragged(self, encoder: bool, x: torch.Tensor, valid_len, what: str) -> torch.Tensor:
+        """Clips sorted longest first (so each conv splits into at most two engine groups), run, put back."""
+        _lib.require_cuda(x, what)
+        if x.dim() != 3 or x.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError(f"{what}: valid_len needs a float32 or bfloat16 [B, C, T] input")
+        out_len = self.latent_length if encoder else self.wav_length
+        lens = _check_valid_len(valid_len, x.shape[0], x.shape[2], out_len, what)
+        order, inverse = ragged_order(lens)
+        xs = x[torch.tensor(order, device=x.device)].contiguous()     # a copy: its padding rows are zeroed in place
+        y = _run_ragged(self, encoder, xs, [lens[b] for b in order])
+        return y if order == sorted(order) else y[torch.tensor(inverse, device=y.device)]
+
     @torch.no_grad()
-    def extract_latents(self, x):
+    def extract_latents(self, x, valid_len=None):
+        """``valid_len`` (host sequence of B ints, 1 <= valid_len[b] <= T, B <= 64): clip b is x[b, :, :valid_len[b]];
+        what x holds past that is ignored.  out[b, :, :latent_length(valid_len[b])] then equals
+        ``extract_latents(x[b:b+1, :, :valid_len[b]])`` bit for bit, and the rest of out[b] is 0."""
+        if valid_len is not None:
+            return self._ragged(True, x, valid_len, "extract_latents")
         return self.audio_encoder(x)
 
     @torch.no_grad()
-    def inference_from_latents(self, x, do_sample=True, noise: Optional[torch.Tensor] = None):
+    def inference_from_latents(self, x, do_sample=True, noise: Optional[torch.Tensor] = None, valid_len=None):
+        """``valid_len`` (host sequence of B ints, frames, 1 <= valid_len[b] <= T, B <= 64): clip b is
+        x[b, :, :valid_len[b]]; what x (and noise) hold past that is ignored.  out[b, :, :wav_length(valid_len[b])]
+        then equals the call on x[b:b+1, :, :valid_len[b]] (noise[b:b+1, :, :valid_len[b]]) bit for bit, and the rest
+        of out[b] is 0."""
         h = self.h
         if h.use_vae and do_sample:
             assert x.size(1) == h.latent_dim * 2, "Input must be like [B, D, H]"
@@ -351,6 +671,8 @@ class BigVGANFlowVAE(nn.Module):
             x = z if z.dtype == x.dtype else z.to(x.dtype)
         else:
             assert x.size(1) == h.latent_dim, "Input must be like [B, D, H]"
+        if valid_len is not None:
+            return self._ragged(False, x, valid_len, "inference_from_latents")
         x = self.conv_pre(x)
         for i in range(self.num_upsamples):
             for up in self.ups[i]:

@@ -15,8 +15,9 @@ exactly once, and ``torch.cat(pushes + [flush])`` equals the whole-utterance dec
   * residual adds / the AMP average / tanh / the Gaussian sample: the library's elementwise kernels on rows that both
     operands have.
 
-The op list comes from one description of the decoder (``_program``) that two interpreters read: the integer one
-behind ``bigvgan_stream_geometry`` (rows available per op, lookahead) and the tensor one behind the decoder.
+The op list comes from one description of the decoder (``bigvgan._program``) that three interpreters read: the integer
+one behind ``bigvgan_stream_geometry`` (rows available per op, lookahead), the tensor one behind the decoder, and the
+ragged whole-clip decode of ``BigVGANFlowVAE.inference_from_latents(valid_len=...)``.
 
 Pushes whose (size, start-up phase) was seen before replay one ``torch.cuda.CUDAGraph``; the op state lives in static
 buffers per phase, so a constant-hop stream in steady state is one graph launch per push.
@@ -24,124 +25,12 @@ buffers per phase, so a constant-hop stream in steady state is one graph launch 
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, Optional
 
 import torch
 
 from . import _lib
-from .bigvgan import BigVGANFlowVAE, _axpby, _k, _unary
-
-_AA_HALO = 5            # Activation1d: y[t] reads x[t - 5 .. t + 5] (12-tap x2 filters, bigvgan.cuh)
-
-
-# ------------------------------------------------------------------------------------------------ the op list
-def _program(h) -> Tuple[List[tuple], str]:
-    """The inference path as a list of ops over named streams (flows.py:506-527 in execution order).
-
-    ("conv", module, src, dst)  ("convT", module, src, dst)  ("act", module, src, dst)
-    ("axpby", a, b, dst, alpha, beta)  ("tanh", src, dst).  Module paths are ``BigVGANFlowVAE`` attribute paths."""
-    ops: List[tuple] = [("conv", "conv_pre", "z", "x0")]
-    nk = len(h["resblock_kernel_sizes"])
-    x = "x0"
-    for i in range(len(h["upsample_rates"])):
-        up = f"u{i}"
-        ops.append(("convT", f"ups.{i}.0", x, up))
-        xs = None
-        for j, dil in enumerate(h["resblock_dilation_sizes"]):
-            rb, cur = f"resblocks.{i * nk + j}", up
-            if h["resblock"] == "1":
-                for q in range(len(dil)):
-                    t = f"{rb}.{q}"
-                    ops += [("act", f"{rb}.activations.{2 * q}", cur, t + "a1"),
-                            ("conv", f"{rb}.convs1.{q}", t + "a1", t + "c1"),
-                            ("act", f"{rb}.activations.{2 * q + 1}", t + "c1", t + "a2"),
-                            ("conv", f"{rb}.convs2.{q}", t + "a2", t + "c2"),
-                            ("axpby", t + "c2", cur, t + "r", 1.0, 1.0)]
-                    cur = t + "r"
-            else:
-                for q in range(len(dil)):
-                    t = f"{rb}.{q}"
-                    ops += [("act", f"{rb}.activations.{q}", cur, t + "a"),
-                            ("conv", f"{rb}.convs.{q}", t + "a", t + "c"),
-                            ("axpby", t + "c", cur, t + "r", 1.0, 1.0)]
-                    cur = t + "r"
-            if xs is None:
-                xs = cur
-            else:
-                ops.append(("axpby", xs, cur, f"s{i}.{j}", 1.0, 1.0))
-                xs = f"s{i}.{j}"
-        x = f"x{i + 1}"
-        ops.append(("axpby", xs, xs, x, 1.0 / nk, 0.0))
-    ops += [("act", "activation_post", x, "ap"), ("conv", "conv_post", "ap", "cp"), ("tanh", "cp", "wav")]
-    return ops, "wav"
-
-
-def _conv_shape(h, path: str) -> Tuple[int, int, int, bool]:
-    """(kernel, dilation, stride, causal) of a conv / transposed conv of the program, from ``h`` alone."""
-    causal = bool(h["causal"])
-    if path == "conv_pre":
-        return 7, 1, 1, False
-    if path == "conv_post":
-        return 7, 1, 1, causal
-    parts = path.split(".")
-    if parts[0] == "ups":
-        i = int(parts[1])
-        return int(h["upsample_kernel_sizes"][i]), 1, int(h["upsample_rates"][i]), causal
-    nk = len(h["resblock_kernel_sizes"])
-    j = int(parts[1]) % nk
-    k = int(h["resblock_kernel_sizes"][j])
-    d = int(h["resblock_dilation_sizes"][j][int(parts[3])]) if parts[2] in ("convs1", "convs") else 1
-    return k, d, 1, causal
-
-
-class _Geom:
-    """Integer form of one op: how many output rows are final once ``R`` input rows have arrived."""
-
-    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False):
-        self.kind, self.K, self.d, self.s, self.causal = kind, K, d, s, causal
-        if kind == "conv":
-            self.span = d * (K - 1)
-            self.pl = self.span if causal else d * (K - 1) // 2        # left zero rows (flows.py:607-608)
-            self.pr = 0 if causal else self.pl                           # right zero rows at the stream end
-        elif kind == "convT":
-            self.span = K - 1
-            self.p = 0 if causal else (K - s) // 2                       # flows.py:336-391
-        elif kind == "act":
-            self.span = 2 * _AA_HALO
-
-    def total(self, R: int) -> int:
-        """Output rows of the whole-utterance op on R input rows."""
-        if self.kind == "conv":
-            return R + self.pl + self.pr - self.span
-        if self.kind == "convT":
-            return R * self.s if self.causal else (R - 1) * self.s - 2 * self.p + self.K
-        return R
-
-    def avail(self, R: int, end: bool) -> int:
-        if end:
-            return max(0, self.total(R)) if R > 0 else 0
-        if self.kind == "conv":
-            return max(0, R + self.pl - self.span)
-        if self.kind == "convT":
-            return max(0, R * self.s - self.p)
-        if self.kind == "act":
-            return max(0, R - _AA_HALO)
-        return R
-
-    def lookahead(self) -> int:
-        """Rows after an output's own position that it reads (in output rows)."""
-        if self.kind == "conv":
-            return self.span - self.pl
-        if self.kind == "convT":
-            return self.p
-        return _AA_HALO if self.kind == "act" else 0
-
-
-def _geom_of(h, op) -> _Geom:
-    if op[0] in ("conv", "convT"):
-        K, d, s, causal = _conv_shape(h, op[1])
-        return _Geom(op[0], K, d, s, causal)
-    return _Geom(op[0])
+from .bigvgan import _AA_HALO, BigVGANFlowVAE, _axpby, _geom_of, _k, _module, _program, _unary
 
 
 def bigvgan_stream_geometry(h) -> Dict[str, object]:
@@ -172,13 +61,6 @@ def bigvgan_stream_geometry(h) -> Dict[str, object]:
 
 
 # ------------------------------------------------------------------------------------------------ the decoder
-def _module(model, path: str):
-    m = model
-    for p in path.split("."):
-        m = m[int(p)] if p.isdigit() else getattr(m, p)
-    return m
-
-
 def _cat(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     if b.shape[2] == 0:
         return a
@@ -263,10 +145,7 @@ class BigVGANStreamingDecoder:
             self._engine, self._packed = {}, {}
             for c in self._convs:
                 m = _module(self.model, c)
-                tc = m.tc_precision is not None and not getattr(m, "_same_extra_right", 0) and \
-                    L.kvae_conv1d_tc_supported(m.in_channels, m.out_channels, m.kernel_size[0], m.stride[0],
-                                               m.dilation[0], int(m.transposed))
-                self._engine[c] = m.tc_precision if tc else None
+                self._engine[c] = m.tc_precision if m.tc_layer() else None
                 code = {None: 0, "bf16": 1, "fp32": 2}[self._engine[c]]
                 K = m.kernel_size[0]
                 nb = L.kvae_conv1d_packed_bytes(m.in_channels, m.out_channels, K, code)

@@ -30,16 +30,27 @@ constexpr long long kAaNoEnd = 1ll << 60;            // t_end of a window whose 
 // Everything inside a tile is indexed relative to the tile start in 32 bits; 64-bit arithmetic only places the tile
 // and clamps at the two ends of the row (the first version did every tap's index in 64 bits and spent ~60 % of its
 // instructions there: 21 of the 60 ms of the bench decode).  Same operations in the same order per sample.
+// kRagged (a batch of clips of different lengths): clip b = row / C ends at its own lens.v[b] instead of t_end, and
+// outputs t >= lens.v[b] are stored as 0, so a following conv reads the zero padding the clip's own call would have.
+// Otherwise lens is not read; the window and whole-row calls compile to the code they had before.
+template <bool kRagged>
 __global__ void __launch_bounds__(256) aa_act_kernel(const void* x, long long ldx, long long x0, long long nx, void* y,
                                                      long long ldy, long long o0, long long o1, long long t_end,
                                                      const float* alpha, const float* beta, int logscale,
-                                                     const float* fu, const float* fd, int C, int f32) {
+                                                     const float* fu, const float* fd, int C, int f32, RaggedLens lens) {
   __shared__ float xs[kAaTile + 16];
   __shared__ float vs[2 * kAaTile + kAaK];
   __shared__ float f_up[kAaK], f_dn[kAaK];
   const int c = blockIdx.y % C;
   const size_t row_x = static_cast<size_t>(blockIdx.y) * ldx, row_y = static_cast<size_t>(blockIdx.y) * ldy;
   const long long t0 = o0 + static_cast<long long>(blockIdx.x) * kAaTile;   // absolute
+  if constexpr (kRagged) {
+    t_end = lens.v[blockIdx.y / C];
+    if (t0 >= t_end) {                                          // a tile past the clip's end: zeros only
+      for (int tl = threadIdx.x; tl < kAaTile && t0 + tl < o1; tl += 256) st_elem(y, row_y + (t0 + tl - o0), f32, 0.f);
+      return;
+    }
+  }
   if (threadIdx.x < kAaK) { f_up[threadIdx.x] = fu[threadIdx.x]; f_dn[threadIdx.x] = fd[threadIdx.x]; }
   float a = alpha[c], bt = beta ? beta[c] : alpha[c];          // Snake: 1/alpha; SnakeBeta: 1/beta
   if (logscale) { a = expf(a); bt = expf(bt); }
@@ -75,7 +86,7 @@ __global__ void __launch_bounds__(256) aa_act_kernel(const void* x, long long ld
       float acc = 0.f;
 #pragma unroll
       for (int m = 0; m < kAaK; ++m) acc = fmaf(vs[2 * tl + m], f_dn[m], acc);
-      st_elem(y, row_y + (t0 + tl - o0), f32, acc);
+      st_elem(y, row_y + (t0 + tl - o0), f32, !kRagged || t0 + tl < t_end ? acc : 0.f);
     }
   }
 }

@@ -346,6 +346,15 @@ __global__ void zero_tail_rows_kernel(uint8_t* base, long long clip_bytes, int r
     for (size_t i = i0; i < nbytes / 2; i += step) q[i] = 0;
   }
 }
+// Channels-first, pitched sibling (the BigVGANFlowVAE ragged path): y[b, c, t] lives at y + (b * C + c) * ldy + t and is
+// set to 0 for t in [v[b], T).  grid: (blocks over the longest tail, C, clips)
+__global__ void zero_tail_cf_kernel(void* y, int C, long long T, long long ldy, RaggedLens lens, int f32) {
+  const int b = blockIdx.z;
+  const size_t row = (static_cast<size_t>(b) * C + blockIdx.y) * ldy;
+  const long long step = static_cast<long long>(gridDim.x) * blockDim.x;
+  for (long long t = lens.v[b] + blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < T; t += step)
+    st_elem(y, row + t, f32, 0.f);
+}
 
 // twj_dataset.py:231-235 for a batch of mono clips: librosa.util.normalize(wav) * 0.95 (peak normalisation, clips
 // whose peak is below float32 tiny stay as they are), duplicated to two channels, zero-padded to the batch length.

@@ -2480,6 +2480,21 @@ int kvae_aa_act_fwd(const void* x, void* y, const float* alpha, const float* bet
   return kvae_aa_act_win_fwd(x, T, 0, T, y, T, 0, T, T, alpha, beta, logscale, filt_up, filt_down, B, C, dtype, stream);
 }
 
+// ragged: per-clip ends from lens; otherwise the stream end t_end, kAaNoEnd for none
+static int launch_aa_act(bool ragged, const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy, long long o0,
+                         long long o1, long long t_end, const float* alpha, const float* beta, int logscale,
+                         const float* filt_up, const float* filt_down, int B, int C, int dtype, const RaggedLens& lens,
+                         void* stream) {
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  dim3 grid(static_cast<unsigned>((o1 - o0 + kAaTile - 1) / kAaTile), B * C);
+  (ragged ? aa_act_kernel<true> : aa_act_kernel<false>)<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      x, ldx, x0, nx, y, ldy, o0, o1, t_end, alpha, beta, logscale, filt_up, filt_down, C, dtype == KVAE_F32, lens);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
 int kvae_aa_act_win_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy, long long o0,
                         long long o1, long long t_end, const float* alpha, const float* beta, int logscale,
                         const float* filt_up, const float* filt_down, int B, int C, int dtype, void* stream) {
@@ -2492,11 +2507,49 @@ int kvae_aa_act_win_fwd(const void* x, long long ldx, long long x0, long long nx
     return fail("aa_act window: need 0 <= x0, 0 <= o0 < o1 <= t_end, nx <= ldx, o1 - o0 <= ldy");
   if (std::max(0ll, o0 - kAaHalo) < x0 || std::min(o1 + kAaHalo, te) > x0 + nx)
     return fail("aa_act window: the input rows [o0 - 5, o1 + 5) (clipped to the stream) must be inside [x0, x0 + nx)");
-  DeviceGuard guard(device_of(x));
+  return launch_aa_act(false, x, ldx, x0, nx, y, ldy, o0, o1, te, alpha, beta, logscale, filt_up, filt_down, B, C, dtype,
+                       RaggedLens{}, stream);
+}
+
+// host valid_len -> RaggedLens, each value in [lo, T]
+static int ragged_lens(const int* valid_len, int B, long long T, int lo, RaggedLens* lens) {
+  if (!valid_len) return fail("null valid_len");
+  if (B > kRaggedMaxClips) return fail("ragged batch: at most 64 clips (kRaggedMaxClips) per call");
+  for (int b = 0; b < B; ++b) {
+    if (valid_len[b] < lo || valid_len[b] > T) return fail(lo ? "valid_len out of range (1 .. padded length)"
+                                                              : "valid_len out of range (0 .. padded length)");
+    lens->v[b] = valid_len[b];
+  }
+  return 0;
+}
+
+int kvae_aa_act_ragged_fwd(const void* x, void* y, const float* alpha, const float* beta, int logscale,
+                           const float* filt_up, const float* filt_down, int B, int C, long long T,
+                           const int* valid_len, int dtype, void* stream) {
+  if (!x || !y || !alpha || !filt_up || !filt_down) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || C <= 0 || T <= 0) return 0;
+  if (static_cast<long long>(B) * C > 65535) return fail("B*C too large");
+  RaggedLens lens;
+  if (ragged_lens(valid_len, B, T, 1, &lens)) return -1;
+  return launch_aa_act(true, x, T, 0, T, y, T, 0, T, T, alpha, beta, logscale, filt_up, filt_down, B, C, dtype, lens, stream);
+}
+
+int kvae_zero_tail_cf(void* y, int B, int C, long long T, long long ldy, const int* valid_len, int dtype, void* stream) {
+  if (!y) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || C <= 0 || T <= 0) return 0;
+  if (C > 65535) return fail("C too large");
+  if (ldy < T) return fail("zero_tail_cf: need T <= ldy");
+  RaggedLens lens;
+  if (ragged_lens(valid_len, B, T, 0, &lens)) return -1;
+  long long tail = 0;
+  for (int b = 0; b < B; ++b) tail = std::max(tail, T - lens.v[b]);
+  if (tail == 0) return 0;
+  DeviceGuard guard(device_of(y));
   if (!guard.ok) return fail("cannot select the tensor's device");
-  dim3 grid(static_cast<unsigned>((o1 - o0 + kAaTile - 1) / kAaTile), B * C);
-  aa_act_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, ldx, x0, nx, y, ldy, o0, o1, te, alpha, beta,
-                                                                     logscale, filt_up, filt_down, C, dtype == KVAE_F32);
+  dim3 grid(static_cast<unsigned>(std::min<long long>((tail + 255) / 256, 64)), C, B);
+  zero_tail_cf_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(y, C, T, ldy, lens, dtype == KVAE_F32);
   KV_CUDA(cudaGetLastError());
   ++g_launches;
   return 0;

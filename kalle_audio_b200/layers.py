@@ -144,6 +144,10 @@ class SnakeBeta(nn.Module):
                            self.alpha_logscale)
 
 
+# Inputs shorter than this run on the CUDA cores even when ``tc_precision`` sends the layer to the tensor cores.
+TC_MIN_ROWS = 64
+
+
 def _single(v):
     if isinstance(v, (tuple, list)):
         if len(v) != 1:
@@ -214,7 +218,9 @@ class _WNConvBase(nn.Module):
         return [p for p in self.parameters(recurse=False)]
 
     # --- layer-level forward -------------------------------------------------------------------
-    def forward(self, x):
+    def forward(self, x, tc=True):
+        """``tc=False`` keeps the layer on the CUDA cores whatever ``tc_precision`` says (the short clips of a ragged
+        BigVGANFlowVAE batch, which their own calls run there)."""
         _lib.require_cuda(x, type(self).__name__ + ".forward")
         if x.dim() != 3 or x.shape[1] != self.in_channels:
             raise ValueError(f"expected [B, {self.in_channels}, T], got {tuple(x.shape)}")
@@ -223,7 +229,7 @@ class _WNConvBase(nn.Module):
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.conv_params())):
             wparams = (self.weight_g, self.weight_v) if self.has_weight_norm else (self._parameters["weight"],)
             return _ConvFn.apply(self, x, self.bias, *wparams)
-        y = self._forward_tc(x)
+        y = self._forward_tc(x) if tc else None
         return y if y is not None else self._forward_impl(x)[0]
 
     # Stand-alone layers run fp32 CUDA-core arithmetic by default.  ``tc_precision`` ("bf16" | "fp32") sends layers
@@ -231,11 +237,16 @@ class _WNConvBase(nn.Module):
     # operand split, <= 1e-5); ``keep`` truncates the output to its first ``keep`` samples inside the kernel.
     tc_precision = None
 
+    def tc_layer(self) -> bool:
+        """Whether inputs of >= TC_MIN_ROWS rows go to the tcgen05 conv."""
+        return self.tc_precision is not None and not getattr(self, "_same_extra_right", 0) and \
+            bool(_lib.lib().kvae_conv1d_tc_supported(self.in_channels, self.out_channels, self.kernel_size[0],
+                                                     self.stride[0], self.dilation[0], int(self.transposed)))
+
     def _forward_tc(self, x, keep=0):
         L = _lib.lib()
         K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
-        if self.tc_precision is None or getattr(self, "_same_extra_right", 0) or x.shape[2] < 64 or \
-                not L.kvae_conv1d_tc_supported(self.in_channels, self.out_channels, K, s, d, int(self.transposed)):
+        if x.shape[2] < TC_MIN_ROWS or not self.tc_layer():
             return None
         xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
         xin = xin.contiguous()
