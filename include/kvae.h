@@ -195,21 +195,14 @@ int kvae_snake_fwd(const void* x, void* y, const float* alpha, const float* beta
 /* torch.nn.utils.weight_norm fold, dim=0: w[i,:] = v[i,:] * g[i] / ||v[i,:]||  (fp32). */
 int kvae_weight_norm_fold(const float* v, const float* g, float* w, int dim0, int inner, void* stream);
 /* WNConv1d.forward / WNConvTranspose1d.forward on [B, Cin, T] with a folded fp32 weight in torch
- * layout; fp32 arithmetic; x and y of `dtype`.  transposed = 1 selects ConvTranspose1d. */
+ * layout; fp32 arithmetic; x and y of `dtype`.  transposed = 1 selects ConvTranspose1d.  The weight is packed into
+ * scratch, then the layer runs as kvae_conv1d_win_fwd's engine 0 over all output rows. */
 int kvae_conv1d_fwd(const void* x, void* y, const float* w_folded, const float* bias, int transposed, int B,
                     int Cin, int Cout, long long T, int K, int stride, int dilation, int padding, int dtype,
                     void* scratch, size_t scratch_bytes, void* stream);
 size_t kvae_conv1d_scratch_bytes(int Cin, int Cout, int K);
-/* Same layer on the tensor cores, for channel counts that are multiples of 64 (kvae_conv1d_tc_supported): one
- * layout pass to a channels-last bf16 operand, then the tcgen05 implicit-GEMM conv writing [B, Cout, T_keep]
- * directly.  precision: KVAE_PREC_BF16 (bf16 operands) or KVAE_PREC_F32 (bf16x3 operand split, <= 1e-5).
- * T_keep (0 = all): keep only the first T_keep outputs -- the causal Conv1d / ConvTranspose1d of backup/flows.py
- * (:607-608 left padding d (K - 1); :388-389 last `stride` samples dropped) are the symmetric layer truncated. */
-size_t kvae_conv1d_tc_scratch_bytes(int B, int Cin, int Cout, long long T, int K, int precision);
+/* Whether the tcgen05 engines of kvae_conv1d_win_fwd take this layer (channel counts that are multiples of 64). */
 int kvae_conv1d_tc_supported(int Cin, int Cout, int K, int stride, int dilation, int transposed);
-int kvae_conv1d_tc_fwd(const void* x, void* y, const float* w_folded, const float* bias, int transposed, int B, int Cin,
-                       int Cout, long long T, long long T_keep, int K, int stride, int dilation, int padding, int dtype,
-                       int precision, void* scratch, size_t scratch_bytes, void* stream);
 
 /* ---- training step (BASELINE config 5) --------------------------------------------------------------
  * The reference trains the autoencoder with plain autograd through the module tree
@@ -318,13 +311,16 @@ int kvae_aa_act_ragged_fwd(const void* x, void* y, const float* alpha, const flo
    batch where the next op reads past the clip's end (the input, the input of a non-causal ConvTranspose1d
    (flows.py:336-391), the inputs of the encoder's convs (:139-189), the final output). */
 int kvae_zero_tail_cf(void* y, int B, int C, long long T, long long ldy, const int* valid_len, int dtype, void* stream);
-/* Window form of the conv layers of BigVGANFlowVAE for the streaming decoder (Conv1d / ConvTranspose1d, flows.py:336-391,
-   566-620).  kvae_conv1d_pack packs a folded fp32 weight ([Cout, Cin, K], transposed: [Cin, Cout, K]) once, for engine
-   0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split, into kvae_conv1d_packed_bytes.  kvae_conv1d_win_fwd
-   runs the conv (padding `padding`) of the T-row window x ([B, Cin] rows at pitch ldx) with those weights and writes only
-   its output rows [o0, o1) to y ([B, Cout] rows at pitch ldy, row o0 first); tcgen05 engines need o0 and o1 to be
-   multiples of the stride of a transposed conv and kvae_conv1d_win_scratch_bytes of scratch.  Per output row the
-   arithmetic is that of kvae_conv1d_fwd / kvae_conv1d_tc_fwd. */
+/* The conv layers of BigVGANFlowVAE (Conv1d / ConvTranspose1d, flows.py:336-391, 566-620; the encoder's strided
+   Conv1d).  kvae_conv1d_pack packs a folded fp32 weight ([Cout, Cin, K], transposed: [Cin, Cout, K]) for engine
+   0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split (<= 1e-5), into kvae_conv1d_packed_bytes.
+   kvae_conv1d_win_fwd runs the conv (padding `padding`) of the T-row input x ([B, Cin] rows at pitch ldx) with those
+   weights and writes only its output rows [o0, o1) to y ([B, Cout] rows at pitch ldy, row o0 first).  The whole layer is the range [0, T_out)
+   of a contiguous input; a shorter range [0, T_keep) is the causal Conv1d / ConvTranspose1d of backup/flows.py
+   (:607-608 left padding d (K - 1); :388-389 last `stride` samples dropped), the symmetric layer truncated.  The
+   streaming decoder runs windows of a stream (o0 > 0).  A strided Conv1d takes o0 = 0 only.  tcgen05 engines need
+   kvae_conv1d_tc_supported, o0 and o1 multiples of the stride of a transposed conv, an input length that is a multiple
+   of the stride of a strided conv, and kvae_conv1d_win_scratch_bytes of scratch. */
 size_t kvae_conv1d_packed_bytes(int Cin, int Cout, int K, int engine);
 int kvae_conv1d_pack(const float* w, int transposed, int Cin, int Cout, int K, int engine, void* packed,
                      size_t packed_bytes, void* stream);

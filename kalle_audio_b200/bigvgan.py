@@ -11,12 +11,13 @@ only; kept as a parameter container so checkpoints load), ``conv_pre``, ``ups``,
 Both take ``valid_len`` for a batch of clips of different lengths, each clip bit-identical to its own call (the
 ragged path below ``_run_ragged``; ``latent_length`` / ``wav_length`` give the per-clip output lengths).
 
-Every step runs through libkvae: convolutions and transposed convolutions (causal or not) through the generic conv
-kernels (``kvae_conv1d_fwd``; weight norm folded on the device), the anti-aliased Snake / SnakeBeta activation as ONE
-fused kernel (``kvae_aa_act_fwd``: x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager
-kernels and four double-rate intermediates in the reference), LeakyReLU / tanh / residual adds / the AMP average / the
-Gaussian sample as small elementwise kernels.  ``forward`` (the training pass through the flow) is not built.
-This is the parity-first form of SURVEY section 8(f) item 2: CUDA end to end, not yet on the tensor cores.
+Every step runs through libkvae: convolutions and transposed convolutions (causal or not; weight norm folded on the
+device) through the layer-level conv -- on the tensor cores for the layers whose channel counts are multiples of 64
+(``set_precision``), ``kvae_conv1d_pack`` + ``kvae_conv1d_win_fwd`` over the rows the layer keeps, otherwise the fp32
+CUDA-core ``kvae_conv1d_fwd`` -- the anti-aliased Snake / SnakeBeta activation as ONE fused kernel (``kvae_aa_act_fwd``:
+x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager kernels and four double-rate intermediates
+in the reference), LeakyReLU / tanh / residual adds / the AMP average / the Gaussian sample as small elementwise
+kernels.  ``forward`` (the training pass through the flow) is not built.
 """
 from __future__ import annotations
 
@@ -68,6 +69,17 @@ def _axpby(a: torch.Tensor, b: torch.Tensor, alpha: float, beta: float) -> torch
     _lib.check(_lib.lib().kvae_axpby(ain.data_ptr(), bin_.data_ptr(), out.data_ptr(), ain.numel(), alpha, beta,
                                      _lib.dtype_code(ain.dtype), _lib.stream_ptr(a.device)))
     return out if out.dtype == a.dtype else out.to(a.dtype)
+
+
+def _gauss_sample(mean: torch.Tensor, logs: torch.Tensor, noise: torch.Tensor) -> torch.Tensor:
+    """mean + noise * exp(logs) (flows.py:500-501), in the dtype of ``mean``."""
+    m = _k(mean)
+    lg, nz = _k(logs).to(m.dtype), _k(noise).to(m.dtype)
+    z = torch.empty_like(m)
+    if m.numel():
+        _lib.check(_lib.lib().kvae_gauss_sample(m.data_ptr(), lg.data_ptr(), nz.data_ptr(), z.data_ptr(), m.numel(),
+                                                _lib.dtype_code(m.dtype), _lib.stream_ptr(m.device)))
+    return z if z.dtype == mean.dtype else z.to(mean.dtype)
 
 
 class LeakyReLU(nn.Module):
@@ -125,16 +137,20 @@ class Activation1d(nn.Module):
         self.upsample = _Filter(up_ratio, up_kernel_size)
         self.downsample = _Down(down_ratio, down_kernel_size)
 
+    def _params(self):
+        """(alpha, beta or None, upsampling filter, low-pass filter): the fp32 device vectors the kernels read."""
+        fu = self.upsample.filter.detach().float().reshape(-1).contiguous()
+        fd = self.downsample.lowpass.filter.detach().float().reshape(-1).contiguous()
+        alpha, beta = self.act.alpha.detach().float().contiguous(), getattr(self.act, "beta", None)
+        return alpha, None if beta is None else beta.detach().float().contiguous(), fu, fd
+
     def forward(self, x):
         _lib.require_cuda(x, "Activation1d")
         xin = _k(x)
         B, C, T = xin.shape
         y = torch.empty_like(xin)
-        beta = getattr(self.act, "beta", None)
-        fu = self.upsample.filter.detach().float().reshape(-1).contiguous()
-        fd = self.downsample.lowpass.filter.detach().float().reshape(-1).contiguous()
-        _lib.check(_lib.lib().kvae_aa_act_fwd(xin.data_ptr(), y.data_ptr(), self.act.alpha.detach().float().contiguous().data_ptr(),
-                                              None if beta is None else beta.detach().float().contiguous().data_ptr(),
+        alpha, beta, fu, fd = self._params()
+        _lib.check(_lib.lib().kvae_aa_act_fwd(xin.data_ptr(), y.data_ptr(), alpha.data_ptr(), _lib.ptr(beta),
                                               int(self.act.alpha_logscale), fu.data_ptr(), fd.data_ptr(), B, C, T,
                                               _lib.dtype_code(xin.dtype), _lib.stream_ptr(x.device)))
         return y if y.dtype == x.dtype else y.to(x.dtype)
@@ -144,15 +160,26 @@ class Activation1d(nn.Module):
         forward(x[b:b+1, :, :valid_len[b]]), rows past it are 0.  x: contiguous fp32 / bf16 [B, C, T]."""
         B, C, T = x.shape
         y = torch.empty_like(x)
-        beta = getattr(self.act, "beta", None)
-        fu = self.upsample.filter.detach().float().reshape(-1).contiguous()
-        fd = self.downsample.lowpass.filter.detach().float().reshape(-1).contiguous()
-        _lib.check(_lib.lib().kvae_aa_act_ragged_fwd(x.data_ptr(), y.data_ptr(),
-                                                     self.act.alpha.detach().float().contiguous().data_ptr(),
-                                                     None if beta is None else beta.detach().float().contiguous().data_ptr(),
+        alpha, beta, fu, fd = self._params()
+        _lib.check(_lib.lib().kvae_aa_act_ragged_fwd(x.data_ptr(), y.data_ptr(), alpha.data_ptr(), _lib.ptr(beta),
                                                      int(self.act.alpha_logscale), fu.data_ptr(), fd.data_ptr(), B, C, T,
                                                      (ctypes.c_int * B)(*valid_len), _lib.dtype_code(x.dtype),
                                                      _lib.stream_ptr(x.device)))
+        return y
+
+    def window(self, win, x0, o0, o1, t_end):
+        """Outputs [o0, o1) of the stream whose absolute rows [x0, x0 + W) are the window ``win`` [B, C, W] (fp32 /
+        bf16, rows at any pitch); replicate padding at row 0 and, when t_end >= 0, at the stream end t_end
+        (kvae_aa_act_win_fwd)."""
+        B, C, W = win.shape
+        y = torch.empty((B, C, o1 - o0), dtype=win.dtype, device=win.device)
+        if win.stride(2) != 1 or win.stride(0) != C * win.stride(1):
+            win = win.contiguous()
+        alpha, beta, fu, fd = self._params()
+        _lib.check(_lib.lib().kvae_aa_act_win_fwd(win.data_ptr(), win.stride(1), x0, W, y.data_ptr(), o1 - o0, o0, o1,
+                                                  t_end, alpha.data_ptr(), _lib.ptr(beta), int(self.act.alpha_logscale),
+                                                  fu.data_ptr(), fd.data_ptr(), B, C, _lib.dtype_code(win.dtype),
+                                                  _lib.stream_ptr(win.device)))
         return y
 
 
@@ -663,12 +690,7 @@ class BigVGANFlowVAE(nn.Module):
             m_q, logs_q = torch.split(x, h.latent_dim, dim=1)
             if noise is None:
                 noise = torch.randn_like(m_q)
-            m, lg, nz = _k(m_q), _k(logs_q), _k(noise)
-            z = torch.empty_like(m)
-            _lib.check(_lib.lib().kvae_gauss_sample(m.data_ptr(), lg.to(m.dtype).data_ptr(), nz.to(m.dtype).data_ptr(),
-                                                    z.data_ptr(), m.numel(), _lib.dtype_code(m.dtype),
-                                                    _lib.stream_ptr(x.device)))
-            x = z if z.dtype == x.dtype else z.to(x.dtype)
+            x = _gauss_sample(m_q, logs_q, noise)
         else:
             assert x.size(1) == h.latent_dim, "Input must be like [B, D, H]"
         if valid_len is not None:

@@ -30,7 +30,7 @@ from typing import Dict, List, Optional
 import torch
 
 from . import _lib
-from .bigvgan import _AA_HALO, BigVGANFlowVAE, _axpby, _geom_of, _k, _module, _program, _unary
+from .bigvgan import _AA_HALO, BigVGANFlowVAE, _axpby, _gauss_sample, _geom_of, _k, _module, _program, _unary
 
 
 def bigvgan_stream_geometry(h) -> Dict[str, object]:
@@ -138,7 +138,6 @@ class BigVGANStreamingDecoder:
     def _begin(self, z: torch.Tensor) -> None:
         B, dev, dt = z.shape[0], z.device, z.dtype
         key = self._weights_key()
-        L = _lib.lib()
         if (key, B, dt, dev) != self._graph_key:
             # engines fixed and weights packed once per weight version; the captured graphs hold the packed weights'
             # addresses, so both are replaced together
@@ -147,13 +146,8 @@ class BigVGANStreamingDecoder:
                 m = _module(self.model, c)
                 self._engine[c] = m.tc_precision if m.tc_layer() else None
                 code = {None: 0, "bf16": 1, "fp32": 2}[self._engine[c]]
-                K = m.kernel_size[0]
-                nb = L.kvae_conv1d_packed_bytes(m.in_channels, m.out_channels, K, code)
-                packed = torch.empty(nb, dtype=torch.uint8, device=dev)
-                _lib.check(L.kvae_conv1d_pack(m.folded_weight().data_ptr(), int(m.transposed), m.in_channels,
-                                              m.out_channels, K, code, packed.data_ptr(), nb, _lib.stream_ptr(dev)))
-                bias = None if m.bias is None else m.bias.detach().float().contiguous().clone()
-                self._packed[c] = (packed, code, bias)
+                packed, bias = m.packed_weight(code)
+                self._packed[c] = (packed, None if bias is None else bias.clone(), code)
             self._graphs, self._static, self._graph_key = {}, {}, (key, B, dt, dev)
         self._weights = key
         self._B, self._dtype, self._dev = B, dt, dev
@@ -180,45 +174,6 @@ class BigVGANStreamingDecoder:
         self._in_static = False
 
     # ------------------------------------------------------------------ one step of every op (functional)
-    def _conv_call(self, path: str, x: torch.Tensor, padding: int, o0: int, o1: int) -> torch.Tensor:
-        """Output rows [o0, o1) of the layer's conv (padding ``padding``) of the window ``x`` (pitched rows), with the
-        weights packed at stream start."""
-        m = _module(self.model, path)
-        L = _lib.lib()
-        packed, code, bias = self._packed[path]
-        K, s, d = m.kernel_size[0], m.stride[0], m.dilation[0]
-        B, Cin, T = x.shape
-        if x.stride(2) != 1 or x.stride(0) != Cin * x.stride(1):
-            x = x.contiguous()
-        a0, a1 = o0, o1
-        if code and m.transposed:             # the tcgen05 engine emits whole stride groups
-            a0, a1 = o0 // s * s, -(-o1 // s) * s
-        y = torch.empty((B, m.out_channels, a1 - a0), dtype=x.dtype, device=x.device)
-        ns = L.kvae_conv1d_win_scratch_bytes(B, Cin, T, code)
-        scratch = torch.empty(ns, dtype=torch.uint8, device=x.device) if ns else None
-        _lib.check(L.kvae_conv1d_win_fwd(x.data_ptr(), x.stride(1), y.data_ptr(), a1 - a0, packed.data_ptr(),
-                                         _lib.ptr(bias), int(m.transposed), B, Cin, m.out_channels, T, K, s, d, padding,
-                                         a0, a1, _lib.dtype_code(x.dtype), code, _lib.ptr(scratch), ns,
-                                         _lib.stream_ptr(x.device)))
-        return y if (a0, a1) == (o0, o1) else y[:, :, o0 - a0:o1 - a0]
-
-    def _act_call(self, path: str, win: torch.Tensor, x0: int, o0: int, o1: int, t_end: int) -> torch.Tensor:
-        act = _module(self.model, path)
-        B, C, W = win.shape
-        y = torch.empty((B, C, o1 - o0), dtype=win.dtype, device=win.device)
-        if win.stride(2) != 1 or win.stride(0) != C * win.stride(1):
-            win = win.contiguous()
-        beta = getattr(act.act, "beta", None)
-        fu = act.upsample.filter.detach().float().reshape(-1).contiguous()
-        fd = act.downsample.lowpass.filter.detach().float().reshape(-1).contiguous()
-        alpha = act.act.alpha.detach().float().contiguous()
-        beta = None if beta is None else beta.detach().float().contiguous()
-        _lib.check(_lib.lib().kvae_aa_act_win_fwd(win.data_ptr(), win.stride(1), x0, W, y.data_ptr(), o1 - o0, o0, o1,
-                                                  t_end, alpha.data_ptr(), _lib.ptr(beta), int(act.act.alpha_logscale),
-                                                  fu.data_ptr(), fd.data_ptr(), B, C, _lib.dtype_code(win.dtype),
-                                                  _lib.stream_ptr(win.device)))
-        return y
-
     def _step(self, ints, tens, z: torch.Tensor, end: bool):
         """Runs every op once on its new input rows.  Pure: returns (waveform rows, new ints, new tensors)."""
         vals = {"z": z}
@@ -234,7 +189,7 @@ class BigVGANStreamingDecoder:
                     win = _cat(win, win.new_zeros((win.shape[0], win.shape[1], g.pr)))
                 n_out = win.shape[2] - g.span
                 if n_out > 0:
-                    y = self._conv_call(op[1], win, 0, 0, n_out)
+                    y = _module(self.model, op[1]).conv_rows(win, *self._packed[op[1]], 0, 0, n_out)
                     e += n_out
                     win = _rows(win, n_out)
                 else:
@@ -251,7 +206,7 @@ class BigVGANStreamingDecoder:
                 m = _module(self.model, op[1])
                 if o_max > e:
                     # only the rows not emitted yet: a causal layer skips the first `stride` rows of its window
-                    y = self._conv_call(op[1], win, g.p, e - g.s * j0, o_max - g.s * j0)
+                    y = m.conv_rows(win, *self._packed[op[1]], g.p, e - g.s * j0, o_max - g.s * j0)
                     e = o_max
                 else:
                     y = win.new_zeros((win.shape[0], m.out_channels, 0))
@@ -270,7 +225,7 @@ class BigVGANStreamingDecoder:
                     # a window away from the stream start (its outputs at o >= 5) is addressed window-relative
                     # (include/kvae.h), so a captured graph's kernel arguments hold for every later push of a phase
                     off = a
-                    y = self._act_call(op[1], win, a - off, e - off, o_max - off, R - off if end else -1)
+                    y = _module(self.model, op[1]).window(win, a - off, e - off, o_max - off, R - off if end else -1)
                     e = o_max
                 else:
                     y = win.new_zeros((win.shape[0], win.shape[1], 0))
@@ -307,14 +262,7 @@ class BigVGANStreamingDecoder:
         if not self.sample:
             return _k(z)
         D = self.model.h.latent_dim
-        m, lg = _k(z[:, :D]), _k(z[:, D:])
-        nz = _k(noise).to(m.dtype)
-        out = torch.empty_like(m)
-        if m.numel():
-            _lib.check(_lib.lib().kvae_gauss_sample(m.data_ptr(), lg.to(m.dtype).data_ptr(), nz.data_ptr(),
-                                                    out.data_ptr(), m.numel(), _lib.dtype_code(m.dtype),
-                                                    _lib.stream_ptr(z.device)))
-        return out
+        return _gauss_sample(z[:, :D], z[:, D:], noise)
 
     # ------------------------------------------------------------------ graphs
     def _sig(self) -> tuple:

@@ -1,6 +1,6 @@
 // Leaf kernels of the BigVGANFlowVAE inference path (reference /root/reference/backup/flows.py:396-529): the
 // anti-aliased periodic activation of its AMP blocks and the small elementwise steps between the convolutions.
-// The convolutions themselves run through the generic conv kernels (kvae_conv1d_fwd).
+// The convolutions themselves run through the layer-level conv (kvae_conv1d_pack + kvae_conv1d_win_fwd).
 #pragma once
 #include <cuda_bf16.h>
 #include <cstdint>

@@ -1769,39 +1769,6 @@ size_t kvae_conv1d_scratch_bytes(int Cin, int Cout, int K) {
   return align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
 }
 
-int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, int transposed, int B, int Cin,
-                    int Cout, long long T, int K, int stride, int dilation, int padding, int dtype, void* scratch,
-                    size_t scratch_bytes, void* stream) {
-  if (!x || !y || !w || !scratch) return fail("null argument");
-  if (!check_dtype(dtype)) return fail("bad dtype");
-  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
-  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
-  if (scratch_bytes < kvae_conv1d_scratch_bytes(Cin, Cout, K)) return fail("scratch too small");
-  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
-  const long long T_out = g.out_len(static_cast<int>(T));
-  if (T_out <= 0) return fail("input shorter than the kernel");
-  DeviceGuard guard(device_of(x));
-  if (!guard.ok) return fail("cannot select the tensor's device");
-  DirectLaunch L;
-  std::string err;
-  if (!prepare_direct(g, B, T, T_out, 0, L, err)) return fail(err);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  float* wd = static_cast<float*>(scratch);
-  const size_t n = static_cast<size_t>(Cin) * Cout * K;
-  pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
-      w, transposed, Cout, Cin, K, nullptr, wd);
-  KV_CUDA(cudaGetLastError());
-  DirectParams& d = L.d;
-  d.x = x; d.x_f32 = (dtype == KVAE_F32);
-  d.x_sB = static_cast<long long>(Cin) * T; d.x_sT = 1; d.x_sC = T;
-  d.w = wd; d.bias = bias;
-  d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
-  d.o_sB = static_cast<long long>(Cout) * T_out; d.o_sT = 1; d.o_sC = T_out;
-  KV_CUDA(launch_direct(L, st));
-  g_launches += 2;
-  return 0;
-}
-
 int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, float* dw, float* dbias, int transposed,
                     int B, int Cin, int Cout, long long T, int K, int stride, int dilation, int padding, int dtype,
                     void* scratch, size_t scratch_bytes, void* stream) {
@@ -1874,18 +1841,6 @@ int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, flo
   return 0;
 }
 
-// Tensor-core form of kvae_conv1d_fwd for stand-alone layers whose channel counts are multiples of 64 (the wide
-// layers of BigVGANFlowVAE): [B, Cin, T] -> channels-last bf16 operand (one layout pass) -> conv_umma2_kernel writing
-// [B, Cout, T_keep] directly.  precision KVAE_PREC_BF16: bf16 operands; KVAE_PREC_F32: bf16 x 3 split (<= 1e-5).
-// T_keep <= the conv's natural output length keeps only the first T_keep outputs (causal convs / transposed convs of
-// flows.py: symmetric padding d (K - 1), first T outputs; kernel 2 s, last s outputs dropped) without a slicing copy.
-size_t kvae_conv1d_tc_scratch_bytes(int B, int Cin, int Cout, long long T, int K, int precision) {
-  const size_t n = static_cast<size_t>(Cin) * Cout * K;
-  const int split = precision == KVAE_PREC_F32 ? 2 : 1;
-  return align_up(n * 2 * split, 1024) + (split == 2 ? align_up(n * 4, 1024) : 0) +
-         align_up(static_cast<size_t>(B) * T * Cin * 2 * split, 1024);
-}
-
 int kvae_conv1d_tc_supported(int Cin, int Cout, int K, int stride, int dilation, int transposed) {
   ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, 0};
   if (!umma_supported(g) || stride < 1 || stride > kMaxPhases || K > kMaxTaps) return 0;
@@ -1893,71 +1848,11 @@ int kvae_conv1d_tc_supported(int Cin, int Cout, int K, int stride, int dilation,
   return 1;
 }
 
-int kvae_conv1d_tc_fwd(const void* x, void* y, const float* w, const float* bias, int transposed, int B, int Cin, int Cout,
-                       long long T, long long T_keep, int K, int stride, int dilation, int padding, int dtype,
-                       int precision, void* scratch, size_t scratch_bytes, void* stream) {
-  if (!x || !y || !w || !scratch) return fail("null argument");
-  if (!check_dtype(dtype)) return fail("bad dtype");
-  if (precision != KVAE_PREC_BF16 && precision != KVAE_PREC_F32) return fail("bad precision");
-  if (B <= 0 || T <= 0) return fail("empty input");
-  if (!kvae_conv1d_tc_supported(Cin, Cout, K, stride, dilation, transposed))
-    return fail("kvae_conv1d_tc_fwd: channel counts must be multiples of 64 (use kvae_conv1d_fwd)");
-  if (scratch_bytes < kvae_conv1d_tc_scratch_bytes(B, Cin, Cout, T, K, precision)) return fail("scratch too small");
-  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
-  const long long T_nat = g.out_len(static_cast<int>(T));
-  if (T_nat <= 0) return fail("input shorter than the kernel");
-  if (T_keep <= 0) T_keep = T_nat;
-  const int P_out = transposed ? stride : 1;
-  if (T_keep > T_nat || T_keep % P_out) return fail("T_keep must be <= the output length and a multiple of the stride (transposed)");
-  DeviceGuard guard(device_of(x));
-  if (!guard.ok) return fail("cannot select the tensor's device");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int split = precision == KVAE_PREC_F32 ? 2 : 1;
-  const size_t n = static_cast<size_t>(Cin) * Cout * K;
-  uint8_t* sp = static_cast<uint8_t*>(scratch);
-  __nv_bfloat16* w_umma = reinterpret_cast<__nv_bfloat16*>(sp);
-  sp += align_up(n * 2 * split, 1024);
-  float* w_direct = nullptr;
-  if (split == 2) { w_direct = reinterpret_cast<float*>(sp); sp += align_up(n * 4, 1024); }
-  __nv_bfloat16* xcl = reinterpret_cast<__nv_bfloat16*>(sp);
-  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 4096));
-  pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, split == 2 ? nullptr : w_umma, w_direct);
-  KV_CUDA(cudaGetLastError());
-  if (split == 2) {
-    split_pack_kernel<<<blocks, 256, 0, st>>>(w_direct, K, Cin, Cout, w_umma);
-    KV_CUDA(cudaGetLastError());
-    ++g_launches;
-  }
-  {
-    dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(Cin, 32), B), block(32, 8);
-    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, Cin, static_cast<int>(T), split == 2 ? 1 : 0);
-    KV_CUDA(cudaGetLastError());
-  }
-  ConvEpilogue ep;
-  ep.bias = bias;
-  ep.out_raw = y;
-  ep.out_raw_cf = 1;
-  ep.out_raw_f32 = (dtype == KVAE_F32);
-  if (split == 2) { ep.split3 = 1; ep.precise = 1; }
-  ConvTuning2 tune;
-  ConvLaunch2 L;
-  std::string err;
-  StreamGeom sg;
-  sg.in_rows = static_cast<int>(T);
-  sg.out_q = static_cast<int>(T_keep / P_out);
-  sg.row_bias = 0;
-  const bool truncated = T_keep != T_nat;
-  if (truncated && !transposed && stride != 1) return fail("T_keep with a strided conv is unsupported");
-  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(T), w_umma, ep, tune, L, err, truncated ? &sg : nullptr)) return fail(err);
-  KV_CUDA(launch_conv_umma2(L, st));
-  g_launches += 3;
-  return 0;
-}
-
-// Window form of the layer-level conv for the streaming BigVGAN decoder: weights packed once (kvae_conv1d_pack), input
-// and output pitched, and only the output rows [o0, o1) of the conv of the T-row window computed.  Engines: 0 = CUDA
-// cores fp32 (conv_direct_kernel), 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split -- the arithmetic of kvae_conv1d_fwd /
-// kvae_conv1d_tc_fwd per output row.
+// Layer-level conv with packed weights (kvae_conv1d_pack) on the CUDA cores or the tensor cores: output rows [o0, o1)
+// of the conv of a pitched T-row input, written pitched.  Engines: 0 = CUDA cores fp32 (conv_direct_kernel),
+// 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3 split (<= 1e-5).  A whole layer is the range [0, keep) of a contiguous input:
+// keep = the natural output length, or less for the causal layers of flows.py (symmetric padding d (K - 1), first T
+// outputs; transposed kernel 2 s, last s outputs dropped), which the kernel truncates without a slicing copy.
 namespace {
 size_t win_pack_main_bytes(int Cin, int Cout, int K, int engine) {
   const size_t n = static_cast<size_t>(Cin) * Cout * K;
@@ -2004,49 +1899,40 @@ size_t kvae_conv1d_win_scratch_bytes(int B, int Cin, long long T, int engine) {
   return align_up(static_cast<size_t>(B) * T * Cin * 2 * (engine == 2 ? 2 : 1), 1024);
 }
 
-int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, const void* packed, const float* bias,
-                        int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation,
-                        int padding, long long o0, long long o1, int dtype, int engine, void* scratch,
-                        size_t scratch_bytes, void* stream) {
-  if (!x || !y || !packed) return fail("null argument");
-  if (!check_dtype(dtype)) return fail("bad dtype");
-  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
-  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
-  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
-  if (!transposed && stride != 1) return fail("window form: stride-1 or transposed convs");
-  if (ldx < T) return fail("ldx < T");
-  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
-  const long long T_nat = g.out_len(static_cast<int>(T));
-  if (o0 < 0 || o1 <= o0 || o1 > T_nat) return fail("output rows must satisfy 0 <= o0 < o1 <= the conv's output length");
-  if (ldy < o1 - o0) return fail("ldy < o1 - o0");
-  DeviceGuard guard(device_of(x));
-  if (!guard.ok) return fail("cannot select the tensor's device");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int P_out = transposed ? stride : 1;
+namespace {
+// The layer-level conv: output rows [o0, o1) of the conv of the T-row input x ([B, Cin] rows at pitch ldx) with weights
+// packed for `engine` (kvae_conv1d_pack), written to y ([B, Cout] rows at pitch ldy, row o0 first).  The callers check
+// the arguments and select the device.  A tcgen05 call for the full range [0, natural length) runs with no StreamGeom,
+// which keeps the whole-row set-up of the strided convs.
+int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, void* y, long long ldy, const void* packed,
+                const float* bias, int B, long long T, long long o0, long long o1, int dtype, int engine, void* scratch,
+                size_t scratch_bytes, cudaStream_t st) {
   if (engine == 0) {
     DirectLaunch L;
     std::string err;
     if (!prepare_direct(g, B, T, o1, o0, L, err)) return fail(err);
     DirectParams& d = L.d;
     d.x = x; d.x_f32 = (dtype == KVAE_F32);
-    d.x_sB = static_cast<long long>(Cin) * ldx; d.x_sT = 1; d.x_sC = ldx;
+    d.x_sB = static_cast<long long>(g.Cin) * ldx; d.x_sT = 1; d.x_sC = ldx;
     d.w = static_cast<const float*>(packed); d.bias = bias;
     d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
-    d.o_sB = static_cast<long long>(Cout) * ldy; d.o_sT = 1; d.o_sC = ldy;
+    d.o_sB = static_cast<long long>(g.Cout) * ldy; d.o_sT = 1; d.o_sC = ldy;
     KV_CUDA(launch_direct(L, st));
     ++g_launches;
     return 0;
   }
-  if (!kvae_conv1d_tc_supported(Cin, Cout, K, stride, dilation, transposed))
+  const int transposed = g.kind == kConvT;
+  if (!kvae_conv1d_tc_supported(g.Cin, g.Cout, g.K, g.stride, g.dilation, transposed))
     return fail("kvae_conv1d_win_fwd: the tcgen05 engine needs channel counts that are multiples of 64");
+  const int P_out = transposed ? g.stride : 1;
   if (o0 % P_out || o1 % P_out) return fail("tcgen05 engine: o0 and o1 must be multiples of the stride (transposed)");
-  if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, Cin, T, engine) || !scratch) return fail("scratch too small");
+  if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, g.Cin, T, engine) || !scratch) return fail("scratch too small");
   const int split = engine == 2 ? 2 : 1;
   __nv_bfloat16* xcl = static_cast<__nv_bfloat16*>(scratch);
   {
-    dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(Cin, 32), B), block(32, 8);
-    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, Cin, static_cast<int>(T), split == 2 ? 1 : 0,
-                                                 0, ldx);
+    dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(g.Cin, 32), B), block(32, 8);
+    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, g.Cin, static_cast<int>(T),
+                                                 split == 2 ? 1 : 0, 0, ldx);
     KV_CUDA(cudaGetLastError());
   }
   ConvEpilogue ep;
@@ -2062,12 +1948,58 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
   sg.in_rows = static_cast<int>(T);
   sg.out_q = static_cast<int>((o1 - o0) / P_out);
   sg.row_bias = static_cast<int>(o0 / P_out);
-  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(T), static_cast<const __nv_bfloat16*>(packed), ep, tune, L, err, &sg))
+  const bool full = o0 == 0 && o1 == g.out_len(static_cast<int>(T));
+  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(T), static_cast<const __nv_bfloat16*>(packed), ep, tune, L, err,
+                          full ? nullptr : &sg))
     return fail(err);
   L.p.cf_ld = ldy;
   KV_CUDA(launch_conv_umma2(L, st));
   g_launches += 2;
   return 0;
+}
+}  // namespace
+
+int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, const void* packed, const float* bias,
+                        int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation,
+                        int padding, long long o0, long long o1, int dtype, int engine, void* scratch,
+                        size_t scratch_bytes, void* stream) {
+  if (!x || !y || !packed) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
+  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
+  if (!transposed && stride != 1 && o0 != 0) return fail("a strided conv (not transposed) starts at o0 = 0");
+  if (ldx < T) return fail("ldx < T");
+  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
+  const long long T_nat = g.out_len(static_cast<int>(T));
+  if (o0 < 0 || o1 <= o0 || o1 > T_nat) return fail("output rows must satisfy 0 <= o0 < o1 <= the conv's output length");
+  if (ldy < o1 - o0) return fail("ldy < o1 - o0");
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  return conv1d_rows(g, x, ldx, y, ldy, packed, bias, B, T, o0, o1, dtype, engine, scratch, scratch_bytes,
+                     static_cast<cudaStream_t>(stream));
+}
+
+int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, int transposed, int B, int Cin,
+                    int Cout, long long T, int K, int stride, int dilation, int padding, int dtype, void* scratch,
+                    size_t scratch_bytes, void* stream) {
+  if (!x || !y || !w || !scratch) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
+  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
+  if (scratch_bytes < kvae_conv1d_scratch_bytes(Cin, Cout, K)) return fail("scratch too small");
+  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
+  const long long T_out = g.out_len(static_cast<int>(T));
+  if (T_out <= 0) return fail("input shorter than the kernel");
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t n = static_cast<size_t>(Cin) * Cout * K;
+  pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
+      w, transposed, Cout, Cin, K, nullptr, static_cast<float*>(scratch));
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return conv1d_rows(g, x, T, y, T_out, scratch, bias, B, T, 0, T_out, dtype, 0, nullptr, 0, st);
 }
 
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)

@@ -10,8 +10,9 @@ Parameters are initialised through torch's own ``nn.Conv1d`` / ``nn.ConvTranspos
 the same ``torch.manual_seed`` yields the same random-init ``state_dict`` as the reference.
 
 ``forward`` / ``backward`` of a leaf run the layer-level C-ABI kernels (fp32 arithmetic, autograd nodes
-``_SnakeFn`` / ``_ConvFn``).  The fast path is not here: ``OobleckEncoder`` / ``OobleckDecoder`` hand the whole
-stack to a fused plan (see ``_plan.py``).
+``_SnakeFn`` / ``_ConvFn``); a conv with ``tc_precision`` set runs its forward on the tensor cores through
+``packed_weight`` / ``conv_rows``, which the streaming BigVGAN decoder calls on its windows too.  The fast path is
+not here: ``OobleckEncoder`` / ``OobleckDecoder`` hand the whole stack to a fused plan (see ``_plan.py``).
 """
 from __future__ import annotations
 
@@ -233,8 +234,8 @@ class _WNConvBase(nn.Module):
         return y if y is not None else self._forward_impl(x)[0]
 
     # Stand-alone layers run fp32 CUDA-core arithmetic by default.  ``tc_precision`` ("bf16" | "fp32") sends layers
-    # whose channel counts are multiples of 64 through the tcgen05 conv instead (kvae_conv1d_tc_fwd; "fp32" = bf16x3
-    # operand split, <= 1e-5); ``keep`` truncates the output to its first ``keep`` samples inside the kernel.
+    # whose channel counts are multiples of 64 through the tcgen05 conv instead ("fp32" = bf16x3 operand split,
+    # <= 1e-5); ``keep`` truncates the output to its first ``keep`` samples inside the kernel.
     tc_precision = None
 
     def tc_layer(self) -> bool:
@@ -243,28 +244,52 @@ class _WNConvBase(nn.Module):
             bool(_lib.lib().kvae_conv1d_tc_supported(self.in_channels, self.out_channels, self.kernel_size[0],
                                                      self.stride[0], self.dilation[0], int(self.transposed)))
 
-    def _forward_tc(self, x, keep=0):
+    def packed_weight(self, engine: int):
+        """(the folded weight packed by kvae_conv1d_pack for ``engine``: 0 = CUDA cores fp32, 1 = tcgen05 bf16,
+        2 = tcgen05 bf16x3; the fp32 bias or None)"""
         L = _lib.lib()
+        w = self.folded_weight()
+        K = self.kernel_size[0]
+        nb = L.kvae_conv1d_packed_bytes(self.in_channels, self.out_channels, K, engine)
+        packed = torch.empty(nb, dtype=torch.uint8, device=w.device)
+        _lib.check(L.kvae_conv1d_pack(w.data_ptr(), int(self.transposed), self.in_channels, self.out_channels, K,
+                                      engine, packed.data_ptr(), nb, _lib.stream_ptr(w.device)))
+        return packed, None if self.bias is None else self.bias.detach().float().contiguous()
+
+    def conv_rows(self, x, packed, bias, engine: int, padding: int, o0: int, o1: int) -> torch.Tensor:
+        """Output rows [o0, o1) of this layer's conv (padding ``padding``) of x [B, Cin, T] (fp32 / bf16, rows at any
+        pitch) with the weights of ``packed_weight(engine)``: kvae_conv1d_win_fwd.  The tcgen05 engines emit whole
+        stride groups of a transposed conv; rows outside [o0, o1) are sliced off."""
+        L = _lib.lib()
+        K, s, d = self.kernel_size[0], self.stride[0], self.dilation[0]
+        B, Cin, T = x.shape
+        if x.stride(2) != 1 or x.stride(0) != Cin * x.stride(1):
+            x = x.contiguous()
+        a0, a1 = o0, o1
+        if engine and self.transposed:
+            a0, a1 = o0 // s * s, -(-o1 // s) * s
+        y = torch.empty((B, self.out_channels, a1 - a0), dtype=x.dtype, device=x.device)
+        ns = L.kvae_conv1d_win_scratch_bytes(B, Cin, T, engine)
+        scratch = torch.empty(ns, dtype=torch.uint8, device=x.device) if ns else None
+        _lib.check(L.kvae_conv1d_win_fwd(x.data_ptr(), x.stride(1), y.data_ptr(), a1 - a0, packed.data_ptr(),
+                                         _lib.ptr(bias), int(self.transposed), B, Cin, self.out_channels, T, K, s, d,
+                                         padding, a0, a1, _lib.dtype_code(x.dtype), engine, _lib.ptr(scratch), ns,
+                                         _lib.stream_ptr(x.device)))
+        return y if (a0, a1) == (o0, o1) else y[:, :, o0 - a0:o1 - a0]
+
+    def _forward_tc(self, x, keep=0):
         K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
         if x.shape[2] < TC_MIN_ROWS or not self.tc_layer():
             return None
         xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
         xin = xin.contiguous()
-        B, _, T = xin.shape
+        T = xin.shape[2]
         T_nat = (T - 1) * s - 2 * p + d * (K - 1) + 1 if self.transposed else (T + 2 * p - d * (K - 1) - 1) // s + 1
         keep = int(keep) if keep else T_nat
         if keep != T_nat and not self.transposed and s != 1:
             return None
-        prec = _lib.KVAE_PREC_BF16 if self.tc_precision == "bf16" else _lib.KVAE_PREC_F32
-        w = self.folded_weight()
-        bias = None if self.bias is None else self.bias.detach().float().contiguous()
-        y = torch.empty((B, self.out_channels, keep), dtype=xin.dtype, device=x.device)
-        nscratch = L.kvae_conv1d_tc_scratch_bytes(B, self.in_channels, self.out_channels, T, K, prec)
-        scratch = torch.empty(nscratch, dtype=torch.uint8, device=x.device)
-        _lib.check(L.kvae_conv1d_tc_fwd(xin.data_ptr(), y.data_ptr(), w.data_ptr(), _lib.ptr(bias), int(self.transposed), B,
-                                        self.in_channels, self.out_channels, T, keep, K, s, d, p,
-                                        _lib.dtype_code(xin.dtype), prec, scratch.data_ptr(), nscratch,
-                                        _lib.stream_ptr(x.device)))
+        engine = 1 if self.tc_precision == "bf16" else 2
+        y = self.conv_rows(xin, *self.packed_weight(engine), engine, p, 0, keep)
         return y if y.dtype == x.dtype else y.to(x.dtype)
 
     def _forward_impl(self, x):

@@ -8,6 +8,7 @@ import torch
 
 import helpers  # noqa: F401  (sys.path)
 import kalle_audio_b200 as k
+from kalle_audio_b200 import _lib
 from kalle_audio_b200 import bigvgan as BV
 from kalle_audio_b200.bigvgan_stream import bigvgan_stream_geometry
 from oracle import bigvgan_oracle as BO
@@ -94,3 +95,14 @@ def test_argument_checks_without_gpu():
         sd.push(torch.zeros(1, 16, 3))
     with pytest.raises(ValueError):
         k.BigVGANStreamingDecoder(m, max_frames=0)
+
+
+def test_window_conv_refuses_strided_rows_past_zero():
+    """kvae_conv1d_win_fwd runs a strided Conv1d from output row 0 only; it refuses o0 > 0 before any device access
+    (the placeholder pointers are never dereferenced)."""
+    L = _lib.lib()
+    ptr = 1 << 12
+    # Cin = Cout = 64, T = 88, K = 8, stride 4, padding 2: output rows [0, 22); rows [4, 22) asked for
+    rc = L.kvae_conv1d_win_fwd(ptr, 88, ptr, 18, ptr, None, 0, 1, 64, 64, 88, 8, 4, 1, 2, 4, 22, _lib.KVAE_F32, 1, ptr,
+                               1 << 20, None)
+    assert rc != 0 and b"strided" in L.kvae_last_error()

@@ -202,38 +202,47 @@ def test_window_activation_kernel(dev, T):
     H.report(f"window activation T={T}", "bit-exact")
 
 
+# (transposed, stride, K, dilation, padding, T, output rows [o0, o1); None = the whole natural range)
+WINDOW_CONVS = {
+    "conv": (False, 1, 7, 3, 2, 90, (5, 61)),          # stride-1 conv: rows away from both ends
+    "convT": (True, 4, 8, 1, 2, 90, (12, 68)),         # transposed conv: whole stride groups
+    "strided": (False, 4, 8, 1, 2, 88, None),          # strided conv: full range only, whole stride groups of input
+    "causal": (False, 1, 7, 3, 18, 90, (0, 90)),       # causal conv: the first T rows of the symmetric layer
+    "causalT": (True, 4, 8, 1, 0, 90, (0, 360)),       # causal transposed conv: the last `stride` rows dropped
+}
+
+
 @pytest.mark.parametrize("engine", [0, 1, 2])
-@pytest.mark.parametrize("transposed", [False, True])
-def test_window_conv_rows_equal_whole_layer(dev, engine, transposed):
+@pytest.mark.parametrize("geom", list(WINDOW_CONVS))
+def test_window_conv_rows_equal_whole_layer(dev, engine, geom):
     """kvae_conv1d_win_fwd with weights from kvae_conv1d_pack: output rows [o0, o1) of a pitched window, written to a
-    pitched output, equal those rows of the whole-layer call on the same engine."""
+    pitched output, equal those rows of the whole-layer call on the same engine (engine 0: kvae_conv1d_fwd; tcgen05:
+    the full range of a contiguous input).  The causal cases are the truncated whole-layer calls of BigVGANFlowVAE."""
     torch.manual_seed(engine)
-    Cin, Cout, T, K, s, d, p = 128, 64, 90, (8 if transposed else 7), (4 if transposed else 1), (1 if transposed else 3), 2
+    transposed, s, K, d, p, T, rows = WINDOW_CONVS[geom]
+    Cin, Cout = 128, 64
+    T_nat = (T - 1) * s - 2 * p + d * (K - 1) + 1 if transposed else (T + 2 * p - d * (K - 1) - 1) // s + 1
     w = torch.randn((Cin, Cout, K) if transposed else (Cout, Cin, K), device=dev) * 0.05
     bias = torch.randn(Cout, device=dev)
     xbuf = torch.randn(2, Cin, T + 9, device=dev)
     x = xbuf[:, :, :T]                                   # pitched: 9 spare rows per channel
     L = _lib.lib()
+    nb = L.kvae_conv1d_packed_bytes(Cin, Cout, K, engine)
+    packed = torch.empty(nb, dtype=torch.uint8, device=dev)
+    _lib.check(L.kvae_conv1d_pack(w.data_ptr(), int(transposed), Cin, Cout, K, engine, packed.data_ptr(), nb, 0))
+    ref = torch.empty(2, Cout, T_nat, device=dev)
     if engine == 0:
-        ref = torch.empty(2, Cout, (T - 1) * s - 2 * p + d * (K - 1) + 1 if transposed else T + 2 * p - d * (K - 1),
-                          device=dev)
         ns = L.kvae_conv1d_scratch_bytes(Cin, Cout, K)
         sc = torch.empty(ns, dtype=torch.uint8, device=dev)
         _lib.check(L.kvae_conv1d_fwd(x.contiguous().data_ptr(), ref.data_ptr(), w.data_ptr(), bias.data_ptr(),
                                      int(transposed), 2, Cin, Cout, T, K, s, d, p, _lib.KVAE_F32, sc.data_ptr(), ns, 0))
     else:
-        pc = _lib.KVAE_PREC_BF16 if engine == 1 else _lib.KVAE_PREC_F32
-        T_nat = (T - 1) * s - 2 * p + K if transposed else T + 2 * p - d * (K - 1)
-        ref = torch.empty(2, Cout, T_nat, device=dev)
-        ns = L.kvae_conv1d_tc_scratch_bytes(2, Cin, Cout, T, K, pc)
+        ns = L.kvae_conv1d_win_scratch_bytes(2, Cin, T, engine)
         sc = torch.empty(ns, dtype=torch.uint8, device=dev)
-        _lib.check(L.kvae_conv1d_tc_fwd(x.contiguous().data_ptr(), ref.data_ptr(), w.data_ptr(), bias.data_ptr(),
-                                        int(transposed), 2, Cin, Cout, T, 0, K, s, d, p, _lib.KVAE_F32, pc,
-                                        sc.data_ptr(), ns, 0))
-    nb = L.kvae_conv1d_packed_bytes(Cin, Cout, K, engine)
-    packed = torch.empty(nb, dtype=torch.uint8, device=dev)
-    _lib.check(L.kvae_conv1d_pack(w.data_ptr(), int(transposed), Cin, Cout, K, engine, packed.data_ptr(), nb, 0))
-    o0, o1 = (s * 3, s * 17) if transposed else (5, 61)
+        _lib.check(L.kvae_conv1d_win_fwd(x.contiguous().data_ptr(), T, ref.data_ptr(), T_nat, packed.data_ptr(),
+                                         bias.data_ptr(), int(transposed), 2, Cin, Cout, T, K, s, d, p, 0, T_nat,
+                                         _lib.KVAE_F32, engine, sc.data_ptr(), ns, 0))
+    o0, o1 = rows or (0, T_nat)
     ybuf = torch.full((2, Cout, o1 - o0 + 3), float("nan"), device=dev)
     ns = L.kvae_conv1d_win_scratch_bytes(2, Cin, T, engine)
     sc = torch.empty(max(ns, 1), dtype=torch.uint8, device=dev)
