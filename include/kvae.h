@@ -329,6 +329,22 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
                         int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation,
                         int padding, long long o0, long long o1, int dtype, int engine, void* scratch,
                         size_t scratch_bytes, void* stream);
+/* Stream form of the (non-transposed) Conv1d of BigVGANFlowVAE's encoder, strides 1 to 8 (BigVGANStreamingEncoder;
+   flows.py:139-189).  x holds the stream rows [x0, x0 + nx) ([B, Cin] rows at pitch ldx); x0 must be a multiple of
+   the stride.  The conv runs with the layer's own padding: rows < 0 read as zero and, when t_end >= 0 (the stream
+   end), so do rows >= t_end.  Output rows [o0, o1) are written to y ([B, Cout] rows at pitch ldy, row o0 first).
+   Every input row a requested output reads must lie in the window, below 0 or at or past t_end; the call checks this
+   and refuses otherwise before any device access.  Per output the kernels sum the same taps in the same order as the
+   whole-layer call, so the rows equal kvae_conv1d_win_fwd over [0, T_out) of the whole input bit for bit on every
+   engine.  The tcgen05 engines copy the window rounded up to whole stride groups, with zero rows past nx, into
+   kvae_conv1d_stream_scratch_bytes of scratch.  When no requested output reads a row below the window start, the
+   rows may be given window-relative (x0 = 0, o0 and o1 less x0 / stride, t_end less x0): the result is the same,
+   and a captured graph replays with the same arguments on every push. */
+size_t kvae_conv1d_stream_scratch_bytes(int B, int Cin, long long nx, int stride, int engine);
+int kvae_conv1d_stream_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy,
+                           long long o0, long long o1, long long t_end, const void* packed, const float* bias,
+                           int B, int Cin, int Cout, int K, int stride, int dilation, int padding,
+                           int dtype, int engine, void* scratch, size_t scratch_bytes, void* stream);
 /* op 0: nn.LeakyReLU(param) (flows.py:181-217), op 1: tanh (:527) */
 int kvae_unary_fwd(const void* x, void* y, size_t n, int op, float param, int dtype, void* stream);
 /* out = alpha*a + beta*b: the residual adds of the AMP blocks (:283) and their average (:519-520) */

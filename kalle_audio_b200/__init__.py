@@ -22,7 +22,8 @@ from .hostio import HostPipeline
 from .glue import LatentGlue
 from .dataset import LatentExtractor
 from .bigvgan import BigVGANFlowVAE
-from .bigvgan_stream import BigVGANStreamingDecoder, bigvgan_stream_geometry
+from .bigvgan_stream import (BigVGANStreamingDecoder, BigVGANStreamingEncoder, bigvgan_encode_stream_geometry,
+                             bigvgan_stream_geometry)
 from .losses import MultiResolutionSTFTLoss, SumAndDifferenceSTFTLoss, aw_fir_taps
 from .discriminators import OobleckDiscriminator, get_hinge_losses
 from .utils import load_ckpt_state_dict, prepare_audio, remove_weight_norm_from_model, to_pcm16
@@ -39,4 +40,5 @@ __all__ = [
     "snake_beta", "vae_sample", "to_pcm16", "AutoencoderTrainer", "FlatAdamW", "GradSync", "flatten_parameters",
     "gaussian_nll", "vae_sample_with_grad", "StreamingDecoder", "decoder_context_frames", "HostPipeline", "LatentGlue", "LatentExtractor", "BigVGANFlowVAE",
     "BigVGANStreamingDecoder", "bigvgan_stream_geometry", "StreamingEncoder", "encoder_context_samples",
+    "BigVGANStreamingEncoder", "bigvgan_encode_stream_geometry",
 ]

@@ -103,6 +103,11 @@ SIGNATURES = {
                                       C.c_int, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int,
                                       C.c_int, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
                                       C.c_void_p]),
+    "kvae_conv1d_stream_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int]),
+    "kvae_conv1d_stream_fwd": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_longlong,
+                                         C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int,
+                                         C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                         C.c_void_p, C.c_size_t, C.c_void_p]),
     "kvae_unary_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_int, C.c_void_p]),
     "kvae_axpby": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_int, C.c_void_p]),
     "kvae_gauss_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

@@ -400,14 +400,20 @@ def _conv_shape(h, path: str) -> Tuple[int, int, int, bool]:
 
 
 class _Geom:
-    """Integer form of one op: how many output rows are final once ``R`` input rows have arrived."""
+    """Integer form of one op: how many output rows are final once ``R`` input rows have arrived.  A conv is the strided
+    form with ``pl`` left and ``pr`` right zero rows: the decoder's stride-1 convs (symmetric or causal padding) and,
+    with an explicit ``padding``, the encoder's convs of any stride."""
 
-    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False):
+    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False,
+                 padding: Optional[int] = None):
         self.kind, self.K, self.d, self.s, self.causal = kind, K, d, s, causal
         if kind == "conv":
             self.span = d * (K - 1)
-            self.pl = self.span if causal else d * (K - 1) // 2        # left zero rows (flows.py:607-608)
-            self.pr = 0 if causal else self.pl                           # right zero rows at the stream end
+            if padding is None:
+                self.pl = self.span if causal else d * (K - 1) // 2    # left zero rows (flows.py:607-608)
+                self.pr = 0 if causal else self.pl                       # right zero rows at the stream end
+            else:
+                self.pl = self.pr = int(padding)                         # Conv1d_S (flows.py:139-172)
         elif kind == "convT":
             self.span = K - 1
             self.p = 0 if causal else (K - s) // 2                       # flows.py:336-391
@@ -417,7 +423,7 @@ class _Geom:
     def total(self, R: int) -> int:
         """Output rows of the whole-utterance op on R input rows."""
         if self.kind == "conv":
-            return R + self.pl + self.pr - self.span
+            return (R + self.pl + self.pr - self.span - 1) // self.s + 1
         if self.kind == "convT":
             return R * self.s if self.causal else (R - 1) * self.s - 2 * self.p + self.K
         return R
@@ -425,8 +431,8 @@ class _Geom:
     def avail(self, R: int, end: bool) -> int:
         if end:
             return max(0, self.total(R)) if R > 0 else 0
-        if self.kind == "conv":
-            return max(0, R + self.pl - self.span)
+        if self.kind == "conv":                 # output o reads input rows o s - pl .. o s - pl + span
+            return max(0, (R + self.pl - self.span - 1) // self.s + 1)
         if self.kind == "convT":
             return max(0, R * self.s - self.p)
         if self.kind == "act":
@@ -434,15 +440,27 @@ class _Geom:
         return R
 
     def lookahead(self) -> int:
-        """Rows after an output's own position that it reads (in output rows)."""
+        """Rows after an output's own position that it reads (in output rows; a strided conv: input rows past the
+        last of its own stride group)."""
         if self.kind == "conv":
-            return self.span - self.pl
+            return self.span - self.pl - (self.s - 1)
         if self.kind == "convT":
             return self.p
         return _AA_HALO if self.kind == "act" else 0
 
+    def reach(self) -> int:
+        """Input rows before an output's own first row that it reads (a conv's left padding)."""
+        if self.kind == "conv":
+            return self.pl
+        if self.kind == "convT":
+            return 0
+        return _AA_HALO if self.kind == "act" else 0
+
 
 def _geom_of(h, op) -> _Geom:
+    if op[0] == "conv" and len(op) > 4:                 # an encoder conv: (K, stride, dilation, padding) in the op
+        K, s, d, p = op[4]
+        return _Geom("conv", K, d, s, padding=p)
     if op[0] in ("conv", "convT"):
         K, d, s, causal = _conv_shape(h, op[1])
         return _Geom(op[0], K, d, s, causal)
@@ -474,26 +492,22 @@ def _encoder_program(h) -> Tuple[List[tuple], str]:
     return ops, "lat"
 
 
-def _lengths(h, encoder: bool, n: int) -> Dict[str, int]:
+def _lengths(h, encoder: bool, n: int, end: bool = True) -> Dict[str, int]:
     """Rows of every stream of the encoder's (``encoder``) or the decoder's op list for one clip of ``n`` input rows;
-    0 from the first op on that would get no rows (the clip's own call raises there)."""
+    0 from the first op on that would get no rows (the clip's own call raises there).  ``end=False``: the rows that are
+    final while more input may follow (the streams' integer interpreter)."""
     ops, _ = _encoder_program(h) if encoder else _program(h)
     R = {"x" if encoder else "z": int(n)}
     for op in ops:
         kind = op[0]
-        if kind == "add":
-            R[op[3]] = R[op[1]]
-        elif kind == "axpby":
+        if kind in ("add", "axpby"):
             R[op[3]] = min(R[op[1]], R[op[2]])
         elif kind == "tanh":
             R[op[2]] = R[op[1]]
         elif kind == "lrelu":
             R[op[3]] = R[op[2]]
-        elif kind == "conv" and encoder:
-            K, s, d, p = op[4]
-            R[op[3]] = max(0, (R[op[2]] + 2 * p - d * (K - 1) - 1) // s + 1) if R[op[2]] > 0 else 0
         else:
-            R[op[3]] = max(0, _geom_of(h, op).total(R[op[2]])) if R[op[2]] > 0 else 0
+            R[op[3]] = _geom_of(h, op).avail(R[op[2]], end)
     return R
 
 

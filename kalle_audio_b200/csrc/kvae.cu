@@ -1900,19 +1900,26 @@ size_t kvae_conv1d_win_scratch_bytes(int B, int Cin, long long T, int engine) {
 }
 
 namespace {
-// The layer-level conv: output rows [o0, o1) of the conv of the T-row input x ([B, Cin] rows at pitch ldx) with weights
-// packed for `engine` (kvae_conv1d_pack), written to y ([B, Cout] rows at pitch ldy, row o0 first).  The callers check
-// the arguments and select the device.  A tcgen05 call for the full range [0, natural length) runs with no StreamGeom,
-// which keeps the whole-row set-up of the strided convs.
-int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, void* y, long long ldy, const void* packed,
-                const float* bias, int B, long long T, long long o0, long long o1, int dtype, int engine, void* scratch,
-                size_t scratch_bytes, cudaStream_t st) {
+// The layer-level conv: output rows [o0, o1) of the conv of a stream whose rows [x0, x0 + nx) the window x holds
+// ([B, Cin] rows at pitch ldx), with weights packed for `engine` (kvae_conv1d_pack), written to y ([B, Cout] rows at
+// pitch ldy, row o0 first).  Rows < 0 and, when t_end >= 0, rows >= t_end read as zero; a whole layer is the window
+// x0 = 0, nx = t_end = T.  The callers check the arguments (every row the outputs read lies in the window or reads as
+// zero; x0 a multiple of the stride of a strided conv) and select the device.  A tcgen05 call for the full range of a
+// whole layer runs with no StreamGeom, which keeps the whole-row set-up of the strided convs; any other call copies its
+// window into scratch rounded up to whole stride groups, the rows that read as zero written as zeros.
+int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, long long x0, long long nx, long long t_end, void* y,
+                long long ldy, const void* packed, const float* bias, int B, long long o0, long long o1, int dtype,
+                int engine, void* scratch, size_t scratch_bytes, cudaStream_t st) {
   if (engine == 0) {
     DirectLaunch L;
     std::string err;
-    if (!prepare_direct(g, B, T, o1, o0, L, err)) return fail(err);
+    const long long x_hi = t_end < 0 ? x0 + nx : std::min(t_end, x0 + nx);
+    if (!prepare_direct(g, B, x_hi, o1, o0, L, err)) return fail(err);
     DirectParams& d = L.d;
-    d.x = x; d.x_f32 = (dtype == KVAE_F32);
+    // stream row ti is column ti - x0 of the window: the kernel reads x moved back by x0 rows.  It reads rows
+    // [0, x_hi) only; rows below the window are never read, because the lowest row of each tile's slab is a tap of
+    // its first output, and the callers check that every row a requested output reads is in the window or < 0.
+    d.x = static_cast<const char*>(x) - x0 * (dtype == KVAE_F32 ? 4 : 2); d.x_f32 = (dtype == KVAE_F32);
     d.x_sB = static_cast<long long>(g.Cin) * ldx; d.x_sT = 1; d.x_sC = ldx;
     d.w = static_cast<const float*>(packed); d.bias = bias;
     d.out_raw = y; d.out_raw_f32 = (dtype == KVAE_F32);
@@ -1923,16 +1930,25 @@ int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, void* y, long l
   }
   const int transposed = g.kind == kConvT;
   if (!kvae_conv1d_tc_supported(g.Cin, g.Cout, g.K, g.stride, g.dilation, transposed))
-    return fail("kvae_conv1d_win_fwd: the tcgen05 engine needs channel counts that are multiples of 64");
-  const int P_out = transposed ? g.stride : 1;
+    return fail("tcgen05 engine: the layer needs channel counts that are multiples of 64");
+  const int P_out = transposed ? g.stride : 1, P_in = transposed ? 1 : g.stride;
   if (o0 % P_out || o1 % P_out) return fail("tcgen05 engine: o0 and o1 must be multiples of the stride (transposed)");
-  if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, g.Cin, T, engine) || !scratch) return fail("scratch too small");
+  const bool full = x0 == 0 && t_end == nx && o0 == 0 && o1 == g.out_len(static_cast<int>(nx));
+  const long long W = full ? nx : (nx + P_in - 1) / P_in * P_in;
+  StreamGeom sg;                 // rows q of the window's output from o0 / P_out on: taps shifted by that many rows
+  sg.in_rows = static_cast<int>(W);
+  sg.out_q = static_cast<int>((o1 - o0) / P_out);
+  sg.row_bias = static_cast<int>(o0 / P_out - x0 / P_in);
+  if (sg.row_bias < -16384 || sg.row_bias > 16384) return fail("tcgen05 engine: outputs too far from the window origin");
+  if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, g.Cin, W, engine) || !scratch) return fail("scratch too small");
   const int split = engine == 2 ? 2 : 1;
   __nv_bfloat16* xcl = static_cast<__nv_bfloat16*>(scratch);
   {
-    dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(g.Cin, 32), B), block(32, 8);
-    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, g.Cin, static_cast<int>(T),
-                                                 split == 2 ? 1 : 0, 0, ldx);
+    const long long lo = std::max(0LL, -x0), hi = t_end < 0 ? nx : std::min(nx, t_end - x0);
+    dim3 grid(ceil_div(static_cast<int>(W), 32), ceil_div(g.Cin, 32), B), block(32, 8);
+    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, g.Cin, static_cast<int>(W),
+                                                 split == 2 ? 1 : 0, 0, ldx, static_cast<int>(lo),
+                                                 static_cast<int>(std::max(lo, hi)));
     KV_CUDA(cudaGetLastError());
   }
   ConvEpilogue ep;
@@ -1944,12 +1960,7 @@ int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, void* y, long l
   ConvTuning2 tune;
   ConvLaunch2 L;
   std::string err;
-  StreamGeom sg;                 // rows q of the window's output from o0 / P_out on: taps shifted by that many rows
-  sg.in_rows = static_cast<int>(T);
-  sg.out_q = static_cast<int>((o1 - o0) / P_out);
-  sg.row_bias = static_cast<int>(o0 / P_out);
-  const bool full = o0 == 0 && o1 == g.out_len(static_cast<int>(T));
-  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(T), static_cast<const __nv_bfloat16*>(packed), ep, tune, L, err,
+  if (!prepare_conv_umma2(g, xcl, B, static_cast<int>(W), static_cast<const __nv_bfloat16*>(packed), ep, tune, L, err,
                           full ? nullptr : &sg))
     return fail(err);
   L.p.cf_ld = ldy;
@@ -1976,7 +1987,43 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
   if (ldy < o1 - o0) return fail("ldy < o1 - o0");
   DeviceGuard guard(device_of(x));
   if (!guard.ok) return fail("cannot select the tensor's device");
-  return conv1d_rows(g, x, ldx, y, ldy, packed, bias, B, T, o0, o1, dtype, engine, scratch, scratch_bytes,
+  return conv1d_rows(g, x, ldx, 0, T, T, y, ldy, packed, bias, B, o0, o1, dtype, engine, scratch, scratch_bytes,
+                     static_cast<cudaStream_t>(stream));
+}
+
+size_t kvae_conv1d_stream_scratch_bytes(int B, int Cin, long long nx, int stride, int engine) {
+  if (stride < 1 || nx < 0) return 0;
+  return kvae_conv1d_win_scratch_bytes(B, Cin, (nx + stride - 1) / stride * stride, engine);
+}
+
+int kvae_conv1d_stream_fwd(const void* x, long long ldx, long long x0, long long nx, void* y, long long ldy,
+                           long long o0, long long o1, long long t_end, const void* packed, const float* bias,
+                           int B, int Cin, int Cout, int K, int stride, int dilation, int padding,
+                           int dtype, int engine, void* scratch, size_t scratch_bytes, void* stream) {
+  if (!x || !y || !packed) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || nx <= 0) return fail("empty input");
+  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
+  if (dilation < 1 || padding < 0) return fail("dilation >= 1 and padding >= 0");
+  if (x0 % stride) return fail("the window origin x0 must be a multiple of the stride");
+  if (ldx < nx) return fail("ldx < nx");
+  if (o0 < 0 || o1 <= o0) return fail("output rows must satisfy 0 <= o0 < o1");
+  if (ldy < o1 - o0) return fail("ldy < o1 - o0");
+  const long long lim = 1LL << 30;   // the kernels address rows in 32 bits
+  if (x0 <= -lim || x0 + nx >= lim || o1 * stride >= lim || t_end >= lim) return fail("rows beyond 2^30");
+  ConvGeom g{kConv, Cin, Cout, K, stride, dilation, padding};
+  if (t_end >= 0 && o1 > g.out_len(static_cast<int>(t_end))) return fail("output rows past the stream's output length");
+  // every input row a requested output reads, [o0 s - p, (o1 - 1) s - p + d (K - 1)], that does not read as zero
+  // must lie in the window
+  const long long lo = std::max(0LL, o0 * stride - padding);
+  long long hi = (o1 - 1) * stride - padding + static_cast<long long>(dilation) * (K - 1);
+  if (t_end >= 0) hi = std::min(hi, t_end - 1);
+  if (lo <= hi && (lo < x0 || hi >= x0 + nx))
+    return fail("the window does not hold every input row the requested outputs read");
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  return conv1d_rows(g, x, ldx, x0, nx, t_end, y, ldy, packed, bias, B, o0, o1, dtype, engine, scratch, scratch_bytes,
                      static_cast<cudaStream_t>(stream));
 }
 
@@ -1999,7 +2046,7 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
       w, transposed, Cout, Cin, K, nullptr, static_cast<float*>(scratch));
   KV_CUDA(cudaGetLastError());
   ++g_launches;
-  return conv1d_rows(g, x, T, y, T_out, scratch, bias, B, T, 0, T_out, dtype, 0, nullptr, 0, st);
+  return conv1d_rows(g, x, T, 0, T, T, y, T_out, scratch, bias, B, 0, T_out, dtype, 0, nullptr, 0, st);
 }
 
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)

@@ -277,6 +277,27 @@ class _WNConvBase(nn.Module):
                                          _lib.stream_ptr(x.device)))
         return y if (a0, a1) == (o0, o1) else y[:, :, o0 - a0:o1 - a0]
 
+    def conv_window(self, win, packed, bias, engine: int, x0: int, o0: int, o1: int, t_end: int) -> torch.Tensor:
+        """Output rows [o0, o1) of this Conv1d (its own stride and padding) over a stream whose rows [x0, x0 + W) the
+        window ``win`` [B, Cin, W] holds (fp32 / bf16, rows at any pitch; x0 a multiple of the stride), with the weights
+        of ``packed_weight(engine)``: kvae_conv1d_stream_fwd.  Rows < 0 and, when t_end >= 0, rows >= t_end read as
+        zero."""
+        if self.transposed:
+            raise ValueError("conv_window: a Conv1d only (transposed convs stream through conv_rows)")
+        L = _lib.lib()
+        K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
+        B, Cin, W = win.shape
+        if win.stride(2) != 1 or win.stride(0) != Cin * win.stride(1):
+            win = win.contiguous()
+        y = torch.empty((B, self.out_channels, o1 - o0), dtype=win.dtype, device=win.device)
+        ns = L.kvae_conv1d_stream_scratch_bytes(B, Cin, W, s, engine)
+        scratch = torch.empty(ns, dtype=torch.uint8, device=win.device) if ns else None
+        _lib.check(L.kvae_conv1d_stream_fwd(win.data_ptr(), win.stride(1), x0, W, y.data_ptr(), o1 - o0, o0, o1, t_end,
+                                            packed.data_ptr(), _lib.ptr(bias), B, Cin, self.out_channels, K, s, d, p,
+                                            _lib.dtype_code(win.dtype), engine, _lib.ptr(scratch), ns,
+                                            _lib.stream_ptr(win.device)))
+        return y
+
     def _forward_tc(self, x, keep=0):
         K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
         if x.shape[2] < TC_MIN_ROWS or not self.tc_layer():
