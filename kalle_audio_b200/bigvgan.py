@@ -23,7 +23,7 @@ from __future__ import annotations
 
 import ctypes
 import math
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 from torch import nn
@@ -340,80 +340,16 @@ class _FlowParams(nn.Module):
 _AA_HALO = 5            # Activation1d: y[t] reads x[t - 5 .. t + 5] (12-tap x2 filters, bigvgan.cuh)
 
 
-def _program(h) -> Tuple[List[tuple], str]:
-    """The inference path as a list of ops over named streams (flows.py:506-527 in execution order).
-
-    ("conv", module, src, dst)  ("convT", module, src, dst)  ("act", module, src, dst)
-    ("axpby", a, b, dst, alpha, beta)  ("tanh", src, dst).  Module paths are ``BigVGANFlowVAE`` attribute paths."""
-    ops: List[tuple] = [("conv", "conv_pre", "z", "x0")]
-    nk = len(h["resblock_kernel_sizes"])
-    x = "x0"
-    for i in range(len(h["upsample_rates"])):
-        up = f"u{i}"
-        ops.append(("convT", f"ups.{i}.0", x, up))
-        xs = None
-        for j, dil in enumerate(h["resblock_dilation_sizes"]):
-            rb, cur = f"resblocks.{i * nk + j}", up
-            if h["resblock"] == "1":
-                for q in range(len(dil)):
-                    t = f"{rb}.{q}"
-                    ops += [("act", f"{rb}.activations.{2 * q}", cur, t + "a1"),
-                            ("conv", f"{rb}.convs1.{q}", t + "a1", t + "c1"),
-                            ("act", f"{rb}.activations.{2 * q + 1}", t + "c1", t + "a2"),
-                            ("conv", f"{rb}.convs2.{q}", t + "a2", t + "c2"),
-                            ("axpby", t + "c2", cur, t + "r", 1.0, 1.0)]
-                    cur = t + "r"
-            else:
-                for q in range(len(dil)):
-                    t = f"{rb}.{q}"
-                    ops += [("act", f"{rb}.activations.{q}", cur, t + "a"),
-                            ("conv", f"{rb}.convs.{q}", t + "a", t + "c"),
-                            ("axpby", t + "c", cur, t + "r", 1.0, 1.0)]
-                    cur = t + "r"
-            if xs is None:
-                xs = cur
-            else:
-                ops.append(("axpby", xs, cur, f"s{i}.{j}", 1.0, 1.0))
-                xs = f"s{i}.{j}"
-        x = f"x{i + 1}"
-        ops.append(("axpby", xs, xs, x, 1.0 / nk, 0.0))
-    ops += [("act", "activation_post", x, "ap"), ("conv", "conv_post", "ap", "cp"), ("tanh", "cp", "wav")]
-    return ops, "wav"
-
-
-def _conv_shape(h, path: str) -> Tuple[int, int, int, bool]:
-    """(kernel, dilation, stride, causal) of a conv / transposed conv of the program, from ``h`` alone."""
-    causal = bool(h["causal"])
-    if path == "conv_pre":
-        return 7, 1, 1, False
-    if path == "conv_post":
-        return 7, 1, 1, causal
-    parts = path.split(".")
-    if parts[0] == "ups":
-        i = int(parts[1])
-        return int(h["upsample_kernel_sizes"][i]), 1, int(h["upsample_rates"][i]), causal
-    nk = len(h["resblock_kernel_sizes"])
-    j = int(parts[1]) % nk
-    k = int(h["resblock_kernel_sizes"][j])
-    d = int(h["resblock_dilation_sizes"][j][int(parts[3])]) if parts[2] in ("convs1", "convs") else 1
-    return k, d, 1, causal
-
-
 class _Geom:
     """Integer form of one op: how many output rows are final once ``R`` input rows have arrived.  A conv is the strided
-    form with ``pl`` left and ``pr`` right zero rows: the decoder's stride-1 convs (symmetric or causal padding) and,
-    with an explicit ``padding``, the encoder's convs of any stride."""
+    form with ``pl`` left and ``pr`` right zero rows (``padding`` on both sides, or on the left only when causal)."""
 
-    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False,
-                 padding: Optional[int] = None):
+    def __init__(self, kind: str, K: int = 1, d: int = 1, s: int = 1, causal: bool = False, padding: int = 0):
         self.kind, self.K, self.d, self.s, self.causal = kind, K, d, s, causal
         if kind == "conv":
             self.span = d * (K - 1)
-            if padding is None:
-                self.pl = self.span if causal else d * (K - 1) // 2    # left zero rows (flows.py:607-608)
-                self.pr = 0 if causal else self.pl                       # right zero rows at the stream end
-            else:
-                self.pl = self.pr = int(padding)                         # Conv1d_S (flows.py:139-172)
+            self.pl = padding
+            self.pr = 0 if causal else padding
         elif kind == "convT":
             self.span = K - 1
             self.p = 0 if causal else (K - s) // 2                       # flows.py:336-391
@@ -435,60 +371,125 @@ class _Geom:
             return max(0, (R + self.pl - self.span - 1) // self.s + 1)
         if self.kind == "convT":
             return max(0, R * self.s - self.p)
-        if self.kind == "act":
-            return max(0, R - _AA_HALO)
-        return R
+        return max(0, R - _AA_HALO)
 
     def lookahead(self) -> int:
         """Rows after an output's own position that it reads (in output rows; a strided conv: input rows past the
         last of its own stride group)."""
         if self.kind == "conv":
             return self.span - self.pl - (self.s - 1)
-        if self.kind == "convT":
-            return self.p
-        return _AA_HALO if self.kind == "act" else 0
+        return self.p if self.kind == "convT" else _AA_HALO
 
     def reach(self) -> int:
         """Input rows before an output's own first row that it reads (a conv's left padding)."""
         if self.kind == "conv":
             return self.pl
+        return 0 if self.kind == "convT" else _AA_HALO
+
+    def first_read(self, e: int) -> int:
+        """First input row that the outputs from row e on read (a conv: rounded down to a whole stride group)."""
+        if self.kind == "conv":
+            return max(0, e * self.s - self.pl) // self.s * self.s
         if self.kind == "convT":
-            return 0
-        return _AA_HALO if self.kind == "act" else 0
+            return max(0, -(-(e + self.p - self.K + 1) // self.s))
+        return max(0, e - _AA_HALO)
+
+    def origin(self, a: int) -> int:
+        """Output row that a window starting at input row a (a conv: a multiple of the stride) numbers 0 when its rows
+        are passed window-relative."""
+        if self.kind == "conv":
+            return a // self.s
+        return a * self.s if self.kind == "convT" else a
 
 
-def _geom_of(h, op) -> _Geom:
-    if op[0] == "conv" and len(op) > 4:                 # an encoder conv: (K, stride, dilation, padding) in the op
-        K, s, d, p = op[4]
-        return _Geom("conv", K, d, s, padding=p)
-    if op[0] in ("conv", "convT"):
-        K, d, s, causal = _conv_shape(h, op[1])
-        return _Geom(op[0], K, d, s, causal)
-    return _Geom(op[0])
+class _Op(NamedTuple):
+    """One op of a program over named streams.  ``kind``: conv, convT, act (``geom`` set), lrelu, tanh, or axpby
+    (``coef`` = (alpha, beta): alpha * srcs[0] + beta * srcs[1]).  ``module``: the ``BigVGANFlowVAE`` attribute path
+    of the layer that holds the weights, None for tanh / axpby."""
+    kind: str
+    module: Optional[str]
+    srcs: Tuple[str, ...]
+    dst: str
+    geom: Optional[_Geom] = None
+    coef: Optional[Tuple[float, float]] = None
 
 
-def _encoder_program(h) -> Tuple[List[tuple], str]:
-    """Encoder.generator (flows.py:191-241) as a list of ops over named streams, in execution order:
+def _program(h) -> Tuple[List[_Op], str]:
+    """The inference path as a list of ops over named streams (flows.py:506-527 in execution order), from the input
+    stream "z" to the returned output stream."""
+    causal = bool(h["causal"])
 
-    ("conv", module, src, dst, (K, stride, dilation, padding))  ("lrelu", module, src, dst)  ("add", a, b, dst).
-    Conv1d_S pads d (K - 1) // 2, so the strided conv (K = 2 f, stride f) maps L rows to (L - 2) // f + 1; the ResStack
-    has 6 layers at dilations 1 .. 32 (``Encoder``'s stacks / stack_dilation_base)."""
+    def conv(path, src, dst, K, d=1, causal=causal):
+        pad = d * (K - 1) if causal else d * (K - 1) // 2                  # Conv1d (flows.py:607-608)
+        return _Op("conv", path, (src,), dst, _Geom("conv", K, d, 1, causal, pad))
+
+    def act(path, src, dst):
+        return _Op("act", path, (src,), dst, _Geom("act"))
+
+    def add(a, b, dst, alpha=1.0, beta=1.0):
+        return _Op("axpby", None, (a, b), dst, coef=(alpha, beta))
+
+    ops = [conv("conv_pre", "z", "x0", 7, causal=False)]
+    nk = len(h["resblock_kernel_sizes"])
+    x = "x0"
+    for i, (u, ku) in enumerate(zip(h["upsample_rates"], h["upsample_kernel_sizes"])):
+        up = f"u{i}"
+        ops.append(_Op("convT", f"ups.{i}.0", (x,), up, _Geom("convT", int(ku), 1, int(u), causal)))
+        xs = None
+        for j, (k, dil) in enumerate(zip(h["resblock_kernel_sizes"], h["resblock_dilation_sizes"])):
+            rb, cur, k = f"resblocks.{i * nk + j}", up, int(k)
+            for q, d in enumerate(dil):
+                t = f"{rb}.{q}"
+                if h["resblock"] == "1":
+                    ops += [act(f"{rb}.activations.{2 * q}", cur, t + "a1"),
+                            conv(f"{rb}.convs1.{q}", t + "a1", t + "c1", k, int(d)),
+                            act(f"{rb}.activations.{2 * q + 1}", t + "c1", t + "a2"),
+                            conv(f"{rb}.convs2.{q}", t + "a2", t + "c2", k),
+                            add(t + "c2", cur, t + "r")]
+                else:
+                    ops += [act(f"{rb}.activations.{q}", cur, t + "a"),
+                            conv(f"{rb}.convs.{q}", t + "a", t + "c", k, int(d)),
+                            add(t + "c", cur, t + "r")]
+                cur = t + "r"
+            if xs is None:
+                xs = cur
+            else:
+                ops.append(add(xs, cur, f"s{i}.{j}"))
+                xs = f"s{i}.{j}"
+        x = f"x{i + 1}"
+        ops.append(add(xs, xs, x, 1.0 / nk, 0.0))
+    ops += [act("activation_post", x, "ap"), conv("conv_post", "ap", "cp", 7),
+            _Op("tanh", None, ("cp",), "wav")]
+    return ops, "wav"
+
+
+def _encoder_program(h) -> Tuple[List[_Op], str]:
+    """Encoder.generator (flows.py:191-241) as a list of ops over named streams, in execution order, from the input
+    stream "x" to "lat".  Conv1d_S pads d (K - 1) // 2, so the strided conv (K = 2 f, stride f) maps L rows to
+    (L - 2) // f + 1; the ResStack has 6 layers at dilations 1 .. 32 (``Encoder``'s stacks / stack_dilation_base)."""
     p = "audio_encoder.generator"
-    ops: List[tuple] = [("conv", f"{p}.0.layer", "x", "h", (3, 1, 1, 1)), ("lrelu", f"{p}.1", "h", "a0")]
+
+    def conv(path, src, dst, K, s=1, d=1):
+        return _Op("conv", path, (src,), dst, _Geom("conv", K, d, s, padding=d * (K - 1) // 2))
+
+    def lrelu(path, src, dst):
+        return _Op("lrelu", path, (src,), dst)
+
+    ops = [conv(f"{p}.0.layer", "x", "h", 3), lrelu(f"{p}.1", "h", "a0")]
     x, idx = "a0", 2
     for i, f in enumerate(h["downsample_rates"]):
         f = int(f)
-        ops.append(("conv", f"{p}.{idx}.layer", x, f"s{i}", (2 * f, f, 1, f - 1)))
+        ops.append(conv(f"{p}.{idx}.layer", x, f"s{i}", 2 * f, f))
         x = f"s{i}"
         for j in range(6):
             rs, t = f"{p}.{idx + 1}.layers.{j}", f"s{i}.{j}"
-            ops += [("lrelu", f"{rs}.0", x, t + "a"), ("conv", f"{rs}.1", t + "a", t + "c", (3, 1, 2 ** j, 2 ** j)),
-                    ("lrelu", f"{rs}.2", t + "c", t + "b"), ("conv", f"{rs}.3", t + "b", t + "d", (3, 1, 1, 1)),
-                    ("add", x, t + "d", t + "r")]
+            ops += [lrelu(f"{rs}.0", x, t + "a"), conv(f"{rs}.1", t + "a", t + "c", 3, d=2 ** j),
+                    lrelu(f"{rs}.2", t + "c", t + "b"), conv(f"{rs}.3", t + "b", t + "d", 3),
+                    _Op("axpby", None, (x, t + "d"), t + "r", coef=(1.0, 1.0))]
             x = t + "r"
-        ops.append(("lrelu", f"{p}.{idx + 2}", x, f"a{i + 1}"))
+        ops.append(lrelu(f"{p}.{idx + 2}", x, f"a{i + 1}"))
         x, idx = f"a{i + 1}", idx + 3
-    ops.append(("conv", f"{p}.{idx}.layer", x, "lat", (3, 1, 1, 1)))
+    ops.append(conv(f"{p}.{idx}.layer", x, "lat", 3))
     return ops, "lat"
 
 
@@ -499,15 +500,8 @@ def _lengths(h, encoder: bool, n: int, end: bool = True) -> Dict[str, int]:
     ops, _ = _encoder_program(h) if encoder else _program(h)
     R = {"x" if encoder else "z": int(n)}
     for op in ops:
-        kind = op[0]
-        if kind in ("add", "axpby"):
-            R[op[3]] = min(R[op[1]], R[op[2]])
-        elif kind == "tanh":
-            R[op[2]] = R[op[1]]
-        elif kind == "lrelu":
-            R[op[3]] = R[op[2]]
-        else:
-            R[op[3]] = _geom_of(h, op).avail(R[op[2]], end)
+        rows = min(R[s] for s in op.srcs)
+        R[op.dst] = op.geom.avail(rows, end) if op.geom else rows
     return R
 
 
@@ -583,28 +577,25 @@ def _run_ragged(model, encoder: bool, x: torch.Tensor, lens: List[int]) -> torch
     src = "x" if encoder else "z"
     last = {}                                     # stream -> index of the op that reads it last
     for i, op in enumerate(ops):
-        for name in {"add": op[1:3], "axpby": op[1:3], "tanh": op[1:2]}.get(op[0], op[2:3]):
+        for name in op.srcs:
             last[name] = i
     vals = {src: x}
     _zero_tail(x, [r[src] for r in R])
     for i, op in enumerate(ops):
-        kind = op[0]
-        if kind in ("conv", "convT"):
-            m, xin = _module(model, op[1]), vals[op[2]]
-            rows = [r[op[2]] for r in R]
-            if encoder and op[2] != src or kind == "convT" and not m.causal:
+        xin = vals[op.srcs[0]]
+        if op.kind in ("conv", "convT"):
+            rows = [r[op.srcs[0]] for r in R]
+            if encoder and op.srcs[0] != src or op.kind == "convT" and not op.geom.causal:
                 _zero_tail(xin, rows)
-            vals[op[3]] = _conv_ragged(m, xin, rows)
-        elif kind == "act":
-            vals[op[3]] = _module(model, op[1]).ragged(vals[op[2]], [r[op[2]] for r in R])
-        elif kind == "lrelu":
-            vals[op[3]] = _module(model, op[1])(vals[op[2]])
-        elif kind == "add":
-            vals[op[3]] = _axpby(vals[op[1]], vals[op[2]], 1.0, 1.0)
-        elif kind == "axpby":
-            vals[op[3]] = _axpby(vals[op[1]], vals[op[2]], op[4], op[5])
+            vals[op.dst] = _conv_ragged(_module(model, op.module), xin, rows)
+        elif op.kind == "act":
+            vals[op.dst] = _module(model, op.module).ragged(xin, [r[op.srcs[0]] for r in R])
+        elif op.kind == "lrelu":
+            vals[op.dst] = _module(model, op.module)(xin)
+        elif op.kind == "axpby":
+            vals[op.dst] = _axpby(xin, vals[op.srcs[1]], *op.coef)
         else:
-            vals[op[2]] = _unary(vals[op[1]], 1)
+            vals[op.dst] = _unary(xin, 1)
         for name in [k for k, j in last.items() if j == i]:
             vals.pop(name, None)
     y = vals[out]

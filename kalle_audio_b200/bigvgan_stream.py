@@ -2,32 +2,29 @@
 ``extract_latents`` (:494-496).
 
 A speech LM emits one latent frame per step; ``BigVGANStreamingDecoder.push`` turns each batch of frames into the
-waveform samples that became final, and ``flush`` returns the rest.  Every op of the decoder keeps the tail of its own
-input between calls and runs in *valid form* on the window ``[carry | new rows]``, so each output row is computed
-exactly once, and ``torch.cat(pushes + [flush])`` equals the whole-utterance decode bit for bit:
+waveform samples that became final, and ``flush`` returns the rest.  ``BigVGANStreamingEncoder`` does the same from
+audio to latent frames.  Both are one interpreter of an op list, the decoder's (``bigvgan._program``) or the
+encoder's (``bigvgan._encoder_program``).  Every op keeps the tail of its own input between calls and runs in *valid
+form* on the window ``[carry | new rows]``, so each output row is computed exactly once, and
+``torch.cat(pushes + [flush])`` equals the whole call bit for bit:
 
-  * convolutions (``conv_pre``, the AMP-block convs, ``conv_post``): the window starts with the left zero padding and
-    the stream end appends the right zero padding; the conv then runs with padding 0.  Per output the kernels sum the
-    same taps in the same order as the padded whole-row call (a zero row contributes ``fma(0, w, acc) == acc``).
+  * convolutions (any stride): the carry holds whole stride groups from a stream row = 0 (mod stride) on, and
+    ``kvae_conv1d_stream_fwd`` runs on ``[carry | new rows]`` with the layer's own padding.  Rows below 0 read as zero,
+    and so do rows at or past the stream end, which is given only at ``flush``.  Per output the kernels sum the same
+    taps in the same order as the whole-layer call.
   * transposed convs (``ups``): the window holds the input rows the next outputs read, the kernel runs with the layer's
     own padding and the needed output rows are kept (a causal layer skips the first ``stride`` rows of its window).
   * ``Activation1d``: ``kvae_aa_act_win_fwd``, the whole-row kernel addressed in absolute stream rows, so its
     replicate padding happens only at the true stream start and end.
-  * residual adds / the AMP average / tanh / the Gaussian sample: the library's elementwise kernels on rows that both
-    operands have.
+  * LeakyReLU / tanh / the AMP average: stateless on the new rows; residual adds: the library's elementwise kernel on
+    the rows that both operands have; the decoder's Gaussian sample: on the pushed frames.
 
-The op list comes from one description of the decoder (``bigvgan._program``) that three interpreters read: the integer
-one behind ``bigvgan_stream_geometry`` (rows available per op, lookahead), the tensor one behind the decoder, and the
-ragged whole-clip decode of ``BigVGANFlowVAE.inference_from_latents(valid_len=...)``.
-
-``BigVGANStreamingEncoder`` runs the encoder's op list (``bigvgan._encoder_program``) the same way: every conv keeps a
-carry of whole stride groups from a stream row = 0 (mod stride) on and runs ``kvae_conv1d_stream_fwd`` on
-``[carry | new rows]`` with the layer's own padding, the stream end given only at ``flush``; LeakyReLU is stateless on
-the new rows; the residual adds keep the pending rows of both operands.
+The same op lists are read by the integer interpreters behind ``bigvgan_stream_geometry`` /
+``bigvgan_encode_stream_geometry`` (rows available per op, lookahead) and by the ragged whole-clip calls of
+``BigVGANFlowVAE``.
 
 Pushes whose (size, start-up phase) was seen before replay one ``torch.cuda.CUDAGraph``; the op state lives in static
-buffers per phase, so a constant-hop stream in steady state is one graph launch per push.  Both streams share that
-machinery (``_GraphedStream``).
+buffers per phase, so a constant-hop stream in steady state is one graph launch per push.
 """
 from __future__ import annotations
 
@@ -37,8 +34,7 @@ from typing import Dict, List, Optional
 import torch
 
 from . import _lib
-from .bigvgan import (_AA_HALO, BigVGANFlowVAE, _axpby, _encoder_program, _gauss_sample, _geom_of, _k, _lengths,
-                      _module, _program, _unary)
+from .bigvgan import BigVGANFlowVAE, _axpby, _encoder_program, _gauss_sample, _k, _lengths, _module, _program, _unary
 
 
 def bigvgan_stream_geometry(h) -> Dict[str, object]:
@@ -50,22 +46,14 @@ def bigvgan_stream_geometry(h) -> Dict[str, object]:
     ratio = int(math.prod(h["upsample_rates"]))
     rate = {"z": 1}
     rows = []
-    n = 64 + 4 * ratio                       # far beyond any start-up effect
-    R = {"z": n}
     for op in ops:
-        if op[0] == "tanh":
-            R[op[2]], rate[op[2]] = R[op[1]], rate[op[1]]
-            continue
-        if op[0] == "axpby":
-            R[op[3]], rate[op[3]] = min(R[op[1]], R[op[2]]), rate[op[1]]
-            continue
-        g = _geom_of(h, op)
-        r_in = rate[op[2]]
-        R[op[3]] = g.avail(R[op[2]], False)
-        rate[op[3]] = r_in * g.s
-        rows.append({"op": op[0], "module": op[1], "rate": r_in, "rows_read": -(-(g.span + 1) // g.s),
-                     "span": g.span, "dilation": g.d, "stride": g.s, "lookahead": g.lookahead()})
-    return {"ops": rows, "ratio": ratio, "lookahead": n * ratio - R[out]}
+        g, r_in = op.geom, rate[op.srcs[0]]
+        rate[op.dst] = r_in * (g.s if g else 1)
+        if g:
+            rows.append({"op": op.kind, "module": op.module, "rate": r_in, "rows_read": -(-(g.span + 1) // g.s),
+                         "span": g.span, "dilation": g.d, "stride": g.s, "lookahead": g.lookahead()})
+    n = 64 + 4 * ratio                       # far beyond any start-up effect
+    return {"ops": rows, "ratio": ratio, "lookahead": n * ratio - _lengths(h, False, n, end=False)[out]}
 
 
 def bigvgan_encode_stream_geometry(h) -> Dict[str, object]:
@@ -81,18 +69,14 @@ def bigvgan_encode_stream_geometry(h) -> Dict[str, object]:
     rows = []
     bound = 0
     for op in ops:
-        if op[0] == "lrelu":
-            rate[op[3]], first[op[3]] = rate[op[2]], first[op[2]]
+        g, r_in = op.geom, rate[op.srcs[0]]
+        if g is None:
+            rate[op.dst], first[op.dst] = r_in, min(first[s] for s in op.srcs)
             continue
-        if op[0] == "add":
-            rate[op[3]], first[op[3]] = rate[op[1]], min(first[op[1]], first[op[2]])
-            continue
-        g = _geom_of(h, op)
-        r_in = rate[op[2]]
-        rate[op[3]] = r_in * g.s
-        first[op[3]] = first[op[2]] - g.reach() * r_in
+        rate[op.dst] = r_in * g.s
+        first[op.dst] = first[op.srcs[0]] - g.reach() * r_in
         bound += g.span * r_in
-        rows.append({"module": op[1], "rate": r_in, "span": g.span, "dilation": g.d, "stride": g.s,
+        rows.append({"module": op.module, "rate": r_in, "span": g.span, "dilation": g.d, "stride": g.s,
                      "padding": g.pl, "lookahead": g.lookahead()})
     # the fewest samples after which F frames are final (the stream's integer interpreter) is F * ratio + lookahead
     F = bound // ratio + 2
@@ -106,7 +90,6 @@ def bigvgan_encode_stream_geometry(h) -> Dict[str, object]:
     return {"ops": rows, "ratio": ratio, "lookahead": lo - F * ratio, "context": -first[out]}
 
 
-# ------------------------------------------------------------------------------------------------ the decoder
 def _cat(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     if b.shape[2] == 0:
         return a
@@ -119,33 +102,57 @@ def _rows(t: torch.Tensor, lo: int, hi: Optional[int] = None) -> torch.Tensor:
     return t[:, :, lo:hi] if (lo, hi) != (0, None) else t
 
 
-class _GraphedStream:
-    """What both streams share: engines fixed and weights packed per weight version, the check that the weights did not
-    change inside a stream, and the CUDA graphs (static state buffers per phase, capture, replay).  A subclass sets
-    ``model``, ``_params`` (the parameters its ops read) and ``_convs`` (their conv module paths), calls
-    ``_init_graphs``, and defines ``_step``, ``_head`` and ``_phase``."""
+class _OpStream:
+    """The stream interpreter of the decoder's or the encoder's op list: per-op state, one step per op kind, engines
+    fixed and weights packed per weight version, the check that the weights did not change inside a stream, and the
+    CUDA graphs (static state buffers per phase, capture, replay).  ``push`` takes [B, ``in_channels``, n] and returns
+    [B, ``out_channels``, m].  A subclass sets ``in_channels``, ``out_channels`` and ``_noun`` (what it is fed, for the
+    error messages) and may override ``_head``, the step on the pushed rows before the first op."""
 
-    def _init_graphs(self) -> None:
+    _noun = ""
+
+    def __init__(self, model: BigVGANFlowVAE, encoder: bool, use_cuda_graphs: bool):
+        if not isinstance(model, BigVGANFlowVAE):
+            raise TypeError(f"{type(self).__name__} wraps a kalle_audio_b200.BigVGANFlowVAE")
+        self.model = model
+        self.use_cuda_graphs = bool(use_cuda_graphs)
+        self._ops, self._out = _encoder_program(model.h) if encoder else _program(model.h)
+        self._src = self._ops[0].srcs[0]
+        # each op's module, resolved once: looking paths up per op and push cost an eager push more host time than
+        # the rest of its interpreter
+        self._mods = [op.module and _module(model, op.module) for op in self._ops]
+        self._convs = {op.module: m for op, m in zip(self._ops, self._mods) if op.kind in ("conv", "convT")}
+        self._params = [p for m in self._mods if m is not None for p in m.parameters()]
         self.graph_captures = 0         # CUDA graphs captured by this stream
         self.graph_replays = 0          # pushes served by replaying one
         self._graphs: Dict[tuple, dict] = {}
         self._static: Dict[tuple, List[torch.Tensor]] = {}
         self._pool = None
         self._graph_key = None
+        self.reset()
+
+    # ------------------------------------------------------------------ stream state
+    def reset(self) -> None:
+        """Drops the stream; the next push starts a new one (captured graphs stay while the weights do)."""
+        self._B = None
+        self._ints: Optional[List[tuple]] = None
+        self._tens: Optional[List[List[torch.Tensor]]] = None
+        self._in_static = False
+        self._weights = None
 
     def _weights_key(self) -> tuple:
         key = [(p.data_ptr(), p._version) for p in self._params]
-        key += [_module(self.model, c).tc_precision for c in self._convs]
+        key += [m.tc_precision for m in self._convs.values()]
         return tuple(key)
 
-    def _fix_engines(self, B: int, dt: torch.dtype, dev: torch.device) -> None:
+    def _begin(self, x: torch.Tensor) -> None:
         """Starts a stream of B clips: engines fixed per layer (``tc_layer()``) and weights packed once per weight
         version; the captured graphs hold the packed weights' addresses, so both are replaced together."""
+        B, dt, dev = x.shape[0], x.dtype, x.device
         key = self._weights_key()
         if (key, B, dt, dev) != self._graph_key:
             self._engine, self._packed = {}, {}
-            for c in self._convs:
-                m = _module(self.model, c)
+            for c, m in self._convs.items():
                 self._engine[c] = m.tc_precision if m.tc_layer() else None
                 code = {None: 0, "bf16": 1, "fp32": 2}[self._engine[c]]
                 packed, bias = m.packed_weight(code)
@@ -153,12 +160,81 @@ class _GraphedStream:
             self._graphs, self._static, self._graph_key = {}, {}, (key, B, dt, dev)
         self._weights = key
         self._B, self._dtype, self._dev = B, dt, dev
+        self._ints, self._tens = [], []
+        for op, m in zip(self._ops, self._mods):
+            if op.geom is not None:                     # (rows in, first carried row, rows out), the carry
+                ch = m.act.alpha.numel() if op.kind == "act" else m.in_channels
+                self._ints.append((0, 0, 0))
+                self._tens.append([torch.zeros((B, ch, 0), dtype=dt, device=dev)])
+            else:                                       # stateless; a residual add keeps the pending rows of both operands
+                self._ints.append(())
+                self._tens.append([None, None] if op.kind == "axpby" and op.srcs[0] != op.srcs[1] else [])
+        self._in_static = False
 
     def _check_weights(self) -> None:
         if self._weights_key() != self._weights:
             raise RuntimeError(f"{type(self).__name__}: the model's weights or precision changed inside a stream; "
                                "call reset() to start a new stream with the new weights")
 
+    # ------------------------------------------------------------------ one step of every op (functional)
+    def _step(self, ints, tens, x: torch.Tensor, end: bool):
+        """Runs every op once on its new input rows.  Pure: returns (output rows, new ints, new tensors)."""
+        vals = {self._src: x}
+        new_ints, new_tens = [], []
+        for op, m, st, ts in zip(self._ops, self._mods, ints, tens):
+            g, xin = op.geom, vals[op.srcs[0]]
+            st1, ts1 = (), []
+            if g is not None:
+                R, a, e = st
+                win = _cat(ts[0], xin)
+                R += xin.shape[2]
+                o_max = g.avail(R, end)
+                if o_max > e:
+                    # window-relative rows (include/kvae.h): no output reads a row below the window except at the
+                    # stream start, where the window starts at row 0, so a captured graph's kernel arguments hold
+                    # for every later push of a phase
+                    q = g.origin(a)
+                    o0, o1, t_end = e - q, o_max - q, R - a if end else -1
+                    if op.kind == "conv":
+                        y = m.conv_window(win, *self._packed[op.module], 0, o0, o1, t_end)
+                    elif op.kind == "convT":
+                        y = m.conv_rows(win, *self._packed[op.module], g.p, o0, o1)
+                    else:
+                        y = m.window(win, 0, o0, o1, t_end)
+                    e = o_max
+                else:
+                    y = win.new_zeros((win.shape[0], win.shape[1] if op.kind == "act" else m.out_channels, 0))
+                a1 = g.first_read(e)
+                st1, ts1 = (R, a1, e), [_rows(win, a1 - a)]
+            elif op.kind == "axpby" and op.srcs[0] != op.srcs[1]:     # a residual add: rows both operands have
+                pa = xin if ts[0] is None else _cat(ts[0], xin)
+                b_in = vals[op.srcs[1]]
+                pb = b_in if ts[1] is None else _cat(ts[1], b_in)
+                n = min(pa.shape[2], pb.shape[2])
+                y = _axpby(_rows(pa, 0, n), _rows(pb, 0, n), *op.coef) if n else pa[:, :, :0]
+                ts1 = [_rows(pa, n), _rows(pb, n)]
+            elif not xin.shape[2]:
+                y = xin
+            elif op.kind == "axpby":                    # the AMP average
+                y = _axpby(xin, xin, *op.coef)
+            elif op.kind == "lrelu":
+                y = m(xin)
+            else:                                       # tanh
+                y = _unary(xin, 1)
+            vals[op.dst] = y
+            new_ints.append(st1)
+            new_tens.append(ts1)
+        return vals[self._out], new_ints, new_tens
+
+    def _head(self, x: torch.Tensor, noise: Optional[torch.Tensor]) -> torch.Tensor:
+        return _k(x)
+
+    def _phase(self) -> tuple:
+        """What a step depends on besides the carried row counts: per op with a window, the position of the next output
+        in it and whether the window still starts at the stream start."""
+        return tuple((st[2] - op.geom.origin(st[1]), st[1] == 0) for op, st in zip(self._ops, self._ints) if op.geom)
+
+    # ------------------------------------------------------------------ CUDA graphs
     def _sig(self) -> tuple:
         return tuple(tuple(t.shape[2] if t is not None else -1 for t in ts) for ts in self._tens)
 
@@ -225,8 +301,50 @@ class _GraphedStream:
         self._tens, self._in_static = G["state"], True
         return G["out"].clone()
 
+    # ------------------------------------------------------------------ public surface
+    def _check(self, x: torch.Tensor) -> None:
+        _lib.require_cuda(x, f"{type(self).__name__}.push")
+        if x.dim() != 3 or x.shape[1] != self.in_channels:
+            raise ValueError(f"expected {self._noun} [B, {self.in_channels}, n], got {tuple(x.shape)}")
+        if x.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError(f"{self._noun} must be float32 or bfloat16")
+        if self._B is not None:
+            if x.shape[0] != self._B:
+                raise ValueError("batch size changed inside a stream")
+            if x.dtype != self._dtype or x.device != self._dev:
+                raise ValueError("dtype or device changed inside a stream")
+            self._check_weights()
 
-class BigVGANStreamingDecoder(_GraphedStream):
+    def _push(self, x: torch.Tensor, noise: Optional[torch.Tensor], chunk: int) -> torch.Tensor:
+        """x [B, in_channels, n] (and the noise of the decoder's head) in steps of at most ``chunk`` rows."""
+        if self._B is None:
+            self._begin(x)
+        pieces = []
+        for i in range(0, x.shape[2], chunk):
+            xi = x[:, :, i:i + chunk]
+            nz = None if noise is None else noise[:, :, i:i + chunk].contiguous()
+            if self.use_cuda_graphs:
+                pieces.append(self._run_graph(xi.contiguous(), nz))
+            else:
+                out, self._ints, self._tens = self._step(self._ints, self._tens, self._head(xi, nz), False)
+                pieces.append(out)
+        if not pieces:
+            return x.new_zeros((x.shape[0], self.out_channels, 0))
+        return pieces[0] if len(pieces) == 1 else torch.cat(pieces, dim=2)
+
+    @torch.no_grad()
+    def flush(self) -> torch.Tensor:
+        """The output rows still held back (right edge as in the whole call); then resets the stream."""
+        if self._B is None:
+            raise ValueError("nothing was pushed")
+        self._check_weights()
+        x = torch.zeros((self._B, self.in_channels, 0), dtype=self._dtype, device=self._dev)   # no new rows
+        out, _, _ = self._step(self._ints, self._tens, x, True)
+        self.reset()
+        return out
+
+
+class BigVGANStreamingDecoder(_OpStream):
     """Feed latent frames as they arrive; get waveform back as soon as it is final.
 
         sd = BigVGANStreamingDecoder(model)          # model: BigVGANFlowVAE on a CUDA device
@@ -246,146 +364,21 @@ class BigVGANStreamingDecoder(_GraphedStream):
     With ``do_sample`` and no ``noise``, noise is drawn per push with ``torch.randn``: the samples do not replay the
     RNG stream of one whole ``inference_from_latents`` call.  Pass ``noise`` for a reproducible stream."""
 
+    _noun = "latents"
+
     def __init__(self, model: BigVGANFlowVAE, max_frames: int = 16, use_cuda_graphs: bool = True,
                  do_sample: bool = False):
-        if not isinstance(model, BigVGANFlowVAE):
-            raise TypeError("BigVGANStreamingDecoder wraps a kalle_audio_b200.BigVGANFlowVAE")
+        super().__init__(model, False, use_cuda_graphs)
         if max_frames < 1:
             raise ValueError("max_frames must be >= 1")
-        self.model = model
         self.max_frames = int(max_frames)
-        self.use_cuda_graphs = bool(use_cuda_graphs)
         h = model.h
         self.do_sample = bool(do_sample)
         self.sample = bool(h.use_vae and do_sample)
         self.in_channels = h.latent_dim * (2 if self.sample else 1)
+        self.out_channels = 1
         self.ratio = int(math.prod(h.upsample_rates))
-        self._ops, self._out = _program(h)
-        self._geoms = [_geom_of(h, op) for op in self._ops]
         self.lookahead = int(bigvgan_stream_geometry(h)["lookahead"])
-        self._convs = sorted({op[1] for op in self._ops if op[0] in ("conv", "convT")})
-        self._params = [p for name in ("conv_pre", "ups", "resblocks", "activation_post", "conv_post")
-                        for p in getattr(model, name).parameters()]
-        self._init_graphs()
-        self.reset()
-
-    # ------------------------------------------------------------------ stream state
-    def reset(self) -> None:
-        """Drops the stream; the next push starts a new one (captured graphs stay while the weights do)."""
-        self._B = None
-        self._ints: Optional[List[tuple]] = None
-        self._tens: Optional[List[List[torch.Tensor]]] = None
-        self._in_static = False
-        self._weights = None
-
-    def _begin(self, z: torch.Tensor) -> None:
-        B, dev, dt = z.shape[0], z.device, z.dtype
-        self._fix_engines(B, dt, dev)
-        self._ints, self._tens = [], []
-        for op, g in zip(self._ops, self._geoms):
-            if op[0] == "conv":
-                ch = _module(self.model, op[1]).in_channels
-                self._ints.append((0, 0))                               # (rows in, rows out)
-                self._tens.append([torch.zeros((B, ch, g.pl), dtype=dt, device=dev)])
-            elif op[0] == "convT":
-                ch = _module(self.model, op[1]).in_channels
-                self._ints.append((0, 0, 0))                            # (rows in, first carried row, rows out)
-                self._tens.append([torch.zeros((B, ch, 0), dtype=dt, device=dev)])
-            elif op[0] == "act":
-                ch = _module(self.model, op[1]).act.alpha.numel()
-                self._ints.append((0, 0))
-                self._tens.append([torch.zeros((B, ch, 0), dtype=dt, device=dev)])
-            elif op[0] == "axpby" and op[1] != op[2]:
-                self._ints.append((0,))
-                self._tens.append([None, None])                         # pending rows of each operand
-            else:
-                self._ints.append(())
-                self._tens.append([])
-        self._in_static = False
-
-    # ------------------------------------------------------------------ one step of every op (functional)
-    def _step(self, ints, tens, z: torch.Tensor, end: bool):
-        """Runs every op once on its new input rows.  Pure: returns (waveform rows, new ints, new tensors)."""
-        vals = {"z": z}
-        new_ints, new_tens = [], []
-        for op, g, st, ts in zip(self._ops, self._geoms, ints, tens):
-            kind = op[0]
-            if kind == "conv":
-                R, e = st
-                x = vals[op[2]]
-                win = _cat(ts[0], x)
-                R += x.shape[2]
-                if end and g.pr:
-                    win = _cat(win, win.new_zeros((win.shape[0], win.shape[1], g.pr)))
-                n_out = win.shape[2] - g.span
-                if n_out > 0:
-                    y = _module(self.model, op[1]).conv_rows(win, *self._packed[op[1]], 0, 0, n_out)
-                    e += n_out
-                    win = _rows(win, n_out)
-                else:
-                    y = win.new_zeros((win.shape[0], _module(self.model, op[1]).out_channels, 0))
-                vals[op[3]] = y
-                new_ints.append((R, e))
-                new_tens.append([win])
-            elif kind == "convT":
-                R, j0, e = st
-                x = vals[op[2]]
-                win = _cat(ts[0], x)
-                R += x.shape[2]
-                o_max = g.avail(R, end)
-                m = _module(self.model, op[1])
-                if o_max > e:
-                    # only the rows not emitted yet: a causal layer skips the first `stride` rows of its window
-                    y = m.conv_rows(win, *self._packed[op[1]], g.p, e - g.s * j0, o_max - g.s * j0)
-                    e = o_max
-                else:
-                    y = win.new_zeros((win.shape[0], m.out_channels, 0))
-                j1 = max(0, -(-(e + g.p - g.K + 1) // g.s))
-                vals[op[3]] = y
-                new_ints.append((R, j1, e))
-                new_tens.append([_rows(win, j1 - j0)])
-            elif kind == "act":
-                R, e = st
-                x = vals[op[2]]
-                a = max(0, e - _AA_HALO)
-                win = _cat(ts[0], x)
-                R += x.shape[2]
-                o_max = g.avail(R, end)
-                if o_max > e:
-                    # a window away from the stream start (its outputs at o >= 5) is addressed window-relative
-                    # (include/kvae.h), so a captured graph's kernel arguments hold for every later push of a phase
-                    off = a
-                    y = _module(self.model, op[1]).window(win, a - off, e - off, o_max - off, R - off if end else -1)
-                    e = o_max
-                else:
-                    y = win.new_zeros((win.shape[0], win.shape[1], 0))
-                a1 = max(0, e - _AA_HALO)
-                vals[op[3]] = y
-                new_ints.append((R, e))
-                new_tens.append([_rows(win, a1 - a)])
-            elif kind == "axpby":
-                a_in, b_in = vals[op[1]], vals[op[2]]
-                if op[1] == op[2]:                                      # the AMP average: stateless
-                    vals[op[3]] = _axpby(a_in, b_in, op[4], op[5]) if a_in.shape[2] else a_in
-                    new_ints.append(())
-                    new_tens.append([])
-                    continue
-                pa = a_in if ts[0] is None else _cat(ts[0], a_in)
-                pb = b_in if ts[1] is None else _cat(ts[1], b_in)
-                n = min(pa.shape[2], pb.shape[2])
-                if n:
-                    y = _axpby(_rows(pa, 0, n), _rows(pb, 0, n), op[4], op[5])
-                else:
-                    y = pa[:, :, :0]
-                vals[op[3]] = y
-                new_ints.append((st[0] + n,))
-                new_tens.append([_rows(pa, n), _rows(pb, n)])
-            else:                                                       # tanh
-                x = vals[op[1]]
-                vals[op[2]] = _unary(x, 1) if x.shape[2] else x
-                new_ints.append(())
-                new_tens.append([])
-        return vals[self._out], new_ints, new_tens
 
     def _head(self, z: torch.Tensor, noise: Optional[torch.Tensor]) -> torch.Tensor:
         """The Gaussian sample of the do_sample branch (flows.py:500-501) on the pushed frames."""
@@ -394,77 +387,23 @@ class BigVGANStreamingDecoder(_GraphedStream):
         D = self.model.h.latent_dim
         return _gauss_sample(z[:, :D], z[:, D:], noise)
 
-    def _phase(self) -> tuple:
-        """What a step depends on besides the carried row counts: the position of the next output inside the window
-        and whether the window still touches the stream start."""
-        ph = []
-        for op, g, st in zip(self._ops, self._geoms, self._ints):
-            if op[0] == "convT":
-                ph.append((st[2] - g.s * st[1], st[1] == 0))
-            elif op[0] == "act":
-                a = max(0, st[1] - _AA_HALO)
-                ph.append((st[1] - a, a == 0))
-        return tuple(ph)
-
-    # ------------------------------------------------------------------ public surface
-    def _check(self, z: torch.Tensor, noise: Optional[torch.Tensor]) -> None:
-        _lib.require_cuda(z, "BigVGANStreamingDecoder.push")
-        if z.dim() != 3 or z.shape[1] != self.in_channels:
-            raise ValueError(f"expected latents [B, {self.in_channels}, n], got {tuple(z.shape)}")
-        if z.dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("latents must be float32 or bfloat16")
-        if self._B is not None:
-            if z.shape[0] != self._B:
-                raise ValueError("batch size changed inside a stream")
-            if z.dtype != self._dtype or z.device != self._dev:
-                raise ValueError("dtype or device changed inside a stream")
-            self._check_weights()
+    @torch.no_grad()
+    def push(self, latents: torch.Tensor, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """latents [B, D, n] (or [B, 2 D, n] with do_sample), n >= 0 -> the [B, 1, m] samples that became final."""
+        self._check(latents)
         if noise is not None:
             if not self.sample:
                 raise ValueError("noise is only used with do_sample on a use_vae model")
             _lib.require_cuda(noise, "BigVGANStreamingDecoder.push")
-            if tuple(noise.shape) != (z.shape[0], self.model.h.latent_dim, z.shape[2]):
+            if tuple(noise.shape) != (latents.shape[0], self.model.h.latent_dim, latents.shape[2]):
                 raise ValueError("noise must be [B, D, n] like the mean half of the latents")
-
-    @torch.no_grad()
-    def push(self, latents: torch.Tensor, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """latents [B, D, n] (or [B, 2 D, n] with do_sample), n >= 0 -> the [B, 1, m] samples that became final."""
-        self._check(latents, noise)
-        if self._B is None:
-            self._begin(latents)
         if self.sample and noise is None:
             noise = torch.randn((latents.shape[0], self.model.h.latent_dim, latents.shape[2]), dtype=latents.dtype,
                                 device=latents.device)
-        pieces = []
-        for i in range(0, latents.shape[2], self.max_frames):
-            z = latents[:, :, i:i + self.max_frames]
-            nz = None if noise is None else noise[:, :, i:i + self.max_frames].contiguous()
-            if self.use_cuda_graphs:
-                pieces.append(self._run_graph(z.contiguous(), nz))
-            else:
-                out, self._ints, self._tens = self._step(self._ints, self._tens, self._head(z, nz), False)
-                pieces.append(out)
-        if not pieces:
-            return latents.new_zeros((latents.shape[0], 1, 0))
-        return pieces[0] if len(pieces) == 1 else torch.cat(pieces, dim=2)
-
-    @torch.no_grad()
-    def flush(self) -> torch.Tensor:
-        """The samples still held back (right edge as in the whole decode); then resets the stream."""
-        if self._B is None:
-            raise ValueError("nothing was pushed")
-        self._check_weights()
-        D = self.in_channels
-        z = torch.zeros((self._B, D, 0), dtype=self._dtype, device=self._dev)
-        nz = None if not self.sample else torch.zeros((self._B, self.model.h.latent_dim, 0), dtype=self._dtype,
-                                                      device=self._dev)
-        out, _, _ = self._step(self._ints, self._tens, self._head(z, nz), True)
-        self.reset()
-        return out
+        return self._push(latents, noise, self.max_frames)
 
 
-# ------------------------------------------------------------------------------------------------ the encoder
-class BigVGANStreamingEncoder(_GraphedStream):
+class BigVGANStreamingEncoder(_OpStream):
     """Feed audio as it arrives; get latent frames back as soon as they are final.
 
         se = BigVGANStreamingEncoder(model)          # model: BigVGANFlowVAE on a CUDA device
@@ -483,147 +422,28 @@ class BigVGANStreamingEncoder(_GraphedStream):
     input length divisible by its stride; for other clips the stream equals the ragged call
     ``extract_latents(x_padded, valid_len=[L])[..., :latent_length(L)]`` on the clip padded to whole frames."""
 
+    _noun = "audio"
+
     def __init__(self, model: BigVGANFlowVAE, max_samples: Optional[int] = None, use_cuda_graphs: bool = True):
-        if not isinstance(model, BigVGANFlowVAE):
-            raise TypeError("BigVGANStreamingEncoder wraps a kalle_audio_b200.BigVGANFlowVAE")
+        super().__init__(model, True, use_cuda_graphs)
         h = model.h
         self.ratio = int(math.prod(h.downsample_rates))
         max_samples = 16 * self.ratio if max_samples is None else int(max_samples)
         if max_samples < 1:
             raise ValueError("max_samples must be >= 1")
-        self.model = model
         self.max_samples = max_samples
-        self.use_cuda_graphs = bool(use_cuda_graphs)
-        self._ops, self._out = _encoder_program(h)
-        self._geoms = [_geom_of(h, op) for op in self._ops]
         geo = bigvgan_encode_stream_geometry(h)
         self.lookahead, self.context = int(geo["lookahead"]), int(geo["context"])
-        self._convs = sorted({op[1] for op in self._ops if op[0] == "conv"})
-        self.out_channels = _module(model, self._ops[-1][1]).out_channels
-        self._params = list(model.audio_encoder.parameters())
-        self._init_graphs()
-        self.reset()
+        self.in_channels = 1
+        self.out_channels = self._mods[-1].out_channels
 
     def frames(self, n_samples: int, end: bool = False) -> int:
         """Latent frames final after ``n_samples`` samples; with ``end``, the frames of the whole clip
         (``latent_length``)."""
         return _lengths(self.model.h, True, n_samples, end)[self._out]
 
-    # ------------------------------------------------------------------ stream state
-    def reset(self) -> None:
-        """Drops the stream; the next push starts a new one (captured graphs stay while the weights do)."""
-        self._B = None
-        self._ints: Optional[List[tuple]] = None
-        self._tens: Optional[List[List[torch.Tensor]]] = None
-        self._in_static = False
-        self._weights = None
-
-    def _begin(self, x: torch.Tensor) -> None:
-        B, dev, dt = x.shape[0], x.device, x.dtype
-        self._fix_engines(B, dt, dev)
-        self._ints, self._tens = [], []
-        for op in self._ops:
-            if op[0] == "conv":
-                ch = _module(self.model, op[1]).in_channels
-                self._ints.append((0, 0, 0))                            # (rows in, first carried row, rows out)
-                self._tens.append([torch.zeros((B, ch, 0), dtype=dt, device=dev)])
-            elif op[0] == "add":
-                self._ints.append((0,))
-                self._tens.append([None, None])                         # pending rows of each operand
-            else:
-                self._ints.append(())
-                self._tens.append([])
-        self._in_static = False
-
-    # ------------------------------------------------------------------ one step of every op (functional)
-    def _step(self, ints, tens, x: torch.Tensor, end: bool):
-        """Runs every op once on its new input rows.  Pure: returns (latent rows, new ints, new tensors)."""
-        vals = {"x": x}
-        new_ints, new_tens = [], []
-        for op, g, st, ts in zip(self._ops, self._geoms, ints, tens):
-            kind = op[0]
-            if kind == "conv":
-                R, a, e = st
-                xin = vals[op[2]]
-                win = _cat(ts[0], xin)
-                R += xin.shape[2]
-                o_max = g.avail(R, end)
-                m = _module(self.model, op[1])
-                if o_max > e:
-                    # window-relative rows (include/kvae.h): the window starts at a row = 0 (mod stride), and no
-                    # output reads a row below it except at the stream start, where the window starts at row 0
-                    q = a // g.s
-                    y = m.conv_window(win, *self._packed[op[1]], 0, e - q, o_max - q, R - a if end else -1)
-                    e = o_max
-                else:
-                    y = win.new_zeros((win.shape[0], m.out_channels, 0))
-                a1 = max(0, e * g.s - g.pl) // g.s * g.s                # first row the next output reads, whole groups
-                vals[op[3]] = y
-                new_ints.append((R, a1, e))
-                new_tens.append([_rows(win, a1 - a)])
-            elif kind == "lrelu":
-                xin = vals[op[2]]
-                vals[op[3]] = _module(self.model, op[1])(xin) if xin.shape[2] else xin
-                new_ints.append(())
-                new_tens.append([])
-            else:                                                       # add: rows both operands have
-                a_in, b_in = vals[op[1]], vals[op[2]]
-                pa = a_in if ts[0] is None else _cat(ts[0], a_in)
-                pb = b_in if ts[1] is None else _cat(ts[1], b_in)
-                n = min(pa.shape[2], pb.shape[2])
-                vals[op[3]] = _axpby(_rows(pa, 0, n), _rows(pb, 0, n), 1.0, 1.0) if n else pa[:, :, :0]
-                new_ints.append((st[0] + n,))
-                new_tens.append([_rows(pa, n), _rows(pb, n)])
-        return vals[self._out], new_ints, new_tens
-
-    def _head(self, x: torch.Tensor) -> torch.Tensor:
-        return _k(x)
-
-    def _phase(self) -> tuple:
-        """What a step depends on besides the carried row counts: per conv, the next output's position in its window
-        and whether the window still starts at the stream start."""
-        return tuple((st[2] - st[1] // g.s, st[1] == 0) for op, g, st in zip(self._ops, self._geoms, self._ints)
-                     if op[0] == "conv")
-
-    # ------------------------------------------------------------------ public surface
-    def _check(self, x: torch.Tensor) -> None:
-        _lib.require_cuda(x, "BigVGANStreamingEncoder.push")
-        if x.dim() != 3 or x.shape[1] != 1:
-            raise ValueError(f"expected audio [B, 1, n], got {tuple(x.shape)}")
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("audio must be float32 or bfloat16")
-        if self._B is not None:
-            if x.shape[0] != self._B:
-                raise ValueError("batch size changed inside a stream")
-            if x.dtype != self._dtype or x.device != self._dev:
-                raise ValueError("dtype or device changed inside a stream")
-            self._check_weights()
-
     @torch.no_grad()
     def push(self, audio: torch.Tensor) -> torch.Tensor:
         """audio [B, 1, n], n >= 0 -> the [B, C_lat, m] latent frames that became final."""
         self._check(audio)
-        if self._B is None:
-            self._begin(audio)
-        pieces = []
-        for i in range(0, audio.shape[2], self.max_samples):
-            x = audio[:, :, i:i + self.max_samples]
-            if self.use_cuda_graphs:
-                pieces.append(self._run_graph(x.contiguous()))
-            else:
-                out, self._ints, self._tens = self._step(self._ints, self._tens, self._head(x), False)
-                pieces.append(out)
-        if not pieces:
-            return audio.new_zeros((audio.shape[0], self.out_channels, 0))
-        return pieces[0] if len(pieces) == 1 else torch.cat(pieces, dim=2)
-
-    @torch.no_grad()
-    def flush(self) -> torch.Tensor:
-        """The frames still held back (right edge as in the whole encode); then resets the stream."""
-        if self._B is None:
-            raise ValueError("nothing was pushed")
-        self._check_weights()
-        x = torch.zeros((self._B, 1, 0), dtype=self._dtype, device=self._dev)
-        out, _, _ = self._step(self._ints, self._tens, x, True)
-        self.reset()
-        return out
+        return self._push(audio, None, self.max_samples)

@@ -161,9 +161,11 @@ def test_weight_change_and_errors(dev):
     assert torch.equal(y, m.extract_latents(x))
 
 
-# (stride, K, dilation, padding, T): the encoder's k3 convs up to dilation 32 and its strided convs (K = 2 s)
+# (stride, K, dilation, padding, T): the encoder's k3 convs up to dilation 32 and its strided convs (K = 2 s), and the
+# decoder's stride-1 convs: a causal layer (padding d (K - 1); the stream keeps its first T rows) and a non-causal one
 STREAM_CONVS = {"k3d1": (1, 3, 1, 1, 200), "k3d32": (1, 3, 32, 32, 300), "s2": (2, 4, 1, 1, 301),
-                "s4": (4, 8, 1, 3, 403), "s5": (5, 10, 1, 4, 502)}
+                "s4": (4, 8, 1, 3, 403), "s5": (5, 10, 1, 4, 502), "causal_k7d5": (1, 7, 5, 30, 250),
+                "k11d5": (1, 11, 5, 25, 260)}
 
 
 @pytest.mark.parametrize("engine", [0, 1, 2])
