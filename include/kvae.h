@@ -319,8 +319,11 @@ int kvae_zero_tail_cf(void* y, int B, int C, long long T, long long ldy, const i
    of a contiguous input; a shorter range [0, T_keep) is the causal Conv1d / ConvTranspose1d of backup/flows.py
    (:607-608 left padding d (K - 1); :388-389 last `stride` samples dropped), the symmetric layer truncated.  The
    streaming decoder runs windows of a stream (o0 > 0).  A strided Conv1d takes o0 = 0 only.  tcgen05 engines need
-   kvae_conv1d_tc_supported, o0 and o1 multiples of the stride of a transposed conv, an input length that is a multiple
-   of the stride of a strided conv, and kvae_conv1d_win_scratch_bytes of scratch. */
+   kvae_conv1d_tc_supported and o0 and o1 multiples of the stride of a transposed conv; o1 may then reach T_out rounded
+   up to a whole stride group (a non-causal ConvTranspose1d with odd K - stride), the rows past T_out being the conv
+   continued over zero input rows.  A strided Conv1d takes any input length: its input is staged rounded up to whole
+   stride groups, zero rows past T, so the tcgen05 engines need kvae_conv1d_stream_scratch_bytes(B, Cin, T, stride,
+   engine) of scratch (kvae_conv1d_win_scratch_bytes(B, Cin, T, engine) for the other layers, the same value). */
 size_t kvae_conv1d_packed_bytes(int Cin, int Cout, int K, int engine);
 int kvae_conv1d_pack(const float* w, int transposed, int Cin, int Cout, int K, int engine, void* packed,
                      size_t packed_bytes, void* stream);

@@ -417,10 +417,10 @@ class BigVGANStreamingEncoder(_OpStream):
     samples from ``t * ratio - context`` on; ``frames(n)`` counts the frames final after n samples.  Each sample is
     encoded once: the stream keeps per-op carries, not the clip.
 
-    Engines are fixed per layer when a stream starts, as in ``BigVGANStreamingDecoder``.  ``extract_latents`` puts a
-    conv on the tensor cores only for inputs of >= 64 rows, and a strided tensor-core conv of the whole call needs an
-    input length divisible by its stride; for other clips the stream equals the ragged call
-    ``extract_latents(x_padded, valid_len=[L])[..., :latent_length(L)]`` on the clip padded to whole frames."""
+    Engines are fixed per layer when a stream starts, as in ``BigVGANStreamingDecoder``: ``extract_latents`` puts a
+    conv on the tensor cores only for inputs of >= 64 rows.  Clips that are not whole frames need nothing more: a
+    strided tensor-core conv of the whole call stages its input rounded up to whole stride groups with zero rows, as
+    the stream does."""
 
     _noun = "audio"
 

@@ -1905,8 +1905,9 @@ namespace {
 // pitch ldy, row o0 first).  Rows < 0 and, when t_end >= 0, rows >= t_end read as zero; a whole layer is the window
 // x0 = 0, nx = t_end = T.  The callers check the arguments (every row the outputs read lies in the window or reads as
 // zero; x0 a multiple of the stride of a strided conv) and select the device.  A tcgen05 call for the full range of a
-// whole layer runs with no StreamGeom, which keeps the whole-row set-up of the strided convs; any other call copies its
-// window into scratch rounded up to whole stride groups, the rows that read as zero written as zeros.
+// whole layer whose input is whole stride groups runs with no StreamGeom, which keeps the whole-row set-up of the
+// strided convs; any other call (a strided conv's input of any length included) copies its window into scratch rounded
+// up to whole stride groups, the rows that read as zero written as zeros.
 int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, long long x0, long long nx, long long t_end, void* y,
                 long long ldy, const void* packed, const float* bias, int B, long long o0, long long o1, int dtype,
                 int engine, void* scratch, size_t scratch_bytes, cudaStream_t st) {
@@ -1933,7 +1934,7 @@ int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, long long x0, l
     return fail("tcgen05 engine: the layer needs channel counts that are multiples of 64");
   const int P_out = transposed ? g.stride : 1, P_in = transposed ? 1 : g.stride;
   if (o0 % P_out || o1 % P_out) return fail("tcgen05 engine: o0 and o1 must be multiples of the stride (transposed)");
-  const bool full = x0 == 0 && t_end == nx && o0 == 0 && o1 == g.out_len(static_cast<int>(nx));
+  const bool full = x0 == 0 && t_end == nx && nx % P_in == 0 && o0 == 0 && o1 == g.out_len(static_cast<int>(nx));
   const long long W = full ? nx : (nx + P_in - 1) / P_in * P_in;
   StreamGeom sg;                 // rows q of the window's output from o0 / P_out on: taps shifted by that many rows
   sg.in_rows = static_cast<int>(W);
@@ -1983,7 +1984,12 @@ int kvae_conv1d_win_fwd(const void* x, long long ldx, void* y, long long ldy, co
   if (ldx < T) return fail("ldx < T");
   ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
   const long long T_nat = g.out_len(static_cast<int>(T));
-  if (o0 < 0 || o1 <= o0 || o1 > T_nat) return fail("output rows must satisfy 0 <= o0 < o1 <= the conv's output length");
+  // the tcgen05 engines write whole stride groups of a transposed conv: its last group may run past T_nat (odd K - s
+  // without causal truncation), those rows being the conv's own continuation over zero input rows
+  const long long o_max = transposed && engine ? (T_nat + stride - 1) / stride * stride : T_nat;
+  if (o0 < 0 || o1 <= o0 || o1 > o_max)
+    return fail("output rows must satisfy 0 <= o0 < o1 <= the conv's output length (rounded up to whole stride groups "
+                "for a transposed conv on the tcgen05 engines)");
   if (ldy < o1 - o0) return fail("ldy < o1 - o0");
   DeviceGuard guard(device_of(x));
   if (!guard.ok) return fail("cannot select the tensor's device");

@@ -269,7 +269,8 @@ class _WNConvBase(nn.Module):
         if engine and self.transposed:
             a0, a1 = o0 // s * s, -(-o1 // s) * s
         y = torch.empty((B, self.out_channels, a1 - a0), dtype=x.dtype, device=x.device)
-        ns = L.kvae_conv1d_win_scratch_bytes(B, Cin, T, engine)
+        # a strided conv's input is staged rounded up to whole stride groups
+        ns = L.kvae_conv1d_stream_scratch_bytes(B, Cin, T, 1 if self.transposed else s, engine)
         scratch = torch.empty(ns, dtype=torch.uint8, device=x.device) if ns else None
         _lib.check(L.kvae_conv1d_win_fwd(x.data_ptr(), x.stride(1), y.data_ptr(), a1 - a0, packed.data_ptr(),
                                          _lib.ptr(bias), int(self.transposed), B, Cin, self.out_channels, T, K, s, d,

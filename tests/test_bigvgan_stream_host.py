@@ -106,3 +106,26 @@ def test_window_conv_refuses_strided_rows_past_zero():
     rc = L.kvae_conv1d_win_fwd(ptr, 88, ptr, 18, ptr, None, 0, 1, 64, 64, 88, 8, 4, 1, 2, 4, 22, _lib.KVAE_F32, 1, ptr,
                                1 << 20, None)
     assert rc != 0 and b"strided" in L.kvae_last_error()
+
+
+def test_window_conv_takes_the_last_stride_group_of_a_transposed_conv():
+    """A non-causal ConvTranspose1d with odd K - stride (the bench kernel 10 at rate 5) has T_out = 5 T + 1 rows, and
+    the tcgen05 engines write whole stride groups: o1 = 5 T + 5 passes the argument checks, one row more is refused,
+    and the CUDA-core engine, which writes single rows, still stops at T_out.  No scratch is passed, so an accepted
+    call stops before any launch: at device selection without a GPU, at the scratch check with one (the placeholder
+    pointers are never dereferenced)."""
+    L = _lib.lib()
+    ptr = 1 << 12
+
+    def call(o1, engine):
+        # Cin 512 -> Cout 256, T = 70, K = 10, stride 5, padding (10 - 5) // 2 = 2: T_out = 351
+        rc = L.kvae_conv1d_win_fwd(ptr, 70, ptr, o1, ptr, None, 1, 1, 512, 256, 70, 10, 5, 1, 2, 0, o1, _lib.KVAE_F32,
+                                   engine, None, 0, None)
+        assert rc != 0
+        return L.kvae_last_error()
+
+    for engine in (1, 2):
+        err = call(355, engine)
+        assert b"output rows" not in err and (b"device" in err or b"scratch" in err), err
+        assert b"output rows" in call(356, engine)
+    assert b"output rows" in call(352, 0)

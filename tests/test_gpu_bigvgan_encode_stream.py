@@ -1,5 +1,5 @@
 """GPU checks of BigVGANStreamingEncoder: the concatenated stream equals ``extract_latents`` of the whole clip with
-``torch.equal`` (frame count included), or its ragged call for clips that are not whole frames, and the stream-form
+``torch.equal`` (frame count included), for clips that are not whole frames its ragged call too, and the stream-form
 conv kvae_conv1d_stream_fwd equals the whole-layer rows on every engine."""
 import os
 import random
@@ -102,13 +102,15 @@ def test_small_tensor_core_encoder(dev, prec):
 @pytest.mark.parametrize("prec", [None, "bf16"])
 @pytest.mark.parametrize("L", [803, 1001])
 def test_non_frame_lengths_equal_the_ragged_call(dev, prec, L):
-    """A clip that is not whole frames: the stream equals the ragged call on the clip padded to whole frames."""
+    """A clip that is not whole frames: the stream equals the whole-clip call, whose strided tensor-core convs read
+    inputs that are not whole stride groups, and the ragged call on the clip padded to whole frames."""
     m = _model(SMALL_TC, dev).set_precision(prec)
     x = 0.3 * torch.randn(1, 1, L, device=dev)
     xp = torch.nn.functional.pad(x, (0, -L % 8))
     ref = m.extract_latents(xp, valid_len=[L])[:, :, :m.latent_length(L)]
     y, _ = _stream(k.BigVGANStreamingEncoder(m), x, [L // 3, 0, L - L // 3])
     assert torch.equal(y, ref), f"max diff {(y - ref).abs().max()}"
+    assert torch.equal(m.extract_latents(x), ref)
 
 
 @pytest.mark.parametrize("prec", ["bf16", "fp32"])
