@@ -355,6 +355,50 @@ int kvae_axpby(const void* a, const void* b, void* out, size_t n, float alpha, f
 /* z = mean + noise * exp(logs) (:500-501) */
 int kvae_gauss_sample(const void* mean, const void* logs, const void* noise, void* out, size_t n, int dtype, void* stream);
 
+/* ---- BigVGANFlowVAE decoder backward (BigVGANFlowVAE.decode_with_grad: autograd of inference_from_latents,
+ * flows.py:498-529, through AMPBlock1 / AMPBlock2 :243-335) ----
+ * Backward of kvae_aa_act_fwd over whole rows (alias_free_torch Activation1d, flows.py:266, 312, 443): from the saved
+ * input x and gy ([B, C, T], both of `dtype`) gx (same dtype) and the per-channel fp32 dalpha, dbeta (SnakeBeta; Snake,
+ * beta == NULL: dalpha only, both terms of a = b).  The double-rate signal is rebuilt from x tile by tile, as the
+ * forward builds it.  dalpha / dbeta are reduced from one partial per (row, 1024-output tile) in a fixed order: two
+ * calls give the same bits.  dalpha == NULL (frozen parameters): gx only, no scratch.  scratch:
+ * kvae_aa_act_bwd_scratch_bytes. */
+size_t kvae_aa_act_bwd_scratch_bytes(int B, int C, long long T);
+int kvae_aa_act_bwd(const void* x, const void* gy, void* gx, const float* alpha, const float* beta, int logscale,
+                    const float* filt_up, const float* filt_down, float* dalpha, float* dbeta, int B, int C, long long T,
+                    int dtype, void* scratch, size_t scratch_bytes, void* stream);
+/* Backward of kvae_unary_fwd: op 0 (LeakyReLU, :181-217) takes the forward's input t = x, gx = gy * (x > 0 ? 1 :
+ * param); op 1 (tanh, :527) takes the forward's output t = y, gx = gy * (1 - y^2). */
+int kvae_unary_bwd(const void* t, const void* gy, void* gx, size_t n, int op, float param, int dtype, void* stream);
+/* Backward of the Gaussian sample (:500-501) on the latents x = [B, 2 D, T] (mean | logs): gz and noise [B, D, T];
+ * gx[:, :D] = gz, gx[:, D:] = gz * noise * exp(logs).  (The residual adds and the AMP average differentiate through
+ * kvae_axpby itself.) */
+int kvae_gauss_sample_bwd(const void* x, const void* noise, const void* gz, void* gx, int B, int D, long long T, int dtype,
+                          void* stream);
+/* Backward of a BigVGANFlowVAE conv layer (Conv1d :566-620, ConvTranspose1d :336-391; the layer geometry is the
+ * forward's: padding on both sides, a causal layer being the symmetric-padded one truncated).  gy: the gradient of
+ * the layer's output rows [0, T_gy) ([B, Cout, T_gy] of `dtype`); rows past T_gy (a causal layer's dropped rows) have
+ * none.  x: the layer's input [B, Cin, T].  w: the folded fp32 weight.  Each product is optional (NULL = skipped):
+ *   gx [B, Cin, T] (`dtype`)  the forward conv kernels under the data-gradient geometry (kvae_conv1d_dgrad_geom) on
+ *                             `engine`: 0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3;
+ *   dv (fp32, torch layout)   with g != NULL the gradients of weight_v and (dg) weight_g of the weight norm (v, g: the
+ *                             fp32 parameters), else of the plain weight.  Engine 1: tcgen05 weight gradient from
+ *                             channels-last bf16 copies of x and gy; engines 0 and 2: fp32 CUDA cores;
+ *   dbias [Cout] (fp32).
+ * A frozen layer (dv = dbias = NULL) runs no weight-gradient kernel.  tcgen05 engines: kvae_conv1d_tc_supported.
+ * scratch: kvae_conv1d_win_bwd_scratch_bytes. */
+size_t kvae_conv1d_win_bwd_scratch_bytes(int transposed, int B, int Cin, int Cout, long long T, long long T_gy, int K,
+                                         int stride, int engine);
+int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const float* w, const float* v, const float* g,
+                        void* gx, float* dv, float* dg, float* dbias, int transposed, int B, int Cin, int Cout, long long T,
+                        int K, int stride, int dilation, int padding, int dtype, int engine, void* scratch,
+                        size_t scratch_bytes, void* stream);
+/* The data-gradient geometry kvae_conv1d_win_bwd runs: gx = rows [0, T) of the Conv1d (out[0] input channels, out[1]
+ * output channels, stride out[2], dilation out[3], left padding out[4], zero rows past the end of gy) of gy with the
+ * layer's weight transposed to [Cin, Cout, K] with its taps reversed (out[5] = 1: a Conv1d of stride 1, new left
+ * padding d (K - 1) - padding), or as it is (out[5] = 0: a ConvTranspose1d, stride s, padding p). */
+int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]);
+
 /* ---- post-decode tail ---- */
 /* audio.to(float32).div(max|audio|).clamp(-1,1).mul(32767).to(int16) -- the peak-normalised PCM conversion every
  * caller of the decoder repeats (infer_0828_sigma.py:298, train_offline.py:302,319); bit-exact with torch's

@@ -111,6 +111,20 @@ SIGNATURES = {
     "kvae_unary_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_int, C.c_void_p]),
     "kvae_axpby": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_int, C.c_void_p]),
     "kvae_gauss_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "kvae_aa_act_bwd_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong]),
+    "kvae_aa_act_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p,
+                                  C.c_size_t, C.c_void_p]),
+    "kvae_unary_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_int, C.c_void_p]),
+    "kvae_gauss_sample_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong,
+                                        C.c_int, C.c_void_p]),
+    "kvae_conv1d_win_bwd_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_longlong,
+                                                       C.c_int, C.c_int, C.c_int]),
+    "kvae_conv1d_win_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                      C.c_size_t, C.c_void_p]),
+    "kvae_conv1d_dgrad_geom": (C.c_int, [C.c_int] * 7 + [C.POINTER(C.c_int * 6)]),
     "kvae_plan_out_length": (C.c_longlong, [C.c_void_p, C.c_longlong]),
     "kvae_mrstft_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int]),
     "kvae_mrstft_loss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p,

@@ -7,8 +7,10 @@ only; kept as a parameter container so checkpoints load), ``conv_pre``, ``ups``,
 
     extract_latents(x)                      :494-496   waveform [B, 1, L] -> [B, 2 D, L / prod(downsample_rates)]
     inference_from_latents(x, do_sample)    :498-529   latents -> waveform [B, 1, T * prod(upsample_rates)]
+    decode_with_grad(x, do_sample)          :498-529   the same under autograd (gradients to the latents and the
+                                                       decoder's parameters)
 
-Both take ``valid_len`` for a batch of clips of different lengths, each clip bit-identical to its own call (the
+The first two take ``valid_len`` for a batch of clips of different lengths, each clip bit-identical to its own call (the
 ragged path below ``_run_ragged``; ``latent_length`` / ``wav_length`` give the per-clip output lengths).
 
 Every step runs through libkvae: convolutions and transposed convolutions (causal or not; weight norm folded on the
@@ -17,7 +19,8 @@ device) through the layer-level conv -- on the tensor cores for the layers whose
 CUDA-core ``kvae_conv1d_fwd`` -- the anti-aliased Snake / SnakeBeta activation as ONE fused kernel (``kvae_aa_act_fwd``:
 x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager kernels and four double-rate intermediates
 in the reference), LeakyReLU / tanh / residual adds / the AMP average / the Gaussian sample as small elementwise
-kernels.  ``forward`` (the training pass through the flow) is not built.
+kernels.  Under grad mode each of them has an autograd node whose backward is a libkvae call too (the ``_*Fn`` classes
+below; ``decode_with_grad``).  ``forward`` (the training pass through the flow) is not built.
 """
 from __future__ import annotations
 
@@ -54,8 +57,15 @@ def _k(t: torch.Tensor) -> torch.Tensor:
     return t.contiguous()
 
 
+def _grad_on(*ts) -> bool:
+    """Whether a step under the current grad mode gets an autograd node: some input or parameter requires grad."""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in ts)
+
+
 def _unary(x: torch.Tensor, op: int, param: float = 0.0) -> torch.Tensor:
     _lib.require_cuda(x, "bigvgan")
+    if torch.is_grad_enabled() and _grad_on(x):
+        return _UnaryFn.apply(x, op, param)
     xin = _k(x)
     y = torch.empty_like(xin)
     _lib.check(_lib.lib().kvae_unary_fwd(xin.data_ptr(), y.data_ptr(), xin.numel(), op, float(param),
@@ -64,6 +74,8 @@ def _unary(x: torch.Tensor, op: int, param: float = 0.0) -> torch.Tensor:
 
 
 def _axpby(a: torch.Tensor, b: torch.Tensor, alpha: float, beta: float) -> torch.Tensor:
+    if torch.is_grad_enabled() and _grad_on(a, b):
+        return _AxpbyFn.apply(a, b, alpha, beta)
     ain, bin_ = _k(a), _k(b).to(_k(a).dtype)
     out = torch.empty_like(ain)
     _lib.check(_lib.lib().kvae_axpby(ain.data_ptr(), bin_.data_ptr(), out.data_ptr(), ain.numel(), alpha, beta,
@@ -73,6 +85,8 @@ def _axpby(a: torch.Tensor, b: torch.Tensor, alpha: float, beta: float) -> torch
 
 def _gauss_sample(mean: torch.Tensor, logs: torch.Tensor, noise: torch.Tensor) -> torch.Tensor:
     """mean + noise * exp(logs) (flows.py:500-501), in the dtype of ``mean``."""
+    if _grad_on(mean, logs):
+        raise RuntimeError("_gauss_sample: differentiate through _GaussSampleFn on the whole latents (decode_with_grad)")
     m = _k(mean)
     lg, nz = _k(logs).to(m.dtype), _k(noise).to(m.dtype)
     z = torch.empty_like(m)
@@ -80,6 +94,179 @@ def _gauss_sample(mean: torch.Tensor, logs: torch.Tensor, noise: torch.Tensor) -
         _lib.check(_lib.lib().kvae_gauss_sample(m.data_ptr(), lg.data_ptr(), nz.data_ptr(), z.data_ptr(), m.numel(),
                                                 _lib.dtype_code(m.dtype), _lib.stream_ptr(m.device)))
     return z if z.dtype == mean.dtype else z.to(mean.dtype)
+
+
+# ------------------------------------------------------------------------------------------------- autograd nodes
+# The backward of every step is a libkvae call (decode_with_grad; the flows.py interfaces each differentiates are cited
+# in include/kvae.h).  Forward values are those of the no-grad calls: the same kernels on the same engines.
+class _UnaryFn(torch.autograd.Function):
+    """LeakyReLU (op 0) / tanh (op 1): kvae_unary_fwd / kvae_unary_bwd (tanh's backward reads the output)."""
+
+    @staticmethod
+    def forward(ctx, x, op, param):
+        y = _unary(x, op, param)
+        ctx.op, ctx.param, ctx.x_dtype = op, param, x.dtype
+        ctx.save_for_backward(_k(x) if op == 0 else _k(y))
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        t, = ctx.saved_tensors
+        g = gy.detach().to(t.dtype).contiguous()
+        gx = torch.empty_like(t)
+        _lib.check(_lib.lib().kvae_unary_bwd(t.data_ptr(), g.data_ptr(), gx.data_ptr(), t.numel(), ctx.op, float(ctx.param),
+                                             _lib.dtype_code(t.dtype), _lib.stream_ptr(t.device)))
+        return gx.to(ctx.x_dtype), None, None
+
+
+class _AxpbyFn(torch.autograd.Function):
+    """out = alpha a + beta b: ga = alpha g and gb = beta g through kvae_axpby itself (g as is for a coefficient 1,
+    nothing for 0)."""
+
+    @staticmethod
+    def forward(ctx, a, b, alpha, beta):
+        ctx.coef, ctx.dtypes = (alpha, beta), (a.dtype, b.dtype)
+        return _axpby(a, b, alpha, beta)
+
+    @staticmethod
+    def backward(ctx, gout):
+        g = _k(gout.detach())
+        out = []
+        for c, dt, need in zip(ctx.coef, ctx.dtypes, ctx.needs_input_grad[:2]):
+            if not need or c == 0.0:
+                out.append(None)
+            elif c == 1.0:
+                out.append(g.to(dt))
+            else:
+                r = torch.empty_like(g)
+                _lib.check(_lib.lib().kvae_axpby(g.data_ptr(), g.data_ptr(), r.data_ptr(), g.numel(), c, 0.0,
+                                                 _lib.dtype_code(g.dtype), _lib.stream_ptr(g.device)))
+                out.append(r.to(dt))
+        return out[0], out[1], None, None
+
+
+class _GaussSampleFn(torch.autograd.Function):
+    """z = mean + noise exp(logs) on the latents x = [B, 2 D, T] (mean | logs): kvae_gauss_sample /
+    kvae_gauss_sample_bwd (gmean = gz, glogs = gz noise exp(logs))."""
+
+    @staticmethod
+    def forward(ctx, x, noise, D):
+        m_q, logs_q = torch.split(x, D, dim=1)
+        z = _gauss_sample(m_q, logs_q, noise)
+        xin = _k(x)
+        ctx.save_for_backward(xin, _k(noise).to(xin.dtype))
+        ctx.x_dtype = x.dtype
+        return z
+
+    @staticmethod
+    def backward(ctx, gz):
+        xin, nz = ctx.saved_tensors
+        B, D2, T = xin.shape
+        g = gz.detach().to(xin.dtype).contiguous()
+        gx = torch.empty_like(xin)
+        _lib.check(_lib.lib().kvae_gauss_sample_bwd(xin.data_ptr(), nz.data_ptr(), g.data_ptr(), gx.data_ptr(), B, D2 // 2,
+                                                    T, _lib.dtype_code(xin.dtype), _lib.stream_ptr(xin.device)))
+        return gx.to(ctx.x_dtype), None, None
+
+
+class _AaActFn(torch.autograd.Function):
+    """Activation1d: kvae_aa_act_fwd / kvae_aa_act_bwd (x saved; the double-rate signal is rebuilt in the backward)."""
+
+    @staticmethod
+    def forward(ctx, x, alpha, beta, mod):
+        y = mod(x)
+        ctx.mod, ctx.x_dtype = mod, x.dtype
+        ctx.p_dtypes = (alpha.dtype, None if beta is None else beta.dtype)
+        ctx.save_for_backward(_k(x))
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        xin, = ctx.saved_tensors
+        mod = ctx.mod
+        B, C, T = xin.shape
+        L = _lib.lib()
+        g = gy.detach().to(xin.dtype).contiguous()
+        gx = torch.empty_like(xin)
+        alpha, beta, fu, fd = mod._params()
+        want_p = any(ctx.needs_input_grad[1:3])         # frozen parameters: gx only
+        da = torch.empty(C, dtype=torch.float32, device=xin.device) if want_p else None
+        db = None if beta is None or not want_p else torch.empty_like(da)
+        ns = L.kvae_aa_act_bwd_scratch_bytes(B, C, T) if want_p else 0
+        scratch = torch.empty(ns, dtype=torch.uint8, device=xin.device) if want_p else None
+        _lib.check(L.kvae_aa_act_bwd(xin.data_ptr(), g.data_ptr(), gx.data_ptr(), alpha.data_ptr(), _lib.ptr(beta),
+                                     int(mod.act.alpha_logscale), fu.data_ptr(), fd.data_ptr(), _lib.ptr(da),
+                                     _lib.ptr(db), B, C, T, _lib.dtype_code(xin.dtype), _lib.ptr(scratch), ns,
+                                     _lib.stream_ptr(xin.device)))
+        if not want_p:
+            return gx.to(ctx.x_dtype), None, None, None
+        return (gx.to(ctx.x_dtype), da.to(ctx.p_dtypes[0]), None if db is None else db.to(ctx.p_dtypes[1]), None)
+
+
+class _BVConvFn(torch.autograd.Function):
+    """Conv1d / ConvTranspose1d of BigVGANFlowVAE: the forward is the no-grad call (grad mode is off inside),
+    the backward through kvae_conv1d_win_bwd on the same engine (0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05
+    bf16x3); no weight-gradient work when no conv parameter requires grad."""
+
+    @staticmethod
+    def forward(ctx, mod, x, tc, bias, *wparams):
+        y, engine = mod(x, tc), _engine_of(mod, x, tc)
+        ctx.mod, ctx.engine, ctx.x_dtype, ctx.T_gy = mod, engine, x.dtype, y.shape[2]
+        ctx.has_bias = bias is not None
+        xin = _k(x)
+        ctx.save_for_backward(xin, mod.folded_weight(), *[p.detach() for p in wparams])
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        mod = ctx.mod
+        xin, w, *wparams = ctx.saved_tensors
+        L = _lib.lib()
+        B, Cin, T = xin.shape
+        K, s, d, p = mod.kernel_size[0], mod.stride[0], mod.dilation[0], mod.padding[0]
+        Cout, tr = mod.out_channels, int(mod.transposed)
+        g = gy.detach().to(xin.dtype).contiguous()
+        need = ctx.needs_input_grad
+        gx = torch.empty_like(xin) if need[1] else None
+        db = torch.empty(Cout, dtype=torch.float32, device=xin.device) if ctx.has_bias and need[3] else None
+        dv = dg = vf = gf = None
+        if any(need[4:]):
+            if len(wparams) == 2:                  # (weight_g, weight_v): the weight norm's backward too
+                gf, vf = (t.float().contiguous() for t in wparams)
+                dg = torch.empty(vf.shape[0], dtype=torch.float32, device=vf.device)
+            dv = torch.empty(w.shape, dtype=torch.float32, device=w.device)
+        if gx is None and dv is None and db is None:
+            return (None,) * (4 + len(wparams))
+        ns = L.kvae_conv1d_win_bwd_scratch_bytes(tr, B, Cin, Cout, T, ctx.T_gy, K, s, ctx.engine)
+        scratch = torch.empty(ns, dtype=torch.uint8, device=xin.device)
+        _lib.check(L.kvae_conv1d_win_bwd(xin.data_ptr(), g.data_ptr(), ctx.T_gy, w.data_ptr(), _lib.ptr(vf), _lib.ptr(gf),
+                                         _lib.ptr(gx), _lib.ptr(dv), _lib.ptr(dg), _lib.ptr(db), tr, B, Cin, Cout, T, K,
+                                         s, d, p, _lib.dtype_code(xin.dtype), ctx.engine, scratch.data_ptr(), ns,
+                                         _lib.stream_ptr(xin.device)))
+        if dv is None:
+            wgrads = (None,) * len(wparams)
+        elif len(wparams) == 2:
+            wgrads = (dg.view_as(wparams[0]).to(wparams[0].dtype), dv.to(wparams[1].dtype))
+        else:
+            wgrads = (dv.to(wparams[0].dtype),)
+        return (None, None if gx is None else gx.to(ctx.x_dtype), None, db, *wgrads)
+
+
+def _conv_grad(mod, x, tc):
+    """mod(x) under autograd when the input or a conv parameter requires grad (grad mode on), else None."""
+    wparams = (mod.weight_g, mod.weight_v) if mod.has_weight_norm else (mod._parameters["weight"],)
+    if not _grad_on(x, mod.bias, *wparams):
+        return None
+    _lib.require_cuda(x, type(mod).__name__ + ".forward")
+    return _BVConvFn.apply(mod, x, tc, mod.bias, *wparams)
+
+
+def _engine_of(mod, x, tc) -> int:
+    """The engine the no-grad call runs the layer on: _forward_tc's condition for the tensor cores (the decoder's convs
+    have stride 1, so a truncated output never sends them back to the CUDA cores)."""
+    if tc and x.shape[2] >= TC_MIN_ROWS and mod.tc_layer():
+        return 1 if mod.tc_precision == "bf16" else 2
+    return 0
 
 
 class LeakyReLU(nn.Module):
@@ -146,6 +333,8 @@ class Activation1d(nn.Module):
 
     def forward(self, x):
         _lib.require_cuda(x, "Activation1d")
+        if torch.is_grad_enabled() and _grad_on(x, self.act.alpha, getattr(self.act, "beta", None)):
+            return _AaActFn.apply(x, self.act.alpha, getattr(self.act, "beta", None), self)
         xin = _k(x)
         B, C, T = xin.shape
         y = torch.empty_like(xin)
@@ -193,6 +382,9 @@ class Conv1d(WNConv1d):
         super().__init__(in_channels, out_channels, kernel_size, stride=stride, padding=pad, dilation=dilation, bias=bias)
 
     def forward(self, x, tc=True):
+        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
+        if y is not None:
+            return y
         if self.causal and self.kernel_size[0] > 1:
             y = self._forward_tc(x, keep=x.shape[2]) if tc else None   # tensor-core layers truncate inside the kernel
             if y is not None:
@@ -213,6 +405,9 @@ class ConvTranspose1d(WNConvTranspose1d):
         self._drop = stride if causal else 0
 
     def forward(self, x, tc=True):
+        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
+        if y is not None:
+            return y
         if self._drop:
             y = self._forward_tc(x, keep=x.shape[2] * self.stride[0]) if tc else None
             if y is not None:
@@ -689,13 +884,32 @@ class BigVGANFlowVAE(nn.Module):
         x[b, :, :valid_len[b]]; what x (and noise) hold past that is ignored.  out[b, :, :wav_length(valid_len[b])]
         then equals the call on x[b:b+1, :, :valid_len[b]] (noise[b:b+1, :, :valid_len[b]]) bit for bit, and the rest
         of out[b] is 0."""
+        return self._decode(x, do_sample, noise, valid_len)
+
+    def decode_with_grad(self, x, do_sample=True, noise: Optional[torch.Tensor] = None, valid_len=None):
+        """``inference_from_latents`` under autograd: the same kernels on the same engines, so the output is
+        ``torch.equal`` to it (same ``noise``) under every ``set_precision``, and ``backward`` reaches the latents (mean
+        and log-scale when sampling) and every parameter of the decoder that requires grad -- the convs' ``weight_g`` /
+        ``weight_v`` / ``bias`` and the activations' ``alpha`` / ``beta``.  Each backward step is a libkvae kernel: the
+        fused anti-aliased activation backward, the convs' data and weight gradients on the engine their forward ran on
+        (tensor cores for the wide layers), no weight-gradient work for a frozen decoder.  Ragged batches and the streams
+        are inference-only.  Under ``torch.no_grad`` it is ``inference_from_latents``."""
+        if valid_len is not None:
+            raise NotImplementedError("decode_with_grad: valid_len (ragged batches) has no backward; decode each clip "
+                                      "on its own or pad the batch")
+        return self._decode(x, do_sample, noise, None)
+
+    def _decode(self, x, do_sample, noise, valid_len):
         h = self.h
         if h.use_vae and do_sample:
             assert x.size(1) == h.latent_dim * 2, "Input must be like [B, D, H]"
             m_q, logs_q = torch.split(x, h.latent_dim, dim=1)
             if noise is None:
                 noise = torch.randn_like(m_q)
-            x = _gauss_sample(m_q, logs_q, noise)
+            if _grad_on(x):
+                x = _GaussSampleFn.apply(x, noise, h.latent_dim)
+            else:
+                x = _gauss_sample(m_q, logs_q, noise)
         else:
             assert x.size(1) == h.latent_dim, "Input must be like [B, D, H]"
         if valid_len is not None:

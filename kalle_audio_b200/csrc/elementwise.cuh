@@ -123,12 +123,14 @@ __global__ void weight_norm_fold_kernel(const float* v, const float* g, float* w
 // ---------------------------------------------------------------- weight packing
 // torch Conv1d weight [Cout][Cin][K] (transposed=0) or ConvTranspose1d weight [Cin][Cout][K]
 // (transposed=1) -> tensor-core operand [K][Cout][Cin] bf16 and CUDA-core operand [K][Cin][Cout] fp32.
+// kFlipTaps: tap k of w lands at K - 1 - k (the data gradient of a Conv1d, kvae_conv1d_win_bwd).
+template <bool kFlipTaps = false>
 __global__ void pack_weights_kernel(const float* w, int transposed, int Cout, int Cin, int K,
                                     __nv_bfloat16* w_umma, float* w_direct) {
   const size_t n = static_cast<size_t>(Cout) * Cin * K;
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n;
        i += static_cast<size_t>(gridDim.x) * blockDim.x) {
-    const int k = static_cast<int>(i % K);
+    const int k = kFlipTaps ? K - 1 - static_cast<int>(i % K) : static_cast<int>(i % K);
     const size_t r = i / K;
     int co, ci;
     if (transposed) { co = static_cast<int>(r % Cout); ci = static_cast<int>(r / Cout); }

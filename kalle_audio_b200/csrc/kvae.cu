@@ -1440,6 +1440,38 @@ int run_backward(kvae_plan* p, const void* x, int x_dtype, const void* gy, int g
 
 bool check_dtype(int d) { return d == KVAE_F32 || d == KVAE_BF16; }
 
+// fp32 CUDA-core weight gradient of a layer-level Conv1d / ConvTranspose1d straight from the API layout [B, C, T]:
+// dw (torch layout, overwritten) from x (T rows) and gy, the gradient of the output rows [0, T_gy) (rows past T_gy,
+// a causal layer's dropped rows, have none).
+cudaError_t launch_wgrad_direct_cf(const void* x, const void* gy, int f32, float* dw, int transposed, int B, int Cin, int Cout,
+                                   long long T, long long T_gy, int K, int stride, int dilation, int padding, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(dw, 0, static_cast<size_t>(Cin) * Cout * K * 4, st);
+  if (e != cudaSuccess) return e;
+  const long long xsB = static_cast<long long>(Cin) * T, gsB = static_cast<long long>(Cout) * T_gy;
+  WgradParams wp;
+  std::memset(&wp, 0, sizeof(wp));
+  if (!transposed) {
+    wp.D = gy; wp.D_sB = gsB; wp.D_sT = 1; wp.D_sC = T_gy; wp.Td = static_cast<int>(T_gy); wp.Cd = Cout;
+    wp.S = x; wp.S_sB = xsB; wp.S_sT = 1; wp.S_sC = T; wp.Ts = static_cast<int>(T); wp.Cs = Cin;
+  } else {
+    wp.D = x; wp.D_sB = xsB; wp.D_sT = 1; wp.D_sC = T; wp.Td = static_cast<int>(T); wp.Cd = Cin;
+    wp.S = gy; wp.S_sB = gsB; wp.S_sT = 1; wp.S_sC = T_gy; wp.Ts = static_cast<int>(T_gy); wp.Cs = Cout;
+  }
+  wp.D_f32 = wp.S_f32 = f32;
+  wp.dW = dw; wp.B = B; wp.K = K; wp.stride = stride; wp.dil = dilation; wp.pad = padding;
+  const int tiles = ceil_div(wp.Cd, 64) * ceil_div(wp.Cs, 64);
+  const long long rows = static_cast<long long>(B) * wp.Td;
+  long long nsplit = std::max<long long>(1, (4ll * sm_count()) / (static_cast<long long>(tiles) * K));
+  nsplit = std::max<long long>(1, std::min<long long>(std::min(nsplit, (rows + 4 * kWgRows - 1) / (4 * kWgRows)), 65535));
+  long long rps = (rows + nsplit - 1) / nsplit;
+  rps = (rps + kWgRows - 1) / kWgRows * kWgRows;
+  nsplit = (rows + rps - 1) / rps;
+  wp.rows_per_split = rps;
+  wgrad_direct_kernel<<<dim3(tiles, K, static_cast<unsigned>(nsplit)), 256, 0, st>>>(wp);
+  ++g_launches;
+  return cudaGetLastError();
+}
+
 #include "stream.inc.cuh"
 
 }  // namespace
@@ -1788,33 +1820,7 @@ int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, flo
   // ---- weight gradient (torch layout), straight from the API layout through element strides
   const size_t n = static_cast<size_t>(Cin) * Cout * K;
   const long long xsB = static_cast<long long>(Cin) * T, gsB = static_cast<long long>(Cout) * T_out;
-  if (dw) {
-  KV_CUDA(cudaMemsetAsync(dw, 0, n * 4, st));
-  WgradParams wp;
-  std::memset(&wp, 0, sizeof(wp));
-  if (!transposed) {
-    wp.D = gy; wp.D_sB = gsB; wp.D_sT = 1; wp.D_sC = T_out; wp.Td = static_cast<int>(T_out); wp.Cd = Cout;
-    wp.S = x; wp.S_sB = xsB; wp.S_sT = 1; wp.S_sC = T; wp.Ts = static_cast<int>(T); wp.Cs = Cin;
-  } else {
-    wp.D = x; wp.D_sB = xsB; wp.D_sT = 1; wp.D_sC = T; wp.Td = static_cast<int>(T); wp.Cd = Cin;
-    wp.S = gy; wp.S_sB = gsB; wp.S_sT = 1; wp.S_sC = T_out; wp.Ts = static_cast<int>(T_out); wp.Cs = Cout;
-  }
-  wp.D_f32 = wp.S_f32 = f32;
-  wp.dW = dw; wp.B = B; wp.K = K; wp.stride = stride; wp.dil = dilation; wp.pad = padding;
-  {
-    const int tiles = ceil_div(wp.Cd, 64) * ceil_div(wp.Cs, 64);
-    const long long rows = static_cast<long long>(B) * wp.Td;
-    long long nsplit = std::max<long long>(1, (4ll * sm_count()) / (static_cast<long long>(tiles) * K));
-    nsplit = std::max<long long>(1, std::min<long long>(std::min(nsplit, (rows + 4 * kWgRows - 1) / (4 * kWgRows)), 65535));
-    long long rps = (rows + nsplit - 1) / nsplit;
-    rps = (rps + kWgRows - 1) / kWgRows * kWgRows;
-    nsplit = (rows + rps - 1) / rps;
-    wp.rows_per_split = rps;
-    wgrad_direct_kernel<<<dim3(tiles, K, static_cast<unsigned>(nsplit)), 256, 0, st>>>(wp);
-    KV_CUDA(cudaGetLastError());
-    ++g_launches;
-  }
-  }  // dw
+  if (dw) KV_CUDA(launch_wgrad_direct_cf(x, gy, f32, dw, transposed, B, Cin, Cout, T, T_out, K, stride, dilation, padding, st));
   if (dbias) {
     bias_grad_cf_kernel<<<Cout, 256, 0, st>>>(gy, f32, dbias, B, Cout, T_out);
     KV_CUDA(cudaGetLastError());
@@ -1858,6 +1864,31 @@ size_t win_pack_main_bytes(int Cin, int Cout, int K, int engine) {
   const size_t n = static_cast<size_t>(Cin) * Cout * K;
   return engine == 0 ? align_up(n * 4, 1024) : align_up(n * 2 * (engine == 2 ? 2 : 1), 1024);
 }
+
+// kvae_conv1d_pack's layout for `engine`; w is read as [Cin, Cout, K] (transposed) or [Cout, Cin, K], tap k packed at
+// K - 1 - k when flip_taps.  The data gradient of a layer packs the layer's weight under the opposite kind with Cin and
+// Cout exchanged (kvae_conv1d_win_bwd).
+int pack_conv_weights(const float* w, int transposed, int Cin, int Cout, int K, int engine, int flip_taps, void* packed,
+                      cudaStream_t st) {
+  const size_t n = static_cast<size_t>(Cin) * Cout * K;
+  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 4096));
+  uint8_t* base = static_cast<uint8_t*>(packed);
+  auto pack = flip_taps ? pack_weights_kernel<true> : pack_weights_kernel<false>;
+  if (engine == 0) {
+    pack<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, reinterpret_cast<float*>(base));
+  } else if (engine == 1) {
+    pack<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, reinterpret_cast<__nv_bfloat16*>(base), nullptr);
+  } else {
+    float* w_direct = reinterpret_cast<float*>(base + win_pack_main_bytes(Cin, Cout, K, 2));
+    pack<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, w_direct);
+    KV_CUDA(cudaGetLastError());
+    split_pack_kernel<<<blocks, 256, 0, st>>>(w_direct, K, Cin, Cout, reinterpret_cast<__nv_bfloat16*>(base));
+    ++g_launches;
+  }
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
 }  // namespace
 
 size_t kvae_conv1d_packed_bytes(int Cin, int Cout, int K, int engine) {
@@ -1874,24 +1905,7 @@ int kvae_conv1d_pack(const float* w, int transposed, int Cin, int Cout, int K, i
   if (packed_bytes < kvae_conv1d_packed_bytes(Cin, Cout, K, engine)) return fail("packed buffer too small");
   DeviceGuard guard(device_of(w));
   if (!guard.ok) return fail("cannot select the tensor's device");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t n = static_cast<size_t>(Cin) * Cout * K;
-  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 4096));
-  uint8_t* base = static_cast<uint8_t*>(packed);
-  if (engine == 0) {
-    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, reinterpret_cast<float*>(base));
-  } else if (engine == 1) {
-    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, reinterpret_cast<__nv_bfloat16*>(base), nullptr);
-  } else {
-    float* w_direct = reinterpret_cast<float*>(base + win_pack_main_bytes(Cin, Cout, K, 2));
-    pack_weights_kernel<<<blocks, 256, 0, st>>>(w, transposed, Cout, Cin, K, nullptr, w_direct);
-    KV_CUDA(cudaGetLastError());
-    split_pack_kernel<<<blocks, 256, 0, st>>>(w_direct, K, Cin, Cout, reinterpret_cast<__nv_bfloat16*>(base));
-    ++g_launches;
-  }
-  KV_CUDA(cudaGetLastError());
-  ++g_launches;
-  return 0;
+  return pack_conv_weights(w, transposed, Cin, Cout, K, engine, 0, packed, static_cast<cudaStream_t>(stream));
 }
 
 size_t kvae_conv1d_win_scratch_bytes(int B, int Cin, long long T, int engine) {
@@ -1907,10 +1921,11 @@ namespace {
 // zero; x0 a multiple of the stride of a strided conv) and select the device.  A tcgen05 call for the full range of a
 // whole layer whose input is whole stride groups runs with no StreamGeom, which keeps the whole-row set-up of the
 // strided convs; any other call (a strided conv's input of any length included) copies its window into scratch rounded
-// up to whole stride groups, the rows that read as zero written as zeros.
+// up to whole stride groups, the rows that read as zero written as zeros.  staged (tcgen05, split 1 only): scratch
+// already holds that channels-last window (kvae_conv1d_win_bwd shares it with the weight gradient).
 int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, long long x0, long long nx, long long t_end, void* y,
                 long long ldy, const void* packed, const float* bias, int B, long long o0, long long o1, int dtype,
-                int engine, void* scratch, size_t scratch_bytes, cudaStream_t st) {
+                int engine, void* scratch, size_t scratch_bytes, cudaStream_t st, bool staged = false) {
   if (engine == 0) {
     DirectLaunch L;
     std::string err;
@@ -1944,7 +1959,7 @@ int conv1d_rows(const ConvGeom& g, const void* x, long long ldx, long long x0, l
   if (scratch_bytes < kvae_conv1d_win_scratch_bytes(B, g.Cin, W, engine) || !scratch) return fail("scratch too small");
   const int split = engine == 2 ? 2 : 1;
   __nv_bfloat16* xcl = static_cast<__nv_bfloat16*>(scratch);
-  {
+  if (!staged) {
     const long long lo = std::max(0LL, -x0), hi = t_end < 0 ? nx : std::min(nx, t_end - x0);
     dim3 grid(ceil_div(static_cast<int>(W), 32), ceil_div(g.Cin, 32), B), block(32, 8);
     cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, dtype == KVAE_F32, xcl, g.Cin, static_cast<int>(W),
@@ -2053,6 +2068,141 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
   KV_CUDA(cudaGetLastError());
   ++g_launches;
   return conv1d_rows(g, x, T, 0, T, T, y, T_out, scratch, bias, B, 0, T_out, dtype, 0, nullptr, 0, st);
+}
+
+// ------------------------------------------------------------------ BigVGANFlowVAE conv backward
+namespace {
+// The data gradient of a layer as a forward Conv1d over the layer's output gradient gy (run by conv1d_rows, rows of gy
+// past its end reading as zero):
+//   Conv1d, stride 1, left padding pl <= d (K - 1): gx = the conv of gy with the weight transposed ([Cin, Cout, K]) and
+//     its taps reversed, same dilation, left padding d (K - 1) - pl;
+//   ConvTranspose1d, stride s, padding p: gx = the strided Conv1d of gy with the same weight, stride s, padding p.
+struct DgradGeom {
+  ConvGeom g;      // kConv, Cin = the layer's Cout, Cout = the layer's Cin
+  int flip;        // the weight's taps reversed (Conv1d)
+};
+bool dgrad_conv_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, DgradGeom& d,
+                     std::string& err) {
+  if (Cin <= 0 || Cout <= 0 || K <= 0 || dilation < 1) { err = "conv backward: empty layer"; return false; }
+  if (stride < 1 || stride > kMaxPhases) { err = "stride out of range (1..8)"; return false; }
+  if (!transposed) {
+    if (stride != 1) { err = "conv backward: a Conv1d of stride 1 only"; return false; }
+    if (padding < 0 || padding > dilation * (K - 1)) { err = "conv backward: Conv1d padding outside 0 .. d (K - 1)"; return false; }
+    d.g = ConvGeom{kConv, Cout, Cin, K, 1, dilation, dilation * (K - 1) - padding};
+    d.flip = 1;
+  } else {
+    if (dilation != 1) { err = "conv backward: ConvTranspose1d of dilation 1 only"; return false; }
+    if (padding < 0 || padding >= K) { err = "conv backward: ConvTranspose1d padding outside 0 .. K - 1"; return false; }
+    d.g = ConvGeom{kConv, Cout, Cin, K, stride, 1, padding};
+    d.flip = 0;
+  }
+  return true;
+}
+
+long long round_up_ll(long long v, long long m) { return (v + m - 1) / m * m; }
+}  // namespace
+
+int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]) {
+  if (!out) return fail("null argument");
+  DgradGeom d;
+  std::string err;
+  if (!dgrad_conv_geom(transposed, Cin, Cout, K, stride, dilation, padding, d, err)) return fail(err);
+  const int v[6] = {d.g.Cin, d.g.Cout, d.g.stride, d.g.dilation, d.g.pad, d.flip};
+  std::memcpy(out, v, sizeof(v));
+  return 0;
+}
+
+size_t kvae_conv1d_win_bwd_scratch_bytes(int transposed, int B, int Cin, int Cout, long long T, long long T_gy, int K,
+                                         int stride, int engine) {
+  if (engine < 0 || engine > 2 || B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0 || T_gy <= 0 || stride < 1) return 0;
+  const long long Tg = round_up_ll(T_gy, transposed ? stride : 1);
+  size_t bytes = kvae_conv1d_packed_bytes(Cout, Cin, K, engine) + kvae_conv1d_win_scratch_bytes(B, Cout, Tg, engine) +
+                 align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
+  if (engine == 1) bytes += align_up(static_cast<size_t>(B) * T * Cin * 2, 1024);
+  return bytes;
+}
+
+int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const float* w, const float* v, const float* g,
+                        void* gx, float* dv, float* dg, float* dbias, int transposed, int B, int Cin, int Cout, long long T,
+                        int K, int stride, int dilation, int padding, int dtype, int engine, void* scratch,
+                        size_t scratch_bytes, void* stream) {
+  if (!gy) return fail("null argument");
+  if (!gx && !dv && !dbias) return fail("nothing to compute (gx, dv and dbias are all null)");
+  if ((gx && !w) || (dv && !x) || (g && (!v || !dg))) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (engine < 0 || engine > 2) return fail("engine: 0 = CUDA cores, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3");
+  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
+  DgradGeom dgg;
+  std::string err;
+  if (!dgrad_conv_geom(transposed, Cin, Cout, K, stride, dilation, padding, dgg, err)) return fail(err);
+  const ConvGeom lg{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
+  if (T >= (1LL << 30) || lg.out_len(static_cast<int>(T)) >= (1LL << 30)) return fail("rows beyond 2^30");
+  if (T_gy < 1 || T_gy > lg.out_len(static_cast<int>(T))) return fail("T_gy outside 1 .. the layer's output length");
+  if (engine && !kvae_conv1d_tc_supported(Cin, Cout, K, stride, dilation, transposed))
+    return fail("tcgen05 engine: the layer needs channel counts that are multiples of 64");
+  if (!scratch || scratch_bytes < kvae_conv1d_win_bwd_scratch_bytes(transposed, B, Cin, Cout, T, T_gy, K, stride, engine))
+    return fail("scratch too small");
+  DeviceGuard guard(device_of(gy));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int f32 = dtype == KVAE_F32;
+  const long long Tg = round_up_ll(T_gy, dgg.g.stride);     // gy staged in whole stride groups of the data-gradient conv
+  uint8_t* base = static_cast<uint8_t*>(scratch);
+  void* wpk = base;
+  base += kvae_conv1d_packed_bytes(Cout, Cin, K, engine);
+  __nv_bfloat16* gcl = reinterpret_cast<__nv_bfloat16*>(base);
+  const size_t gcl_bytes = kvae_conv1d_win_scratch_bytes(B, Cout, Tg, engine);
+  base += gcl_bytes;
+  float* dW = reinterpret_cast<float*>(base);
+  base += align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
+  __nv_bfloat16* xcl = reinterpret_cast<__nv_bfloat16*>(base);
+  if (dbias) {
+    bias_grad_cf_kernel<<<Cout, 256, 0, st>>>(gy, f32, dbias, B, Cout, T_gy);
+    KV_CUDA(cudaGetLastError());
+    ++g_launches;
+  }
+  // engine 1: gy channels-last bf16 once, the data-gradient conv's input and a weight-gradient operand
+  if (engine == 1 && (gx || dv)) {
+    dim3 grid(ceil_div(static_cast<int>(Tg), 32), ceil_div(Cout, 32), B), block(32, 8);
+    cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(gy, f32, gcl, Cout, static_cast<int>(Tg), 0, 0, T_gy, 0,
+                                                 static_cast<int>(T_gy));
+    KV_CUDA(cudaGetLastError());
+    ++g_launches;
+  }
+  if (dv) {
+    const int R = transposed ? Cin : Cout, Cc = transposed ? Cout : Cin;   // dim 0 of the torch weight and the rest
+    if (engine == 1) {
+      // tensor-core weight gradient into the packed [K][R][Cc] layout, then the weight-norm backward from it
+      dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(Cin, 32), B), block(32, 8);
+      cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, f32, xcl, Cin, static_cast<int>(T), 0);
+      KV_CUDA(cudaGetLastError());
+      ++g_launches;
+      KV_CUDA(cudaMemsetAsync(dW, 0, static_cast<size_t>(Cin) * Cout * K * 4, st));
+      WgradLaunch L;
+      const bool ok = transposed
+          ? prepare_wgrad_umma(xcl, static_cast<int>(T), Cin, gcl, static_cast<int>(Tg), Cout, B, K, stride, dilation, padding, dW, L, err)
+          : prepare_wgrad_umma(gcl, static_cast<int>(T_gy), Cout, xcl, static_cast<int>(T), Cin, B, K, stride, dilation, padding, dW, L, err);
+      if (!ok) return fail(err);
+      KV_CUDA(launch_wgrad_umma(L, st));
+      ++g_launches;
+      weight_norm_bwd_packed_kernel<<<R, 256, 0, st>>>(v, g, dW, dv, g ? dg : nullptr, R, Cc, K);
+      KV_CUDA(cudaGetLastError());
+      ++g_launches;
+    } else {
+      // fp32 CUDA cores (engine 0, and engine 2, whose bf16x3 split would take three tensor-core passes)
+      KV_CUDA(launch_wgrad_direct_cf(x, gy, f32, g ? dW : dv, transposed, B, Cin, Cout, T, T_gy, K, stride, dilation,
+                                     padding, st));
+      if (g) {
+        weight_norm_bwd_kernel<<<R, 256, 0, st>>>(v, g, dW, dv, dg, Cc * K);
+        KV_CUDA(cudaGetLastError());
+        ++g_launches;
+      }
+    }
+  }
+  if (!gx) return 0;
+  if (pack_conv_weights(w, !transposed, Cout, Cin, K, engine, dgg.flip, wpk, st)) return -1;
+  return conv1d_rows(dgg.g, gy, T_gy, 0, T_gy, T_gy, gx, T, wpk, nullptr, B, 0, T, dtype, engine, gcl, gcl_bytes, st,
+                     engine == 1);
 }
 
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)
@@ -2575,6 +2725,67 @@ int kvae_gauss_sample(const void* mean, const void* logs, const void* noise, voi
   if (!guard.ok) return fail("cannot select the tensor's device");
   const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 148 * 16));
   gauss_sample_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(mean, logs, noise, out, n, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+// ------------------------------------------------------------------ BigVGANFlowVAE leaf backward (bigvgan.cuh)
+size_t kvae_aa_act_bwd_scratch_bytes(int B, int C, long long T) {
+  if (B <= 0 || C <= 0 || T <= 0) return 0;
+  return align_up(static_cast<size_t>(B) * C * ((T + kAaTile - 1) / kAaTile) * 2 * sizeof(double), 1024);
+}
+
+int kvae_aa_act_bwd(const void* x, const void* gy, void* gx, const float* alpha, const float* beta, int logscale,
+                    const float* filt_up, const float* filt_down, float* dalpha, float* dbeta, int B, int C, long long T,
+                    int dtype, void* scratch, size_t scratch_bytes, void* stream) {
+  if (!x || !gy || !gx || !alpha || !filt_up || !filt_down || (dalpha && beta && !dbeta)) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || C <= 0 || T <= 0) return fail("empty input");
+  if (static_cast<long long>(B) * C > 65535) return fail("B*C too large");
+  if (T >= (1LL << 40)) return fail("rows beyond 2^40");
+  if (dalpha && (!scratch || scratch_bytes < kvae_aa_act_bwd_scratch_bytes(B, C, T))) return fail("scratch too small");
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int tiles = static_cast<int>((T + kAaTile - 1) / kAaTile);
+  double* part = dalpha ? static_cast<double*>(scratch) : nullptr;
+  aa_act_bwd_kernel<<<dim3(tiles, B * C), 256, 0, st>>>(x, gy, gx, part, T, alpha, beta, logscale, filt_up, filt_down, C,
+                                                        dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  if (!dalpha) return 0;
+  aa_act_bwd_params_kernel<<<C, 256, 0, st>>>(part, alpha, beta, logscale, dalpha, dbeta, B, C, tiles);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_unary_bwd(const void* t, const void* gy, void* gx, size_t n, int op, float param, int dtype, void* stream) {
+  if (!t || !gy || !gx) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (op != 0 && op != 1) return fail("unary op: 0 = leaky_relu, 1 = tanh");
+  if (n == 0) return 0;
+  DeviceGuard guard(device_of(t));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 148 * 16));
+  unary_bwd_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(t, gy, gx, n, op, param, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_gauss_sample_bwd(const void* x, const void* noise, const void* gz, void* gx, int B, int D, long long T, int dtype,
+                          void* stream) {
+  if (!x || !noise || !gz || !gx) return fail("null argument");
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || D <= 0 || T <= 0) return 0;
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  const size_t n = static_cast<size_t>(B) * D * T;
+  const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 148 * 16));
+  gauss_sample_bwd_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, noise, gz, gx, static_cast<long long>(D) * T,
+                                                                                 n, dtype == KVAE_F32);
   KV_CUDA(cudaGetLastError());
   ++g_launches;
   return 0;

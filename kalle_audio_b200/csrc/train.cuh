@@ -868,6 +868,13 @@ __device__ __forceinline__ void weight_norm_bwd_packed_row(float (*red)[32], con
   if (g && threadIdx.x == 0) dg[i] = dot / n;
 }
 
+// One layer (kvae_conv1d_win_bwd): one block per dim-0 row, 256 threads.
+__global__ void __launch_bounds__(256) weight_norm_bwd_packed_kernel(const float* v, const float* g, const float* dwp,
+                                                                     float* dv, float* dg, int R, int Cc, int K) {
+  __shared__ float red[2][32];
+  weight_norm_bwd_packed_row(red, v, g, dwp, dv, dg, R, Cc, K, blockIdx.x);
+}
+
 // All layers of a plan in ONE launch (72 launches of ~16 us each before): grid = sum of dim-0 rows, a block finds its
 // layer by binary search in the prefix table.  params == nullptr: packed gradients are only re-ordered.
 struct WnBwdDesc {
