@@ -375,15 +375,20 @@ int kvae_unary_bwd(const void* t, const void* gy, void* gx, size_t n, int op, fl
  * kvae_axpby itself.) */
 int kvae_gauss_sample_bwd(const void* x, const void* noise, const void* gz, void* gx, int B, int D, long long T, int dtype,
                           void* stream);
-/* Backward of a BigVGANFlowVAE conv layer (Conv1d :566-620, ConvTranspose1d :336-391; the layer geometry is the
- * forward's: padding on both sides, a causal layer being the symmetric-padded one truncated).  gy: the gradient of
+/* Backward of a BigVGANFlowVAE conv layer (Conv1d :566-620, ConvTranspose1d :336-391, and the encoder's Conv1d_S
+ * :139-172, whose downsampling convs have stride 2 .. 8; the layer geometry is the forward's: padding on both sides, a
+ * causal layer being the symmetric-padded one truncated; a strided Conv1d has dilation 1).  gy: the gradient of
  * the layer's output rows [0, T_gy) ([B, Cout, T_gy] of `dtype`); rows past T_gy (a causal layer's dropped rows) have
  * none.  x: the layer's input [B, Cin, T].  w: the folded fp32 weight.  Each product is optional (NULL = skipped):
- *   gx [B, Cin, T] (`dtype`)  the forward conv kernels under the data-gradient geometry (kvae_conv1d_dgrad_geom) on
- *                             `engine`: 0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3;
+ *   gx [B, Cin, T] (`dtype`)  the forward conv kernels under the data-gradient geometry (kvae_conv1d_dgrad_form) on
+ *                             `engine`: 0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16 x 3.  A strided
+ *                             Conv1d's is a ConvTranspose1d continued to all T input rows (rows past its natural
+ *                             length are rows the forward read); the tcgen05 engines compute it in whole stride groups,
+ *                             through scratch when T is not a multiple of the stride;
  *   dv (fp32, torch layout)   with g != NULL the gradients of weight_v and (dg) weight_g of the weight norm (v, g: the
  *                             fp32 parameters), else of the plain weight.  Engine 1: tcgen05 weight gradient from
- *                             channels-last bf16 copies of x and gy; engines 0 and 2: fp32 CUDA cores;
+ *                             channels-last bf16 copies of x (rounded up to whole stride groups
+ *                             with zero rows) and gy; engines 0 and 2: fp32 CUDA cores;
  *   dbias [Cout] (fp32).
  * A frozen layer (dv = dbias = NULL) runs no weight-gradient kernel.  tcgen05 engines: kvae_conv1d_tc_supported.
  * scratch: kvae_conv1d_win_bwd_scratch_bytes. */
@@ -398,6 +403,12 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
  * layer's weight transposed to [Cin, Cout, K] with its taps reversed (out[5] = 1: a Conv1d of stride 1, new left
  * padding d (K - 1) - padding), or as it is (out[5] = 0: a ConvTranspose1d, stride s, padding p). */
 int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]);
+/* The same for every layer kvae_conv1d_win_bwd accepts, the kind of conv first: gx = rows [0, T) of the Conv1d
+ * (out[0] = 0, as kvae_conv1d_dgrad_geom's out[0 .. 5] in out[1 .. 6]) or the ConvTranspose1d (out[0] = 1: a strided
+ * Conv1d's; out[1] input channels = the layer's Cout, out[2] output channels = the layer's Cin, stride out[3], dilation
+ * out[4] = 1, padding out[5] = the layer's, out[6] = 0: the layer's weight as it is, read as [out[1], out[2], K]) of gy,
+ * continued past its natural length to T rows (torch's output_padding T - that length). */
+int kvae_conv1d_dgrad_form(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[7]);
 
 /* ---- post-decode tail ---- */
 /* audio.to(float32).div(max|audio|).clamp(-1,1).mul(32767).to(int16) -- the peak-normalised PCM conversion every

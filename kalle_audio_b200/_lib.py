@@ -125,6 +125,7 @@ SIGNATURES = {
                                       C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                       C.c_size_t, C.c_void_p]),
     "kvae_conv1d_dgrad_geom": (C.c_int, [C.c_int] * 7 + [C.POINTER(C.c_int * 6)]),
+    "kvae_conv1d_dgrad_form": (C.c_int, [C.c_int] * 7 + [C.POINTER(C.c_int * 7)]),
     "kvae_plan_out_length": (C.c_longlong, [C.c_void_p, C.c_longlong]),
     "kvae_mrstft_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int]),
     "kvae_mrstft_loss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p,

@@ -9,6 +9,8 @@ only; kept as a parameter container so checkpoints load), ``conv_pre``, ``ups``,
     inference_from_latents(x, do_sample)    :498-529   latents -> waveform [B, 1, T * prod(upsample_rates)]
     decode_with_grad(x, do_sample)          :498-529   the same under autograd (gradients to the latents and the
                                                        decoder's parameters)
+    encode_with_grad(x)                     :494-496   extract_latents under autograd (gradients to the audio and the
+                                                       encoder's parameters)
 
 The first two take ``valid_len`` for a batch of clips of different lengths, each clip bit-identical to its own call (the
 ragged path below ``_run_ragged``; ``latent_length`` / ``wav_length`` give the per-clip output lengths).
@@ -20,7 +22,7 @@ CUDA-core ``kvae_conv1d_fwd`` -- the anti-aliased Snake / SnakeBeta activation a
 x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager kernels and four double-rate intermediates
 in the reference), LeakyReLU / tanh / residual adds / the AMP average / the Gaussian sample as small elementwise
 kernels.  Under grad mode each of them has an autograd node whose backward is a libkvae call too (the ``_*Fn`` classes
-below; ``decode_with_grad``).  ``forward`` (the training pass through the flow) is not built.
+below; ``decode_with_grad``, ``encode_with_grad``).  ``forward`` (the training pass through the flow) is not built.
 """
 from __future__ import annotations
 
@@ -262,8 +264,9 @@ def _conv_grad(mod, x, tc):
 
 
 def _engine_of(mod, x, tc) -> int:
-    """The engine the no-grad call runs the layer on: _forward_tc's condition for the tensor cores (the decoder's convs
-    have stride 1, so a truncated output never sends them back to the CUDA cores)."""
+    """The engine the no-grad call runs the layer on: _forward_tc's condition for the tensor cores (only a strided conv
+    with a truncated output goes back to the CUDA cores there, and no strided conv is truncated: the decoder's convs
+    have stride 1, the encoder's are never causal)."""
     if tc and x.shape[2] >= TC_MIN_ROWS and mod.tc_layer():
         return 1 if mod.tc_precision == "bf16" else 2
     return 0
@@ -416,13 +419,26 @@ class ConvTranspose1d(WNConvTranspose1d):
         return super().forward(x, tc)
 
 
+class _EncConv1d(WNConv1d):
+    """The encoder's convs (``Conv1d_S.layer``, the ResStack convs): ``layers.WNConv1d`` with an autograd node of its
+    own.  ``WNConv1d`` differentiates through ``_ConvFn``, fp32 on the CUDA cores whatever ``set_precision`` says; here
+    grad mode runs ``_BVConvFn``, whose forward is the no-grad call (``extract_latents``' engine and bits) and whose
+    backward runs on that engine."""
+
+    def forward(self, x, tc=True):
+        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
+        if y is not None:
+            return y
+        return super().forward(x, tc)
+
+
 class Conv1d_S(nn.Module):
     """flows.py:139-172 (weight_norm form): ``self.layer`` = weight-normed Conv1d with padding d (k - 1) // 2."""
 
     def __init__(self, in_channels, out_channels, kernel_size=1, stride=1, dilation=1):
         super().__init__()
-        self.layer = WNConv1d(in_channels, out_channels, kernel_size, stride=stride, padding=dilation * (kernel_size - 1) // 2,
-                              dilation=dilation)
+        self.layer = _EncConv1d(in_channels, out_channels, kernel_size, stride=stride,
+                                padding=dilation * (kernel_size - 1) // 2, dilation=dilation)
 
     def forward(self, x):
         return self.layer(x)
@@ -434,8 +450,8 @@ class ResStack(nn.Module):
     def __init__(self, channel, kernel_size=3, base=3, nums=4):
         super().__init__()
         self.layers = nn.ModuleList([
-            nn.Sequential(LeakyReLU(), WNConv1d(channel, channel, kernel_size, dilation=base ** i, padding=base ** i),
-                          LeakyReLU(), WNConv1d(channel, channel, kernel_size, dilation=1, padding=1))
+            nn.Sequential(LeakyReLU(), _EncConv1d(channel, channel, kernel_size, dilation=base ** i, padding=base ** i),
+                          LeakyReLU(), _EncConv1d(channel, channel, kernel_size, dilation=1, padding=1))
             for i in range(nums)])
 
     def forward(self, x):
@@ -876,6 +892,19 @@ class BigVGANFlowVAE(nn.Module):
         ``extract_latents(x[b:b+1, :, :valid_len[b]])`` bit for bit, and the rest of out[b] is 0."""
         if valid_len is not None:
             return self._ragged(True, x, valid_len, "extract_latents")
+        return self.audio_encoder(x)
+
+    def encode_with_grad(self, x, valid_len=None):
+        """``extract_latents`` under autograd: the same kernels on the same engines, so the output is ``torch.equal`` to
+        it under every ``set_precision``, and ``backward`` reaches the audio (when it requires grad) and every parameter
+        of the encoder that requires grad (the convs' ``weight_g`` / ``weight_v`` / ``bias``).  The convs' data and
+        weight gradients run on the engine their forward ran on: tensor cores for the wide layers, the strided
+        downsampling convs included; no weight-gradient work for a frozen encoder.  ``decode_with_grad(
+        encode_with_grad(x), noise=...)`` is the whole autoencoder under autograd.  Ragged batches and the streams are
+        inference-only.  Under ``torch.no_grad`` it is ``extract_latents``."""
+        if valid_len is not None:
+            raise NotImplementedError("encode_with_grad: valid_len (ragged batches) has no backward; encode each clip "
+                                      "on its own or pad the batch")
         return self.audio_encoder(x)
 
     @torch.no_grad()

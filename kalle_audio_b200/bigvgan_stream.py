@@ -306,7 +306,8 @@ class _OpStream:
         _lib.require_cuda(x, f"{type(self).__name__}.push")
         if x.requires_grad:
             raise ValueError(f"{type(self).__name__}.push: streams are inference-only and return no gradient; use "
-                             "BigVGANFlowVAE.decode_with_grad for gradients (or pass a tensor that does not require grad)")
+                             "BigVGANFlowVAE.encode_with_grad / decode_with_grad for gradients (or pass a tensor that does not "
+                             "require grad)")
         if x.dim() != 3 or x.shape[1] != self.in_channels:
             raise ValueError(f"expected {self._noun} [B, {self.in_channels}, n], got {tuple(x.shape)}")
         if x.dtype not in (torch.float32, torch.bfloat16):

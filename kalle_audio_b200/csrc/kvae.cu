@@ -2072,21 +2072,28 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
 
 // ------------------------------------------------------------------ BigVGANFlowVAE conv backward
 namespace {
-// The data gradient of a layer as a forward Conv1d over the layer's output gradient gy (run by conv1d_rows, rows of gy
-// past its end reading as zero):
+// The data gradient of a layer as a conv over the layer's output gradient gy (run by conv1d_rows, rows of gy past its
+// end reading as zero):
 //   Conv1d, stride 1, left padding pl <= d (K - 1): gx = the conv of gy with the weight transposed ([Cin, Cout, K]) and
 //     its taps reversed, same dilation, left padding d (K - 1) - pl;
+//   Conv1d, stride s > 1, dilation 1, padding p < K: gx = the ConvTranspose1d of gy with the same weight (read as the
+//     transposed conv's [Cin', Cout', K] = [Cout, Cin, K]), stride s, padding p, continued past its natural length to
+//     the layer's T input rows (torch's output_padding): those rows are input rows the forward read;
 //   ConvTranspose1d, stride s, padding p: gx = the strided Conv1d of gy with the same weight, stride s, padding p.
 struct DgradGeom {
-  ConvGeom g;      // kConv, Cin = the layer's Cout, Cout = the layer's Cin
-  int flip;        // the weight's taps reversed (Conv1d)
+  ConvGeom g;      // Cin = the layer's Cout, Cout = the layer's Cin; kConvT for a strided Conv1d, else kConv
+  int flip;        // the weight's taps reversed (Conv1d of stride 1)
 };
 bool dgrad_conv_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, DgradGeom& d,
                      std::string& err) {
   if (Cin <= 0 || Cout <= 0 || K <= 0 || dilation < 1) { err = "conv backward: empty layer"; return false; }
   if (stride < 1 || stride > kMaxPhases) { err = "stride out of range (1..8)"; return false; }
-  if (!transposed) {
-    if (stride != 1) { err = "conv backward: a Conv1d of stride 1 only"; return false; }
+  if (!transposed && stride > 1) {
+    if (dilation != 1) { err = "conv backward: a strided Conv1d of dilation 1 only"; return false; }
+    if (padding < 0 || padding >= K) { err = "conv backward: strided Conv1d padding outside 0 .. K - 1"; return false; }
+    d.g = ConvGeom{kConvT, Cout, Cin, K, stride, 1, padding};
+    d.flip = 0;
+  } else if (!transposed) {
     if (padding < 0 || padding > dilation * (K - 1)) { err = "conv backward: Conv1d padding outside 0 .. d (K - 1)"; return false; }
     d.g = ConvGeom{kConv, Cout, Cin, K, 1, dilation, dilation * (K - 1) - padding};
     d.flip = 1;
@@ -2104,10 +2111,20 @@ long long round_up_ll(long long v, long long m) { return (v + m - 1) / m * m; }
 
 int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]) {
   if (!out) return fail("null argument");
+  if (!transposed && stride != 1)
+    return fail("conv backward: a strided Conv1d's data gradient is a ConvTranspose1d (kvae_conv1d_dgrad_form)");
+  int f[7];
+  if (kvae_conv1d_dgrad_form(transposed, Cin, Cout, K, stride, dilation, padding, f)) return -1;
+  std::memcpy(out, f + 1, 6 * sizeof(int));
+  return 0;
+}
+
+int kvae_conv1d_dgrad_form(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[7]) {
+  if (!out) return fail("null argument");
   DgradGeom d;
   std::string err;
   if (!dgrad_conv_geom(transposed, Cin, Cout, K, stride, dilation, padding, d, err)) return fail(err);
-  const int v[6] = {d.g.Cin, d.g.Cout, d.g.stride, d.g.dilation, d.g.pad, d.flip};
+  const int v[7] = {d.g.kind == kConvT, d.g.Cin, d.g.Cout, d.g.stride, d.g.dilation, d.g.pad, d.flip};
   std::memcpy(out, v, sizeof(v));
   return 0;
 }
@@ -2115,10 +2132,11 @@ int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride,
 size_t kvae_conv1d_win_bwd_scratch_bytes(int transposed, int B, int Cin, int Cout, long long T, long long T_gy, int K,
                                          int stride, int engine) {
   if (engine < 0 || engine > 2 || B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0 || T_gy <= 0 || stride < 1) return 0;
-  const long long Tg = round_up_ll(T_gy, transposed ? stride : 1);
+  const long long Tg = round_up_ll(T_gy, transposed ? stride : 1), Tx = round_up_ll(T, transposed ? 1 : stride);
   size_t bytes = kvae_conv1d_packed_bytes(Cout, Cin, K, engine) + kvae_conv1d_win_scratch_bytes(B, Cout, Tg, engine) +
                  align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
-  if (engine == 1) bytes += align_up(static_cast<size_t>(B) * T * Cin * 2, 1024);
+  if (engine == 1) bytes += align_up(static_cast<size_t>(B) * Tx * Cin * 2, 1024);
+  if (engine && Tx != T) bytes += align_up(static_cast<size_t>(B) * Cin * Tx * 4, 1024);   // gx in whole stride groups
   return bytes;
 }
 
@@ -2146,7 +2164,10 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
   if (!guard.ok) return fail("cannot select the tensor's device");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int f32 = dtype == KVAE_F32;
-  const long long Tg = round_up_ll(T_gy, dgg.g.stride);     // gy staged in whole stride groups of the data-gradient conv
+  // gy staged in whole stride groups of the data-gradient conv (a strided Conv1d; a transposed one reads single rows),
+  // x (the weight gradient's strided operand) in whole stride groups of the layer
+  const long long Tg = round_up_ll(T_gy, dgg.g.kind == kConv ? dgg.g.stride : 1);
+  const long long Tx = round_up_ll(T, transposed ? 1 : stride);
   uint8_t* base = static_cast<uint8_t*>(scratch);
   void* wpk = base;
   base += kvae_conv1d_packed_bytes(Cout, Cin, K, engine);
@@ -2156,6 +2177,8 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
   float* dW = reinterpret_cast<float*>(base);
   base += align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
   __nv_bfloat16* xcl = reinterpret_cast<__nv_bfloat16*>(base);
+  if (engine == 1) base += align_up(static_cast<size_t>(B) * Tx * Cin * 2, 1024);
+  void* gx_groups = base;     // tcgen05 data gradient of a strided Conv1d whose T is not whole stride groups
   if (dbias) {
     bias_grad_cf_kernel<<<Cout, 256, 0, st>>>(gy, f32, dbias, B, Cout, T_gy);
     KV_CUDA(cudaGetLastError());
@@ -2173,15 +2196,16 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
     const int R = transposed ? Cin : Cout, Cc = transposed ? Cout : Cin;   // dim 0 of the torch weight and the rest
     if (engine == 1) {
       // tensor-core weight gradient into the packed [K][R][Cc] layout, then the weight-norm backward from it
-      dim3 grid(ceil_div(static_cast<int>(T), 32), ceil_div(Cin, 32), B), block(32, 8);
-      cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, f32, xcl, Cin, static_cast<int>(T), 0);
+      // rows [T, Tx) (a strided layer's last stride group) written as zeros
+      dim3 grid(ceil_div(static_cast<int>(Tx), 32), ceil_div(Cin, 32), B), block(32, 8);
+      cf_to_cl_bf16_kernel<<<grid, block, 0, st>>>(x, f32, xcl, Cin, static_cast<int>(Tx), 0, 0, T, 0, static_cast<int>(T));
       KV_CUDA(cudaGetLastError());
       ++g_launches;
       KV_CUDA(cudaMemsetAsync(dW, 0, static_cast<size_t>(Cin) * Cout * K * 4, st));
       WgradLaunch L;
       const bool ok = transposed
           ? prepare_wgrad_umma(xcl, static_cast<int>(T), Cin, gcl, static_cast<int>(Tg), Cout, B, K, stride, dilation, padding, dW, L, err)
-          : prepare_wgrad_umma(gcl, static_cast<int>(T_gy), Cout, xcl, static_cast<int>(T), Cin, B, K, stride, dilation, padding, dW, L, err);
+          : prepare_wgrad_umma(gcl, static_cast<int>(T_gy), Cout, xcl, static_cast<int>(Tx), Cin, B, K, stride, dilation, padding, dW, L, err);
       if (!ok) return fail(err);
       KV_CUDA(launch_wgrad_umma(L, st));
       ++g_launches;
@@ -2201,8 +2225,19 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
   }
   if (!gx) return 0;
   if (pack_conv_weights(w, !transposed, Cout, Cin, K, engine, dgg.flip, wpk, st)) return -1;
-  return conv1d_rows(dgg.g, gy, T_gy, 0, T_gy, T_gy, gx, T, wpk, nullptr, B, 0, T, dtype, engine, gcl, gcl_bytes, st,
-                     engine == 1);
+  // the tcgen05 engines emit whole stride groups of a transposed conv: a strided Conv1d's gx of T rows not whole groups
+  // goes through scratch and its rows [0, T) are copied out
+  const bool groups = engine && Tx != T;
+  const long long To = groups ? Tx : T;
+  if (conv1d_rows(dgg.g, gy, T_gy, 0, T_gy, T_gy, groups ? gx_groups : gx, To, wpk, nullptr, B, 0, To, dtype, engine, gcl,
+                  gcl_bytes, st, engine == 1))
+    return -1;
+  if (groups) {
+    const size_t es = f32 ? 4 : 2;
+    KV_CUDA(cudaMemcpy2DAsync(gx, T * es, gx_groups, To * es, T * es, static_cast<size_t>(B) * Cin,
+                              cudaMemcpyDeviceToDevice, st));
+  }
+  return 0;
 }
 
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)
