@@ -254,13 +254,6 @@ int kvae_gaussian_nll(const void* x, const void* xhat, void* gxhat, float* loss,
 int kvae_adamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, size_t n, float lr,
                     float beta1, float beta2, float eps, float weight_decay, int step, float grad_scale, void* stream);
 
-/* Backward of kvae_conv1d_fwd (autograd of F.conv1d / F.conv_transpose1d on the stand-alone WNConv1d /
- * WNConvTranspose1d modules): dw = gradient of the folded weight (torch layout, overwritten), dbias [Cout] and gx
- * (same shape as x); each of the three is optional (NULL = not computed).  fp32 arithmetic; x, gy, gx of `dtype`.  scratch as for kvae_conv1d_fwd. */
-int kvae_conv1d_bwd(const void* x, const void* gy, const float* w_folded, void* gx, float* dw, float* dbias,
-                    int transposed, int B, int Cin, int Cout, long long T, int K, int stride, int dilation, int padding,
-                    int dtype, void* scratch, size_t scratch_bytes, void* stream);
-
 /* ---- Multi-resolution STFT loss of the autoencoder training wrapper (SURVEY section 8f item 4, loss half) ----
  * training/losses/auraloss.py: MultiResolutionSTFTLoss (443-531) / SumAndDifferenceSTFTLoss (534-606) over STFTLoss
  * (220-441: torch.stft with reflect padding and a periodic Hann window, magnitude sqrt(clamp(re^2 + im^2, 1e-8)),
@@ -375,9 +368,11 @@ int kvae_unary_bwd(const void* t, const void* gy, void* gx, size_t n, int op, fl
  * kvae_axpby itself.) */
 int kvae_gauss_sample_bwd(const void* x, const void* noise, const void* gz, void* gx, int B, int D, long long T, int dtype,
                           void* stream);
-/* Backward of a BigVGANFlowVAE conv layer (Conv1d :566-620, ConvTranspose1d :336-391, and the encoder's Conv1d_S
- * :139-172, whose downsampling convs have stride 2 .. 8; the layer geometry is the forward's: padding on both sides, a
- * causal layer being the symmetric-padded one truncated; a strided Conv1d has dilation 1).  gy: the gradient of
+/* Backward of a conv layer of kvae_conv1d_fwd / kvae_conv1d_win_fwd: the stand-alone WNConv1d / WNConvTranspose1d
+ * (autograd of F.conv1d / F.conv_transpose1d and weight_norm) and the conv layers of BigVGANFlowVAE (Conv1d :566-620,
+ * ConvTranspose1d :336-391, and the encoder's Conv1d_S :139-172, whose downsampling convs have stride 2 .. 8).  The
+ * layer geometry is the forward's: padding >= 0 on both sides, a causal layer being the symmetric-padded one truncated;
+ * a strided Conv1d and a ConvTranspose1d have dilation 1; the tcgen05 engines take padding <= d (K - 1).  gy: the gradient of
  * the layer's output rows [0, T_gy) ([B, Cout, T_gy] of `dtype`); rows past T_gy (a causal layer's dropped rows) have
  * none.  x: the layer's input [B, Cin, T].  w: the folded fp32 weight.  Each product is optional (NULL = skipped):
  *   gx [B, Cin, T] (`dtype`)  the forward conv kernels under the data-gradient geometry (kvae_conv1d_dgrad_form) on
@@ -401,7 +396,8 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
 /* The data-gradient geometry kvae_conv1d_win_bwd runs: gx = rows [0, T) of the Conv1d (out[0] input channels, out[1]
  * output channels, stride out[2], dilation out[3], left padding out[4], zero rows past the end of gy) of gy with the
  * layer's weight transposed to [Cin, Cout, K] with its taps reversed (out[5] = 1: a Conv1d of stride 1, new left
- * padding d (K - 1) - padding), or as it is (out[5] = 0: a ConvTranspose1d, stride s, padding p). */
+ * padding d (K - 1) - padding, negative when padding > d (K - 1): gx then reads gy ahead), or as it is (out[5] = 0: a
+ * ConvTranspose1d, stride s, padding p). */
 int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]);
 /* The same for every layer kvae_conv1d_win_bwd accepts, the kind of conv first: gx = rows [0, T) of the Conv1d
  * (out[0] = 0, as kvae_conv1d_dgrad_geom's out[0 .. 5] in out[1 .. 6]) or the ConvTranspose1d (out[0] = 1: a strided
@@ -447,8 +443,8 @@ int kvae_vae_sample(const void* mean, const void* scale, const void* noise, void
  * stable_audio_tools/models/discriminators.py: SharedDiscriminatorConvNet (62-116), MultiScaleDiscriminator (119-138),
  * MultiPeriodDiscriminator (140-168), MultiDiscriminator (171-238), OobleckDiscriminator.loss (240-297),
  * get_hinge_losses (11-14); wired at training/autoencoders.py:133-134, 288.  Every net is a stack of strided
- * convolutions + SiLU; they run on kvae_disc_conv15_* / kvae_disc_conv1x1_* below (kvae_conv1d_fwd / kvae_conv1d_bwd for
- * any other kernel size / stride; dw may be NULL when only the data gradient is wanted).  The multi-period nets' 15 x 15 Conv2d over [N, C, ceil(T / n), n] becomes a Conv1d over the folded
+ * convolutions + SiLU; they run on kvae_disc_conv15_* / kvae_disc_conv1x1_* below (kvae_conv1d_fwd / kvae_conv1d_win_bwd on
+ * engine 0 for any other kernel size / stride; the weight gradient may be NULL when only the data gradient is wanted).  The multi-period nets' 15 x 15 Conv2d over [N, C, ceil(T / n), n] becomes a Conv1d over the folded
  * channels (c, w): same products, minus those with padding zeros.  All tensors fp32, contiguous; `backward` = 1 runs the
  * adjoint with the roles of the two tensor arguments exchanged (first = incoming gradient, second = outgoing). */
 /* MultiPeriodDiscriminator.fold (:164-168): y[b, c n + w, h] = x[b, c, h n + w] (0 past T); x [N, C, T], y [N, C n, ceil(T / n)] */
@@ -480,8 +476,9 @@ int kvae_disc_feature_match(const float* const* feats, const long long* half, in
                             const float* g_loss, float* const* grads, void* scratch, size_t scratch_bytes, void* stream);
 
 /* The nets' own conv geometry -- Conv1d(k = 15, stride 4, padding 7) on [N, Cin, T] fp32 with a folded weight in torch
- * layout (discriminators.py:70-71, 85-100) -- on register-tiled kernels written for it; same contract as kvae_conv1d_fwd /
- * kvae_conv1d_bwd (scratch: kvae_conv1d_scratch_bytes(Cin, Cout, 15); dw, dbias, gx each optional). */
+ * layout (discriminators.py:70-71, 85-100) -- on register-tiled kernels written for it; the forward has kvae_conv1d_fwd's
+ * contract, the backward writes dw (the gradient of the folded weight, torch layout), dbias and gx, each optional
+ * (scratch for both: kvae_conv1d_scratch_bytes(Cin, Cout, 15)). */
 int kvae_disc_conv15_supported(int K, int stride, int pad);
 int kvae_disc_conv15_fwd(const float* x, float* y, const float* w, const float* bias, int N, int Cin, int Cout, long long T,
                          void* scratch, size_t scratch_bytes, void* stream);

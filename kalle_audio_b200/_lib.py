@@ -145,9 +145,6 @@ SIGNATURES = {
     "kvae_conv1d_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                   C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                   C.c_void_p, C.c_size_t, C.c_void_p]),
-    "kvae_conv1d_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
-                                  C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                  C.c_void_p, C.c_size_t, C.c_void_p]),
     "kvae_conv1d_tc_supported": (C.c_int, [C.c_int] * 6),
     "kvae_conv1d_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "kvae_plan_param_count": (C.c_longlong, [C.c_void_p]),

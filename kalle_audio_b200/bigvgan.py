@@ -21,8 +21,10 @@ device) through the layer-level conv -- on the tensor cores for the layers whose
 CUDA-core ``kvae_conv1d_fwd`` -- the anti-aliased Snake / SnakeBeta activation as ONE fused kernel (``kvae_aa_act_fwd``:
 x2 Kaiser-sinc upsampling, activation, low-pass + x2 decimation -- six eager kernels and four double-rate intermediates
 in the reference), LeakyReLU / tanh / residual adds / the AMP average / the Gaussian sample as small elementwise
-kernels.  Under grad mode each of them has an autograd node whose backward is a libkvae call too (the ``_*Fn`` classes
-below; ``decode_with_grad``, ``encode_with_grad``).  ``forward`` (the training pass through the flow) is not built.
+kernels.  Under grad mode each of them has an autograd node whose backward is a libkvae call too (``decode_with_grad``,
+``encode_with_grad``): the ``_*Fn`` classes below, and for the convs the node every ``layers`` conv uses, whose backward
+is ``kvae_conv1d_win_bwd`` on the engine the forward ran on.  The causal layers set ``keep``, the output rows they keep.
+``forward`` (the training pass through the flow) is not built.
 """
 from __future__ import annotations
 
@@ -205,73 +207,6 @@ class _AaActFn(torch.autograd.Function):
         return (gx.to(ctx.x_dtype), da.to(ctx.p_dtypes[0]), None if db is None else db.to(ctx.p_dtypes[1]), None)
 
 
-class _BVConvFn(torch.autograd.Function):
-    """Conv1d / ConvTranspose1d of BigVGANFlowVAE: the forward is the no-grad call (grad mode is off inside),
-    the backward through kvae_conv1d_win_bwd on the same engine (0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05
-    bf16x3); no weight-gradient work when no conv parameter requires grad."""
-
-    @staticmethod
-    def forward(ctx, mod, x, tc, bias, *wparams):
-        y, engine = mod(x, tc), _engine_of(mod, x, tc)
-        ctx.mod, ctx.engine, ctx.x_dtype, ctx.T_gy = mod, engine, x.dtype, y.shape[2]
-        ctx.has_bias = bias is not None
-        xin = _k(x)
-        ctx.save_for_backward(xin, mod.folded_weight(), *[p.detach() for p in wparams])
-        return y
-
-    @staticmethod
-    def backward(ctx, gy):
-        mod = ctx.mod
-        xin, w, *wparams = ctx.saved_tensors
-        L = _lib.lib()
-        B, Cin, T = xin.shape
-        K, s, d, p = mod.kernel_size[0], mod.stride[0], mod.dilation[0], mod.padding[0]
-        Cout, tr = mod.out_channels, int(mod.transposed)
-        g = gy.detach().to(xin.dtype).contiguous()
-        need = ctx.needs_input_grad
-        gx = torch.empty_like(xin) if need[1] else None
-        db = torch.empty(Cout, dtype=torch.float32, device=xin.device) if ctx.has_bias and need[3] else None
-        dv = dg = vf = gf = None
-        if any(need[4:]):
-            if len(wparams) == 2:                  # (weight_g, weight_v): the weight norm's backward too
-                gf, vf = (t.float().contiguous() for t in wparams)
-                dg = torch.empty(vf.shape[0], dtype=torch.float32, device=vf.device)
-            dv = torch.empty(w.shape, dtype=torch.float32, device=w.device)
-        if gx is None and dv is None and db is None:
-            return (None,) * (4 + len(wparams))
-        ns = L.kvae_conv1d_win_bwd_scratch_bytes(tr, B, Cin, Cout, T, ctx.T_gy, K, s, ctx.engine)
-        scratch = torch.empty(ns, dtype=torch.uint8, device=xin.device)
-        _lib.check(L.kvae_conv1d_win_bwd(xin.data_ptr(), g.data_ptr(), ctx.T_gy, w.data_ptr(), _lib.ptr(vf), _lib.ptr(gf),
-                                         _lib.ptr(gx), _lib.ptr(dv), _lib.ptr(dg), _lib.ptr(db), tr, B, Cin, Cout, T, K,
-                                         s, d, p, _lib.dtype_code(xin.dtype), ctx.engine, scratch.data_ptr(), ns,
-                                         _lib.stream_ptr(xin.device)))
-        if dv is None:
-            wgrads = (None,) * len(wparams)
-        elif len(wparams) == 2:
-            wgrads = (dg.view_as(wparams[0]).to(wparams[0].dtype), dv.to(wparams[1].dtype))
-        else:
-            wgrads = (dv.to(wparams[0].dtype),)
-        return (None, None if gx is None else gx.to(ctx.x_dtype), None, db, *wgrads)
-
-
-def _conv_grad(mod, x, tc):
-    """mod(x) under autograd when the input or a conv parameter requires grad (grad mode on), else None."""
-    wparams = (mod.weight_g, mod.weight_v) if mod.has_weight_norm else (mod._parameters["weight"],)
-    if not _grad_on(x, mod.bias, *wparams):
-        return None
-    _lib.require_cuda(x, type(mod).__name__ + ".forward")
-    return _BVConvFn.apply(mod, x, tc, mod.bias, *wparams)
-
-
-def _engine_of(mod, x, tc) -> int:
-    """The engine the no-grad call runs the layer on: _forward_tc's condition for the tensor cores (only a strided conv
-    with a truncated output goes back to the CUDA cores there, and no strided conv is truncated: the decoder's convs
-    have stride 1, the encoder's are never causal)."""
-    if tc and x.shape[2] >= TC_MIN_ROWS and mod.tc_layer():
-        return 1 if mod.tc_precision == "bf16" else 2
-    return 0
-
-
 class LeakyReLU(nn.Module):
     def __init__(self, negative_slope: float = 0.01, inplace: bool = False):
         super().__init__()
@@ -384,16 +319,8 @@ class Conv1d(WNConv1d):
         pad = dilation * (kernel_size - 1) if causal else int((kernel_size * dilation - dilation) / 2)
         super().__init__(in_channels, out_channels, kernel_size, stride=stride, padding=pad, dilation=dilation, bias=bias)
 
-    def forward(self, x, tc=True):
-        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
-        if y is not None:
-            return y
-        if self.causal and self.kernel_size[0] > 1:
-            y = self._forward_tc(x, keep=x.shape[2]) if tc else None   # tensor-core layers truncate inside the kernel
-            if y is not None:
-                return y
-            return super().forward(x, tc=False)[:, :, :x.shape[2]].contiguous()
-        return super().forward(x, tc)
+    def keep(self, T: int) -> int:
+        return T if self.causal and self.kernel_size[0] > 1 else self.out_len(T)
 
 
 class ConvTranspose1d(WNConvTranspose1d):
@@ -407,29 +334,8 @@ class ConvTranspose1d(WNConvTranspose1d):
                          padding=0 if causal else (kernel_size - stride) // 2)
         self._drop = stride if causal else 0
 
-    def forward(self, x, tc=True):
-        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
-        if y is not None:
-            return y
-        if self._drop:
-            y = self._forward_tc(x, keep=x.shape[2] * self.stride[0]) if tc else None
-            if y is not None:
-                return y
-            return super().forward(x, tc=False)[:, :, :-self._drop].contiguous()
-        return super().forward(x, tc)
-
-
-class _EncConv1d(WNConv1d):
-    """The encoder's convs (``Conv1d_S.layer``, the ResStack convs): ``layers.WNConv1d`` with an autograd node of its
-    own.  ``WNConv1d`` differentiates through ``_ConvFn``, fp32 on the CUDA cores whatever ``set_precision`` says; here
-    grad mode runs ``_BVConvFn``, whose forward is the no-grad call (``extract_latents``' engine and bits) and whose
-    backward runs on that engine."""
-
-    def forward(self, x, tc=True):
-        y = _conv_grad(self, x, tc) if torch.is_grad_enabled() else None     # autograd node (_BVConvFn)
-        if y is not None:
-            return y
-        return super().forward(x, tc)
+    def keep(self, T: int) -> int:
+        return self.out_len(T) - self._drop
 
 
 class Conv1d_S(nn.Module):
@@ -437,8 +343,8 @@ class Conv1d_S(nn.Module):
 
     def __init__(self, in_channels, out_channels, kernel_size=1, stride=1, dilation=1):
         super().__init__()
-        self.layer = _EncConv1d(in_channels, out_channels, kernel_size, stride=stride,
-                                padding=dilation * (kernel_size - 1) // 2, dilation=dilation)
+        self.layer = WNConv1d(in_channels, out_channels, kernel_size, stride=stride,
+                              padding=dilation * (kernel_size - 1) // 2, dilation=dilation)
 
     def forward(self, x):
         return self.layer(x)
@@ -450,8 +356,8 @@ class ResStack(nn.Module):
     def __init__(self, channel, kernel_size=3, base=3, nums=4):
         super().__init__()
         self.layers = nn.ModuleList([
-            nn.Sequential(LeakyReLU(), _EncConv1d(channel, channel, kernel_size, dilation=base ** i, padding=base ** i),
-                          LeakyReLU(), _EncConv1d(channel, channel, kernel_size, dilation=1, padding=1))
+            nn.Sequential(LeakyReLU(), WNConv1d(channel, channel, kernel_size, dilation=base ** i, padding=base ** i),
+                          LeakyReLU(), WNConv1d(channel, channel, kernel_size, dilation=1, padding=1))
             for i in range(nums)])
 
     def forward(self, x):

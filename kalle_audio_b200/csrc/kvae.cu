@@ -1801,52 +1801,6 @@ size_t kvae_conv1d_scratch_bytes(int Cin, int Cout, int K) {
   return align_up(static_cast<size_t>(Cin) * Cout * K * 4, 1024);
 }
 
-int kvae_conv1d_bwd(const void* x, const void* gy, const float* w, void* gx, float* dw, float* dbias, int transposed,
-                    int B, int Cin, int Cout, long long T, int K, int stride, int dilation, int padding, int dtype,
-                    void* scratch, size_t scratch_bytes, void* stream) {
-  if (!x || !gy || !w || !scratch) return fail("null argument");
-  if (!dw && !gx && !dbias) return fail("nothing to compute (dw, dbias and gx are all null)");
-  if (!check_dtype(dtype)) return fail("bad dtype");
-  if (B <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || T <= 0) return fail("empty input");
-  if (stride < 1 || stride > kMaxPhases) return fail("stride out of range (1..8)");
-  if (scratch_bytes < kvae_conv1d_scratch_bytes(Cin, Cout, K)) return fail("scratch too small");
-  ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
-  const long long T_out = g.out_len(static_cast<int>(T));
-  if (T_out <= 0) return fail("input shorter than the kernel");
-  DeviceGuard guard(device_of(x));
-  if (!guard.ok) return fail("cannot select the tensor's device");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int f32 = (dtype == KVAE_F32);
-  // ---- weight gradient (torch layout), straight from the API layout through element strides
-  const size_t n = static_cast<size_t>(Cin) * Cout * K;
-  const long long xsB = static_cast<long long>(Cin) * T, gsB = static_cast<long long>(Cout) * T_out;
-  if (dw) KV_CUDA(launch_wgrad_direct_cf(x, gy, f32, dw, transposed, B, Cin, Cout, T, T_out, K, stride, dilation, padding, st));
-  if (dbias) {
-    bias_grad_cf_kernel<<<Cout, 256, 0, st>>>(gy, f32, dbias, B, Cout, T_out);
-    KV_CUDA(cudaGetLastError());
-    ++g_launches;
-  }
-  if (!gx) return 0;
-  // ---- data gradient: the forward kernel under the opposite kind, same weight tensor
-  const ConvGeom gd = dgrad_geom(g, static_cast<int>(T));
-  DirectLaunch L;
-  std::string err;
-  if (!prepare_direct(gd, B, T_out, T, 0, L, err)) return fail(err);
-  float* wd = static_cast<float*>(scratch);
-  pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(
-      w, gd.kind == kConvT, gd.Cout, gd.Cin, K, nullptr, wd);
-  KV_CUDA(cudaGetLastError());
-  DirectParams& d = L.d;
-  d.x = gy; d.x_f32 = f32;
-  d.x_sB = gsB; d.x_sT = 1; d.x_sC = T_out;
-  d.w = wd;
-  d.out_raw = gx; d.out_raw_f32 = f32;
-  d.o_sB = xsB; d.o_sT = 1; d.o_sC = T;
-  KV_CUDA(launch_direct(L, st));
-  g_launches += 2;
-  return 0;
-}
-
 int kvae_conv1d_tc_supported(int Cin, int Cout, int K, int stride, int dilation, int transposed) {
   ConvGeom g{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, 0};
   if (!umma_supported(g) || stride < 1 || stride > kMaxPhases || K > kMaxTaps) return 0;
@@ -2070,16 +2024,17 @@ int kvae_conv1d_fwd(const void* x, void* y, const float* w, const float* bias, i
   return conv1d_rows(g, x, T, 0, T, T, y, T_out, scratch, bias, B, 0, T_out, dtype, 0, nullptr, 0, st);
 }
 
-// ------------------------------------------------------------------ BigVGANFlowVAE conv backward
+// ------------------------------------------------------------------ layer-level conv backward
 namespace {
 // The data gradient of a layer as a conv over the layer's output gradient gy (run by conv1d_rows, rows of gy past its
 // end reading as zero):
-//   Conv1d, stride 1, left padding pl <= d (K - 1): gx = the conv of gy with the weight transposed ([Cin, Cout, K]) and
-//     its taps reversed, same dilation, left padding d (K - 1) - pl;
-//   Conv1d, stride s > 1, dilation 1, padding p < K: gx = the ConvTranspose1d of gy with the same weight (read as the
-//     transposed conv's [Cin', Cout', K] = [Cout, Cin, K]), stride s, padding p, continued past its natural length to
-//     the layer's T input rows (torch's output_padding): those rows are input rows the forward read;
+//   Conv1d, stride 1, padding pl: gx = the conv of gy with the weight transposed ([Cin, Cout, K]) and its taps
+//     reversed, same dilation, left padding d (K - 1) - pl (negative when pl > d (K - 1): gx reads gy ahead);
+//   Conv1d, stride s > 1, dilation 1, padding p: gx = the ConvTranspose1d of gy with the same weight (read as the
+//     transposed conv's [Cin', Cout', K] = [Cout, Cin, K]), stride s, padding p, continued past its natural length over
+//     zero gy rows to the layer's T input rows (torch's output_padding): those rows are input rows the forward read;
 //   ConvTranspose1d, stride s, padding p: gx = the strided Conv1d of gy with the same weight, stride s, padding p.
+// conv_direct_kernel takes any tap offset; the tcgen05 engines take padding <= d (K - 1) only (kvae_conv1d_win_bwd).
 struct DgradGeom {
   ConvGeom g;      // Cin = the layer's Cout, Cout = the layer's Cin; kConvT for a strided Conv1d, else kConv
   int flip;        // the weight's taps reversed (Conv1d of stride 1)
@@ -2088,18 +2043,16 @@ bool dgrad_conv_geom(int transposed, int Cin, int Cout, int K, int stride, int d
                      std::string& err) {
   if (Cin <= 0 || Cout <= 0 || K <= 0 || dilation < 1) { err = "conv backward: empty layer"; return false; }
   if (stride < 1 || stride > kMaxPhases) { err = "stride out of range (1..8)"; return false; }
+  if (padding < 0) { err = "conv backward: negative padding"; return false; }
   if (!transposed && stride > 1) {
     if (dilation != 1) { err = "conv backward: a strided Conv1d of dilation 1 only"; return false; }
-    if (padding < 0 || padding >= K) { err = "conv backward: strided Conv1d padding outside 0 .. K - 1"; return false; }
     d.g = ConvGeom{kConvT, Cout, Cin, K, stride, 1, padding};
     d.flip = 0;
   } else if (!transposed) {
-    if (padding < 0 || padding > dilation * (K - 1)) { err = "conv backward: Conv1d padding outside 0 .. d (K - 1)"; return false; }
     d.g = ConvGeom{kConv, Cout, Cin, K, 1, dilation, dilation * (K - 1) - padding};
     d.flip = 1;
   } else {
     if (dilation != 1) { err = "conv backward: ConvTranspose1d of dilation 1 only"; return false; }
-    if (padding < 0 || padding >= K) { err = "conv backward: ConvTranspose1d padding outside 0 .. K - 1"; return false; }
     d.g = ConvGeom{kConv, Cout, Cin, K, stride, 1, padding};
     d.flip = 0;
   }
@@ -2107,6 +2060,27 @@ bool dgrad_conv_geom(int transposed, int Cin, int Cout, int K, int stride, int d
 }
 
 long long round_up_ll(long long v, long long m) { return (v + m - 1) / m * m; }
+
+// gx [B, Cin, T] of `dtype` of a layer (`transposed`, its data-gradient geometry d) from gy [B, Cout, T_gy] on
+// `engine`: the layer's weight w packed under the opposite kind into wpk (kvae_conv1d_packed_bytes(Cout, Cin, K,
+// engine)), then rows [0, T) of the conv d.g of gy.  gcl / gcl_bytes: conv1d_rows' scratch; engine 1 expects gy already
+// staged there channels-last.  The tcgen05 engines emit whole stride groups of a transposed conv: a strided Conv1d's gx
+// of T rows not whole groups is computed into gx_groups and its rows [0, T) are copied out.
+int conv1d_dgrad(int transposed, const DgradGeom& d, const void* gy, long long T_gy, const float* w, void* gx, int B,
+                 long long T, int dtype, int engine, void* wpk, void* gcl, size_t gcl_bytes, void* gx_groups,
+                 cudaStream_t st) {
+  if (pack_conv_weights(w, !transposed, d.g.Cin, d.g.Cout, d.g.K, engine, d.flip, wpk, st)) return -1;
+  const long long To = engine && d.g.kind == kConvT ? round_up_ll(T, d.g.stride) : T;
+  if (conv1d_rows(d.g, gy, T_gy, 0, T_gy, T_gy, To != T ? gx_groups : gx, To, wpk, nullptr, B, 0, To, dtype, engine, gcl,
+                  gcl_bytes, st, engine == 1))
+    return -1;
+  if (To != T) {
+    const size_t es = dtype == KVAE_F32 ? 4 : 2;
+    KV_CUDA(cudaMemcpy2DAsync(gx, T * es, gx_groups, To * es, T * es, static_cast<size_t>(B) * d.g.Cout,
+                              cudaMemcpyDeviceToDevice, st));
+  }
+  return 0;
+}
 }  // namespace
 
 int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[6]) {
@@ -2153,6 +2127,7 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
   DgradGeom dgg;
   std::string err;
   if (!dgrad_conv_geom(transposed, Cin, Cout, K, stride, dilation, padding, dgg, err)) return fail(err);
+  if (engine && padding > dilation * (K - 1)) return fail("tcgen05 engines: conv backward padding outside 0 .. d (K - 1)");
   const ConvGeom lg{transposed ? kConvT : kConv, Cin, Cout, K, stride, dilation, padding};
   if (T >= (1LL << 30) || lg.out_len(static_cast<int>(T)) >= (1LL << 30)) return fail("rows beyond 2^30");
   if (T_gy < 1 || T_gy > lg.out_len(static_cast<int>(T))) return fail("T_gy outside 1 .. the layer's output length");
@@ -2224,20 +2199,7 @@ int kvae_conv1d_win_bwd(const void* x, const void* gy, long long T_gy, const flo
     }
   }
   if (!gx) return 0;
-  if (pack_conv_weights(w, !transposed, Cout, Cin, K, engine, dgg.flip, wpk, st)) return -1;
-  // the tcgen05 engines emit whole stride groups of a transposed conv: a strided Conv1d's gx of T rows not whole groups
-  // goes through scratch and its rows [0, T) are copied out
-  const bool groups = engine && Tx != T;
-  const long long To = groups ? Tx : T;
-  if (conv1d_rows(dgg.g, gy, T_gy, 0, T_gy, T_gy, groups ? gx_groups : gx, To, wpk, nullptr, B, 0, To, dtype, engine, gcl,
-                  gcl_bytes, st, engine == 1))
-    return -1;
-  if (groups) {
-    const size_t es = f32 ? 4 : 2;
-    KV_CUDA(cudaMemcpy2DAsync(gx, T * es, gx_groups, To * es, T * es, static_cast<size_t>(B) * Cin,
-                              cudaMemcpyDeviceToDevice, st));
-  }
-  return 0;
+  return conv1d_dgrad(transposed, dgg, gy, T_gy, w, gx, B, T, dtype, engine, wpk, gcl, gcl_bytes, gx_groups, st);
 }
 
 // ------------------------------------------------------------------ multi-resolution STFT loss (mrstft.cuh)
@@ -3226,9 +3188,12 @@ int kvae_disc_conv15_bwd(const float* x, const float* gy, const float* w, float*
     ++g_launches;
     return 0;
   }
-  if (Cin < 32)
-    return kvae_conv1d_bwd(x, gy, w, gx, nullptr, nullptr, 0, N, Cin, Cout, T, kDK, kDS, 1, kDP, KVAE_F32, scratch,
-                           scratch_bytes, stream);
+  if (Cin < 32) {        // the layer-level data gradient on the CUDA cores: a ConvTranspose1d of stride 4
+    DgradGeom d;
+    std::string err;
+    if (!dgrad_conv_geom(0, Cin, Cout, kDK, kDS, 1, kDP, d, err)) return fail(err);
+    return conv1d_dgrad(0, d, gy, To, w, gx, N, T, KVAE_F32, 0, scratch, nullptr, 0, nullptr, st);
+  }
   float* wT = static_cast<float*>(scratch);
   pack_weights_kernel<<<static_cast<int>(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, st>>>(w, 1, Cin, Cout, kDK, nullptr, wT);
   KV_CUDA(cudaGetLastError());

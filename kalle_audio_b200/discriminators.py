@@ -12,7 +12,7 @@ the same ``torch.manual_seed`` gives the reference's random-init ``state_dict``.
 
 Compute: every net is ONE autograd node (``_SharedNetFn``) whose forward and backward chain libkvae kernels -- the
 strided convolutions on ``kvae_disc_conv15_fwd`` / ``kvae_disc_conv15_bwd`` (fp32 kernels written for the nets' k = 15 /
-stride 4 geometry; any other geometry on ``kvae_conv1d_fwd`` / ``kvae_conv1d_bwd``), everything between them on the
+stride 4 geometry; any other geometry on ``kvae_conv1d_fwd`` / ``kvae_conv1d_win_bwd``), everything between them on the
 other ``kvae_disc_*`` entry points (csrc/disc.cuh).  The multi-period nets' 15 x 15 ``Conv2d`` over ``[N, C, ceil(T / n), n]``
 runs as a ``Conv1d`` over the folded channels ``(c, w)``: identical products, without the ones that only ever meet the
 zero padding of the width axis (n <= 11 < 15).  ``EncodecDiscriminator`` and ``DACGANLoss`` wrap un-vendored packages
@@ -38,7 +38,7 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
     return t.contiguous() if t.dtype == torch.float32 else t.float().contiguous()
 
 
-# KVAE_DISC_GENERIC=1: development switch -- every conv on the generic layer kernels (kvae_conv1d_fwd / kvae_conv1d_bwd)
+# KVAE_DISC_GENERIC=1: development switch -- every conv on the generic layer kernels (kvae_conv1d_fwd / kvae_conv1d_win_bwd)
 # instead of the kernels written for the nets' own k = 15 / stride 4 / padding 7 geometry (same results to fp32 rounding)
 _GENERIC = os.environ.get("KVAE_DISC_GENERIC", "0") == "1"
 
@@ -78,15 +78,18 @@ def _conv_bwd(x, gy, w, Cin, Cout, K, stride, pad, want_gx, want_dw, want_db):
         _lib.check(L.kvae_disc_conv1x1_bwd(x.data_ptr(), gy.data_ptr(), w.data_ptr(), _lib.ptr(gx), _lib.ptr(dw), _lib.ptr(db),
                                            N, Cin, Cout, T, _lib.stream_ptr(x.device)))
         return gx, dw, db
-    ns = L.kvae_conv1d_scratch_bytes(Cin, Cout, K)
-    scratch = torch.empty(ns, dtype=torch.uint8, device=x.device)
     if not _GENERIC and L.kvae_disc_conv15_supported(K, stride, pad):
+        ns = L.kvae_conv1d_scratch_bytes(Cin, Cout, K)
+        scratch = torch.empty(ns, dtype=torch.uint8, device=x.device)
         _lib.check(L.kvae_disc_conv15_bwd(x.data_ptr(), gy.data_ptr(), w.data_ptr(), _lib.ptr(gx), _lib.ptr(dw), _lib.ptr(db),
                                           N, Cin, Cout, T, scratch.data_ptr(), ns, _lib.stream_ptr(x.device)))
         return gx, dw, db
-    _lib.check(L.kvae_conv1d_bwd(x.data_ptr(), gy.data_ptr(), w.data_ptr(), _lib.ptr(gx), _lib.ptr(dw), _lib.ptr(db), 0, N,
-                                 Cin, Cout, T, K, stride, 1, pad, _lib.KVAE_F32, scratch.data_ptr(), ns,
-                                 _lib.stream_ptr(x.device)))
+    T_gy = gy.shape[2]
+    ns = L.kvae_conv1d_win_bwd_scratch_bytes(0, N, Cin, Cout, T, T_gy, K, stride, 0)
+    scratch = torch.empty(ns, dtype=torch.uint8, device=x.device)
+    _lib.check(L.kvae_conv1d_win_bwd(x.data_ptr(), gy.data_ptr(), T_gy, w.data_ptr(), None, None, _lib.ptr(gx), _lib.ptr(dw),
+                                     None, _lib.ptr(db), 0, N, Cin, Cout, T, K, stride, 1, pad, _lib.KVAE_F32, 0,
+                                     scratch.data_ptr(), ns, _lib.stream_ptr(x.device)))
     return gx, dw, db
 
 

@@ -9,10 +9,13 @@ reference:
 Parameters are initialised through torch's own ``nn.Conv1d`` / ``nn.ConvTranspose1d`` constructors, so
 the same ``torch.manual_seed`` yields the same random-init ``state_dict`` as the reference.
 
-``forward`` / ``backward`` of a leaf run the layer-level C-ABI kernels (fp32 arithmetic, autograd nodes
-``_SnakeFn`` / ``_ConvFn``); a conv with ``tc_precision`` set runs its forward on the tensor cores through
-``packed_weight`` / ``conv_rows``, which the streaming BigVGAN decoder calls on its windows too.  The fast path is
-not here: ``OobleckEncoder`` / ``OobleckDecoder`` hand the whole stack to a fused plan (see ``_plan.py``).
+``forward`` / ``backward`` of a leaf run the layer-level C-ABI kernels (fp32 arithmetic by default, autograd nodes
+``_SnakeFn`` / ``_ConvLayerFn``).  A conv with ``tc_precision`` set runs its forward on the tensor cores through
+``packed_weight`` / ``conv_rows``, which the streaming BigVGAN decoder calls on its windows too.  ``engine`` picks the
+engine of a call, and ``keep`` the output rows a layer keeps (BigVGANFlowVAE's causal layers keep the first ones).
+Every conv layer, BigVGANFlowVAE's included, differentiates through ``_ConvLayerFn``: its forward is the no-grad call,
+its backward ``kvae_conv1d_win_bwd`` on the same engine.  The fast path is not here: ``OobleckEncoder`` /
+``OobleckDecoder`` hand the whole stack to a fused plan (see ``_plan.py``).
 """
 from __future__ import annotations
 
@@ -56,17 +59,23 @@ class _SnakeFn(torch.autograd.Function):
                 None)
 
 
-class _ConvFn(torch.autograd.Function):
-    """WNConv1d / WNConvTranspose1d forward / backward on [B, C, T]: kvae_conv1d_fwd, kvae_conv1d_bwd and the
-    weight-norm backward (autograd of torch.nn.utils.weight_norm + F.conv1d / F.conv_transpose1d)."""
+class _ConvLayerFn(torch.autograd.Function):
+    """Every conv layer under autograd (WNConv1d / WNConvTranspose1d and BigVGANFlowVAE's layers built on them): the
+    forward is the layer's no-grad call (grad mode is off inside), so it runs the same kernels on the same engine; the
+    backward is kvae_conv1d_win_bwd on that engine (0 = CUDA cores fp32, 1 = tcgen05 bf16, 2 = tcgen05 bf16x3), with no
+    weight-gradient work when no conv parameter requires grad.  A 'same' conv with an even kernel differentiates its
+    padded input (one more zero row on the right) and returns the gradient of the first T rows."""
 
     @staticmethod
-    def forward(ctx, mod, x, bias, *wparams):
-        y, xin, w = mod._forward_impl(x.detach())
-        ctx.mod = mod
-        ctx.save_for_backward(xin, w, *[p.detach() for p in wparams])
+    def forward(ctx, mod, x, tc, bias, *wparams):
+        T = x.shape[2]
+        y = mod(x, tc)
+        ctx.mod, ctx.engine, ctx.x_dtype, ctx.T, ctx.T_gy = mod, mod.engine(T, tc, mod.keep(T)), x.dtype, T, y.shape[2]
         ctx.has_bias = bias is not None
-        ctx.x_dtype = x.dtype
+        xin = x.detach() if x.dtype in (torch.float32, torch.bfloat16) else x.detach().float()
+        if mod._same_extra_right:
+            xin = torch.nn.functional.pad(xin, (0, mod._same_extra_right))
+        ctx.save_for_backward(xin.contiguous(), mod.folded_weight(), *[p.detach() for p in wparams])
         return y
 
     @staticmethod
@@ -74,28 +83,34 @@ class _ConvFn(torch.autograd.Function):
         mod = ctx.mod
         xin, w, *wparams = ctx.saved_tensors
         L = _lib.lib()
-        g = gy.detach().to(xin.dtype).contiguous()
-        B, _, T = xin.shape
+        B, Cin, T = xin.shape
         K, s, d, p = mod.kernel_size[0], mod.stride[0], mod.dilation[0], mod.padding[0]
-        gx = torch.empty_like(xin) if ctx.needs_input_grad[1] else None
-        dw = torch.empty_like(w)
-        db = torch.empty(mod.out_channels, dtype=torch.float32, device=xin.device) if ctx.has_bias else None
-        nscratch = L.kvae_conv1d_scratch_bytes(mod.in_channels, mod.out_channels, K)
-        scratch = torch.empty(nscratch, dtype=torch.uint8, device=xin.device)
-        _lib.check(L.kvae_conv1d_bwd(xin.data_ptr(), g.data_ptr(), w.data_ptr(), _lib.ptr(gx), dw.data_ptr(), _lib.ptr(db),
-                                     int(mod.transposed), B, mod.in_channels, mod.out_channels, T, K, s, d, p,
-                                     _lib.dtype_code(xin.dtype), scratch.data_ptr(), nscratch, _lib.stream_ptr(xin.device)))
-        if len(wparams) == 2:     # (weight_g, weight_v): weight-norm backward
-            gparam, v = wparams
-            vf, gf = v.float().contiguous(), gparam.float().contiguous()
-            dv, dg = torch.empty_like(vf), torch.empty(vf.shape[0], dtype=torch.float32, device=vf.device)
-            _lib.check(L.kvae_weight_norm_bwd(vf.data_ptr(), gf.data_ptr(), dw.data_ptr(), dv.data_ptr(), dg.data_ptr(),
-                                              vf.shape[0], vf[0].numel(), _lib.stream_ptr(vf.device)))
-            wgrads = (dg.view_as(gparam).to(gparam.dtype), dv.to(v.dtype))
-        else:                     # plain weight (weight norm removed)
-            wgrads = (dw.to(wparams[0].dtype),)
-        gxo = None if gx is None else gx.to(ctx.x_dtype)
-        return (None, gxo, None if db is None else db, *wgrads)
+        Cout, tr = mod.out_channels, int(mod.transposed)
+        g = gy.detach().to(xin.dtype).contiguous()
+        need = ctx.needs_input_grad
+        gx = torch.empty_like(xin) if need[1] else None
+        db = torch.empty(Cout, dtype=torch.float32, device=xin.device) if ctx.has_bias and need[3] else None
+        dv = dg = vf = gf = None
+        if any(need[4:]):
+            if len(wparams) == 2:                  # (weight_g, weight_v): the weight norm's backward too
+                gf, vf = (t.float().contiguous() for t in wparams)
+                dg = torch.empty(vf.shape[0], dtype=torch.float32, device=vf.device)
+            dv = torch.empty(w.shape, dtype=torch.float32, device=w.device)
+        if gx is None and dv is None and db is None:
+            return (None,) * (4 + len(wparams))
+        ns = L.kvae_conv1d_win_bwd_scratch_bytes(tr, B, Cin, Cout, T, ctx.T_gy, K, s, ctx.engine)
+        scratch = torch.empty(ns, dtype=torch.uint8, device=xin.device)
+        _lib.check(L.kvae_conv1d_win_bwd(xin.data_ptr(), g.data_ptr(), ctx.T_gy, w.data_ptr(), _lib.ptr(vf), _lib.ptr(gf),
+                                         _lib.ptr(gx), _lib.ptr(dv), _lib.ptr(dg), _lib.ptr(db), tr, B, Cin, Cout, T, K,
+                                         s, d, p, _lib.dtype_code(xin.dtype), ctx.engine, scratch.data_ptr(), ns,
+                                         _lib.stream_ptr(xin.device)))
+        if dv is None:
+            wgrads = (None,) * len(wparams)
+        elif len(wparams) == 2:
+            wgrads = (dg.view_as(wparams[0]).to(wparams[0].dtype), dv.to(wparams[1].dtype))
+        else:
+            wgrads = (dv.to(wparams[0].dtype),)
+        return (None, None if gx is None else gx[:, :, :ctx.T].to(ctx.x_dtype), None, db, *wgrads)
 
 
 def snake_beta(x, alpha, beta):
@@ -229,20 +244,51 @@ class _WNConvBase(nn.Module):
             raise ValueError("empty input")
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.conv_params())):
             wparams = (self.weight_g, self.weight_v) if self.has_weight_norm else (self._parameters["weight"],)
-            return _ConvFn.apply(self, x, self.bias, *wparams)
-        y = self._forward_tc(x) if tc else None
-        return y if y is not None else self._forward_impl(x)[0]
+            return _ConvLayerFn.apply(self, x, tc, self.bias, *wparams)
+        T = x.shape[2]
+        keep = self.keep(T)
+        engine = self.engine(T, tc, keep)
+        xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
+        if engine:       # the tensor cores truncate inside the kernel
+            y = self.conv_rows(xin.contiguous(), *self.packed_weight(engine), engine, self.padding[0], 0, keep)
+        else:
+            y = self._forward_impl(xin)
+            if keep < y.shape[2]:
+                y = y[:, :, :keep].contiguous()
+        return y if y.dtype == x.dtype else y.to(x.dtype)
 
     # Stand-alone layers run fp32 CUDA-core arithmetic by default.  ``tc_precision`` ("bf16" | "fp32") sends layers
     # whose channel counts are multiples of 64 through the tcgen05 conv instead ("fp32" = bf16x3 operand split,
-    # <= 1e-5); ``keep`` truncates the output to its first ``keep`` samples inside the kernel.
+    # <= 1e-5).
     tc_precision = None
+    _same_extra_right = 0     # WNConv1d(padding='same') with an even kernel: one more zero row on the right
 
     def tc_layer(self) -> bool:
         """Whether inputs of >= TC_MIN_ROWS rows go to the tcgen05 conv."""
-        return self.tc_precision is not None and not getattr(self, "_same_extra_right", 0) and \
+        return self.tc_precision is not None and not self._same_extra_right and \
             bool(_lib.lib().kvae_conv1d_tc_supported(self.in_channels, self.out_channels, self.kernel_size[0],
                                                      self.stride[0], self.dilation[0], int(self.transposed)))
+
+    def out_len(self, T: int) -> int:
+        """Output rows of the conv on an input of T rows."""
+        K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
+        T += self._same_extra_right
+        return (T - 1) * s - 2 * p + d * (K - 1) + 1 if self.transposed else (T + 2 * p - d * (K - 1) - 1) // s + 1
+
+    def keep(self, T: int) -> int:
+        """Output rows the layer keeps of an input of T rows: all of them here; BigVGANFlowVAE's causal layers keep
+        the first ones only."""
+        return self.out_len(T)
+
+    def engine(self, T: int, tc: bool, keep: int) -> int:
+        """The engine the layer runs an input of T rows on (keeping ``keep`` output rows): 0 = CUDA cores fp32,
+        1 = tcgen05 bf16, 2 = tcgen05 bf16x3.  The tensor cores take a ``tc_layer`` from TC_MIN_ROWS rows on, unless
+        ``tc`` is False or the layer is a strided Conv1d whose output is truncated."""
+        if not tc or T < TC_MIN_ROWS or not self.tc_layer():
+            return 0
+        if not self.transposed and self.stride[0] != 1 and keep != self.out_len(T):
+            return 0
+        return 1 if self.tc_precision == "bf16" else 2
 
     def packed_weight(self, engine: int):
         """(the folded weight packed by kvae_conv1d_pack for ``engine``: 0 = CUDA cores fp32, 1 = tcgen05 bf16,
@@ -299,47 +345,27 @@ class _WNConvBase(nn.Module):
                                             _lib.stream_ptr(win.device)))
         return y
 
-    def _forward_tc(self, x, keep=0):
-        K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
-        if x.shape[2] < TC_MIN_ROWS or not self.tc_layer():
-            return None
-        xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
-        xin = xin.contiguous()
-        T = xin.shape[2]
-        T_nat = (T - 1) * s - 2 * p + d * (K - 1) + 1 if self.transposed else (T + 2 * p - d * (K - 1) - 1) // s + 1
-        keep = int(keep) if keep else T_nat
-        if keep != T_nat and not self.transposed and s != 1:
-            return None
-        engine = 1 if self.tc_precision == "bf16" else 2
-        y = self.conv_rows(xin, *self.packed_weight(engine), engine, p, 0, keep)
-        return y if y.dtype == x.dtype else y.to(x.dtype)
-
-    def _forward_impl(self, x):
-        """(y, the contiguous input actually used, the folded fp32 weight)"""
-        xin = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
-        if getattr(self, "_same_extra_right", 0):     # 'same' with an even kernel: one more zero on the right
+    def _forward_impl(self, xin):
+        """All output rows of the conv of xin (fp32 / bf16) on the CUDA cores (kvae_conv1d_fwd), in xin's dtype."""
+        T_out = self.out_len(xin.shape[2])
+        if T_out <= 0:
+            raise RuntimeError("Kernel size can't be greater than actual input size")
+        if self._same_extra_right:     # 'same' with an even kernel: one more zero on the right
             xin = torch.nn.functional.pad(xin, (0, self._same_extra_right))
         xin = xin.contiguous()
         w = self.folded_weight()
         bias = None if self.bias is None else self.bias.detach().float().contiguous()
         B, _, T = xin.shape
         K, s, d, p = self.kernel_size[0], self.stride[0], self.dilation[0], self.padding[0]
-        if self.transposed:
-            T_out = (T - 1) * s - 2 * p + d * (K - 1) + 1
-        else:
-            T_out = (T + 2 * p - d * (K - 1) - 1) // s + 1
-        if T_out <= 0:
-            raise RuntimeError("Kernel size can't be greater than actual input size")
         L = _lib.lib()
-        y = torch.empty((B, self.out_channels, T_out), dtype=xin.dtype, device=x.device)
+        y = torch.empty((B, self.out_channels, T_out), dtype=xin.dtype, device=xin.device)
         nscratch = L.kvae_conv1d_scratch_bytes(self.in_channels, self.out_channels, K)
-        scratch = torch.empty(nscratch, dtype=torch.uint8, device=x.device)
+        scratch = torch.empty(nscratch, dtype=torch.uint8, device=xin.device)
         _lib.check(L.kvae_conv1d_fwd(xin.data_ptr(), y.data_ptr(), w.data_ptr(), _lib.ptr(bias), int(self.transposed),
                                      B, self.in_channels, self.out_channels, T, K, s, d, p,
                                      _lib.dtype_code(xin.dtype), scratch.data_ptr(), nscratch,
-                                     _lib.stream_ptr(x.device)))
-        y = y if y.dtype == x.dtype else y.to(x.dtype)
-        return y, xin, w
+                                     _lib.stream_ptr(xin.device)))
+        return y
 
     def extra_repr(self):
         return (f"{self.in_channels}, {self.out_channels}, kernel_size={self.kernel_size}, stride={self.stride}, "
@@ -359,14 +385,11 @@ class WNConv1d(_WNConvBase):
         # padding='same' (the conv of DecoderBlock's use_nearest_upsample branch, autoencoders.py:90-95): torch pads
         # d(K-1) in total, the smaller half on the left
         self.same_padding = isinstance(padding, str)
+        conv_padding = padding
         if self.same_padding:
             total = _single(dilation) * (_single(kernel_size) - 1)
             self._same_extra_right = total - 2 * (total // 2)
-            conv_padding = padding
             padding = total // 2
-        else:
-            self._same_extra_right = 0
-            conv_padding = padding
         conv = nn.Conv1d(in_channels, out_channels, kernel_size, stride=stride, padding=conv_padding, dilation=dilation,
                          bias=bias, device=device, dtype=dtype)
         self.in_channels, self.out_channels = in_channels, out_channels

@@ -50,21 +50,26 @@ class FakeLib:
         self.calls.append(("conv_fwd", Cin, Cout, K))
         return 0
 
-    def kvae_conv1d_bwd(self, x, gy, w, gx, dw, dbias, transposed, B, Cin, Cout, Tn, K, stride, dil, pad, dtype, scratch, ns, st):
-        assert not transposed and dtype == 0
+    def kvae_conv1d_win_bwd_scratch_bytes(self, transposed, B, Cin, Cout, Tn, T_gy, K, stride, engine):
+        return 1024
+
+    def kvae_conv1d_win_bwd(self, x, gy, T_gy, w, v, g, gx, dv, dg, dbias, transposed, B, Cin, Cout, Tn, K, stride, dil,
+                            pad, dtype, engine, scratch, ns, st):
+        assert not transposed and dtype == 0 and engine == 0 and v is None and g is None
         with torch.enable_grad():
             xx = T(x, B, Cin, Tn).clone().requires_grad_(True)
             ww = T(w, Cout, Cin, K).clone().requires_grad_(True)
             out = F.conv1d(xx, ww, None, stride=stride, padding=pad, dilation=dil)
-            g = T(gy, *out.shape)
-            gxx, gww = torch.autograd.grad(out, (xx, ww), g)
+            assert out.shape[2] == T_gy
+            gr = T(gy, *out.shape)
+            gxx, gww = torch.autograd.grad(out, (xx, ww), gr)
         if gx is not None:
             T(gx, B, Cin, Tn).copy_(gxx)
-        if dw is not None:
-            T(dw, Cout, Cin, K).copy_(gww)
+        if dv is not None:
+            T(dv, Cout, Cin, K).copy_(gww)
         if dbias is not None:
-            T(dbias, Cout).copy_(g.sum((0, 2)))
-        self.calls.append(("conv_bwd", gx is not None, dw is not None))
+            T(dbias, Cout).copy_(gr.sum((0, 2)))
+        self.calls.append(("conv_bwd", gx is not None, dv is not None))
         return 0
 
     def kvae_disc_conv15_supported(self, K, stride, pad):
@@ -74,7 +79,8 @@ class FakeLib:
         return self.kvae_conv1d_fwd(x, y, w, bias, 0, N, Cin, Cout, Tn, 15, 4, 1, 7, 0, scratch, ns, st)
 
     def kvae_disc_conv15_bwd(self, x, gy, w, gx, dw, dbias, N, Cin, Cout, Tn, scratch, ns, st):
-        return self.kvae_conv1d_bwd(x, gy, w, gx, dw, dbias, 0, N, Cin, Cout, Tn, 15, 4, 1, 7, 0, scratch, ns, st)
+        return self.kvae_conv1d_win_bwd(x, gy, (Tn - 1) // 4 + 1, w, None, None, gx, dw, None, dbias, 0, N, Cin, Cout, Tn,
+                                        15, 4, 1, 7, 0, 0, scratch, ns, st)
 
     def kvae_disc_conv1x1_supported(self, K, stride, pad, Cout):
         return int(K == 1 and stride == 1 and pad == 0 and 1 <= Cout <= 8)
@@ -83,7 +89,8 @@ class FakeLib:
         return self.kvae_conv1d_fwd(x, y, w, bias, 0, N, Cin, Cout, Tn, 1, 1, 1, 0, 0, None, 0, st)
 
     def kvae_disc_conv1x1_bwd(self, x, gy, w, gx, dw, dbias, N, Cin, Cout, Tn, st):
-        return self.kvae_conv1d_bwd(x, gy, w, gx, dw, dbias, 0, N, Cin, Cout, Tn, 1, 1, 1, 0, 0, None, 0, st)
+        return self.kvae_conv1d_win_bwd(x, gy, Tn, w, None, None, gx, dw, None, dbias, 0, N, Cin, Cout, Tn, 1, 1, 1, 0, 0, 0,
+                                        None, 0, st)
 
     # ---- csrc/disc.cuh
     def kvae_disc_period_fold(self, x, y, N, Cc, Tn, n, backward, st):

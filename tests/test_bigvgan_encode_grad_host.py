@@ -5,8 +5,9 @@
     layer's T input rows (output_padding), it equals torch.autograd.grad of F.conv1d for every strided conv of the
     golden and bench encoders and every T mod s, the rows past the transposed conv's natural length included;
   * kvae_conv1d_win_bwd's argument checks with placeholder pointers (refused before any device access): a strided
-    Conv1d is accepted and sized, a strided dilated conv and a T_gy out of range are refused, and the scratch size of
-    the geometries accepted before (stride-1 convs, transposed convs) is unchanged."""
+    Conv1d is accepted and sized, a strided dilated conv and a T_gy out of range are refused, padding past d (K - 1)
+    is accepted on the CUDA cores only, and the scratch size of the geometries accepted before (stride-1 convs,
+    transposed convs) is unchanged."""
 import ctypes
 import os
 import sys
@@ -134,6 +135,15 @@ def test_win_bwd_arguments_without_gpu():
     for engine in (0, 1, 2):
         assert call(False, 64, 64, 400, 100, 4, 4, 2, 3, engine, 1 << 30) != 0
         assert b"dilation" in L.kvae_last_error()
+    # padding past d (K - 1) (a stride-1 Conv1d, a strided one, a ConvTranspose1d): the CUDA cores only
+    for tr, K, s, d, p, T, T_gy in ((False, 3, 1, 2, 5, 400, 406), (False, 4, 2, 1, 4, 400, 203),
+                                    (True, 4, 2, 1, 4, 100, 194)):
+        for engine in (0, 1, 2):
+            n = size(tr, 64, 64, T, T_gy, K, s, engine)
+            assert call(tr, 64, 64, T, T_gy, K, s, d, p, engine, n - 1) != 0
+            assert (b"scratch too small" if engine == 0 else b"padding") in L.kvae_last_error(), (tr, engine)
+            assert call(tr, 64, 64, T, T_gy + 1, K, s, d, p, engine, n) != 0
+            assert (b"T_gy" if engine == 0 else b"padding") in L.kvae_last_error(), (tr, engine)
     # the geometries accepted before keep their scratch size: stride-1 convs (one with a non-multiple-of-64 T) and the
     # decoder's transposed convs
     for tr, Cin, Cout, T, T_gy, K, s in ((False, 768, 768, 401, 401, 3, 1), (False, 64, 64, 1000, 1000, 7, 1),

@@ -3,7 +3,8 @@
   * the data-gradient geometry that kvae_conv1d_win_bwd runs (kvae_conv1d_dgrad_geom): applied as a plain F.conv1d of
     the output gradient with the transposed / tap-reversed weight, the stated left padding and zeros past the end, it
     equals torch.autograd.grad of the layer for every conv and transposed conv of the golden and bench decoders,
-    causal and not (the bench rates include K = 10 at rate 5, odd K - s);
+    causal and not (the bench rates include K = 10 at rate 5, odd K - s), and for the paddings past d (K - 1) that the
+    stand-alone layers accept (kvae_conv1d_dgrad_form);
   * the backward chain of the anti-aliased activation as aa_act_bwd_kernel computes it (adjoint of the decimation,
     replicate padding folded back, the Snake derivative, adjoint of the up-filter, folded again; the parameter terms)
     against autograd through oracle.bigvgan_oracle.aa_activation."""
@@ -96,11 +97,52 @@ def test_data_gradient_geometry_vs_autograd(tag, causal):
     assert len(seen) >= (4 if tag == "golden" else 10)
 
 
-def test_data_gradient_geometry_refusals():
+@pytest.mark.parametrize("transposed,K,s,d,p", [(0, 3, 1, 1, 3), (0, 3, 1, 2, 7), (0, 4, 2, 1, 4), (0, 3, 3, 1, 5),
+                                               (1, 4, 2, 1, 4), (1, 3, 1, 1, 3)])
+def test_large_padding_data_gradient_vs_autograd(transposed, K, s, d, p):
+    """Padding past d (K - 1), which the stand-alone WNConv1d / WNConvTranspose1d accept (CUDA cores only): a stride-1
+    Conv1d's form reads gy ahead (negative left padding), a strided Conv1d's is the ConvTranspose1d continued over zero
+    gy rows, a ConvTranspose1d's the strided Conv1d; each against torch.autograd.grad in float64."""
+    Cin, Cout = 3, 2
+    out = (ctypes.c_int * 7)()
+    _lib.check(_lib.lib().kvae_conv1d_dgrad_form(transposed, Cin, Cout, K, s, d, p, ctypes.byref(out)))
+    kind, cin, cout, s2, d2, p2, flip = out
+    assert (cin, cout) == (Cout, Cin)
+    if not kind:        # the stride-1 / transposed contract of kvae_conv1d_dgrad_geom
+        assert [kind] + _dgrad_geom(transposed, Cin, Cout, K, s, d, p) == list(out)
+    gen = torch.Generator().manual_seed(5)
+    w = torch.randn(*((Cin, Cout, K) if transposed else (Cout, Cin, K)), dtype=torch.float64, generator=gen)
+    checked = 0
+    for T in range(1, 4 * K + 3 * s):
+        x = torch.randn(2, Cin, T, dtype=torch.float64, generator=gen, requires_grad=True)
+        T_out = (T - 1) * s - 2 * p + K if transposed else (T + 2 * p - d * (K - 1) - 1) // s + 1
+        if T_out < 1:
+            continue
+        y = (F.conv_transpose1d(x, w, stride=s, padding=p) if transposed
+             else F.conv1d(x, w, stride=s, padding=p, dilation=d))
+        gy = torch.randn(y.shape, dtype=torch.float64, generator=gen)
+        ref, = torch.autograd.grad(y, x, gy)
+        if kind:        # ConvTranspose1d of gy with the weight as it is, over enough zero rows of gy past its end
+            z = max(0, -(-(T + 2 * p2 - K) // s2) + 1 - T_out)
+            gx = F.conv_transpose1d(F.pad(gy, (0, z)), w, stride=s2, padding=p2)[:, :, :T]
+        else:           # Conv1d of gy, left padding p2 (< 0: the first -p2 rows are skipped), zeros past its end
+            W = w.transpose(0, 1).flip(-1) if flip else w
+            right = max(0, (T - 1) * s2 - p2 + d2 * (K - 1) + 1 - T_out)
+            gx = F.conv1d(F.pad(gy, (p2, right)), W, stride=s2, dilation=d2)[:, :, :T]
+        assert gx.shape == ref.shape, T
+        assert torch.allclose(gx, ref, rtol=1e-12, atol=1e-12), T
+        checked += 1
+    assert checked >= 5
+    if not transposed and s == 1:
+        assert p2 < 0
+
+
+def test_data_gradient_geometry_still_refused():
+    """What kvae_conv1d_dgrad_geom still refuses: a strided Conv1d (its form is a ConvTranspose1d, through
+    kvae_conv1d_dgrad_form) and a dilated transposed conv.  Padding past d (K - 1) is accepted (see above)."""
     L = _lib.lib()
     out = (ctypes.c_int * 6)()
     assert L.kvae_conv1d_dgrad_geom(0, 64, 64, 3, 2, 1, 1, ctypes.byref(out)) != 0          # strided Conv1d
-    assert L.kvae_conv1d_dgrad_geom(0, 64, 64, 3, 1, 1, 3, ctypes.byref(out)) != 0          # padding > d (K - 1)
     assert L.kvae_conv1d_dgrad_geom(1, 64, 64, 4, 2, 2, 1, ctypes.byref(out)) != 0          # dilated transposed conv
     assert L.kvae_conv1d_dgrad_geom(1, 64, 64, 10, 5, 1, 2, ctypes.byref(out)) == 0
     assert list(out) == [64, 64, 5, 1, 2, 0]

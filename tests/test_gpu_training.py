@@ -131,7 +131,9 @@ def test_snake_beta_module_backward(dev):
 @pytest.mark.parametrize("transposed,cin,cout,K,stride,dil,pad,T", [
     (0, 5, 7, 7, 1, 1, 3, 50), (0, 16, 16, 7, 1, 9, 27, 300), (0, 8, 16, 8, 4, 1, 2, 64), (0, 8, 4, 10, 5, 1, 3, 45),
     (0, 6, 6, 1, 1, 1, 0, 33), (0, 2, 32, 7, 1, 1, 3, 200), (1, 8, 4, 4, 2, 1, 1, 33), (1, 6, 3, 11, 5, 1, 3, 11),
-    (1, 16, 8, 8, 4, 1, 2, 20)])
+    (1, 16, 8, 8, 4, 1, 2, 20),
+    # 'same' with an even kernel (one more zero row on the right); padding past d (K - 1) on each kind of layer
+    (0, 6, 5, 8, 1, 1, "same", 40), (0, 5, 7, 3, 1, 2, 6, 50), (0, 8, 4, 4, 2, 1, 5, 45), (1, 6, 4, 4, 2, 1, 4, 40)])
 def test_wnconv_modules_backward(dev, transposed, cin, cout, K, stride, dil, pad, T):
     torch.manual_seed(5)
     if transposed:

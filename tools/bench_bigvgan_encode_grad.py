@@ -6,9 +6,7 @@ Cases per clip length:
     gradient only), per precision;
   * the whole autoencoder: encode_with_grad -> decode_with_grad (Gaussian sample) -> MultiResolutionSTFTLoss against
     the input, backward to every encoder and decoder parameter, per precision;
-  * baselines: model.audio_encoder(x) under grad through layers.WNConv1d's own autograd node (_ConvFn: fp32 CUDA
-    cores for every layer, what grad mode ran before encode_with_grad), and torch eager autograd through
-    oracle/bigvgan_oracle.extract_latents in fp32 on the same GPU.
+  * baseline: torch eager autograd through oracle/bigvgan_oracle.extract_latents in fp32 on the same GPU.
 Per case: p50 / p10 / p90 of the step (CUDA events around each step, after warm-up) and peak memory; the encoder cases
 also get a per-kernel-class split from torch.profiler in a separate run (the forward profiled on its own and
 subtracted).  Writes one JSON file (--out).
@@ -26,26 +24,10 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from bench_bigvgan_grad import H, _gpu_info, _split, _time  # noqa: E402  (also puts the repository on sys.path)
 
 from kalle_audio_b200 import bigvgan as BV  # noqa: E402
-from kalle_audio_b200.layers import WNConv1d  # noqa: E402
 from kalle_audio_b200.losses import MultiResolutionSTFTLoss  # noqa: E402
 from oracle import bigvgan_oracle as BO  # noqa: E402
 
 SAMPLE_RATE = 16000
-
-
-class _ConvFnEncoder:
-    """The encoder's convs as plain layers.WNConv1d while inside: their grad-mode forward is _ConvFn."""
-
-    def __init__(self, m):
-        self.mods = [mod for mod in m.audio_encoder.modules() if isinstance(mod, BV._EncConv1d)]
-
-    def __enter__(self):
-        for mod in self.mods:
-            mod.__class__ = WNConv1d
-
-    def __exit__(self, *a):
-        for mod in self.mods:
-            mod.__class__ = BV._EncConv1d
 
 
 def _with_split(step, fwd, case):
@@ -118,15 +100,6 @@ def main():
             m.requires_grad_(True)
             record(dict(base, what="round trip (encode, decode, MR-STFT loss) fwd+bwd", precision=prec, frozen=False),
                    round_trip)
-        m.requires_grad_(False)
-        for p in enc_params:
-            p.requires_grad_(True)
-        with _ConvFnEncoder(m):
-            def convfn_step():
-                zero()
-                (m.audio_encoder(xg) * r).sum().backward()
-            record(dict(base, what="encoder fwd+bwd, audio_encoder(x) under grad (_ConvFn, fp32 CUDA cores)",
-                        precision="_ConvFn", frozen=False), convfn_step)
         sd = {n: p.detach().clone().requires_grad_(True) for n, p in m.state_dict().items()
               if n.startswith("audio_encoder.")}
         xe = x.clone().requires_grad_(True)
@@ -140,7 +113,6 @@ def main():
 
         record(dict(base, what="encoder fwd+bwd, torch eager autograd through the fp32 oracle",
                     precision="torch eager fp32 (oracle)", frozen=False), eager, 2, max(5, args.steps // 2))
-        m.requires_grad_(True)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         json.dump(res, f, indent=1)
