@@ -406,6 +406,44 @@ int kvae_conv1d_dgrad_geom(int transposed, int Cin, int Cout, int K, int stride,
  * continued past its natural length to T rows (torch's output_padding T - that length). */
 int kvae_conv1d_dgrad_form(int transposed, int Cin, int Cout, int K, int stride, int dilation, int padding, int out[7]);
 
+/* ---- BigVGANFlowVAE flow (backup/flows.py:613-792, the VITS ResidualCouplingBlock with mean_only coupling layers and
+ * an unconditioned WN) ----
+ * Elementwise steps between the flow's convolutions (which run through kvae_conv1d_win_fwd / kvae_conv1d_win_bwd).
+ * Tensors are contiguous [B, C, T] of `dtype` (fp32 or bf16; fp32 arithmetic, one rounding per stored value); x_mask is
+ * [B, 1, T] of the same dtype.  Every backward is a pass of its own with no reduction.  A NULL output gradient reads
+ * as 0 (an output autograd did not use).
+ *
+ * torch.split(x, [C/2] * 2, 1)[0] (ResidualCouplingLayer.forward) and torch.flip(x, [1]) (Flip.forward): xs = x, or x
+ * with its C channels reversed (flip), and x0 = xs[:, :C/2] as a contiguous [B, C/2, T] copy unless x0 == NULL.  The
+ * backward: gx = the reversal (flip) of gxs + (gx0 on the first C/2 channels). */
+int kvae_flow_split(const void* x, void* xs, void* x0, int B, int C, long long T, int flip, int dtype, void* stream);
+int kvae_flow_split_bwd(const void* gxs, const void* gx0, void* gx, int B, int C, long long T, int flip, int dtype,
+                        void* stream);
+/* h = pre(x0) * x_mask (ResidualCouplingLayer.forward): y = x * mask over C channels; also its backward (gx = gy * mask). */
+int kvae_flow_mask(const void* x, const void* mask, void* y, int B, int C, long long T, int dtype, void* stream);
+/* commons.fused_add_tanh_sigmoid_multiply(x_in, 0, H) (WN.forward): acts [B, H, T] = tanh(a[:, :H]) sigmoid(a[:, H:])
+ * of a [B, 2H, T].  The backward reads the saved a and writes both halves of ga [B, 2H, T]. */
+int kvae_wn_gate_fwd(const void* a, void* acts, int B, int H, long long T, int dtype, void* stream);
+int kvae_wn_gate_bwd(const void* a, const void* g, void* ga, int B, int H, long long T, int dtype, void* stream);
+/* WN.forward's residual / skip update of one layer from rs = res_skip_layers[i](acts) and the running skip sum (skip ==
+ * NULL: 0, the first layer).  last == 0 (rs [B, 2H, T]): x_out = (x + rs[:, :H]) * mask, skip_out = skip + rs[:, H:].
+ * last != 0 (rs [B, H, T]): skip_out = (skip + rs) * mask, WN's output (x, x_out unused).  The backward from g_xout and
+ * g_skipout: gx = g_xout * mask and grs = (g_xout * mask | g_skipout), or for the last layer grs = g_skipout * mask; the
+ * skip input's gradient is g_skipout (g_skipout * mask for the last layer), written to gskip unless it is NULL. */
+int kvae_wn_update_fwd(const void* x, const void* rs, const void* skip, const void* mask, void* x_out, void* skip_out,
+                       int B, int H, int last, long long T, int dtype, void* stream);
+int kvae_wn_update_bwd(const void* g_xout, const void* g_skipout, const void* mask, void* gx, void* grs, void* gskip,
+                       int B, int H, int last, long long T, int dtype, void* stream);
+/* ResidualCouplingLayer.forward's update (mean_only: logs = 0, the log-determinant 0) followed by Flip: from the layer
+ * input x [B, C, T] and m = post(h) [B, C/2, T], mm = m * mask and x1' = mm + x1 * mask (reverse == 0) or (x1 - mm) *
+ * mask (reverse != 0); y = cat(x0, x1'), written with its channels reversed when flip, and y0 = y[:, :C/2] as a
+ * contiguous copy (the next layer's `pre` input) unless y0 == NULL.  The backward from gy and gy0 (either may be NULL):
+ * gx [B, C, T] and gm [B, C/2, T]; it reads neither x nor m. */
+int kvae_flow_coupling_fwd(const void* x, const void* m, const void* mask, void* y, void* y0, int B, int C, long long T,
+                           int flip, int reverse, int dtype, void* stream);
+int kvae_flow_coupling_bwd(const void* gy, const void* gy0, const void* mask, void* gx, void* gm, int B, int C,
+                           long long T, int flip, int reverse, int dtype, void* stream);
+
 /* ---- post-decode tail ---- */
 /* audio.to(float32).div(max|audio|).clamp(-1,1).mul(32767).to(int16) -- the peak-normalised PCM conversion every
  * caller of the decoder repeats (infer_0828_sigma.py:298, train_offline.py:302,319); bit-exact with torch's

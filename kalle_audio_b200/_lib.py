@@ -126,6 +126,17 @@ SIGNATURES = {
                                       C.c_size_t, C.c_void_p]),
     "kvae_conv1d_dgrad_geom": (C.c_int, [C.c_int] * 7 + [C.POINTER(C.c_int * 6)]),
     "kvae_conv1d_dgrad_form": (C.c_int, [C.c_int] * 7 + [C.POINTER(C.c_int * 7)]),
+    "kvae_flow_split": (C.c_int, [C.c_void_p] * 3 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
+    "kvae_flow_split_bwd": (C.c_int, [C.c_void_p] * 3 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
+    "kvae_flow_mask": (C.c_int, [C.c_void_p] * 3 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_wn_gate_fwd": (C.c_int, [C.c_void_p] * 2 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_wn_gate_bwd": (C.c_int, [C.c_void_p] * 3 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_wn_update_fwd": (C.c_int, [C.c_void_p] * 6 + [C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_wn_update_bwd": (C.c_int, [C.c_void_p] * 6 + [C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p]),
+    "kvae_flow_coupling_fwd": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int,
+                                                            C.c_void_p]),
+    "kvae_flow_coupling_bwd": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int,
+                                                            C.c_void_p]),
     "kvae_plan_out_length": (C.c_longlong, [C.c_void_p, C.c_longlong]),
     "kvae_mrstft_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int]),
     "kvae_mrstft_loss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_void_p,

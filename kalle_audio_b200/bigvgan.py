@@ -1,9 +1,10 @@
 """Drop-in for the inference path of the reference's 12.5 Hz VAE, ``BigVGANFlowVAE`` (/root/reference/backup/flows.py).
 
 Module tree, constructor argument (the hyper-parameter object ``h``) and ``state_dict`` keys mirror the reference:
-``audio_encoder`` (Encoder :191-241: Conv1d_S / LeakyReLU / ResStack), ``flow`` (ResidualCouplingBlock -- training
-only; kept as a parameter container so checkpoints load), ``conv_pre``, ``ups``, ``resblocks`` (AMPBlock1 / AMPBlock2
-:243-330 with their anti-aliased ``Activation1d``), ``activation_post``, ``conv_post``.  Implemented:
+``audio_encoder`` (Encoder :191-241: Conv1d_S / LeakyReLU / ResStack), ``flow`` (VITS's ResidualCouplingBlock
+:613-792, the training objective's flow: ``flow(z, x_mask, reverse=False)`` under autograd), ``conv_pre``, ``ups``,
+``resblocks`` (AMPBlock1 / AMPBlock2 :243-330 with their anti-aliased ``Activation1d``), ``activation_post``,
+``conv_post``.  Implemented:
 
     extract_latents(x)                      :494-496   waveform [B, 1, L] -> [B, 2 D, L / prod(downsample_rates)]
     inference_from_latents(x, do_sample)    :498-529   latents -> waveform [B, 1, T * prod(upsample_rates)]
@@ -24,7 +25,8 @@ in the reference), LeakyReLU / tanh / residual adds / the AMP average / the Gaus
 kernels.  Under grad mode each of them has an autograd node whose backward is a libkvae call too (``decode_with_grad``,
 ``encode_with_grad``): the ``_*Fn`` classes below, and for the convs the node every ``layers`` conv uses, whose backward
 is ``kvae_conv1d_win_bwd`` on the engine the forward ran on.  The causal layers set ``keep``, the output rows they keep.
-``forward`` (the training pass through the flow) is not built.
+The flow's steps between its convs are the flow.cuh kernels (see "the flow" below).  ``forward`` (the reference's
+training pass, whose return contract is not recorded here) is not built.
 """
 from __future__ import annotations
 
@@ -36,7 +38,7 @@ import torch
 from torch import nn
 
 from . import _lib
-from .layers import TC_MIN_ROWS, WNConv1d, WNConvTranspose1d
+from .layers import TC_MIN_ROWS, WNConv1d, WNConvTranspose1d, _WNConvBase
 
 _RAGGED_MAX_CLIPS = 64       # kRaggedMaxClips (elementwise.cuh): lengths travel by value into the kernels
 
@@ -426,31 +428,335 @@ class AMPBlock2(nn.Module):
         return x
 
 
-class _FlowParams(nn.Module):
-    """Parameter container with the keys of ResidualCouplingBlock (flows.py:622-792).  The flow only runs in the
-    reference's training ``forward``; neither inference entry point touches it."""
+# ------------------------------------------------------------------------------------------------- the flow
+# ResidualCouplingBlock (flows.py:613-792, VITS): coupling layers with an unconditioned WaveNet, each followed by Flip.
+# Between the convs every step is one flow.cuh kernel with its own autograd node: the split of x0 off the block input,
+# the mask after `pre`, WN's gate and residual / skip update, and the coupling update, which writes its output with the
+# following Flip applied and also the next layer's `pre` input, so channel splits, concatenations and flips are no pass
+# of their own.
+def _flow_call(name, *args):
+    _lib.check(getattr(_lib.lib(), name)(*args))
 
-    def __init__(self, channels, hidden, kernel_size, n_layers, n_flows=4):
+
+def _flow_split(x, flip):
+    B, C, T = x.shape
+    xs = torch.empty_like(x)
+    x0 = torch.empty((B, C // 2, T), dtype=x.dtype, device=x.device)
+    _flow_call("kvae_flow_split", x.data_ptr(), xs.data_ptr(), x0.data_ptr(), B, C, T, int(flip),
+               _lib.dtype_code(x.dtype), _lib.stream_ptr(x.device))
+    return xs, x0
+
+
+def _flow_mask(x, mask):
+    B, C, T = x.shape
+    y = torch.empty_like(x)
+    _flow_call("kvae_flow_mask", x.data_ptr(), mask.data_ptr(), y.data_ptr(), B, C, T, _lib.dtype_code(x.dtype),
+               _lib.stream_ptr(x.device))
+    return y
+
+
+def _wn_gate(a):
+    B, H2, T = a.shape
+    acts = torch.empty((B, H2 // 2, T), dtype=a.dtype, device=a.device)
+    _flow_call("kvae_wn_gate_fwd", a.data_ptr(), acts.data_ptr(), B, H2 // 2, T, _lib.dtype_code(a.dtype),
+               _lib.stream_ptr(a.device))
+    return acts
+
+
+def _wn_update(x, rs, skip, mask, last):
+    B, H, T = x.shape
+    x_out = None if last else torch.empty_like(x)
+    skip_out = torch.empty_like(x)
+    _flow_call("kvae_wn_update_fwd", x.data_ptr(), rs.data_ptr(), _lib.ptr(skip), mask.data_ptr(), _lib.ptr(x_out),
+               skip_out.data_ptr(), B, H, int(last), T, _lib.dtype_code(x.dtype), _lib.stream_ptr(x.device))
+    return x_out, skip_out
+
+
+def _flow_coupling(x, m, mask, flip, reverse, want_y0):
+    B, C, T = x.shape
+    y = torch.empty_like(x)
+    y0 = torch.empty((B, C // 2, T), dtype=x.dtype, device=x.device) if want_y0 else None
+    _flow_call("kvae_flow_coupling_fwd", x.data_ptr(), m.data_ptr(), mask.data_ptr(), y.data_ptr(), _lib.ptr(y0), B, C,
+               T, int(flip), int(reverse), _lib.dtype_code(x.dtype), _lib.stream_ptr(x.device))
+    return y, y0
+
+
+def _g(t):
+    return None if t is None else t.detach().contiguous()
+
+
+class _FlowSplitFn(torch.autograd.Function):
+    """(xs, x0) = (x or flip(x), its first half): kvae_flow_split / kvae_flow_split_bwd."""
+
+    @staticmethod
+    def forward(ctx, x, flip):
+        ctx.set_materialize_grads(False)
+        ctx.flip = flip
+        return _flow_split(x, flip)
+
+    @staticmethod
+    def backward(ctx, gxs, gx0):
+        gxs, gx0 = _g(gxs), _g(gx0)
+        ref = gxs if gxs is not None else gx0
+        if ref is None:
+            return None, None
+        B, C, T = gxs.shape if gxs is not None else (gx0.shape[0], 2 * gx0.shape[1], gx0.shape[2])
+        gx = torch.empty((B, C, T), dtype=ref.dtype, device=ref.device)
+        _flow_call("kvae_flow_split_bwd", _lib.ptr(gxs), _lib.ptr(gx0), gx.data_ptr(), B, C, T, int(ctx.flip),
+                   _lib.dtype_code(ref.dtype), _lib.stream_ptr(ref.device))
+        return gx, None
+
+
+class _FlowMaskFn(torch.autograd.Function):
+    """y = x * mask: kvae_flow_mask both ways (no gradient to the mask)."""
+
+    @staticmethod
+    def forward(ctx, x, mask):
+        ctx.save_for_backward(mask)
+        return _flow_mask(x, mask)
+
+    @staticmethod
+    def backward(ctx, gy):
+        mask, = ctx.saved_tensors
+        return _flow_mask(gy.detach().contiguous(), mask), None
+
+
+class _WNGateFn(torch.autograd.Function):
+    """acts = tanh(a[:, :H]) sigmoid(a[:, H:]): kvae_wn_gate_fwd / kvae_wn_gate_bwd (a saved)."""
+
+    @staticmethod
+    def forward(ctx, a):
+        ctx.save_for_backward(a)
+        return _wn_gate(a)
+
+    @staticmethod
+    def backward(ctx, g):
+        a, = ctx.saved_tensors
+        B, H2, T = a.shape
+        g = g.detach().contiguous()
+        ga = torch.empty_like(a)
+        _flow_call("kvae_wn_gate_bwd", a.data_ptr(), g.data_ptr(), ga.data_ptr(), B, H2 // 2, T,
+                   _lib.dtype_code(a.dtype), _lib.stream_ptr(a.device))
+        return ga
+
+
+class _WNUpdateFn(torch.autograd.Function):
+    """WN's residual / skip update of one layer: kvae_wn_update_fwd / kvae_wn_update_bwd.  Returns (x_out, skip_out), or
+    skip_out * mask (WN's output) for the last layer."""
+
+    @staticmethod
+    def forward(ctx, x, rs, skip, mask, last):
+        ctx.set_materialize_grads(False)
+        ctx.last, ctx.has_skip, ctx.shape = last, skip is not None, x.shape
+        ctx.save_for_backward(mask)
+        x_out, skip_out = _wn_update(x, rs, skip, mask, last)
+        return skip_out if last else (x_out, skip_out)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        mask, = ctx.saved_tensors
+        g_x, g_s = (None, _g(grads[0])) if ctx.last else (_g(grads[0]), _g(grads[1]))
+        B, H, T = ctx.shape
+        ref = g_s if g_s is not None else g_x
+        if ref is None:
+            return None, None, None, None, None
+        gx = None if ctx.last else torch.empty((B, H, T), dtype=ref.dtype, device=ref.device)
+        grs = torch.empty((B, H if ctx.last else 2 * H, T), dtype=ref.dtype, device=ref.device)
+        # the skip input's gradient: g_skipout itself (written only where it is masked or missing)
+        write_skip = ctx.has_skip and (ctx.last or g_s is None)
+        gskip = torch.empty((B, H, T), dtype=ref.dtype, device=ref.device) if write_skip else None
+        _flow_call("kvae_wn_update_bwd", _lib.ptr(g_x), _lib.ptr(g_s), mask.data_ptr(), _lib.ptr(gx), grs.data_ptr(),
+                   _lib.ptr(gskip), B, H, int(ctx.last), T, _lib.dtype_code(ref.dtype), _lib.stream_ptr(ref.device))
+        if ctx.has_skip and not write_skip:
+            gskip = g_s
+        return gx, grs, gskip, None, None
+
+
+class _FlowCouplingFn(torch.autograd.Function):
+    """(y, y0) of the coupling update (+ Flip): kvae_flow_coupling_fwd / kvae_flow_coupling_bwd (reads only the mask)."""
+
+    @staticmethod
+    def forward(ctx, x, m, mask, flip, reverse, want_y0):
+        ctx.set_materialize_grads(False)
+        ctx.flip, ctx.reverse, ctx.shape = flip, reverse, x.shape
+        ctx.save_for_backward(mask)
+        return _flow_coupling(x, m, mask, flip, reverse, want_y0)
+
+    @staticmethod
+    def backward(ctx, gy, gy0):
+        mask, = ctx.saved_tensors
+        gy, gy0 = _g(gy), _g(gy0)
+        ref = gy if gy is not None else gy0
+        if ref is None:
+            return (None,) * 6
+        B, C, T = ctx.shape
+        gx = torch.empty((B, C, T), dtype=ref.dtype, device=ref.device)
+        gm = torch.empty((B, C // 2, T), dtype=ref.dtype, device=ref.device)
+        _flow_call("kvae_flow_coupling_bwd", _lib.ptr(gy), _lib.ptr(gy0), mask.data_ptr(), gx.data_ptr(), gm.data_ptr(),
+                   B, C, T, int(ctx.flip), int(ctx.reverse), _lib.dtype_code(ref.dtype), _lib.stream_ptr(ref.device))
+        return gx, gm, None, None, None, None
+
+
+def _flow_inputs(x, x_mask, g, what):
+    """x as a contiguous fp32 / bf16 [B, C, T] tensor and the mask [B, 1, T] as a detached contiguous tensor of x's
+    dtype."""
+    if g is not None:
+        raise NotImplementedError(f"{what}: conditioning (g) is not supported: the flow has no cond_layer")
+    _lib.require_cuda(x, what)
+    if x.dim() != 3 or x.dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError(f"{what}: x must be a float32 or bfloat16 [B, C, T] tensor, got {x.dtype} {tuple(x.shape)}")
+    B, _, T = x.shape
+    if tuple(x_mask.shape) != (B, 1, T):
+        raise ValueError(f"{what}: x_mask must be [B, 1, T] = {(B, 1, T)}, got {tuple(x_mask.shape)}")
+    if x_mask.device != x.device:
+        raise ValueError(f"{what}: x_mask is on {x_mask.device}, x on {x.device}")
+    return x.contiguous(), x_mask.detach().to(x.dtype).contiguous()
+
+
+class _PlainConv1d(_WNConvBase):
+    """nn.Conv1d(in, out, 1) with its plain ``weight`` / ``bias`` (the coupling layers' ``pre`` and ``post``) on the
+    layer-level conv: the engine choice of ``set_precision`` and the conv autograd node of every other layer."""
+    transposed = False
+
+    def __init__(self, in_channels, out_channels, kernel_size=1):
         super().__init__()
+        conv = nn.Conv1d(in_channels, out_channels, kernel_size)
+        self.in_channels, self.out_channels = in_channels, out_channels
+        self.kernel_size, self.stride, self.padding, self.dilation = (int(kernel_size),), (1,), (0,), (1,)
+        self.groups = 1
+        self._parameters["weight"] = nn.Parameter(conv.weight.detach().clone())     # nn.Conv1d's key order
+        self._parameters["bias"] = nn.Parameter(conv.bias.detach().clone())
 
-        class _WN(nn.Module):
-            def __init__(self):
-                super().__init__()
-                self.in_layers = nn.ModuleList([WNConv1d(hidden, 2 * hidden, kernel_size) for _ in range(n_layers)])
-                self.res_skip_layers = nn.ModuleList([WNConv1d(hidden, 2 * hidden if i < n_layers - 1 else hidden, 1)
-                                                      for i in range(n_layers)])
 
-        class _Layer(nn.Module):
-            def __init__(self):
-                super().__init__()
-                self.pre = nn.Conv1d(channels // 2, hidden, 1)
-                self.enc = _WN()
-                self.post = nn.Conv1d(hidden, channels // 2, 1)
+class Flip(nn.Module):
+    """flows.py Flip: torch.flip(x, [1]) (kvae_flow_split).  Inside ResidualCouplingBlock the coupling kernels apply
+    it; called on its own it is one pass.  The forward direction returns (x, logdet = 0) as VITS does."""
 
+    def forward(self, x, *args, reverse=False, **kwargs):
+        _lib.require_cuda(x, "Flip")
+        if x.dim() != 3 or x.dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("Flip: x must be a float32 or bfloat16 [B, C, T] tensor")
+        x = x.contiguous()
+        if x.shape[1] % 2:
+            raise ValueError("Flip: the flow's channel count is even")
+        y = (_FlowSplitFn.apply(x, True) if _grad_on(x) else _flow_split(x, True))[0]
+        return y if reverse else (y, torch.zeros(x.size(0), dtype=x.dtype, device=x.device))
+
+
+class WN(nn.Module):
+    """VITS modules.WN without conditioning: ``in_layers`` (hidden -> 2 hidden, kernel K, dilation rate^i) and
+    ``res_skip_layers`` (hidden -> 2 hidden, the last hidden -> hidden), built interleaved as VITS builds them."""
+
+    def __init__(self, hidden_channels, kernel_size, dilation_rate, n_layers, gin_channels=0, p_dropout=0):
+        super().__init__()
+        if gin_channels:
+            raise NotImplementedError("WN: conditioning (gin_channels > 0) is not supported")
+        if p_dropout:
+            raise NotImplementedError("WN: dropout is not supported (the flow uses p_dropout = 0)")
+        assert kernel_size % 2 == 1
+        self.hidden_channels, self.kernel_size = hidden_channels, kernel_size
+        self.dilation_rate, self.n_layers = dilation_rate, n_layers
+        self.in_layers = nn.ModuleList()
+        self.res_skip_layers = nn.ModuleList()
+        for i in range(n_layers):
+            d = dilation_rate ** i
+            self.in_layers.append(WNConv1d(hidden_channels, 2 * hidden_channels, kernel_size, dilation=d,
+                                           padding=int((kernel_size * d - d) / 2)))
+            self.res_skip_layers.append(WNConv1d(hidden_channels, 2 * hidden_channels if i < n_layers - 1
+                                                 else hidden_channels, 1))
+
+    def forward(self, x, x_mask, g=None, **kwargs):
+        x, mask = _flow_inputs(x, x_mask, g, "WN")
+        return self._run(x, mask)
+
+    def _run(self, x, mask):
+        skip = None
+        for i, (cin, crs) in enumerate(zip(self.in_layers, self.res_skip_layers)):
+            a = cin(x)
+            acts = _WNGateFn.apply(a) if _grad_on(a) else _wn_gate(a)
+            rs = crs(acts)
+            last = i == self.n_layers - 1
+            if _grad_on(x, rs, skip):
+                out = _WNUpdateFn.apply(x, rs, skip, mask, last)
+            else:
+                out = _wn_update(x, rs, skip, mask, last)
+                out = out[1] if last else out
+            if last:
+                return out
+            x, skip = out
+
+
+class ResidualCouplingLayer(nn.Module):
+    """VITS ResidualCouplingLayer with mean_only = True (``post`` zeroed at construction): x0, x1 = split(x);
+    h = pre(x0) mask; h = WN(h, mask); m = post(h) mask; x1' = m + x1 mask (reverse: (x1 - m) mask); cat(x0, x1').
+    The forward direction returns (x, logdet = 0), the reverse direction x, as VITS does."""
+
+    def __init__(self, channels, hidden_channels, kernel_size, dilation_rate, n_layers, p_dropout=0, gin_channels=0,
+                 mean_only=True):
+        super().__init__()
+        assert channels % 2 == 0, "channels should be divisible by 2"
+        if not mean_only:
+            raise NotImplementedError("ResidualCouplingLayer: mean_only=True only (the flow's coupling layers)")
+        self.channels, self.hidden_channels, self.half_channels = channels, hidden_channels, channels // 2
+        self.mean_only = True
+        self.pre = _PlainConv1d(self.half_channels, hidden_channels, 1)
+        self.enc = WN(hidden_channels, kernel_size, dilation_rate, n_layers, p_dropout=p_dropout,
+                      gin_channels=gin_channels)
+        self.post = _PlainConv1d(hidden_channels, self.half_channels, 1)
+        self.post._parameters["weight"].data.zero_()
+        self.post._parameters["bias"].data.zero_()
+
+    def forward(self, x, x_mask, g=None, reverse=False):
+        x, mask = _flow_inputs(x, x_mask, g, "ResidualCouplingLayer")
+        if x.shape[1] != self.channels:
+            raise ValueError(f"ResidualCouplingLayer: expected {self.channels} channels, got {x.shape[1]}")
+        x, x0 = _FlowSplitFn.apply(x, False) if _grad_on(x) else _flow_split(x, False)
+        y, _ = self._run(x, x0, mask, reverse, flip=False, want_y0=False)
+        return y if reverse else (y, torch.zeros(x.size(0), dtype=x.dtype, device=x.device))
+
+    def _run(self, x, x0, mask, reverse, flip, want_y0):
+        """(y, y0): the layer on x with its first half x0 already split off; ``flip``: y with the following Flip
+        applied; ``want_y0``: y's first half too (the next layer's x0)."""
+        h = self.pre(x0)
+        h = _FlowMaskFn.apply(h, mask) if _grad_on(h) else _flow_mask(h, mask)
+        h = self.enc._run(h, mask)
+        m = self.post(h)
+        if _grad_on(x, m):
+            return _FlowCouplingFn.apply(x, m, mask, flip, reverse, want_y0)
+        return _flow_coupling(x, m, mask, flip, reverse, want_y0)
+
+
+class ResidualCouplingBlock(nn.Module):
+    """VITS ResidualCouplingBlock (flows.py:613-792): ``flows`` = [coupling layer, Flip] x n_flows.
+    forward(x, x_mask, reverse=False): the layers in list order; reverse=True: in reversed order (each coupling layer
+    then runs its inverse).  x [B, C, T] fp32 / bf16 (the result has x's dtype), x_mask [B, 1, T] (no gradient).
+    Under autograd every coupling layer differentiates to x and its parameters (the WN convs' ``weight_g`` /
+    ``weight_v`` / ``bias``, ``pre`` / ``post``'s ``weight`` / ``bias``); under ``torch.no_grad`` the same kernels run."""
+
+    def __init__(self, channels, hidden_channels, kernel_size, dilation_rate, n_layers, n_flows=4, gin_channels=0):
+        super().__init__()
+        if gin_channels:
+            raise NotImplementedError("ResidualCouplingBlock: conditioning (gin_channels > 0) is not supported")
+        self.channels, self.hidden_channels, self.kernel_size = channels, hidden_channels, kernel_size
+        self.dilation_rate, self.n_layers, self.n_flows, self.gin_channels = dilation_rate, n_layers, n_flows, 0
         self.flows = nn.ModuleList()
         for _ in range(n_flows):
-            self.flows.append(_Layer())
-            self.flows.append(nn.Module())      # Flip: no parameters
+            self.flows.append(ResidualCouplingLayer(channels, hidden_channels, kernel_size, dilation_rate, n_layers,
+                                                    gin_channels=gin_channels, mean_only=True))
+            self.flows.append(Flip())
+
+    def forward(self, x, x_mask, g=None, reverse=False):
+        x, mask = _flow_inputs(x, x_mask, g, "ResidualCouplingBlock")
+        if x.shape[1] != self.channels:
+            raise ValueError(f"ResidualCouplingBlock: expected {self.channels} channels, got {x.shape[1]}")
+        layers = list(self.flows[0::2])
+        if reverse:          # Flip, L_{n-1}^-1, Flip, ..., Flip, L_0^-1: each flip is applied by the kernel before it
+            layers = layers[::-1]
+        x, x0 = _FlowSplitFn.apply(x, reverse) if _grad_on(x) else _flow_split(x, reverse)
+        for i, layer in enumerate(layers):
+            more = i < len(layers) - 1
+            x, x0 = layer._run(x, x0, mask, reverse, flip=more or not reverse, want_y0=more)
+        return x
 
 
 # ------------------------------------------------------------------------------------------------- layer descriptions
@@ -734,7 +1040,9 @@ class BigVGANFlowVAE(nn.Module):
         causal = h.causal
         self.audio_encoder = Encoder(out_channels=h.latent_dim, use_vae=h.use_vae, channels=list(h.downsample_channels),
                                      down_sample_factors=list(h.downsample_rates))
-        self.flow = _FlowParams(h.latent_dim, h.flow_hidden_channels, 5, 4)
+        # VITS builds this block as ResidualCouplingBlock(inter, hidden, 5, 1, 4); the checkpoint fixes everything but the
+        # dilation rate 1, which changes no parameter shape (DESIGN §4.10g)
+        self.flow = ResidualCouplingBlock(h.latent_dim, h.flow_hidden_channels, 5, 1, 4)
         self.num_kernels = len(h.resblock_kernel_sizes)
         self.num_upsamples = len(h.upsample_rates)
         self.conv_pre = Conv1d(h.latent_dim, h.upsample_initial_channel, 7, 1, causal=False)
@@ -752,8 +1060,8 @@ class BigVGANFlowVAE(nn.Module):
         self.activation_post = _make_act(h, ch)
         self.conv_post = Conv1d(ch, 1, 7, 1, causal=causal)
         self.set_precision("fp32")
-        for m in self.modules():           # inference-only model: fold weight norm once per weight version (layers.py)
-            if isinstance(m, (WNConv1d, WNConvTranspose1d)):
+        for m in self.modules():           # no-grad calls fold weight norm once per weight version (layers.py)
+            if isinstance(m, _WNConvBase):
                 m._cache_fold = True
 
     def set_precision(self, precision: Optional[str]):
@@ -763,13 +1071,14 @@ class BigVGANFlowVAE(nn.Module):
         if precision not in (None, "fp32", "bf16"):
             raise ValueError("precision must be None, 'fp32' or 'bf16'")
         for m in self.modules():
-            if isinstance(m, (WNConv1d, WNConvTranspose1d)):
+            if isinstance(m, _WNConvBase):
                 m.tc_precision = precision
         return self
 
     def forward(self, x):
         raise NotImplementedError("BigVGANFlowVAE.forward (the training pass through the flow, flows.py:454-492) is "
-                                  "outside the hot path; use extract_latents / inference_from_latents")
+                                  "not built; use extract_latents / inference_from_latents, or compose encode_with_grad, "
+                                  "flow and decode_with_grad for training")
 
     def latent_length(self, n_samples: int) -> int:
         """Latent frames ``extract_latents`` returns for a clip of ``n_samples`` samples (0: too short for any)."""

@@ -27,6 +27,7 @@
 #include "elementwise.cuh"
 #include "glue.cuh"
 #include "bigvgan.cuh"
+#include "flow.cuh"
 #include "mrstft.cuh"
 #include "disc.cuh"
 #include "train.cuh"
@@ -2783,6 +2784,143 @@ int kvae_gauss_sample_bwd(const void* x, const void* noise, const void* gz, void
   const int blocks = static_cast<int>(std::min<size_t>((n + 255) / 256, 148 * 16));
   gauss_sample_bwd_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, noise, gz, gx, static_cast<long long>(D) * T,
                                                                                  n, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+// ------------------------------------------------------------------ BigVGANFlowVAE flow (flow.cuh)
+namespace {
+// shared argument checks of the flow kernels: rows = the grid's (b, channel) rows, each of T frames
+int flow_launch_check(int B, int rows_per_clip, long long T, int dtype, dim3* grid) {
+  if (!check_dtype(dtype)) return fail("bad dtype");
+  if (B <= 0 || rows_per_clip <= 0 || T <= 0) return fail("empty input");
+  if (static_cast<long long>(B) * rows_per_clip > 65535) return fail("B * channels too large");
+  if (T >= (1LL << 40)) return fail("rows beyond 2^40");
+  *grid = dim3(static_cast<unsigned>((T + kFlowThreads - 1) / kFlowThreads), static_cast<unsigned>(B * rows_per_clip));
+  return 0;
+}
+}  // namespace
+
+int kvae_flow_split(const void* x, void* xs, void* x0, int B, int C, long long T, int flip, int dtype, void* stream) {
+  if (!x || !xs) return fail("null argument");
+  if (C % 2) return fail("flow: odd channel count");
+  dim3 grid;
+  if (flow_launch_check(B, C, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  flow_split_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(x, xs, x0, C, T, flip, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_flow_split_bwd(const void* gxs, const void* gx0, void* gx, int B, int C, long long T, int flip, int dtype,
+                        void* stream) {
+  if (!gx) return fail("null argument");
+  if (C % 2) return fail("flow: odd channel count");
+  dim3 grid;
+  if (flow_launch_check(B, C, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(gx));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  flow_split_bwd_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(gxs, gx0, gx, C, T, flip,
+                                                                                      dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_flow_mask(const void* x, const void* mask, void* y, int B, int C, long long T, int dtype, void* stream) {
+  if (!x || !mask || !y) return fail("null argument");
+  dim3 grid;
+  if (flow_launch_check(B, C, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  flow_mask_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(x, mask, y, C, T, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_wn_gate_fwd(const void* a, void* acts, int B, int H, long long T, int dtype, void* stream) {
+  if (!a || !acts) return fail("null argument");
+  dim3 grid;
+  if (flow_launch_check(B, H, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(a));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  wn_gate_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(a, acts, H, T, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_wn_gate_bwd(const void* a, const void* g, void* ga, int B, int H, long long T, int dtype, void* stream) {
+  if (!a || !g || !ga) return fail("null argument");
+  dim3 grid;
+  if (flow_launch_check(B, H, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(a));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  wn_gate_bwd_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(a, g, ga, H, T, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_wn_update_fwd(const void* x, const void* rs, const void* skip, const void* mask, void* x_out, void* skip_out,
+                       int B, int H, int last, long long T, int dtype, void* stream) {
+  if (!rs || !mask || !skip_out || (!last && (!x || !x_out))) return fail("null argument");
+  dim3 grid;
+  if (flow_launch_check(B, H, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(rs));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  wn_update_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(x, rs, skip, mask, x_out, skip_out, H,
+                                                                                 last ? 1 : 0, T, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_wn_update_bwd(const void* g_xout, const void* g_skipout, const void* mask, void* gx, void* grs, void* gskip,
+                       int B, int H, int last, long long T, int dtype, void* stream) {
+  if (!mask || !grs || (!last && !gx)) return fail("null argument");
+  dim3 grid;
+  if (flow_launch_check(B, H, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(grs));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  wn_update_bwd_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(g_xout, g_skipout, mask, gx, grs,
+                                                                                     gskip, H, last ? 1 : 0, T,
+                                                                                     dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_flow_coupling_fwd(const void* x, const void* m, const void* mask, void* y, void* y0, int B, int C, long long T,
+                           int flip, int reverse, int dtype, void* stream) {
+  if (!x || !m || !mask || !y) return fail("null argument");
+  if (C % 2) return fail("flow: odd channel count");
+  dim3 grid;
+  if (flow_launch_check(B, C / 2, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(x));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  flow_coupling_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(x, m, mask, y, y0, C / 2, T, flip,
+                                                                                     reverse, dtype == KVAE_F32);
+  KV_CUDA(cudaGetLastError());
+  ++g_launches;
+  return 0;
+}
+
+int kvae_flow_coupling_bwd(const void* gy, const void* gy0, const void* mask, void* gx, void* gm, int B, int C,
+                           long long T, int flip, int reverse, int dtype, void* stream) {
+  if (!mask || !gx || !gm) return fail("null argument");
+  if (C % 2) return fail("flow: odd channel count");
+  dim3 grid;
+  if (flow_launch_check(B, C / 2, T, dtype, &grid)) return -1;
+  DeviceGuard guard(device_of(gx));
+  if (!guard.ok) return fail("cannot select the tensor's device");
+  flow_coupling_bwd_kernel<<<grid, kFlowThreads, 0, static_cast<cudaStream_t>(stream)>>>(gy, gy0, mask, gx, gm, C / 2, T,
+                                                                                         flip, reverse,
+                                                                                         dtype == KVAE_F32);
   KV_CUDA(cudaGetLastError());
   ++g_launches;
   return 0;
